@@ -1,6 +1,7 @@
 """bench.py — N-best PLL hypotheses/sec of the MLM-PLL scoring path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c1|c2|c4|c5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -34,6 +35,14 @@ cpu_baseline / --impl reference: the reference's own CPU code from baseline/_ref
           rescore.find_best_weight under the jiwer stand-in), all host threads, bounded sample;
           falls back to the oracle port (kind "port") only when baseline/_ref is absent.
 stdout  : exactly one JSON line (library banners are redirected to stderr).
+--dump-outputs DIR: after the timed steps, what the last timed step computed, as rank 0's caller
+          receives it, goes to DIR/<name>.npy: pll (per-hypothesis PLL, float64; N > 1 strong: every
+          hypothesis in global order after the gather; not for c5, where it is an input), distance
+          (per-hypothesis Levenshtein distance, float32), argmax ([weight, utterance] index of the
+          chosen hypothesis, float32), edit_sums (per-weight edit sum, float64; N > 1 strong: after the
+          all_reduce).  Inputs are seeded, so two builds run with the same arguments can be compared
+          file by file.  Over 64 MB in all, an array keeps a fixed, seeded sample of its last axis
+          (positions in <name>_index.npy).
 """
 from __future__ import annotations
 
@@ -96,7 +105,14 @@ def parse_args(argv=None):
     ap.add_argument("--operand-dtype", default=None,
                     help="GEMM operand type; default = the workload's (bf16 encoder + fp16 MLM head; fp16 for c4), always "
                          "reported in `dtype`")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (--impl b200)")
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the timed path of --impl b200")
+    return args
 
 
 def model_cfg(name):
@@ -353,6 +369,26 @@ def _emit(line: dict):
     os.write(_JSON_FD if _JSON_FD is not None else 1, (json.dumps(line) + "\n").encode())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir: str, arrays: dict, limit: int = DUMP_LIMIT_BYTES):
+    """arrays: {name: float32 / float64 ndarray} -> out_dir/<name>.npy.  When they exceed `limit` bytes
+    together, an array larger than its equal share keeps a fixed, seeded sample of its last axis, and the
+    sampled positions are written to out_dir/<name>_index.npy (float64), so the files stay within `limit`."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = limit // max(len(arrays), 1)
+    over = sum(a.nbytes for a in arrays.values()) > limit
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if over and a.nbytes > share:
+            per_position = a.nbytes // a.shape[-1] + 8            # the values at one position + its index
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[-1], size=share // per_position, replace=False))
+            a = a[..., idx]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 # ------------------------------------------------------------------------------------ GPU arm
 def main(argv=None):
     args = parse_args(argv)
@@ -527,6 +563,14 @@ def main(argv=None):
             dist.barrier()
         torch.cuda.synchronize(dev)
 
+    def in_global_order(gathered):
+        """The device gather (rank-major, padded to n_max) laid out in global hypothesis order."""
+        g = gathered.reshape(world, n_max)
+        full = np.zeros(n_total, np.float64)
+        for r in range(world):
+            full[shard.global_hyp_index(parts[r], n_best)] = g[r, :counts_per_rank[r]]
+        return full
+
     # ------------------------------------------------------------------ value (device resident)
     for _ in range(args.warmup):
         step_device()
@@ -545,6 +589,13 @@ def main(argv=None):
     barrier()
     ms_value = e0.elapsed_time(e1) / args.steps
     clocks = sampler.stop()
+    last_step = None
+    if args.dump_outputs and rank == 0:              # the last timed step's results, copied after the timed region
+        last_step = {"distance": d_dist[:n_hyp].cpu().numpy().astype(np.float32),
+                     "argmax": d_arg[:W * N].cpu().numpy().reshape(W, N).astype(np.float32),
+                     "edit_sums": (d_counts_all if strong else d_counts)[:W].cpu().numpy().astype(np.float64)}
+        if not combiner_only:
+            last_step = {"pll": in_global_order(d_gather.cpu().numpy()) if strong else d_pll.cpu().numpy(), **last_step}
     launches = 2 * args.steps + (int(scorer.stats()["kernel_launches"]) if scorer else 0)
 
     # one extra, untimed-for-`value` step with per-launch CUDA events: the per-kind GEMM breakdown
@@ -574,12 +625,8 @@ def main(argv=None):
     # ------------------------------------------------------------------ checks + max over ranks
     checks = {}
     if not combiner_only:
-        if strong:                                   # the device gather, laid out in global order on the host
-            g = d_gather.cpu().numpy().reshape(world, n_max)
-            all_idx = [shard.global_hyp_index(p, n_best) for p in parts]
-            full_dev = np.zeros(n_total, np.float64)
-            for r in range(world):
-                full_dev[all_idx[r]] = g[r, :counts_per_rank[r]]
+        if strong:
+            full_dev = in_global_order(d_gather.cpu().numpy())
             checks["device_gather_equals_host_gather"] = bool(np.array_equal(full_dev, full_host))
         else:
             full_dev = d_pll.cpu().numpy()
@@ -704,6 +751,8 @@ def main(argv=None):
                                        "sample": f"first {n_cpu} hypotheses ({copies} masked copies) of the same workload; "
                                                  f"{arm.describe()}; {dt:.1f} s",
                                        "max_abs_dpll_vs_gpu": float(err.max()), "mean_abs_dpll_vs_gpu": float(err.mean())}
+        if last_step is not None:
+            write_outputs(args.dump_outputs, last_step)
     if scorer:
         scorer.close()
     if world > 1:

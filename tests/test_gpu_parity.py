@@ -461,6 +461,40 @@ def test_drop_in_cli_end_to_end():
     assert "rescore.log matches the oracle" in out.stdout
 
 
+def test_bench_dump_outputs_are_the_timed_results_and_repeat_across_runs(tmp_path):
+    """bench.py --dump-outputs: what the last timed step computed, identical for 1 and 2 timed steps
+    (seeded inputs), consistent with the JSON line, and the same scores as a direct scoring call."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    lines = {}
+    for steps in (1, 2):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "c1", "--steps", str(steps),
+                              "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / str(steps))],
+                             capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines[steps] = json.loads([l for l in out.stdout.splitlines() if l.strip()][-1])
+        assert lines[steps]["steps"] == steps
+    names = ["argmax.npy", "distance.npy", "edit_sums.npy", "pll.npy"]
+    assert sorted(os.listdir(tmp_path / "1")) == names == sorted(os.listdir(tmp_path / "2"))
+    d = {n[:-4]: np.load(tmp_path / "2" / n) for n in names}
+    for n in names:
+        assert np.array_equal(np.load(tmp_path / "1" / n), d[n[:-4]]), n
+    assert d["pll"].dtype == np.float64 and d["pll"].shape == (1000,) and d["argmax"].shape == (101, 100)
+    assert d["distance"].dtype == np.float32 and d["edit_sums"].dtype == np.float64
+    assert float(np.sum(d["pll"])) == lines[2]["pll_checksum"]
+    assert float(np.arange(0.0, 1.01, 0.01)[int(np.argmin(d["edit_sums"]))]) == lines[2]["best_weight"]
+    nb = synth.make_nbest(100, 10, seed=0)
+    dist = oracle.levenshtein_strings([r for r in nb.refs for _ in range(10)], [h for hs in nb.hyps for h in hs])
+    assert np.array_equal(d["distance"], dist.astype(np.float32))
+    chosen = np.take_along_axis(dist.reshape(100, 10), d["argmax"].T.astype(np.int64), axis=1)
+    assert np.array_equal(d["edit_sums"], chosen.sum(0).astype(np.float64))
+    tok, off = nb.packed_tokens()
+    with engine.PllScorer(synth.random_init_state_dict(synth.BERT_BASE_CHINESE, 10), synth.BERT_BASE_CHINESE,
+                          operand_dtype=lines[2]["dtype"]) as sc:
+        assert np.array_equal(sc.score_packed(tok, off), d["pll"])
+
+
 def test_text_front_end_matches_the_host_tokenizer(tmp_path):
     """pllb_tokenize_host (+ host path for flagged hypotheses) == BertTokenizer-style encode, per string."""
     from asr_rescoring_b200.tokenizer import BertCharTokenizer, SyntheticCharTokenizer, encode_batch

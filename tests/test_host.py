@@ -333,6 +333,36 @@ def test_bench_reference_arm_combiner_workload():
     assert d["impl"] == "reference" and d["value"] > 0 and 0.0 <= d["best_weight"] <= 1.0 and d["dtype"] == "f64"
 
 
+def test_bench_rejects_zero_steps_and_dump_outputs_of_the_reference_arm():
+    import bench
+    assert bench.parse_args(["--steps", "2", "--dump-outputs", "d"]).steps == 2
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"]):
+        with pytest.raises(SystemExit):
+            bench.parse_args(argv)
+
+
+def test_bench_write_outputs_keeps_a_seeded_sample_within_the_limit(tmp_path):
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {"pll": rng.normal(size=5000), "argmax": rng.integers(0, 10, (101, 300)).astype(np.float32)}
+    bench.write_outputs(str(tmp_path / "all"), arrays)
+    for name, a in arrays.items():
+        assert np.array_equal(np.load(tmp_path / "all" / f"{name}.npy"), a)
+    assert sorted(os.listdir(tmp_path / "all")) == ["argmax.npy", "pll.npy"]
+    limit = 60000                                       # both arrays (161 200 bytes) over it
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), arrays, limit=limit)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["argmax.npy", "argmax_index.npy", "pll.npy", "pll_index.npy"] == sorted(os.listdir(tmp_path / "b"))
+    assert sum(np.load(tmp_path / "a" / f).nbytes for f in files) <= limit
+    for name, a in arrays.items():
+        idx = np.load(tmp_path / "a" / f"{name}_index.npy")
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert got.dtype == a.dtype and np.array_equal(got, a[..., idx.astype(np.int64)])
+        assert np.array_equal(got, np.load(tmp_path / "b" / f"{name}.npy"))
+        assert np.all(np.diff(idx) > 0)
+
+
 def test_pack_stripped_equals_strip_then_pack():
     """The combiner's one-pass packing (raw lengths for rescore.py:28-35, stripped code points for the
     CER) against the plain per-string strip(), incl. every whitespace code point str.strip() knows."""
