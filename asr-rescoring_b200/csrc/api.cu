@@ -96,34 +96,6 @@ int get_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int 
   return PLLB_OK;
 }
 
-int get_tmap_blocked(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols) {
-  const uint64_t row_tiles = (rows + 31) / 32, col_tiles = cols / 64;
-  // same cache, keyed with a box shape no 2-D map uses
-  const TmapKey key{base, row_tiles, col_tiles, 0xB10Cu, 0xB10Cu, ((uint32_t)CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 << 8) | 2u};
-  auto it = g_tmaps.find(key);
-  if (it != g_tmaps.end()) {
-    *out = it->second;
-    return PLLB_OK;
-  }
-  if (cols % 64 != 0) return fail(PLLB_ERR_INVALID, "blocked tensor map: cols % 64 != 0");
-  typedef CUresult (*Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                         const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                         CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  Fn fn = reinterpret_cast<Fn>(encode_tiled_fn());
-  if (!fn) return fail(PLLB_ERR_CUDA, "cuTensorMapEncodeTiled entry point unavailable");
-  cuuint64_t gdim[4] = {64, 32, col_tiles, row_tiles};
-  cuuint64_t gstride[3] = {128, 4096, 4096 * col_tiles};
-  cuuint32_t box[4] = {64, 32, 1, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), gdim, gstride, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(PLLB_ERR_CUDA, "cuTensorMapEncodeTiled (blocked) failed, CUresult " + std::to_string((int)r));
-  if (g_tmaps.size() >= 4096) g_tmaps.clear();
-  g_tmaps.emplace(key, *out);
-  return PLLB_OK;
-}
-
 }  // namespace pllb
 
 using namespace pllb;
@@ -172,10 +144,7 @@ struct pllb_context {
   // FFN2 of layer l writes the 16-bit copy that layer l + 1 (or the head) consumes: in THAT type
   int ldt_ffn2(int l, bool next_fp16) const { return lfp16(l) ? DT_FP16 : (next_fp16 ? DT_BF16_OUT16 : DT_BF16); }
   bool has_head = false;             // MLM head weights were supplied (PLL scoring available)
-  bool fused_ln = true;              // residual + LayerNorm inside the GEMM epilogue (PLLB_FUSED_LN=0 disables)
-  bool prune_q = true;               // last layer: Q projection + attention for the consumed row only (PLLB_PRUNE_Q=0 disables)
   bool share_l0 = true;              // embeddings + layer-0 QKV on the unique rows of a hypothesis (PLLB_SHARE_L0=0 disables)
-  bool ffn_blocked = false;          // experiment (PLLB_FFN_BLOCKED=1): the FFN intermediate (FFN1 out = FFN2 in) K-blocked; measured slower
   int64_t cap_rows = 0, cap_copies = 0, cap_hyps = 0;
   int vocab_pad = 0, tiles_v = 0;
   std::vector<void*> owned;          // every cudaMalloc of this handle
@@ -253,8 +222,10 @@ int conv_16(pllb_context* c, __nv_bfloat16** dst, const float* src, int64_t n, b
     if (_rc) return _rc;    \
   } while (0)
 
-int timed_gemm(pllb_context* c, int kind, const void* A, const void* W, const float* bias, void* C, int64_t M, int N,
-               int K, int epi, const LseArgs* lse, cudaStream_t s, int dt, bool c_blocked = false) {
+// Enqueues one GEMM launch (`launch`) on s between the timing events of a timed call, and counts
+// its FLOPs towards the stats and its kind.
+template <typename Launch>
+int timed_launch(pllb_context* c, int kind, double flops, cudaStream_t s, Launch&& launch) {
   TimedLaunch* tl = nullptr;
   if (c->timing) {
     if (c->timed_used == c->timed.size()) {
@@ -267,43 +238,27 @@ int timed_gemm(pllb_context* c, int kind, const void* A, const void* W, const fl
     tl->kind = kind;
     PLLB_CUDA(cudaEventRecord(tl->start, s));
   }
-  RC(launch_gemm_tcgen05(A, W, bias, C, M, N, K, epi, lse, dt, s, c_blocked));
+  RC(launch());
   if (tl) PLLB_CUDA(cudaEventRecord(tl->stop, s));
-  const double fl = 2.0 * (double)M * (double)(epi == EPI_LSE && lse ? lse->vocab : N) * (double)K;
-  c->stats.gemm_flops += fl;
-  c->gemm_flops_kind[kind] += fl;
+  c->stats.gemm_flops += flops;
+  c->gemm_flops_kind[kind] += flops;
   c->stats.last_gemm_launches += 1;
   return PLLB_OK;
 }
 
-// GEMM + bias + residual + LayerNorm: fused kernel, or (PLLB_FUSED_LN=0) GEMM -> fp32 -> LayerNorm kernel.
+int timed_gemm(pllb_context* c, int kind, const void* A, const void* W, const float* bias, void* C, int64_t M, int N,
+               int K, int epi, const LseArgs* lse, cudaStream_t s, int dt) {
+  const double fl = 2.0 * (double)M * (double)(epi == EPI_LSE && lse ? lse->vocab : N) * (double)K;
+  return timed_launch(c, kind, fl, s, [&] { return launch_gemm_tcgen05(A, W, bias, C, M, N, K, epi, lse, dt, s); });
+}
+
+// GEMM + bias + residual + LayerNorm in one kernel (gemm_ln_tcgen05.cu).
 int timed_gemm_ln(pllb_context* c, int kind, const void* A, const void* W, const float* bias, const float* g,
-                  const float* be, float* hid32, void* hid16, int64_t M, int K, cudaStream_t s, int dt,
-                  bool a_blocked = false) {
+                  const float* be, float* hid32, void* hid16, int64_t M, int K, cudaStream_t s, int dt) {
   const int H = c->d.hidden;
-  if (!c->fused_ln) {
-    RC(timed_gemm(c, kind, A, W, bias, c->y_f32, M, H, K, EPI_BIAS_F32, nullptr, s, dt == DT_BF16_OUT16 ? DT_BF16 : dt));
-    return launch_residual_ln(c->y_f32, hid32, hid16, g, be, c->d.ln_eps, M, H, (dt & 4) != 0, s);
-  }
-  TimedLaunch* tl = nullptr;
-  if (c->timing) {
-    if (c->timed_used == c->timed.size()) {
-      TimedLaunch t{};
-      PLLB_CUDA(cudaEventCreate(&t.start));
-      PLLB_CUDA(cudaEventCreate(&t.stop));
-      c->timed.push_back(t);
-    }
-    tl = &c->timed[c->timed_used++];
-    tl->kind = kind;
-    PLLB_CUDA(cudaEventRecord(tl->start, s));
-  }
-  RC(launch_gemm_ln(A, W, bias, g, be, c->d.ln_eps, hid32, hid16, M, H, K, dt, s, a_blocked));
-  if (tl) PLLB_CUDA(cudaEventRecord(tl->stop, s));
   const double fl = 2.0 * (double)M * (double)H * (double)K;
-  c->stats.gemm_flops += fl;
-  c->gemm_flops_kind[kind] += fl;
-  c->stats.last_gemm_launches += 1;
-  return PLLB_OK;
+  return timed_launch(c, kind, fl, s,
+                      [&] { return launch_gemm_ln(A, W, bias, g, be, c->d.ln_eps, hid32, hid16, M, H, K, dt, s); });
 }
 
 // Encoder + head over one chunk whose metadata (tok_off / copy_base / row_base, each
@@ -349,7 +304,7 @@ int run_chunk(pllb_context* c, const int32_t* tokens, const int32_t* tok_off, co
     const int dt = c->ldt(l);
     // type of the 16-bit copy this layer's FFN2 leaves behind: the next layer's, or the head's
     const int dt_ffn2 = c->ldt_ffn2(l, l + 1 < d.num_layers ? c->lfp16(l + 1) : (cls ? f16 : c->head_fp16));
-    if (last && !shared_rows && c->prune_q) {
+    if (last && !shared_rows) {
       // The pruned last layer consumes one attention row per copy: K|V for every row, Q for that
       // row only (1/3 of the projection saved), then a single-query attention straight into hg.
       RC(timed_gemm(c, G_QKV, c->hidden_bf16, L.qkv_w + (size_t)H * H, L.qkv_b + H, c->wide, n_rows, 2 * H, H,
@@ -360,22 +315,21 @@ int run_chunk(pllb_context* c, const int32_t* tokens, const int32_t* tok_off, co
     } else {
       RC(timed_gemm(c, G_QKV, shared_rows ? c->ctx : c->hidden_bf16, L.qkv_w, L.qkv_b, c->wide,
                     shared_rows ? n_unique : n_rows, 3 * H, H, EPI_BIAS_BF16, nullptr, s, dt));
-      RC(launch_attention(c->wide, c->ctx, c->plan, n_copies, H, d.num_heads, max_T, f16, shared_rows, c->cap_rows, s));
+      RC(launch_attention(c->wide, c->ctx, c->plan, n_copies, H, d.num_heads, f16, shared_rows, s));
       if (last) RC(launch_gather_rows_bf16(c->ctx, c->plan.mask_row, n_copies, H, c->hg, s));
     }
     if (last) {
       RC(launch_gather_rows_f32(c->hidden_f32, c->plan.mask_row, n_copies, H, c->hid_c, s));
       RC(timed_gemm_ln(c, G_AO, c->hg, L.ao_w, L.ao_b, L.ao_g, L.ao_be, c->hid_c, c->t_bf16, n_copies, H, s, dt));
-      RC(timed_gemm(c, G_FF1, c->t_bf16, L.ff1_w, L.ff1_b, c->wide, n_copies, I, H, EPI_BIAS_GELU_BF16, nullptr, s, dt, c->ffn_blocked));
+      RC(timed_gemm(c, G_FF1, c->t_bf16, L.ff1_w, L.ff1_b, c->wide, n_copies, I, H, EPI_BIAS_GELU_BF16, nullptr, s, dt));
       // its 16-bit copy is the MLM head's input: written in the head's operand type
-      RC(timed_gemm_ln(c, G_FF2, c->wide, L.ff2_w, L.ff2_b, L.out_g, L.out_be, c->hid_c, c->t_bf16, n_copies, I, s, dt_ffn2,
-                       c->ffn_blocked));
+      RC(timed_gemm_ln(c, G_FF2, c->wide, L.ff2_w, L.ff2_b, L.out_g, L.out_be, c->hid_c, c->t_bf16, n_copies, I, s, dt_ffn2));
       break;
     }
     RC(timed_gemm_ln(c, G_AO, c->ctx, L.ao_w, L.ao_b, L.ao_g, L.ao_be, c->hidden_f32, c->hidden_bf16, n_rows, H, s, dt));
-    RC(timed_gemm(c, G_FF1, c->hidden_bf16, L.ff1_w, L.ff1_b, c->wide, n_rows, I, H, EPI_BIAS_GELU_BF16, nullptr, s, dt, c->ffn_blocked));
+    RC(timed_gemm(c, G_FF1, c->hidden_bf16, L.ff1_w, L.ff1_b, c->wide, n_rows, I, H, EPI_BIAS_GELU_BF16, nullptr, s, dt));
     RC(timed_gemm_ln(c, G_FF2, c->wide, L.ff2_w, L.ff2_b, L.out_g, L.out_be, c->hidden_f32, c->hidden_bf16, n_rows, I, s,
-                     dt_ffn2, c->ffn_blocked));
+                     dt_ffn2));
   }
   if (upto_layer >= 0) return PLLB_OK;
   r_stage.next("stage3: head at the masked rows");
@@ -628,11 +582,7 @@ int pllb_create(pllb_handle* out, const pllb_model_desc* desc, const pllb_weight
                : d.operand_dtype >= 16 ? d.operand_dtype - 16 : d.num_layers;
   c->head_fp16 = d.operand_dtype >= 1;
   c->dt_head = c->head_fp16 ? DT_FP16 : DT_BF16;
-  if (const char* e = getenv("PLLB_FUSED_LN")) c->fused_ln = atoi(e) != 0;
   if (const char* e = getenv("PLLB_SHARE_L0")) c->share_l0 = atoi(e) != 0;
-  if (const char* e = getenv("PLLB_PRUNE_Q")) c->prune_q = atoi(e) != 0;
-  if (const char* e = getenv("PLLB_FFN_BLOCKED")) c->ffn_blocked = atoi(e) != 0;
-  if (!c->fused_ln) c->ffn_blocked = false;        // the unfused fallback reads the intermediate through the plain GEMM (row-major A)
   cudaStream_t s = 0;
   const int H = d.hidden, I = d.intermediate, V = d.vocab;
   int rc = PLLB_OK;

@@ -43,15 +43,6 @@ int sm_count();   // SMs of the current device (cached)
 int get_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int elt_bytes, uint64_t rows, uint64_t cols,
                 uint32_t box_rows, uint32_t box_cols);
 
-// K-blocked 16-bit activation [rows, cols] (cols % 64 == 0, buffer padded to a multiple of 32 rows): tiles of
-// 32 rows x 64 columns (4 KB) stored contiguously, tile (rb, cb) at ((rb * cols/64 + cb) * 4096) bytes, so
-// that every TMA box of a GEMM operand / epilogue is ONE contiguous burst instead of 32 pieces of 128 bytes at
-// the row pitch (tools/pitch_probe.cu: 6.2-6.6 against 5.2-5.3 TB/s when streaming).  EXPERIMENT, off by
-// default: inside the FFN2 mainloop the row-major form is faster (DESIGN.md 3.1b).  4-D tensor map, coordinates
-// {column in tile, row in tile, column tile, row tile}, box {64, 32, 1, 1}, 128-byte swizzle: the
-// shared-memory image of a box is the one of the 2-D row-major map.
-int get_tmap_blocked(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols);
-
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per kernel (keyed by its address — every
 // instantiation with the same signature has the same pointer TYPE) and device.
 template <typename K>
@@ -98,15 +89,12 @@ struct LseArgs {
 // C[M,N] = A[M,K] * W[N,K]^T (+ epilogue).  A, W bf16 row-major (K contiguous).
 // N % 256 == 0 (pad W rows with zeros), K % 64 == 0.  ldc = N.
 // dt: DT_BF16 or DT_FP16.
-// c_blocked: the 16-bit output C is written in the K-blocked layout (get_tmap_blocked) instead of row-major.
 int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C, int64_t M, int N, int K,
-                        int epilogue, const LseArgs* lse, int dt, cudaStream_t stream, bool c_blocked = false);
+                        int epilogue, const LseArgs* lse, int dt, cudaStream_t stream);
 // hidden_f32 = LayerNorm(A * W^T + bias + hidden_f32) in place, hidden_16 = 16-bit copy
 // (gemm_ln_tcgen05.cu: cluster of H/256 CTAs per 128-row block, row statistics through DSMEM).
-// a_blocked: A is stored in the K-blocked layout.
 int launch_gemm_ln(const void* A, const void* W, const float* bias, const float* gamma, const float* beta, float eps,
-                   float* hidden_f32, void* hidden_16, int64_t M, int H, int K, int dt, cudaStream_t stream,
-                   bool a_blocked = false);
+                   float* hidden_f32, void* hidden_16, int64_t M, int H, int K, int dt, cudaStream_t stream);
 int launch_gemm_simt(const void* A, const void* W, const float* bias, void* C, int64_t M, int N, int K,
                      int epilogue, cudaStream_t stream);
 
@@ -144,16 +132,12 @@ int launch_embed_ln(const int32_t* tokens, const int32_t* hyp_tok_off, CopyPlan 
                     const float* word_emb, const float* pos_emb, const float* type_emb, const float* g,
                     const float* b, float eps, int H, int32_t cls_id, int32_t sep_id, int32_t mask_id, int32_t vocab,
                     float* hidden_f32_rowmajor, void* hidden_bf16, bool fp16, cudaStream_t s);
-// hidden = LN(y + hidden) (in place), hidden_bf16 = bf16(hidden)
-int launch_residual_ln(const float* y, float* hidden_f32, void* hidden_bf16, const float* g, const float* b,
-                       float eps, int64_t rows, int H, bool fp16, cudaStream_t s);
 // out_bf16 = bf16(LN(x)); no residual (MLM head transform)
 int launch_plain_ln_bf16(const float* x, void* out_bf16, const float* g, const float* b, float eps, int64_t rows,
                          int H, bool fp16, cudaStream_t s);
 // shared_rows: qkv holds the unique rows of every hypothesis (2L+2 per hypothesis) instead of one row per packed row
-// qkv_rows: rows of the [rows, 3H] buffer behind qkv_bf16 (extent of the TMA tensor maps)
-int launch_attention(const void* qkv_bf16, void* ctx_bf16, CopyPlan plan, int32_t n_copies, int H, int NH,
-                     int max_T, bool fp16, bool shared_rows, int64_t qkv_rows, cudaStream_t s);
+int launch_attention(const void* qkv_bf16, void* ctx_bf16, CopyPlan plan, int32_t n_copies, int H, int NH, bool fp16,
+                     bool shared_rows, cudaStream_t s);
 // Embeddings of the unique rows of every hypothesis (fp32 row-major + 16-bit), and the packed-row -> unique-row map.
 int launch_embed_unique(const int32_t* tokens, const int32_t* hyp_tok_off, int32_t n_hyp, const float* word_emb,
                         const float* pos_emb, const float* type_emb, const float* g, const float* b, float eps, int H,

@@ -2,14 +2,12 @@
 //   stage 1  masked-copy expansion with varlen packing (replaces MLM_PLL/preprocess.py:9-30
 //            and the padded collate of MLM_PLL/main.py:28-54), fused with BertEmbeddings
 //            (transformers modeling_bert.py:72-112);
-//   LayerNorm with residual (modeling_bert.py:294-298, 352-356), per-sequence varlen
+//   the MLM head's LayerNorm (modeling_bert.py:481-487), per-sequence varlen
 //            self-attention (:168-207), masked-row gather, logsumexp finish and the
 //            per-hypothesis sum of MLM_PLL/main.py:101-107.
 // All kernels are one-warp-per-row (or per sequence/head) with 128-bit accesses; rows of
 // H fp32 are contiguous so every warp access is a fully coalesced 512-byte segment.
 #include <cuda_bf16.h>
-#include <algorithm>
-#include <cstdlib>
 #include <cuda_fp16.h>
 
 #include "common.h"
@@ -130,18 +128,11 @@ __device__ __forceinline__ void ln_normalize(float4 (&x)[VEC], const float* __re
   }
 }
 
-// fp32 goes to the T32 blocked layout (common.h): f32_base + row -> 16-byte group g of the row
-// sits at ((row/32 * H/4 + g) * 32 + row%32) float4s; the 16-bit copy is row-major.
-template <int VEC>
-__device__ __forceinline__ float4* t32_row(float* base, int64_t row) {
-  return reinterpret_cast<float4*>(base) + (size_t)(row >> 5) * (32 * VEC) * 32 + (row & 31);
-}
+// the row-major 16-bit copy of one row
 template <int VEC, bool FP16>
-__device__ __forceinline__ void store_row(const float4 (&x)[VEC], float4* __restrict__ f32_t32,
-                                          __nv_bfloat16* __restrict__ bf_row, int lane) {
+__device__ __forceinline__ void store_row(const float4 (&x)[VEC], __nv_bfloat16* __restrict__ bf_row, int lane) {
 #pragma unroll
   for (int i = 0; i < VEC; ++i) {
-    if (f32_t32) f32_t32[(size_t)(lane + 32 * i) * 32] = x[i];
     if (bf_row) {
       uint2 u;
       u.x = pack16<FP16>(x[i].x, x[i].y);
@@ -197,7 +188,7 @@ embed_ln_kernel(const int32_t* __restrict__ tokens, const int32_t* __restrict__ 
     // re-tiles it into the T32 residual layout with fully coalesced accesses on both sides.
 #pragma unroll
     for (int i = 0; i < VEC; ++i) reinterpret_cast<float4*>(hidden_f32 + row * H)[lane + 32 * i] = x[i];
-    store_row<VEC, FP16>(x, nullptr, hidden_bf16 + row * H, lane);
+    store_row<VEC, FP16>(x, hidden_bf16 + row * H, lane);
   }
 }
 
@@ -236,7 +227,7 @@ embed_unique_kernel(const int32_t* __restrict__ tokens, const int32_t* __restric
     const size_t row = ub + j;
 #pragma unroll
     for (int i = 0; i < VEC; ++i) reinterpret_cast<float4*>(u_f32 + row * H)[lane + 32 * i] = x[i];
-    store_row<VEC, FP16>(x, nullptr, u_bf16 + row * H, lane);
+    store_row<VEC, FP16>(x, u_bf16 + row * H, lane);
   }
 }
 
@@ -250,11 +241,11 @@ __global__ void row_src_kernel(CopyPlan plan, int32_t n_copies) {
   for (int p = lane; p < T; p += 32) plan.row_src[start + p] = p == mpos ? ub + T + mpos - 1 : ub + p;
 }
 
-// hidden = LayerNorm(y + hidden) in place (+ bf16 copy).  One warp per row.
-template <int VEC, bool RESID, bool FP16>
+// out_bf16 = 16-bit(LayerNorm(y)), y row-major fp32.  One warp per row.
+template <int VEC, bool FP16>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32)
-ln_kernel(const float* __restrict__ y, float* __restrict__ hidden_f32, __nv_bfloat16* __restrict__ out_bf16,
-          const float* __restrict__ g, const float* __restrict__ b, float eps, int64_t rows) {
+ln_kernel(const float* __restrict__ y, __nv_bfloat16* __restrict__ out_bf16, const float* __restrict__ g,
+          const float* __restrict__ b, float eps, int64_t rows) {
   constexpr int H = 128 * VEC;
   const int64_t row = (int64_t)blockIdx.x * WARPS_PER_BLOCK + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
@@ -263,16 +254,8 @@ ln_kernel(const float* __restrict__ y, float* __restrict__ hidden_f32, __nv_bflo
   float4 x[VEC];
 #pragma unroll
   for (int i = 0; i < VEC; ++i) x[i] = yr[lane + 32 * i];
-  if (RESID) {
-    const float4* hr = t32_row<VEC>(hidden_f32, row);
-#pragma unroll
-    for (int i = 0; i < VEC; ++i) {
-      const float4 r = hr[(size_t)(lane + 32 * i) * 32];
-      x[i].x += r.x; x[i].y += r.y; x[i].z += r.z; x[i].w += r.w;
-    }
-  }
   ln_normalize<VEC>(x, g, b, eps, lane);
-  store_row<VEC, FP16>(x, RESID ? t32_row<VEC>(hidden_f32, row) : nullptr, out_bf16 + row * H, lane);
+  store_row<VEC, FP16>(x, out_bf16 + row * H, lane);
 }
 
 // ---------------------------------------------------------------- tensor-core varlen attention
@@ -585,7 +568,7 @@ __device__ __forceinline__ void attn_staged(const __nv_bfloat16* __restrict__ ba
 template <bool FP16, bool SHARED>
 __global__ void __launch_bounds__(ATT_WARPS * 32, 2)
 attention_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ ctx, CopyPlan plan,
-                     int32_t n_copies, int H, int NH, int skip_le) {
+                     int32_t n_copies, int H, int NH) {
   extern __shared__ __align__(16) uint8_t att_dyn[];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
   __nv_bfloat16* sm = reinterpret_cast<__nv_bfloat16*>(att_dyn) + (size_t)wib * ATT_STAGE_ELEMS;
@@ -593,7 +576,6 @@ attention_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __res
   if (pair >= (int64_t)n_copies * NH) return;
   const int c = (int)(pair / NH), head = (int)(pair % NH);
   const int start = plan.seq_start[c], T = plan.seq_len[c];
-  if (T <= skip_le) return;                 // done by attention_tma_kernel
   const size_t ld = (size_t)3 * H;
   const __nv_bfloat16* base = qkv + head * 64;
   __nv_bfloat16* ob = ctx + (size_t)start * H + head * 64;
@@ -606,253 +588,6 @@ attention_mma_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __res
     const RowDirect rm{(size_t)start * ld, ld};
     if (T <= ATT_TS) attn_staged<FP16>(base, rm, ob, T, H, lane, sm);
     else attn_stream<FP16>(base, rm, ob, T, H, lane, sm);
-  }
-}
-
-// ---------------------------------------------------------------- TMA-fed varlen attention
-// Persistent form for the layers whose Q|K|V rows are the copy's own packed rows (every layer but
-// the shared layer 0 and the pruned last one), written to test the hypothesis that
-// attention_mma_kernel (one (copy, head) staged per warp, no load in flight while the warp
-// computes) is latency-bound at its 0.67 of the HBM peak.  It is not: this kernel keeps ~100 KB per
-// SM in flight and reaches the same rate, because both spend ~900 warp instructions per (copy,
-// head) and are bound by instruction issue.  Kept as an opt-in (PLLB_ATT_TMA=1), bit-identical to
-// the default kernel.  One CTA walks over whole masked copies:
-//   warp 0        producer — per copy 3*NH TMA box loads (Q, K, V slice of every head: 64 columns x
-//                 R rows, R = T rounded up to 8, 128-byte swizzle) into a byte-granular ring of
-//                 216 KiB with up to four copies in flight, one mbarrier transaction per copy; the
-//                 next copies stream in while this one is computed, so 100-200 KB per SM is always
-//                 in flight;
-//   warps 1..NH   one head each: ldmatrix from the swizzled tiles, the same 16x16 flash blocks on
-//                 mma.sync as above, context rows leave as 16-byte stores.
-// Copies longer than ATT_TMA_ROWS rows are left to attention_mma_kernel (launched with skip_le).
-constexpr int ATT_TMA_ROWS = 32;                    // longest copy it takes (T <= 32: all but 0.03 % of the C2 copies)
-constexpr int ATT_TMA_SLOTS = 4;                    // copies in flight (mbarrier pairs)
-constexpr int ATT_TMA_MAPS = ATT_TMA_ROWS / 8;      // one tensor map per box height 8, 16, 24, 32
-constexpr int ATT_TMA_MAX_HEADS = 12;
-// byte-granular ring: a copy of R = roundup8(T) rows occupies 3*NH*R*128 bytes (36 / 72 / 108 / 144 KiB at
-// NH = 12), placed back to back and wrapping to 0 when it does not fit
-constexpr int ATT_TMA_RING_BYTES = 3 * ATT_TMA_MAX_HEADS * 48 * 128;   // 216 KiB
-
-struct AttTmaMaps {
-  CUtensorMap m[ATT_TMA_MAPS];
-};
-
-// byte offset of element (row, col) inside a 128-byte-swizzled tile whose base is 1024-byte aligned
-__device__ __forceinline__ uint32_t sw128(int row, int col) {
-  return (uint32_t)(row * 128 + ((((col >> 3) ^ row) & 7) << 4) + (col & 7) * 2);
-}
-
-// One head of one copy from swizzled tiles of R rows (R % 8 == 0, T <= R <= 32).  Rows >= R do not
-// exist: fragment loads clamp to the last row (their scores are masked / their p is 0) and the
-// output staging skips them.
-template <bool FP16>
-__device__ __forceinline__ void attn_compute_sw(uint32_t q_addr, uint32_t k_addr, uint32_t v_addr,
-                                                __nv_bfloat16* __restrict__ ob, int T, int R, int H, int lane) {
-  const int g = lane >> 2, cq = lane & 3;
-  constexpr float kScaleLog2 = 0.125f * 1.4426950408889634f;
-  const int lrow = (lane & 7) + ((lane >> 3) & 1) * 8, lcol8 = ((lane >> 4) & 1) * 8;
-  const int rmax = R - 1;
-  // V rows T .. R-1 came from the next sequence (or stale memory): they are multiplied by p = 0 and
-  // must be finite (0 * NaN = NaN)
-  for (int r = T + (lane >> 3); r < R; r += 4)
-    asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(v_addr + (uint32_t)(r * 128 + (lane & 7) * 16)), "r"(0u) : "memory");
-  __syncwarp();
-  for (int m0 = 0; m0 < T; m0 += 16) {
-    uint32_t qf[4][4];
-    {
-      const int row = min(m0 + lrow, rmax);
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks)
-        asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                     : "=r"(qf[ks][0]), "=r"(qf[ks][1]), "=r"(qf[ks][2]), "=r"(qf[ks][3])
-                     : "r"(q_addr + sw128(row, 16 * ks + lcol8)));
-    }
-    float mx[2] = {-INFINITY, -INFINITY}, l[2] = {0.f, 0.f};
-    float o[8][4];
-#pragma unroll
-    for (int n = 0; n < 8; ++n) { o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f; }
-    for (int k0 = 0; k0 < T; k0 += 16) {
-      float s[2][4];
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        s[j][0] = s[j][1] = s[j][2] = s[j][3] = 0.f;
-        if (j == 1 && k0 + 8 >= T) break;               // second key tile fully masked (warp-uniform)
-        const int krow = min(k0 + 8 * j + (lane & 7), rmax);
-#pragma unroll
-        for (int kp = 0; kp < 2; ++kp) {
-          uint32_t b0, b1, b2, b3;
-          asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];"
-                       : "=r"(b0), "=r"(b1), "=r"(b2), "=r"(b3) : "r"(k_addr + sw128(krow, 32 * kp + (lane >> 3) * 8)));
-          mma_16816<FP16>(s[j], qf[2 * kp], b0, b1);
-          mma_16816<FP16>(s[j], qf[2 * kp + 1], b2, b3);
-        }
-      }
-      float bm[2] = {-INFINITY, -INFINITY};
-      const bool tail = k0 + 16 > T;
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const int key = k0 + 8 * j + 2 * cq + (e & 1);
-          s[j][e] = (!tail || key < T) ? s[j][e] * kScaleLog2 : -INFINITY;
-          bm[e >> 1] = fmaxf(bm[e >> 1], s[j][e]);
-        }
-      }
-      float corr[2];
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {
-        bm[r] = fmaxf(bm[r], __shfl_xor_sync(0xffffffffu, bm[r], 1));
-        bm[r] = fmaxf(bm[r], __shfl_xor_sync(0xffffffffu, bm[r], 2));
-        const float nm = fmaxf(mx[r], bm[r]);
-        corr[r] = fast_ex2(mx[r] - nm);
-        mx[r] = nm;
-        l[r] *= corr[r];
-      }
-      uint32_t pf[4];
-      {
-        const float p00 = fast_ex2(s[0][0] - mx[0]), p01 = fast_ex2(s[0][1] - mx[0]);
-        const float p02 = fast_ex2(s[0][2] - mx[1]), p03 = fast_ex2(s[0][3] - mx[1]);
-        const float p10 = fast_ex2(s[1][0] - mx[0]), p11 = fast_ex2(s[1][1] - mx[0]);
-        const float p12 = fast_ex2(s[1][2] - mx[1]), p13 = fast_ex2(s[1][3] - mx[1]);
-        l[0] += (p00 + p01) + (p10 + p11);
-        l[1] += (p02 + p03) + (p12 + p13);
-        pf[0] = pack16<FP16>(p00, p01); pf[1] = pack16<FP16>(p02, p03);
-        pf[2] = pack16<FP16>(p10, p11); pf[3] = pack16<FP16>(p12, p13);
-      }
-      if (k0 > 0) {
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-          o[n][0] *= corr[0]; o[n][1] *= corr[0]; o[n][2] *= corr[1]; o[n][3] *= corr[1];
-        }
-      }
-      const int vrow = min(k0 + lrow, rmax);
-#pragma unroll
-      for (int n = 0; n < 8; n += 2) {
-        uint32_t b0, b1, b2, b3;
-        asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                     : "=r"(b0), "=r"(b1), "=r"(b2), "=r"(b3) : "r"(v_addr + sw128(vrow, 8 * n + lcol8)));
-        mma_16816<FP16>(o[n], pf, b0, b1);
-        mma_16816<FP16>(o[n + 1], pf, b2, b3);
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-      l[r] += __shfl_xor_sync(0xffffffffu, l[r], 1);
-      l[r] += __shfl_xor_sync(0xffffffffu, l[r], 2);
-    }
-    const float inv0 = 1.0f / l[0], inv1 = 1.0f / l[1];
-    // transpose the context block through the (consumed) Q rows of this block: 16-byte row stores
-    __syncwarp();
-    {
-      const int r0 = m0 + g, r1 = m0 + g + 8;
-#pragma unroll
-      for (int n = 0; n < 8; ++n) {
-        if (r0 < R)
-          asm volatile("st.shared.b32 [%0], %1;" ::"r"(q_addr + sw128(r0, 8 * n + 2 * cq)),
-                       "r"(pack16<FP16>(o[n][0] * inv0, o[n][1] * inv0)) : "memory");
-        if (r1 < R)
-          asm volatile("st.shared.b32 [%0], %1;" ::"r"(q_addr + sw128(r1, 8 * n + 2 * cq)),
-                       "r"(pack16<FP16>(o[n][2] * inv1, o[n][3] * inv1)) : "memory");
-      }
-    }
-    __syncwarp();
-    {
-      const int r_off = lane >> 3, ch = lane & 7;
-#pragma unroll
-      for (int rr = 0; rr < 16; rr += 4) {
-        const int q = m0 + rr + r_off;
-        if (q < T) {
-          uint4 v;
-          asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w)
-                       : "r"(q_addr + sw128(q, ch * 8)));
-          *reinterpret_cast<uint4*>(ob + (size_t)q * H + ch * 8) = v;
-        }
-      }
-    }
-  }
-}
-
-template <bool FP16>
-__global__ void __launch_bounds__(32 * (1 + ATT_TMA_MAX_HEADS), 1)
-attention_tma_kernel(const __grid_constant__ AttTmaMaps maps, __nv_bfloat16* __restrict__ ctx, CopyPlan plan,
-                     int32_t n_copies, int H, int NH) {
-  extern __shared__ uint8_t att_tma_dyn[];
-  const uint32_t raw = smem_u32(att_tma_dyn);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  const uint32_t bar_full = base + ATT_TMA_RING_BYTES;               // ATT_TMA_SLOTS x 8 B
-  const uint32_t bar_empty = bar_full + 8 * ATT_TMA_SLOTS;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < ATT_TMA_SLOTS; ++s) {
-      mbar_init(bar_full + 8 * s, 1);
-      mbar_init(bar_empty + 8 * s, (uint32_t)NH);
-    }
-    fence_barrier_init();
-#pragma unroll
-    for (int i = 0; i < ATT_TMA_MAPS; ++i) prefetch_tensormap(&maps.m[i]);
-  }
-  __syncthreads();
-  // Producer and consumers walk the same copies in the same order and place them identically:
-  // copy number i (of the accepted ones) uses barrier slot i % SLOTS and the byte range
-  // [off_i, off_i + size_i) with off_i = (cur + size_i <= RING) ? cur : 0.
-  const uint32_t row_bytes = (uint32_t)(3 * NH * 128);
-  uint32_t cur = 0;
-  int i = 0;
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t beg[ATT_TMA_SLOTS] = {0, 0, 0, 0}, end[ATT_TMA_SLOTS] = {0, 0, 0, 0};   // ranges of the last SLOTS copies
-      for (int c = blockIdx.x; c < n_copies; c += gridDim.x) {
-        const int T = plan.seq_len[c];
-        if (T > ATT_TMA_ROWS) continue;
-        const int start = plan.seq_start[c];
-        const int R = (T + 7) & ~7;
-        const uint32_t size = row_bytes * (uint32_t)R;
-        if (cur + size > (uint32_t)ATT_TMA_RING_BYTES) cur = 0;
-        const uint32_t off = cur;
-        cur += size;
-        const int slot = i % ATT_TMA_SLOTS;
-        // the slot's previous user (copy i - SLOTS) must be released ...
-        mbar_wait(bar_empty + 8 * slot, (uint32_t)(((i / ATT_TMA_SLOTS) & 1) ^ 1));
-        // ... and so must every younger copy whose bytes overlap the new range (releases are FIFO: the
-        // youngest overlapping one is enough)
-        for (int j = i - 1; j > i - ATT_TMA_SLOTS && j >= 0; --j) {
-          const int sj = j % ATT_TMA_SLOTS;
-          if (beg[sj] < off + size && off < end[sj]) {
-            mbar_wait(bar_empty + 8 * sj, (uint32_t)((j / ATT_TMA_SLOTS) & 1));
-            break;
-          }
-        }
-        beg[slot] = off;
-        end[slot] = off + size;
-        const CUtensorMap* m = &maps.m[(R >> 3) - 1];
-        mbar_arrive_expect_tx(bar_full + 8 * slot, size);
-        const uint32_t dst = base + off;
-        for (int sl = 0; sl < 3 * NH; ++sl)
-          tma_load_2d(dst + (uint32_t)(sl * R * 128), m, bar_full + 8 * slot, sl * 64, start);
-        ++i;
-      }
-    }
-  } else if (warp <= NH) {
-    const int head = warp - 1;
-    for (int c = blockIdx.x; c < n_copies; c += gridDim.x) {
-      const int T = plan.seq_len[c];
-      if (T > ATT_TMA_ROWS) continue;
-      const int start = plan.seq_start[c];
-      const int R = (T + 7) & ~7;
-      const uint32_t size = row_bytes * (uint32_t)R;
-      if (cur + size > (uint32_t)ATT_TMA_RING_BYTES) cur = 0;
-      const uint32_t sb = base + cur;
-      cur += size;
-      const int slot = i % ATT_TMA_SLOTS;
-      mbar_wait(bar_full + 8 * slot, (uint32_t)((i / ATT_TMA_SLOTS) & 1));
-      const uint32_t tile = (uint32_t)(R * 128);
-      attn_compute_sw<FP16>(sb + (uint32_t)head * tile, sb + (uint32_t)(NH + head) * tile, sb + (uint32_t)(2 * NH + head) * tile,
-                            ctx + (size_t)start * H + head * 64, T, R, H, lane);
-      fence_proxy_async_smem();      // this warp wrote the tiles (zero fill, output staging) before the next TMA refill
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_empty + 8 * slot);
-      ++i;
-    }
   }
 }
 
@@ -1141,63 +876,22 @@ int launch_row_src(CopyPlan plan, int32_t n_copies, cudaStream_t s) {
   return PLLB_OK;
 }
 
-int launch_residual_ln(const float* y, float* hidden_f32, void* hidden_bf16, const float* g, const float* b, float eps,
-                       int64_t rows, int H, bool fp16, cudaStream_t s) {
-  if (rows <= 0) return PLLB_OK;
-  const unsigned grid = (unsigned)ceil_div(rows, WARPS_PER_BLOCK);
-#define LNR(F) ln_kernel<VEC, true, F><<<grid, WARPS_PER_BLOCK * 32, 0, s>>>(                                  \
-      y, hidden_f32, reinterpret_cast<__nv_bfloat16*>(hidden_bf16), g, b, eps, rows)
-  PLLB_DISPATCH_VEC(H, (fp16 ? LNR(true) : LNR(false)));
-#undef LNR
-  PLLB_LAUNCH_CHECK("ln_kernel<resid>");
-  return PLLB_OK;
-}
-
 int launch_plain_ln_bf16(const float* x, void* out_bf16, const float* g, const float* b, float eps, int64_t rows, int H,
                          bool fp16, cudaStream_t s) {
   if (rows <= 0) return PLLB_OK;
   const unsigned grid = (unsigned)ceil_div(rows, WARPS_PER_BLOCK);
-#define LNP(F) ln_kernel<VEC, false, F><<<grid, WARPS_PER_BLOCK * 32, 0, s>>>(                                 \
-      x, nullptr, reinterpret_cast<__nv_bfloat16*>(out_bf16), g, b, eps, rows)
+#define LNP(F) ln_kernel<VEC, F><<<grid, WARPS_PER_BLOCK * 32, 0, s>>>(                                        \
+      x, reinterpret_cast<__nv_bfloat16*>(out_bf16), g, b, eps, rows)
   PLLB_DISPATCH_VEC(H, (fp16 ? LNP(true) : LNP(false)));
 #undef LNP
   PLLB_LAUNCH_CHECK("ln_kernel<plain>");
   return PLLB_OK;
 }
 
-int launch_attention(const void* qkv_bf16, void* ctx_bf16, CopyPlan plan, int32_t n_copies, int H, int NH, int max_T,
-                     bool fp16, bool shared_rows, int64_t qkv_rows, cudaStream_t s) {
+int launch_attention(const void* qkv_bf16, void* ctx_bf16, CopyPlan plan, int32_t n_copies, int H, int NH, bool fp16,
+                     bool shared_rows, cudaStream_t s) {
   if (n_copies <= 0) return PLLB_OK;
   if (H != NH * 64) return fail(PLLB_ERR_INVALID, "attention: head dim must be 64");
-  // TMA-fed persistent kernel for the copies of at most ATT_TMA_ROWS rows: opt-in (PLLB_ATT_TMA=1).
-  // Measured (round 2, ncu): it moves the same bytes no faster than attention_mma_kernel — both are
-  // bound by instruction issue (~900 warp instructions per (copy, head), issue slots 50 % busy with
-  // the 13-16 warps per SM that 128 registers allow), not by load latency — see DESIGN.md §3.2.
-  const char* tma_env = getenv("PLLB_ATT_TMA");
-  const bool tma_on = tma_env && atoi(tma_env) != 0;
-  int skip_le = 0;
-  if (tma_on && !shared_rows && NH <= ATT_TMA_MAX_HEADS && qkv_rows > 0) {
-    AttTmaMaps maps;
-    for (int i = 0; i < ATT_TMA_MAPS; ++i) {
-      int rc = get_tmap_2d(&maps.m[i], qkv_bf16, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)qkv_rows, (uint64_t)3 * H,
-                           (uint32_t)(8 * (i + 1)), 64);
-      if (rc) return rc;
-    }
-    const int smem = ATT_TMA_RING_BYTES + 16 * ATT_TMA_SLOTS + 1024;
-    const int smem_max = smem;
-    const int grid = (int)std::min<int64_t>(n_copies, sm_count());
-    const int threads = 32 * (1 + NH);
-    if (fp16) {
-      PLLB_CUDA(opt_in_smem(attention_tma_kernel<true>, smem_max));
-      attention_tma_kernel<true><<<grid, threads, smem, s>>>(maps, reinterpret_cast<__nv_bfloat16*>(ctx_bf16), plan, n_copies, H, NH);
-    } else {
-      PLLB_CUDA(opt_in_smem(attention_tma_kernel<false>, smem_max));
-      attention_tma_kernel<false><<<grid, threads, smem, s>>>(maps, reinterpret_cast<__nv_bfloat16*>(ctx_bf16), plan, n_copies, H, NH);
-    }
-    PLLB_LAUNCH_CHECK("attention_tma_kernel");
-    skip_le = ATT_TMA_ROWS;
-    if (max_T <= ATT_TMA_ROWS) return PLLB_OK;          // no longer copy in this chunk
-  }
   const int64_t pairs = (int64_t)n_copies * NH;
   const int smem = ATT_WARPS * ATT_STAGE_ELEMS * 2;
   const unsigned grid = (unsigned)ceil_div(pairs, ATT_WARPS);
@@ -1206,7 +900,7 @@ int launch_attention(const void* qkv_bf16, void* ctx_bf16, CopyPlan plan, int32_
     PLLB_CUDA(opt_in_smem(attention_mma_kernel<F, S>, smem));                                                      \
     attention_mma_kernel<F, S><<<grid, ATT_WARPS * 32, smem, s>>>(reinterpret_cast<const __nv_bfloat16*>(qkv_bf16), \
                                                                   reinterpret_cast<__nv_bfloat16*>(ctx_bf16), plan, \
-                                                                  n_copies, H, NH, skip_le);                       \
+                                                                  n_copies, H, NH);                                \
   } while (0)
   if (fp16) { if (shared_rows) ATT(true, true); else ATT(true, false); }
   else { if (shared_rows) ATT(false, true); else ATT(false, false); }

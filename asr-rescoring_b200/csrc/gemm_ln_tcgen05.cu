@@ -69,11 +69,7 @@ constexpr int smem_without_params() {
 // (the staged single-CTA form at H = 1024 has no 3 KB left: it keeps the global loads)
 template <int CN, bool STAGED, bool PAIR>
 constexpr bool params_in_smem() {
-#ifdef PLLB_LN_PARAMS_GLOBAL
-  return false;                                // A/B builds
-#else
   return smem_without_params<CN, STAGED, PAIR>() + SMEM_PAR <= SMEM_LIMIT;
-#endif
 }
 template <int CN, bool STAGED, bool PAIR>
 constexpr int smem_total() {
@@ -92,9 +88,6 @@ struct LnParams {
   const float* gamma;
   const float* beta;
   float eps;
-  int amc;                // 1: the A tile is TMA-multicast to the CN CTAs of the cluster (each issues a share of its 32-row boxes)
-  int apf;                // 1: the producer prefetches the NEXT row block's A boxes into L2 while this block is multiplied
-  int a_blocked;          // 1: A is stored K-blocked (4-D tensor map: tiles of 32 rows x 64 columns contiguous, common.h)
 };
 
 template <bool FP16>
@@ -202,10 +195,10 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int num_kb = p.K / BK;
   const int n0 = (int)cg * BN;
   // All CN CTAs of a cluster multiply the SAME 128 x K block of A by their own 256 columns of W.
-  // With amc the A stage (four 32-row boxes) is fetched from L2 once per cluster: CTA r issues
+  // With AMC the A stage (four 32-row boxes) is fetched from L2 once per cluster: CTA r issues
   // boxes r, r+CN, ... as TMA multicasts into every CTA's stage, and a stage is reused only after
   // every CTA's MMAs released it (their commits are multicast to all empty barriers).
-  const bool amc = !PAIR && CN > 1 && p.amc != 0;
+  constexpr bool AMC = !PAIR && CN > 1;
   constexpr uint16_t mask_all = (uint16_t)((1u << CN) - 1u);
   constexpr int A_BOX_ROWS = 32, A_BOX_BYTES = A_BOX_ROWS * BK * 2;
 
@@ -217,7 +210,7 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (lane == 0) {
       for (int s = 0; s < STAGES; ++s) {
         mbar_init(bar_full + 8 * s, 1);
-        mbar_init(bar_empty + 8 * s, amc ? CN : 1);          // multicast A: every CTA of the cluster releases the stage
+        mbar_init(bar_empty + 8 * s, AMC ? CN : 1);          // multicast A: every CTA of the cluster releases the stage
       }
       for (int s = 0; s < 2; ++s) {
         mbar_init(bar_tfull + 8 * s, 1);
@@ -254,17 +247,6 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       uint32_t stage = 0, phase = 0;
       for (int mb = cluster; mb < tiles_m; mb += n_clusters) {
         const int m0 = mb * ROWS + (int)rh * BM;
-        // Experiment (PLLB_LN_APF, off by default): request the NEXT row block's A boxes into L2 one
-        // block ahead.  ncu shows the K = H launch waiting 20 % of its epilogue time for the accumulator
-        // (A comes from HBM, 3 stages of 64 columns in flight), but the prefetch made it SLOWER
-        // (attention-output 490 -> 547 ms, FFN2 940 -> 1320 ms in the C2 step): the memory system is
-        // throughput-bound there, extra requests only queue in front of the real loads.
-        if (p.apf && !p.a_blocked && mb + n_clusters < tiles_m) {
-          const int m0n = (mb + n_clusters) * ROWS + (int)rh * BM;
-          const int b0 = amc ? (int)rank : 0, bs = amc ? CN : 1;
-          for (int kb = 0; kb < num_kb; ++kb)
-            for (int b = b0; b < BM / A_BOX_ROWS; b += bs) tma_prefetch_l2_2d(&tmA, kb * BK, m0n + b * A_BOX_ROWS);
-        }
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(bar_empty + 8 * stage, phase ^ 1);
           if constexpr (PAIR) {
@@ -273,32 +255,22 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (rh == 0) mbar_arrive_expect_tx(bar_full + 8 * stage, 2 * (A_STAGE_BYTES + B_BYTES));
 #pragma unroll
             for (int b = 0; b < BM / A_BOX_ROWS; ++b)
-              if (p.a_blocked) tma_load_4d_2sm(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, lead_full, 0, 0, kb, (m0 >> 5) + b);
-              else tma_load_2d_2sm(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, lead_full, kb * BK, m0 + b * A_BOX_ROWS);
+              tma_load_2d_2sm(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, lead_full, kb * BK, m0 + b * A_BOX_ROWS);
             tma_load_2d_2sm(sB + stage * B_BYTES, &tmB, lead_full, kb * BK, n0 + (int)rh * (BN / 2));
             if (++stage == STAGES) { stage = 0; phase ^= 1; }
             continue;
           }
           mbar_arrive_expect_tx(bar_full + 8 * stage, A_STAGE_BYTES + B_STAGE_BYTES);
           tma_load_2d(sB + stage * B_STAGE_BYTES, &tmB, bar_full + 8 * stage, kb * BK, n0);
-          if (amc) {
-            for (int b = (int)rank; b < BM / A_BOX_ROWS; b += CN) {
-              if (p.a_blocked)
-                tma_load_4d_multicast(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, 0, 0, kb,
-                                      (m0 >> 5) + b, mask_all);
-              else
-                tma_load_2d_multicast(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, kb * BK,
-                                      m0 + b * A_BOX_ROWS, mask_all);
-            }
+          if constexpr (AMC) {
+            for (int b = (int)rank; b < BM / A_BOX_ROWS; b += CN)
+              tma_load_2d_multicast(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, kb * BK,
+                                    m0 + b * A_BOX_ROWS, mask_all);
           } else {
 #pragma unroll
-            for (int b = 0; b < BM / A_BOX_ROWS; ++b) {
-              if (p.a_blocked)
-                tma_load_4d(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, 0, 0, kb, (m0 >> 5) + b);
-              else
-                tma_load_2d(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, kb * BK,
-                            m0 + b * A_BOX_ROWS);
-            }
+            for (int b = 0; b < BM / A_BOX_ROWS; ++b)
+              tma_load_2d(sA + stage * A_STAGE_BYTES + b * A_BOX_BYTES, &tmA, bar_full + 8 * stage, kb * BK,
+                          m0 + b * A_BOX_ROWS);
           }
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
@@ -328,7 +300,7 @@ gemm_ln_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                                make_kmajor_sw128_desc(b_addr + k * UMMA_K * 2), idesc, (kb | k) != 0 ? 1u : 0u);
           }
           if constexpr (PAIR) tcgen05_commit_2cta_multicast(bar_empty + 8 * stage, mask_pair);
-          else if (amc) tcgen05_commit_multicast(bar_empty + 8 * stage, mask_all);
+          else if constexpr (AMC) tcgen05_commit_multicast(bar_empty + 8 * stage, mask_all);
           else tcgen05_commit(bar_empty + 8 * stage);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
@@ -568,11 +540,8 @@ int launch_cn(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& t
     }
     mc = n;
   }
-  // PLLB_LN_MAX_CLUSTERS: experiment knob (how does the step react to fewer SMs under the power cap?)
-  static const int cap = [] { const char* e = getenv("PLLB_LN_MAX_CLUSTERS"); return e ? atoi(e) : 0; }();
-  const int limit = cap > 0 && cap < mc ? cap : mc;
   const int64_t tiles_m = ceil_div(M, PAIR ? 2 * BM : BM);
-  const int clusters = (int)(tiles_m < limit ? tiles_m : limit);
+  const int clusters = (int)(tiles_m < mc ? tiles_m : mc);
   cfg.gridDim = dim3(CSIZE * clusters);
   PLLB_CUDA(cudaLaunchKernelEx(&cfg, kern, ta, tb, t16, lp));
   ++g_launch_counter;
@@ -591,17 +560,13 @@ int launch_cn_dt(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap
 }  // namespace
 
 int launch_gemm_ln(const void* A, const void* W, const float* bias, const float* gamma, const float* beta, float eps,
-                   float* hidden_f32, void* hidden_16, int64_t M, int H, int K, int dt, cudaStream_t stream,
-                   bool a_blocked) {
+                   float* hidden_f32, void* hidden_16, int64_t M, int H, int K, int dt, cudaStream_t stream) {
   if (M <= 0) return PLLB_OK;
   if (H % BN != 0 || H / BN > MAX_CN || K % BK != 0 || M > INT32_MAX)
     return fail(PLLB_ERR_INVALID, "gemm_ln: need H in {256,512,768,1024} and K % 64 == 0");
   // epilogue-paced (K <= H): staged 16-bit output; mainloop-paced (K > H): deeper operand ring
-  // PLLB_LN_STAGED (experiment knob): 0 / 1 forces the direct / staged form for every launch
-  static const int staged_force = [] { const char* e = getenv("PLLB_LN_STAGED"); return e ? atoi(e) : -1; }();
-  const bool staged = staged_force >= 0 ? staged_force != 0 : K <= H;
-  // cta_group::2 pairs inside the LayerNorm cluster (PLLB_LN_PAIR: 0 never, 1 default policy, 2 always,
-  // 3 every mainloop-paced launch whatever the hidden size).
+  const bool staged = K <= H;
+  // cta_group::2 pairs inside the LayerNorm cluster (PLLB_LN_PAIR: 0 never, 1 default policy, 2 always).
   // Default: the mainloop-paced launches (K > H, i.e. FFN2) for H = 256 (cluster 2: 148 SMs), H = 768
   // (cluster 6: 132 SMs against 135; measured FFN2 -15.5 %, C2 step -3.0 %) and H = 1024 (cluster 8: 120
   // SMs against 132; measured FFN2 -8.7 %, C4 step -2.0 %).  H = 512 would drop from 148 to 132 SMs
@@ -610,20 +575,13 @@ int launch_gemm_ln(const void* A, const void* W, const float* bias, const float*
   const int pair_policy = pe ? atoi(pe) : 1;
   const int cn = H / BN;
   const bool mainloop_paced = K > H;
-  const bool pair = M > 2 * BM && (pair_policy == 2 || (pair_policy == 3 && mainloop_paced) ||
-                                   (pair_policy == 1 && mainloop_paced && cn != 2));
+  const bool pair = M > 2 * BM && (pair_policy == 2 || (pair_policy == 1 && mainloop_paced && cn != 2));
   CUtensorMap ta, tb, t16;
   int rc;
-  if (a_blocked) {
-    if ((rc = get_tmap_blocked(&ta, A, (uint64_t)M, (uint64_t)K))) return rc;
-  } else if ((rc = tmap2d(&ta, A, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)M, (uint64_t)K, 32, BK))) return rc;   // 32-row boxes
+  if ((rc = tmap2d(&ta, A, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)M, (uint64_t)K, 32, BK))) return rc;   // 32-row boxes
   if ((rc = tmap2d(&tb, W, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)H, (uint64_t)K, pair ? BN / 2 : BN, BK))) return rc;
   if ((rc = tmap2d(&t16, hidden_16, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)M, (uint64_t)H, 32, 64))) return rc;
-  static const int amc = [] { const char* e = getenv("PLLB_LN_AMC"); return e ? atoi(e) : 1; }();
-  // PLLB_LN_APF: L2 prefetch of the next row block's A boxes: 0 never (default: measured slower), 1 the K <= H launches, 2 every launch
-  static const int apf_policy = [] { const char* e = getenv("PLLB_LN_APF"); return e ? atoi(e) : 0; }();
-  const int apf = apf_policy == 2 || (apf_policy == 1 && staged) ? 1 : 0;
-  LnParams lp{(int)M, K, H, hidden_f32, reinterpret_cast<__nv_bfloat16*>(hidden_16), bias, gamma, beta, eps, amc, apf, a_blocked ? 1 : 0};
+  LnParams lp{(int)M, K, H, hidden_f32, reinterpret_cast<__nv_bfloat16*>(hidden_16), bias, gamma, beta, eps};
 #define PLLB_LN(CN_)                                                                                          \
   case CN_:                                                                                                   \
     switch (dt) {                                                                                             \

@@ -22,8 +22,6 @@
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
 #include "common.h"
 #include "ptx.cuh"
 
@@ -34,20 +32,14 @@ namespace {
 constexpr int BM = 128;
 constexpr int BN = 256;
 constexpr int BK = 64;
-#ifndef PLLB_GEMM_STAGES
-#define PLLB_GEMM_STAGES 4
-#endif
-#ifndef PLLB_GEMM_EPI_BUFS
-#define PLLB_GEMM_EPI_BUFS 1
-#endif
-constexpr int STAGES = PLLB_GEMM_STAGES;
+constexpr int STAGES = 4;
 constexpr int UMMA_K = 16;
 constexpr int A_STAGE_BYTES = BM * BK * 2;   // 16 KiB
 constexpr int B_STAGE_BYTES = BN * BK * 2;   // 32 KiB
 constexpr int EPI_WARPS = 8;                 // two per TMEM lane quarter, each owning half of the BN columns
 constexpr int EPI_COLS = BN / 2;             // columns per epilogue warp
 constexpr int EPI_BUF_BYTES = 32 * 128;      // one 32-row x 128-byte swizzled box
-constexpr int EPI_BUFS = PLLB_GEMM_EPI_BUFS;  // per epilogue warp
+constexpr int EPI_BUFS = 1;                  // per epilogue warp
 constexpr int NUM_THREADS = 32 * (2 + EPI_WARPS);
 constexpr int TMEM_COLS = 512;               // 2 accumulator stages x BN columns
 constexpr int SMEM_PIPE = STAGES * (A_STAGE_BYTES + B_STAGE_BYTES);
@@ -59,8 +51,6 @@ struct KParams {
   int M, N, K;
   const float* bias;
   LseArgs lse;
-  int early_release;
-  int c_blocked;          // the 16-bit output goes out in the K-blocked layout (4-D tensor map, common.h)
 };
 
 // HF activations "gelu" = nn.functional.gelu (erf form): 0.5 x (1 + erf(x / sqrt 2)).
@@ -264,9 +254,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const uint32_t my_buf = sEpi + ew * EBUFS * EPI_BUF_BYTES;
     uint32_t acc = 0, acc_phase = 0, buf_i = 0;
     // The accumulator buffer goes back to the MMA warp as soon as its last columns sit in registers
-    // (16-bit epilogues: before the bias / GELU math and the stores of the last 64 columns), not after
-    // them: PLLB_GEMM_EARLY_RELEASE=0 restores the late release.
-    const bool early_release = p.early_release != 0;
+    // (16-bit epilogues: before the bias / GELU math and the stores of the last 64 columns), not after them.
     auto release_acc = [&]() {
       tcgen05_fence_before();
       __syncwarp();
@@ -322,7 +310,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           tmem_ld_32x32b_x32(t_addr + c0, r0);
           tmem_ld_32x32b_x32(t_addr + c0 + 32, r1);
           tcgen05_wait_ld();
-          if (early_release && c0 + 64 >= cbase + EPI_COLS) release_acc();   // last columns are in registers
+          if (c0 + 64 >= cbase + EPI_COLS) release_acc();   // last columns are in registers
           const uint32_t buf = my_buf + (buf_i % EBUFS) * EPI_BUF_BYTES;
           if (lane == 0) tma_store_wait_read<EBUFS - 1>();      // the store that last read this buffer is done
           __syncwarp();
@@ -355,8 +343,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
-            if (p.c_blocked) tma_store_4d(&tmC, buf, 0, 0, (n0 + c0) >> 6, (m0 + q * 32) >> 5);
-            else tma_store_2d(&tmC, buf, n0 + c0, m0 + q * 32);
+            tma_store_2d(&tmC, buf, n0 + c0, m0 + q * 32);
             tma_store_commit();
           }
         }
@@ -394,7 +381,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
       }
       // all tcgen05.ld of this accumulator have completed (wait::ld above): release it
-      if (!(early_release && (EPI == EPI_BIAS_BF16 || EPI == EPI_BIAS_GELU_BF16))) release_acc();
+      if constexpr (EPI != EPI_BIAS_BF16 && EPI != EPI_BIAS_GELU_BF16) release_acc();
       acc ^= 1;
       if (acc == 0) acc_phase ^= 1;
     }
@@ -463,29 +450,15 @@ int launch_epi(const CUtensorMap& a, const CUtensorMap& b, const CUtensorMap& c,
 }
 
 // 0 = one CTA per tile, 1 = CTA pairs with TMA multicast of W, 2 = cta_group::2 MMA.
-// Default: cta_group::2, except for the GELU epilogue — FFN1 is paced by its epilogue's CUDA-core
+// M > 128: cta_group::2, except for the GELU epilogue — FFN1 is paced by its epilogue's CUDA-core
 // math, where the cluster-scope accumulator hand-back of mode 2 costs more than the deeper
 // operand ring gains (measured ABAB inside the C2 step: QKV 671 vs 727 ms, FFN1 905-918 vs 884 ms).
-int pair_mode(int epilogue) {
-  static int v = -2;
-  if (v == -2) {
-    const char* e = getenv("PLLB_GEMM_MODE");
-    v = e ? atoi(e) : -1;
-    if (v < -1 || v > 2) v = -1;
-  }
-  if (v >= 0) return v;
-  if (epilogue == EPI_BIAS_GELU_BF16) {
-    const char* g = getenv("PLLB_GEMM_MODE_GELU");        // experiment knob: pair mode of the FFN1 launch alone
-    if (g && atoi(g) >= 0 && atoi(g) <= 2) return atoi(g);
-    return 1;
-  }
-  return 2;
-}
+int pair_mode(int epilogue) { return epilogue == EPI_BIAS_GELU_BF16 ? 1 : 2; }
 
 }  // namespace
 
 int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C, int64_t M, int N, int K,
-                        int epilogue, const LseArgs* lse, int dt, cudaStream_t stream, bool c_blocked) {
+                        int epilogue, const LseArgs* lse, int dt, cudaStream_t stream) {
   if (M <= 0) return PLLB_OK;
   if (N % BN != 0 || K % BK != 0 || M > INT32_MAX)
     return fail(PLLB_ERR_INVALID, "gemm: need N % 256 == 0 and K % 64 == 0");
@@ -496,26 +469,19 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C
   const bool mc = mode != 0;
   if ((rc = make_tmap(&tb, W, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)N, (uint64_t)K, mc ? BN / 2 : BN, BK))) return rc;
   tc = ta;
-  if (c_blocked && epilogue != EPI_BIAS_BF16 && epilogue != EPI_BIAS_GELU_BF16)
-    return fail(PLLB_ERR_INVALID, "gemm: the K-blocked output layout exists for the 16-bit epilogues only");
-  if (c_blocked) {
-    if ((rc = get_tmap_blocked(&tc, C, (uint64_t)M, (uint64_t)N))) return rc;
-  } else if (epilogue == EPI_BIAS_BF16 || epilogue == EPI_BIAS_GELU_BF16) {
+  if (epilogue == EPI_BIAS_BF16 || epilogue == EPI_BIAS_GELU_BF16) {
     if ((rc = make_tmap(&tc, C, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)M, (uint64_t)N, 32, 64))) return rc;
   } else if (epilogue == EPI_BIAS_F32 || epilogue == EPI_BIAS_GELU_F32) {
     if ((rc = make_tmap(&tc, C, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (uint64_t)M, (uint64_t)N, 32, 32))) return rc;
   }
   KParams kp{};
-  kp.M = (int)M; kp.N = N; kp.K = K; kp.bias = bias; kp.c_blocked = c_blocked ? 1 : 0;
-  { const char* e = getenv("PLLB_GEMM_EARLY_RELEASE"); kp.early_release = e ? atoi(e) : 1; }
+  kp.M = (int)M; kp.N = N; kp.K = K; kp.bias = bias;
   if (epilogue == EPI_LSE) {
     if (!lse) return fail(PLLB_ERR_INVALID, "gemm: LSE epilogue needs LseArgs");
     kp.lse = *lse;
   }
   int grid;
-  // PLLB_GEMM_MAX_CTAS: experiment knob (SM-count sensitivity under the power cap)
-  static const int cta_cap = [] { const char* e = getenv("PLLB_GEMM_MAX_CTAS"); return e ? atoi(e) : 0; }();
-  const int sms = cta_cap > 0 && cta_cap < sm_count() ? cta_cap : sm_count();
+  const int sms = sm_count();
   if (mc) {
     const int64_t units = ceil_div(ceil_div(M, BM), 2) * (N / BN);
     const int64_t clusters = units < sms / 2 ? units : sms / 2;

@@ -81,12 +81,6 @@ __device__ __forceinline__ void fence_proxy_async_smem() {
 __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
 }
-// L2 prefetch of a 2-D tile (no shared-memory destination, no completion tracking): the later
-// cp.async.bulk.tensor load of the same box then pays an L2 hit instead of the HBM latency.
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* m, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1) : "memory");
-}
 // 2-D tile load: coordinates {c0 = innermost (element index), c1 = row}.
 __device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap* m, uint32_t bar, int c0, int c1) {
   asm volatile(
@@ -107,28 +101,6 @@ __device__ __forceinline__ void tma_load_2d_multicast(uint32_t smem_dst, const C
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, uint32_t smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
                ::"l"(reinterpret_cast<uint64_t>(m)), "r"(smem_src), "r"(c0), "r"(c1)
-               : "memory");
-}
-// 4-D forms for K-blocked 16-bit activations (common.h: tiles of 32 rows x 64 columns stored
-// contiguously; coordinates {column in tile, row in tile, column tile, row tile}).
-__device__ __forceinline__ void tma_load_4d(uint32_t smem_dst, const CUtensorMap* m, uint32_t bar, int c0, int c1, int c2,
-                                            int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_multicast(uint32_t smem_dst, const CUtensorMap* m, uint32_t bar, int c0, int c1,
-                                                      int c2, int c3, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(cta_mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, uint32_t smem_src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(smem_src), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
                : "memory");
 }
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
@@ -179,13 +151,6 @@ __device__ __forceinline__ void tma_load_2d_2sm(uint32_t smem_dst, const CUtenso
   asm volatile(
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(cluster_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_2sm(uint32_t smem_dst, const CUtensorMap* m, uint32_t cluster_bar, int c0,
-                                                int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(cluster_bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
       : "memory");
 }
 __device__ __forceinline__ void tmem_alloc_2cta(uint32_t smem_dst, uint32_t ncols) {

@@ -778,30 +778,6 @@ def test_two_gpu_drop_in_outputs_identical_to_one_gpu():
     assert "identical to the 1-GPU files" in out.stdout and "row-list input" in out.stdout and "sharded sweep" in out.stdout
 
 
-def test_tma_fed_attention_kernel_is_bit_identical(monkeypatch):
-    """PLLB_ATT_TMA=1 routes the copies of <= 32 rows through attention_tma_kernel (TMA box loads into
-    a byte-granular ring with up to four copies in flight, producer warp + one warp per head): same
-    blocks, same MMA order, so scores and per-token terms must equal the default kernel's bit for
-    bit — for 4, 8 and 12 heads, with sequences on both sides of the 32-row limit and many ring wraps."""
-    rng = np.random.default_rng(11)
-    for hidden, layers in ((256, 4), (512, 3), (768, 3)):
-        cfg = dict(num_layers=layers, hidden=hidden, num_heads=hidden // 64, intermediate=2 * hidden, vocab=1500,
-                   max_position=80, type_vocab=2, ln_eps=1e-12)
-        sd = synth.random_init_state_dict(cfg, 5, perturb=True)
-        lens = [int(x) for x in rng.integers(1, 31, size=60)] + [22, 23, 24, 29, 30, 31, 47, 6, 30, 30, 1]
-        off = np.zeros(len(lens) + 1, np.int64)
-        np.cumsum(lens, out=off[1:])
-        tok = rng.integers(104, cfg["vocab"], size=int(off[-1])).astype(np.int32)
-        monkeypatch.delenv("PLLB_ATT_TMA", raising=False)
-        with engine.PllScorer(sd, cfg, max_chunk_tokens=4096) as sc:
-            a, ta = sc.score_packed(tok, off, return_token_logp=True)
-        monkeypatch.setenv("PLLB_ATT_TMA", "1")
-        with engine.PllScorer(sd, cfg, max_chunk_tokens=4096) as sc:
-            b, tb = sc.score_packed(tok, off, return_token_logp=True)
-        monkeypatch.delenv("PLLB_ATT_TMA", raising=False)
-        assert np.array_equal(a, b) and np.array_equal(ta, tb) and np.isfinite(a).all(), hidden
-
-
 def test_paired_layernorm_clusters_match_the_single_cta_form(monkeypatch):
     """gemm_ln_kernel<.., PAIR>: cta_group::2 pairs inside the LayerNorm cluster (256-row blocks, M = 256
     MMAs, half of the W box per CTA) against the single-CTA form (PLLB_LN_PAIR=0) and the forced form
