@@ -6,7 +6,8 @@ reference's module — ``bert.*`` (a transformers BertModel) plus ``linear.weigh
 ``linear.bias`` [1] (RescoreBert/model.py:7-11).  ``score_packed`` / ``__call__`` replace the
 forward (model.py:13-21) and the padded batches of RescoreBert/main.py:31-75: every hypothesis
 runs once through the B200 encoder as ``[CLS] t [SEP]`` (varlen packed, no padding) and
-``lm_score = Linear([CLS] state)``.  Training (MD / MWER / MWED losses) is out of scope.
+``lm_score = Linear([CLS] state)``.  Training the student on the teacher's PLLs (MD and MWER losses;
+MWED is not built) is ``RescoreBert/train.py``; the state_dict it returns loads here directly.
 """
 from __future__ import annotations
 

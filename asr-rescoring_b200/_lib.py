@@ -49,6 +49,10 @@ class TrainDesc(ctypes.Structure):
                 ("max_rows", c_int32), ("max_seq", c_int32)]
 
 
+class ClsLossDesc(ctypes.Structure):
+    _fields_ = [("md_weight", c_float), ("mwer_weight", c_float), ("am_weight", c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/pllb.h declares
 SIGNATURES = {
     "pllb_last_error": (c_char_p, []),
@@ -89,6 +93,12 @@ SIGNATURES = {
     "pllb_train_row_losses_host": (c_int, [c_void_p, c_void_p, c_int32]),
     "pllb_train_export": (c_int, [c_void_p, POINTER(Weights)]),
     "pllb_train_export_grads": (c_int, [c_void_p, POINTER(Weights)]),
+    "pllb_cls_train_create": (c_int, [POINTER(c_void_p), POINTER(ModelDesc), POINTER(Weights), c_void_p, c_void_p,
+                                      POINTER(TrainDesc), POINTER(ClsLossDesc), c_int]),
+    "pllb_cls_train_step_host": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32,
+                                         c_int32, c_int32, POINTER(c_float), c_void_p]),
+    "pllb_cls_train_export": (c_int, [c_void_p, POINTER(Weights), c_void_p, c_void_p]),
+    "pllb_cls_train_export_grads": (c_int, [c_void_p, POINTER(Weights), c_void_p, c_void_p]),
 }
 
 _lib = None

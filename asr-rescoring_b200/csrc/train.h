@@ -54,4 +54,14 @@ int launch_train_embed_bwd(const float* dz, const int32_t* ids, int B, int T, in
 int launch_train_adamw(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2, float eps,
                        float wd, const TrainStepParams* scalars, cudaStream_t s);
 
+// RescoreBert head (pllb_cls_train_*): scores[b] = w . h[b*T, :] + b[0] over the fp32 last-layer output h [B*T, H]
+int launch_train_cls_fwd(const float* h, const float* w, const float* b, int B, int T, int H, float* scores, cudaStream_t s);
+// MD + MWER loss of the B scores (group: DEVICE int32[B], 0-based and contiguous); dscore may be null (no backward)
+int launch_train_cls_loss(const float* scores, const float* target, const float* am, const float* err, const int32_t* group,
+                          int B, float md_weight, float mwer_weight, float am_weight, float* dscore, float* out_loss,
+                          cudaStream_t s);
+// dw [H], db [1]: head gradients; dh [B*T, H]: the top-layer gradient the encoder backward starts from
+int launch_train_cls_bwd(const float* h, const float* w, const float* dscore, int B, int T, int H, float* dw, float* db,
+                         float* dh, cudaStream_t s);
+
 }  // namespace pllb

@@ -11,6 +11,9 @@
 //     dX [R, K] = dY [R, N] . (W^T [K, N])^T          dW [N, K] = dY^T [N, R] . (X^T [K, R])^T
 // with R padded to a multiple of 64 by zero columns.  Weight gradients are written by the GEMM
 // epilogue straight into the flat gradient buffer.
+//
+// The same encoder forward / backward also trains the RescoreBert student (pllb_cls_train_*): Linear(H, 1)
+// on the [CLS] row in place of the MLM head, with the MD / MWER loss of include/pllb.h.
 #include <cuda_bf16.h>
 
 #include <algorithm>
@@ -81,6 +84,13 @@ struct pllb_trainer_ctx {
   struct GraphEntry { int seen = 0; cudaGraphExec_t exec = nullptr; int64_t launches = 0; };
   std::unordered_map<uint64_t, GraphEntry> graphs;
   int64_t graph_replays = 0;
+  // RescoreBert trainer (pllb_cls_train_create): Linear(H, 1) on the [CLS] row instead of the MLM head.  The flat
+  // buffers hold the embeddings, the layers and lin_w / lin_b; there are no head / decoder copies and no logits.
+  bool cls = false;
+  Span lin_w, lin_b;
+  pllb_cls_loss_desc loss{};
+  int32_t* group = nullptr;                                                 // [max_rows]
+  float *target = nullptr, *am = nullptr, *err = nullptr, *scores = nullptr, *dscore = nullptr;   // [max_rows] each
 };
 
 namespace {
@@ -130,6 +140,7 @@ int refresh_all(pllb_trainer_ctx* c, cudaStream_t s) {
     RC(refresh_weight(c, l.ff1_w, I, H, l.ff116, l.ff1T16, s));
     RC(refresh_weight(c, l.ff2_w, H, I, l.ff216, l.ff2T16, s));
   }
+  if (c->cls) return PLLB_OK;     // no MLM head, no tied decoder
   RC(refresh_weight(c, c->head_w, H, H, c->head16, c->headT16, s));
   RC(refresh_weight(c, c->word, c->Vp, H, c->E16, c->ET16, s));
   return PLLB_OK;
@@ -150,7 +161,9 @@ int linear_bwd(pllb_trainer_ctx* c, const float* dy32, const __nv_bfloat16* x16,
 }
 
 int copy_in(pllb_trainer_ctx* c, Span dst, const float* src, int64_t n, int64_t dst_off = 0) {
-  if (!src) return fail(PLLB_ERR_INVALID, "pllb_train_create: a weight pointer is null (the MLM head is required)");
+  if (!src)
+    return fail(PLLB_ERR_INVALID, c->cls ? "pllb_cls_train_create: a weight pointer is null"
+                                         : "pllb_train_create: a weight pointer is null (the MLM head is required)");
   PLLB_CUDA(cudaMemcpyAsync(c->P + dst.off + dst_off, src, sizeof(float) * n, cudaMemcpyDeviceToDevice, 0));
   return PLLB_OK;
 }
@@ -160,8 +173,8 @@ int copy_out(const float* buf, Span src, const float* dst, int64_t n, int64_t sr
   return PLLB_OK;
 }
 
-// state_dict tensors <- flat buffer `buf` (parameters or gradients)
-int export_flat(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
+// state_dict tensors <- flat buffer `buf` (parameters or gradients): embeddings and encoder layers
+int export_encoder(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
   const int H = c->d.hidden, I = c->d.intermediate, V = c->d.vocab;
   const int64_t HH = (int64_t)H * H;
   RC(copy_out(buf, c->word, w->word_emb, (int64_t)V * H));
@@ -189,6 +202,14 @@ int export_flat(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
     RC(copy_out(buf, t.out_g, lw.out_ln_g, H));
     RC(copy_out(buf, t.out_be, lw.out_ln_b, H));
   }
+  return PLLB_OK;
+}
+
+// ... plus the MLM head
+int export_flat(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
+  const int H = c->d.hidden, V = c->d.vocab;
+  const int64_t HH = (int64_t)H * H;
+  RC(export_encoder(c, buf, w));
   RC(copy_out(buf, c->head_w, w->head_w, HH));
   RC(copy_out(buf, c->head_b, w->head_b, H));
   RC(copy_out(buf, c->head_g, w->head_ln_g, H));
@@ -213,16 +234,13 @@ TrainDrop make_drop(const pllb_trainer_ctx* c, float p, bool train) {
   return d;
 }
 
-// Every launch of one step (shape-static arguments only; the per-step scalars are read from params_dev).
-// mode 0: loss only (model.eval()); 1: forward + backward + AdamW step; 2: forward + backward, no update
-int enqueue_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
+// The encoder forward of one step: embeddings and every layer.  On return h32 holds the fp32 output of the
+// last layer (and xlast16 its bf16 copy, when the trainer has an MLM head to feed).
+int encoder_fwd(pllb_trainer_ctx* c, int B, int T, const TrainDrop& hd, const TrainDrop& ad, cudaStream_t s) {
   const pllb_model_desc& d = c->d;
-  const int H = d.hidden, I = d.intermediate, NH = d.num_heads, NL = d.num_layers, Vp = c->Vp, V = d.vocab;
-  const int R = B * T, Rp = (int)round_up(R, 64);
-  const bool train = mode != 0;
-  const TrainDrop hd = make_drop(c, c->t.hidden_dropout, train), ad = make_drop(c, c->t.attention_dropout, train);
+  const int H = d.hidden, I = d.intermediate, NH = d.num_heads, NL = d.num_layers;
+  const int R = B * T;
   float* P = c->P;
-  // ---------------- forward
   RC(launch_train_embed(c->ids, T, P + c->word.off, P + c->pos.off, P + c->type.off, P + c->emb_g.off, P + c->emb_b.off,
                         d.ln_eps, R, H, hd, SITE_EMB, c->h32, NL > 0 ? (void*)c->L[0].x16 : (void*)c->xlast16, c->xhat_e,
                         c->rstd_e, s));
@@ -240,6 +258,65 @@ int enqueue_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
     RC(launch_train_ln_fwd(c->y32, c->h32, P + t.out_g.off, P + t.out_be.off, d.ln_eps, R, H, hd, SITE_FF2 + 8 * l, c->h32,
                            x_next, t.xhat2, t.rstd2, s));
   }
+  return PLLB_OK;
+}
+
+// The encoder backward of one step, from dh32 = gradient of the last layer's output (written by the head's
+// backward) down to the embedding gradients.  The word-embedding gradient is ADDED to G[word] (the MLM head
+// has written the tied decoder's part there; a CLS trainer clears it first).
+int encoder_bwd(pllb_trainer_ctx* c, int B, int T, const TrainDrop& hd, const TrainDrop& ad, cudaStream_t s) {
+  const pllb_model_desc& d = c->d;
+  const int H = d.hidden, I = d.intermediate, NH = d.num_heads, NL = d.num_layers;
+  const int R = B * T;
+  float* P = c->P;
+  float* G = c->G;
+  // dh32 = gradient of the layer output through the layer above; dz32 = the part that arrives over the
+  // residual connection (added inside ln_bwd)
+  bool have_res = false;
+  for (int l = NL - 1; l >= 0; --l) {
+    TLayer& t = c->L[l];
+    const bool dr = hd.thresh != 0;
+    // BertOutput: LN(dropout(FFN2(g)) + h1)
+    RC(launch_train_ln_bwd(c->dh32, have_res ? c->dz32 : nullptr, P + t.out_g.off, t.xhat2, t.rstd2, R, H, hd, -1,
+                           dr ? (int)(SITE_FF2 + 8 * l) : -1, c->dz32, dr ? c->dzd32 : nullptr, s));
+    RC(launch_train_colsum(c->dh32, false, t.xhat2, R, H, G + t.out_be.off, G + t.out_g.off, c->colsum_scratch, s));
+    RC(linear_bwd(c, dr ? c->dzd32 : c->dz32, t.g16, t.ff2T16, R, H, I, t.ff2_w, t.ff2_b, c->y32, s));   // y32 = dg [R, I]
+    RC(launch_train_gelu_bwd(c->y32, t.f, (int64_t)R * I, s));
+    RC(linear_bwd(c, c->y32, t.h1_16, t.ff1T16, R, I, H, t.ff1_w, t.ff1_b, c->dh32, s));                 // dh32 = dh1 via the FFN
+    // BertSelfOutput: LN(dropout(AO(ctx)) + x)
+    RC(launch_train_ln_bwd(c->dh32, c->dz32, P + t.ao_g.off, t.xhat1, t.rstd1, R, H, hd, -1,
+                           dr ? (int)(SITE_AO + 8 * l) : -1, c->dz32, dr ? c->dzd32 : nullptr, s));
+    RC(launch_train_colsum(c->dh32, false, t.xhat1, R, H, G + t.ao_be.off, G + t.ao_g.off, c->colsum_scratch, s));
+    RC(linear_bwd(c, dr ? c->dzd32 : c->dz32, t.ctx, t.aoT16, R, H, H, t.ao_w, t.ao_b, c->dh32, s));     // dh32 = dctx
+    RC(launch_train_attn_bwd(t.qkv, c->dh32, t.lse, c->n_valid, R, T, H, NH, ad, SITE_ATT + 8 * l, c->y32, c->Dq, s));
+    RC(linear_bwd(c, c->y32, t.x16, t.qkvT16, R, 3 * H, H, t.qkv_w, t.qkv_b, c->dh32, s));               // dh32 = dx via QKV
+    have_res = true;
+  }
+  // embeddings (dropout sits AFTER the LayerNorm here)
+  RC(launch_train_ln_bwd(c->dh32, have_res ? c->dz32 : nullptr, P + c->emb_g.off, c->xhat_e, c->rstd_e, R, H, hd,
+                         hd.thresh != 0 ? (int)SITE_EMB : -1, -1, c->dz32, nullptr, s));
+  RC(launch_train_colsum(c->dh32, false, c->xhat_e, R, H, G + c->emb_b.off, G + c->emb_g.off, c->colsum_scratch, s));
+  RC(launch_train_embed_bwd(c->dz32, c->ids, B, T, H, d.max_position, c->t.pad_id, G + c->word.off, G + c->pos.off,
+                            G + c->type.off, c->colsum_scratch, s));
+  return PLLB_OK;
+}
+
+int optimizer_update(pllb_trainer_ctx* c, cudaStream_t s) {
+  RC(launch_train_adamw(c->P, c->G, c->M, c->V, c->n_flat, c->t.lr, c->t.beta1, c->t.beta2, c->t.adam_eps,
+                        c->t.weight_decay, c->params_dev, s));
+  return refresh_all(c, s);
+}
+
+// Every launch of one MLM step (shape-static arguments only; the per-step scalars are read from params_dev).
+// mode 0: loss only (model.eval()); 1: forward + backward + AdamW step; 2: forward + backward, no update
+int enqueue_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
+  const pllb_model_desc& d = c->d;
+  const int H = d.hidden, Vp = c->Vp, V = d.vocab;
+  const int R = B * T, Rp = (int)round_up(R, 64);
+  const bool train = mode != 0;
+  const TrainDrop hd = make_drop(c, c->t.hidden_dropout, train), ad = make_drop(c, c->t.attention_dropout, train);
+  float* P = c->P;
+  RC(encoder_fwd(c, B, T, hd, ad, s));
   // MLM head on EVERY row (labels are the whole sequence, MLM_PLL/preprocess.py:24-28)
   RC(gemm(c->xlast16, c->head16, P + c->head_b.off, c->t_f32, R, H, H, EPI_BIAS_F32, s));
   RC(launch_train_gelu_fwd(c->t_f32, (int64_t)R * H, nullptr, c->y32, s));
@@ -264,39 +341,32 @@ int enqueue_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
     RC(launch_train_colsum(c->dh32, false, c->xhat_h, R, H, G + c->head_be.off, G + c->head_g.off, c->colsum_scratch, s));
     RC(launch_train_gelu_bwd(c->dz32, c->t_f32, (int64_t)R * H, s));
     RC(linear_bwd(c, c->dz32, c->xlast16, c->headT16, R, H, H, c->head_w, c->head_b, c->dh32, s));
-    // ---------------- backward: encoder layers.  dh32 = gradient of the layer output through the
-    // layer above; dz32 = the part that arrives over the residual connection (added inside ln_bwd)
-    bool have_res = false;
-    for (int l = NL - 1; l >= 0; --l) {
-      TLayer& t = c->L[l];
-      const bool dr = hd.thresh != 0;
-      // BertOutput: LN(dropout(FFN2(g)) + h1)
-      RC(launch_train_ln_bwd(c->dh32, have_res ? c->dz32 : nullptr, P + t.out_g.off, t.xhat2, t.rstd2, R, H, hd, -1,
-                             dr ? (int)(SITE_FF2 + 8 * l) : -1, c->dz32, dr ? c->dzd32 : nullptr, s));
-      RC(launch_train_colsum(c->dh32, false, t.xhat2, R, H, G + t.out_be.off, G + t.out_g.off, c->colsum_scratch, s));
-      RC(linear_bwd(c, dr ? c->dzd32 : c->dz32, t.g16, t.ff2T16, R, H, I, t.ff2_w, t.ff2_b, c->y32, s));   // y32 = dg [R, I]
-      RC(launch_train_gelu_bwd(c->y32, t.f, (int64_t)R * I, s));
-      RC(linear_bwd(c, c->y32, t.h1_16, t.ff1T16, R, I, H, t.ff1_w, t.ff1_b, c->dh32, s));                 // dh32 = dh1 via the FFN
-      // BertSelfOutput: LN(dropout(AO(ctx)) + x)
-      RC(launch_train_ln_bwd(c->dh32, c->dz32, P + t.ao_g.off, t.xhat1, t.rstd1, R, H, hd, -1,
-                             dr ? (int)(SITE_AO + 8 * l) : -1, c->dz32, dr ? c->dzd32 : nullptr, s));
-      RC(launch_train_colsum(c->dh32, false, t.xhat1, R, H, G + t.ao_be.off, G + t.ao_g.off, c->colsum_scratch, s));
-      RC(linear_bwd(c, dr ? c->dzd32 : c->dz32, t.ctx, t.aoT16, R, H, H, t.ao_w, t.ao_b, c->dh32, s));     // dh32 = dctx
-      RC(launch_train_attn_bwd(t.qkv, c->dh32, t.lse, c->n_valid, R, T, H, NH, ad, SITE_ATT + 8 * l, c->y32, c->Dq, s));
-      RC(linear_bwd(c, c->y32, t.x16, t.qkvT16, R, 3 * H, H, t.qkv_w, t.qkv_b, c->dh32, s));               // dh32 = dx via QKV
-      have_res = true;
-    }
-    // ---------------- backward: embeddings (dropout sits AFTER the LayerNorm here)
-    RC(launch_train_ln_bwd(c->dh32, have_res ? c->dz32 : nullptr, P + c->emb_g.off, c->xhat_e, c->rstd_e, R, H, hd,
-                           hd.thresh != 0 ? (int)SITE_EMB : -1, -1, c->dz32, nullptr, s));
-    RC(launch_train_colsum(c->dh32, false, c->xhat_e, R, H, G + c->emb_b.off, G + c->emb_g.off, c->colsum_scratch, s));
-    RC(launch_train_embed_bwd(c->dz32, c->ids, B, T, H, d.max_position, c->t.pad_id, G + c->word.off, G + c->pos.off,
-                              G + c->type.off, c->colsum_scratch, s));
-    if (mode == 1) {
-      RC(launch_train_adamw(c->P, c->G, c->M, c->V, c->n_flat, c->t.lr, c->t.beta1, c->t.beta2, c->t.adam_eps,
-                            c->t.weight_decay, c->params_dev, s));
-      RC(refresh_all(c, s));
-    }
+    // ---------------- backward: encoder
+    RC(encoder_bwd(c, B, T, hd, ad, s));
+    if (mode == 1) RC(optimizer_update(c, s));
+  }
+  return PLLB_OK;
+}
+
+// Every launch of one RescoreBert step: the same encoder, the Linear(H, 1) head on the [CLS] rows, the MD / MWER
+// loss over the per-hypothesis scores.  The batch's targets, AM scores, errors and group indices are read from
+// device memory, so the graph of a (B, T, mode) serves every batch of that shape.
+int enqueue_cls_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
+  const int H = c->d.hidden;
+  const bool train = mode != 0;
+  const TrainDrop hd = make_drop(c, c->t.hidden_dropout, train), ad = make_drop(c, c->t.attention_dropout, train);
+  float* P = c->P;
+  float* G = c->G;
+  RC(encoder_fwd(c, B, T, hd, ad, s));
+  RC(launch_train_cls_fwd(c->h32, P + c->lin_w.off, P + c->lin_b.off, B, T, H, c->scores, s));
+  RC(launch_train_cls_loss(c->scores, c->target, c->am, c->err, c->group, B, c->loss.md_weight, c->loss.mwer_weight,
+                           c->loss.am_weight, train ? c->dscore : nullptr, c->loss_dev, s));
+  if (train) {
+    RC(launch_train_cls_bwd(c->h32, P + c->lin_w.off, c->dscore, B, T, H, G + c->lin_w.off, G + c->lin_b.off, c->dh32, s));
+    // no tied decoder: the embedding scatter adds to a cleared word-embedding gradient
+    PLLB_CUDA(cudaMemsetAsync(G + c->word.off, 0, sizeof(float) * (size_t)c->word.n, s));
+    RC(encoder_bwd(c, B, T, hd, ad, s));
+    if (mode == 1) RC(optimizer_update(c, s));
   }
   return PLLB_OK;
 }
@@ -327,7 +397,7 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
     }
     const int64_t before = g_launch_counter;
     PLLB_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int rc = enqueue_step(c, B, T, mode, s);
+    const int rc = c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_step(c, B, T, mode, s);
     cudaGraph_t g = nullptr;
     const cudaError_t e = cudaStreamEndCapture(s, &g);
     if (rc) { if (g) cudaGraphDestroy(g); return rc; }
@@ -343,7 +413,7 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
     c->graph_replays += 1;
   } else {
     const int64_t before = g_launch_counter;
-    RC(enqueue_step(c, B, T, mode, s));
+    RC(c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_step(c, B, T, mode, s));
     c->launches += g_launch_counter - before;
     if (ge) ge->seen += 1;
   }
@@ -354,13 +424,24 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
   return PLLB_OK;
 }
 
-}  // namespace
+// state_dict tensors and the Linear(H, 1) head of a CLS trainer <- flat buffer `buf`
+int cls_export(pllb_trainer c, const float* buf, const pllb_weights* dst, float* linear_w, float* linear_b, const char* who) {
+  if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
+  if (!c->cls) return fail(PLLB_ERR_INVALID, std::string(who) + ": an MLM trainer exports with pllb_train_export*");
+  PLLB_CUDA(cudaSetDevice(c->device));
+  PLLB_CUDA(cudaStreamSynchronize(c->stream));
+  RC(export_encoder(c, buf, dst));
+  RC(copy_out(buf, c->lin_w, linear_w, c->d.hidden));
+  RC(copy_out(buf, c->lin_b, linear_b, 1));
+  PLLB_CUDA(cudaStreamSynchronize(0));
+  return PLLB_OK;
+}
 
-extern "C" {
-
-int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td,
-                      int device) {
-  if (!out || !desc || !w || !w->layers || !td) return fail(PLLB_ERR_INVALID, "pllb_train_create: null argument");
+// lin_w / lin_b / loss given: a RescoreBert (CLS) trainer; otherwise an MLM trainer (the head pointers of w are required)
+int create_impl(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td, int device,
+                const float* lin_w, const float* lin_b, const pllb_cls_loss_desc* loss) {
+  const char* who = loss ? "pllb_cls_train_create" : "pllb_train_create";
+  if (!out || !desc || !w || !w->layers || !td) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
   *out = nullptr;
   if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 (B200) device visible; libpllb200 has no CPU fallback");
   const pllb_model_desc& d = *desc;
@@ -370,7 +451,10 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
                                   "intermediate % 256 == 0");
   if (td->max_rows < 1 || td->max_seq < 1 || td->max_seq > d.max_position || td->max_seq > 512 ||
       td->hidden_dropout < 0.f || td->hidden_dropout >= 1.f || td->attention_dropout < 0.f || td->attention_dropout >= 1.f)
-    return fail(PLLB_ERR_INVALID, "pllb_train_create: need max_rows >= 1, 1 <= max_seq <= min(max_position, 512), dropout in [0, 1)");
+    return fail(PLLB_ERR_INVALID, std::string(who) + ": need max_rows >= 1, 1 <= max_seq <= min(max_position, 512), dropout in [0, 1)");
+  if (loss && (!lin_w || !lin_b || !std::isfinite(loss->md_weight) || !std::isfinite(loss->mwer_weight) ||
+               !std::isfinite(loss->am_weight) || loss->md_weight < 0.f || loss->mwer_weight < 0.f))
+    return fail(PLLB_ERR_INVALID, "pllb_cls_train_create: need linear_w, linear_b and finite loss weights, md / mwer >= 0");
   PLLB_CUDA(cudaSetDevice(device));
   int major = 0;
   PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
@@ -379,6 +463,8 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
   c->d = d;
   c->t = *td;
   c->device = device;
+  c->cls = loss != nullptr;
+  if (loss) c->loss = *loss;
   c->Vp = (int)round_up(d.vocab, 256);
   const int H = d.hidden, I = d.intermediate, V = d.vocab, NL = d.num_layers, NH = d.num_heads, Vp = c->Vp;
   const int64_t HH = (int64_t)H * H;
@@ -390,7 +476,7 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
   } while (0)
   // ---- flat layout
   int64_t cur = 0;
-  c->word = take(cur, (int64_t)Vp * H);       // rows >= vocab stay zero (zero gradient, zero moments)
+  c->word = take(cur, (int64_t)(c->cls ? V : Vp) * H);    // MLM: rows >= vocab stay zero (zero gradient, zero moments)
   c->pos = take(cur, (int64_t)d.max_position * H);
   c->type = take(cur, 2 * H);
   c->emb_g = take(cur, H);
@@ -402,8 +488,12 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
     l.ff1_w = take(cur, (int64_t)I * H); l.ff1_b = take(cur, I);
     l.ff2_w = take(cur, (int64_t)H * I); l.ff2_b = take(cur, H); l.out_g = take(cur, H); l.out_be = take(cur, H);
   }
-  c->head_w = take(cur, HH); c->head_b = take(cur, H); c->head_g = take(cur, H); c->head_be = take(cur, H);
-  c->dec_b = take(cur, Vp);
+  if (c->cls) {
+    c->lin_w = take(cur, H); c->lin_b = take(cur, 1);
+  } else {
+    c->head_w = take(cur, HH); c->head_b = take(cur, H); c->head_g = take(cur, H); c->head_be = take(cur, H);
+    c->dec_b = take(cur, Vp);
+  }
   c->n_flat = cur;
   TRY(talloc(c, &c->P, cur, true));
   TRY(talloc(c, &c->G, cur, true));
@@ -426,9 +516,13 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
     TRY(copy_in(c, t.ff2_w, lw.ff2_w, (int64_t)H * I)); TRY(copy_in(c, t.ff2_b, lw.ff2_b, H));
     TRY(copy_in(c, t.out_g, lw.out_ln_g, H)); TRY(copy_in(c, t.out_be, lw.out_ln_b, H));
   }
-  TRY(copy_in(c, c->head_w, w->head_w, HH)); TRY(copy_in(c, c->head_b, w->head_b, H));
-  TRY(copy_in(c, c->head_g, w->head_ln_g, H)); TRY(copy_in(c, c->head_be, w->head_ln_b, H));
-  TRY(copy_in(c, c->dec_b, w->decoder_b, V));
+  if (c->cls) {
+    TRY(copy_in(c, c->lin_w, lin_w, H)); TRY(copy_in(c, c->lin_b, lin_b, 1));
+  } else {
+    TRY(copy_in(c, c->head_w, w->head_w, HH)); TRY(copy_in(c, c->head_b, w->head_b, H));
+    TRY(copy_in(c, c->head_g, w->head_ln_g, H)); TRY(copy_in(c, c->head_be, w->head_ln_b, H));
+    TRY(copy_in(c, c->dec_b, w->decoder_b, V));
+  }
   // ---- operand copies, stash, scratch
   c->cap_rows = td->max_rows;
   c->cap_rows_pad = round_up(c->cap_rows, 64);
@@ -444,41 +538,58 @@ int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb
     TRY(talloc(c, &l.lse, R * NH)); TRY(talloc(c, &l.xhat1, R * H)); TRY(talloc(c, &l.rstd1, R));
     TRY(talloc(c, &l.f, R * I)); TRY(talloc(c, &l.xhat2, R * H)); TRY(talloc(c, &l.rstd2, R));
   }
-  TRY(talloc(c, &c->head16, HH)); TRY(talloc(c, &c->headT16, HH));
-  TRY(talloc(c, &c->E16, (int64_t)Vp * H)); TRY(talloc(c, &c->ET16, (int64_t)Vp * H));
-  TRY(talloc(c, &c->ids, R)); TRY(talloc(c, &c->labels, R)); TRY(talloc(c, &c->n_valid, R));
-  TRY(talloc(c, &c->xhat_e, R * H)); TRY(talloc(c, &c->rstd_e, R)); TRY(talloc(c, &c->t_f32, R * H));
-  TRY(talloc(c, &c->xhat_h, R * H)); TRY(talloc(c, &c->rstd_h, R));
-  TRY(talloc(c, &c->xlast16, R * H)); TRY(talloc(c, &c->tn16, R * H)); TRY(talloc(c, &c->dlogits16, R * Vp));
-  TRY(talloc(c, &c->logits, R * Vp)); TRY(talloc(c, &c->loss_rows, R)); TRY(talloc(c, &c->loss_dev, 1));
+  // the MLM head's operand copies, stash, [R, Vp] logits and their gradient; a CLS trainer has none of them
+  const int Vw = c->cls ? 0 : Vp;       // widest vocabulary-sized GEMM / column sum
+  if (!c->cls) {
+    TRY(talloc(c, &c->head16, HH)); TRY(talloc(c, &c->headT16, HH));
+    TRY(talloc(c, &c->E16, (int64_t)Vp * H)); TRY(talloc(c, &c->ET16, (int64_t)Vp * H));
+    TRY(talloc(c, &c->labels, R));
+    TRY(talloc(c, &c->t_f32, R * H)); TRY(talloc(c, &c->xhat_h, R * H)); TRY(talloc(c, &c->rstd_h, R));
+    TRY(talloc(c, &c->xlast16, R * H)); TRY(talloc(c, &c->tn16, R * H)); TRY(talloc(c, &c->dlogits16, R * Vp));
+    TRY(talloc(c, &c->logits, R * Vp)); TRY(talloc(c, &c->loss_rows, R));
+  } else {
+    TRY(talloc(c, &c->group, R)); TRY(talloc(c, &c->target, R)); TRY(talloc(c, &c->am, R)); TRY(talloc(c, &c->err, R));
+    TRY(talloc(c, &c->scores, R)); TRY(talloc(c, &c->dscore, R));
+  }
+  TRY(talloc(c, &c->ids, R)); TRY(talloc(c, &c->n_valid, R));
+  TRY(talloc(c, &c->xhat_e, R * H)); TRY(talloc(c, &c->rstd_e, R)); TRY(talloc(c, &c->loss_dev, 1));
   TRY(talloc(c, &c->h32, R * H)); TRY(talloc(c, &c->y32, R * wide)); TRY(talloc(c, &c->dh32, R * H));
   TRY(talloc(c, &c->dz32, R * H)); TRY(talloc(c, &c->dzd32, R * H)); TRY(talloc(c, &c->Dq, R * NH));
-  TRY(talloc(c, &c->zeros, std::max(Vp, wide), true));
-  TRY(talloc(c, &c->colsum_scratch, (int64_t)2 * TRAIN_COLSUM_SPLITS * std::max(Vp, wide)));
-  TRY(talloc(c, &c->d16, R * std::max(wide, H))); TRY(talloc(c, &c->dT16, (int64_t)std::max(wide, Vp) * Rp));
+  TRY(talloc(c, &c->zeros, std::max(Vw, wide), true));
+  TRY(talloc(c, &c->colsum_scratch, (int64_t)2 * TRAIN_COLSUM_SPLITS * std::max(Vw, wide)));
+  TRY(talloc(c, &c->d16, R * std::max(wide, H))); TRY(talloc(c, &c->dT16, (int64_t)std::max(wide, Vw) * Rp));
   TRY(talloc(c, &c->xT16, (int64_t)std::max(I, H) * Rp));
   TRY(talloc(c, &c->params_dev, 1, true));
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
     cudaGetLastError();
     pllb_train_destroy(c);
-    return fail(PLLB_ERR_CUDA, "pllb_train_create: cudaStreamCreate failed");
+    return fail(PLLB_ERR_CUDA, std::string(who) + ": cudaStreamCreate failed");
   }
   if (const char* e = getenv("PLLB_TRAIN_GRAPH")) c->use_graph = atoi(e) != 0;
   if (cudaHostAlloc(&c->params_host, sizeof(TrainStepParams), cudaHostAllocDefault) != cudaSuccess ||
-      cudaHostAlloc(&c->host_stage, sizeof(int32_t) * (size_t)(3 * R), cudaHostAllocDefault) != cudaSuccess) {
+      cudaHostAlloc(&c->host_stage, sizeof(int32_t) * (size_t)((c->cls ? 6 : 3) * R), cudaHostAllocDefault) != cudaSuccess) {
     cudaGetLastError();
     pllb_train_destroy(c);
-    return fail(PLLB_ERR_OOM, "pllb_train_create: pinned staging buffer");
+    return fail(PLLB_ERR_OOM, std::string(who) + ": pinned staging buffer");
   }
   TRY(refresh_all(c, 0));
 #undef TRY
   cudaError_t e = cudaStreamSynchronize(0);
   if (e != cudaSuccess) {
     pllb_train_destroy(c);
-    return fail(PLLB_ERR_CUDA, std::string("pllb_train_create: ") + cudaGetErrorString(e));
+    return fail(PLLB_ERR_CUDA, std::string(who) + ": " + cudaGetErrorString(e));
   }
   *out = c;
   return PLLB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td,
+                      int device) {
+  return create_impl(out, desc, w, td, device, nullptr, nullptr, nullptr);
 }
 
 int pllb_train_destroy(pllb_trainer c) {
@@ -512,6 +623,7 @@ int pllb_train_reset_optimizer(pllb_trainer c, float lr) {
 int pllb_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* labels, int32_t B,
                          int32_t T, int32_t mode, float* out_loss) {
   if (!c) return fail(PLLB_ERR_INVALID, "null trainer");
+  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_step_host: a RescoreBert trainer takes pllb_cls_train_step_host");
   if (!input_ids || !n_valid || !labels || B < 1 || T < 1 || mode < 0 || mode > 2)
     return fail(PLLB_ERR_INVALID, "pllb_train_step_host: bad argument");
   if (T > c->t.max_seq)
@@ -545,6 +657,7 @@ int pllb_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t
 }
 
 int pllb_train_row_losses_host(pllb_trainer c, float* out, int32_t n) {
+  if (c && c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_row_losses_host: a RescoreBert trainer has no per-position losses");
   if (!c || !out || n < 0 || n > c->last_rows) return fail(PLLB_ERR_INVALID, "pllb_train_row_losses_host: bad argument (n exceeds the rows of the last step)");
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaMemcpyAsync(out, c->loss_rows, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
@@ -554,6 +667,7 @@ int pllb_train_row_losses_host(pllb_trainer c, float* out, int32_t n) {
 
 int pllb_train_export(pllb_trainer c, const pllb_weights* dst) {
   if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, "pllb_train_export: null argument");
+  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_export: a RescoreBert trainer exports with pllb_cls_train_export");
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaStreamSynchronize(c->stream));
   return export_flat(c, c->P, dst);
@@ -561,9 +675,75 @@ int pllb_train_export(pllb_trainer c, const pllb_weights* dst) {
 
 int pllb_train_export_grads(pllb_trainer c, const pllb_weights* dst) {
   if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, "pllb_train_export_grads: null argument");
+  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_export_grads: a RescoreBert trainer exports with pllb_cls_train_export_grads");
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaStreamSynchronize(c->stream));
   return export_flat(c, c->G, dst);
+}
+
+int pllb_cls_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const float* linear_w,
+                          const float* linear_b, const pllb_train_desc* td, const pllb_cls_loss_desc* loss, int device) {
+  if (!loss) return fail(PLLB_ERR_INVALID, "pllb_cls_train_create: null loss descriptor");
+  return create_impl(out, desc, w, td, device, linear_w, linear_b, loss);
+}
+
+int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* group,
+                             const float* target, const float* am, const float* err, int32_t B, int32_t T, int32_t mode,
+                             float* out_loss, float* out_scores) {
+  if (!c) return fail(PLLB_ERR_INVALID, "null trainer");
+  if (!c->cls) return fail(PLLB_ERR_INVALID, "pllb_cls_train_step_host: an MLM trainer takes pllb_train_step_host");
+  if (!input_ids || !n_valid || !group || !target || !am || !err || B < 1 || T < 1 || mode < 0 || mode > 2)
+    return fail(PLLB_ERR_INVALID, "pllb_cls_train_step_host: bad argument");
+  if (T > c->t.max_seq)
+    return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
+                                       std::to_string(c->t.max_seq));
+  if ((int64_t)B * T > c->cap_rows)
+    return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
+                                  std::to_string(c->cap_rows));
+  const int R = B * T;
+  for (int i = 0; i < R; ++i)
+    if (input_ids[i] < 0 || input_ids[i] >= c->d.vocab)
+      return fail(PLLB_ERR_INVALID, "token id outside the vocabulary at row " + std::to_string(i));
+  for (int b = 0; b < B; ++b) {
+    if (n_valid[b] < 1 || n_valid[b] > T) return fail(PLLB_ERR_INVALID, "n_valid must be in [1, T]");
+    if (b == 0 ? group[0] != 0 : (group[b] != group[b - 1] && group[b] != group[b - 1] + 1))
+      return fail(PLLB_ERR_INVALID, "group must start at 0 and number the utterances in row order (each entry equal to the "
+                                    "previous one or one more); bad entry at row " + std::to_string(b));
+    if (!std::isfinite(target[b]) || !std::isfinite(am[b]) || !std::isfinite(err[b]))
+      return fail(PLLB_ERR_INVALID, "non-finite target, AM score or error at row " + std::to_string(b));
+  }
+  PLLB_CUDA(cudaSetDevice(c->device));
+  cudaStream_t s = c->stream;
+  PLLB_CUDA(cudaStreamSynchronize(s));       // the pinned staging buffer of the previous call is free
+  int32_t* st = c->host_stage;
+  std::memcpy(st, input_ids, sizeof(int32_t) * R);
+  std::memcpy(st + R, n_valid, sizeof(int32_t) * B);
+  std::memcpy(st + R + B, group, sizeof(int32_t) * B);
+  std::memcpy(st + R + 2 * B, target, sizeof(float) * B);
+  std::memcpy(st + R + 3 * B, am, sizeof(float) * B);
+  std::memcpy(st + R + 4 * B, err, sizeof(float) * B);
+  PLLB_CUDA(cudaMemcpyAsync(c->ids, st, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
+  PLLB_CUDA(cudaMemcpyAsync(c->n_valid, st + R, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
+  PLLB_CUDA(cudaMemcpyAsync(c->group, st + R + B, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
+  PLLB_CUDA(cudaMemcpyAsync(c->target, st + R + 2 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+  PLLB_CUDA(cudaMemcpyAsync(c->am, st + R + 3 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+  PLLB_CUDA(cudaMemcpyAsync(c->err, st + R + 4 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+  float loss = 0.f;
+  RC(step_impl(c, B, T, mode, &loss, s));
+  if (out_scores) {
+    PLLB_CUDA(cudaMemcpyAsync(out_scores, c->scores, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+    PLLB_CUDA(cudaStreamSynchronize(s));
+  }
+  if (out_loss) *out_loss = loss;
+  return PLLB_OK;
+}
+
+int pllb_cls_train_export(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
+  return cls_export(c, c ? c->P : nullptr, dst, linear_w, linear_b, "pllb_cls_train_export");
+}
+
+int pllb_cls_train_export_grads(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
+  return cls_export(c, c ? c->G : nullptr, dst, linear_w, linear_b, "pllb_cls_train_export_grads");
 }
 
 }  // extern "C"

@@ -508,6 +508,105 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
   }
 }
 
+// ---------------------------------------------------------------- RescoreBert head (sequence score of the [CLS] row)
+// s_b = linear_w . h[b*T, :] + linear_b; a warp per hypothesis, lane-strided fp32 sums then a fixed butterfly
+template <int NV>
+__global__ void __launch_bounds__(RW * 32)
+cls_fwd_kernel(const float* __restrict__ h, const float* __restrict__ w, const float* __restrict__ bias, int B, int T,
+               float* __restrict__ scores) {
+  constexpr int H = NV * 32;
+  const int b = blockIdx.x * RW + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const float* x = h + (size_t)b * T * H;
+  float a = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) a += x[lane + 32 * i] * w[lane + 32 * i];
+  a = wsum(a);
+  if (lane == 0) scores[b] = a + bias[0];
+}
+
+// Loss over the B scores, one CTA.  Rows of a group are contiguous and group[] numbers them 0, 1, ...
+// (checked on the host), so G = group[B-1] + 1 and one captured graph serves every grouping of B rows.
+//   MD:   L_MD = (1/B) sum_i (s_i - y_i)^2,                         dL_MD/ds_i = (2/B) (s_i - y_i)
+//   MWER: P = softmax_g(am_weight * a + s),  L_MWER = (1/G) sum_g sum_{i in g} P_i (e_i - mean_g e),
+//         dL_MWER/ds_i = (1/G) P_i (e_i - sum_{j in g} P_j e_j)
+// The thread that owns the first row of a group walks the whole group in row order; the loss sums run
+// in double over a fixed tree.  dscore (fp32, the 1/B and 1/G already applied) is written when non-null.
+__global__ void __launch_bounds__(256)
+cls_loss_kernel(const float* __restrict__ scores, const float* __restrict__ target, const float* __restrict__ am,
+                const float* __restrict__ err, const int32_t* __restrict__ group, int B, float md_weight, float mwer_weight,
+                float am_weight, float* __restrict__ dscore, float* __restrict__ out_loss) {
+  __shared__ double red_md[256], red_mw[256];
+  const int tid = threadIdx.x;
+  const int G = group[B - 1] + 1;
+  const float inv_b = 1.f / (float)B, inv_g = 1.f / (float)G;
+  double md = 0.0, mw = 0.0;
+  for (int i = tid; i < B; i += 256) {
+    const float d = scores[i] - target[i];
+    md += (double)d * (double)d;
+    if (dscore) dscore[i] = md_weight * (2.f * inv_b) * d;
+  }
+  __syncthreads();      // every dscore[i] holds its MD part before the group walks add to it
+  if (mwer_weight != 0.f) {
+    for (int i = tid; i < B; i += 256) {
+      if (i > 0 && group[i] == group[i - 1]) continue;
+      int end = i + 1;
+      while (end < B && group[end] == group[i]) ++end;
+      float m = -INFINITY;
+      for (int j = i; j < end; ++j) m = fmaxf(m, am_weight * am[j] + scores[j]);
+      float z = 0.f, pe = 0.f, es = 0.f;
+      for (int j = i; j < end; ++j) {
+        const float p = __expf(am_weight * am[j] + scores[j] - m);
+        z += p;
+        pe += p * err[j];
+        es += err[j];
+      }
+      const float inv_z = 1.f / z, ebar_p = pe * inv_z, ebar = es / (float)(end - i);
+      float lg = 0.f;
+      for (int j = i; j < end; ++j) {
+        const float p = __expf(am_weight * am[j] + scores[j] - m) * inv_z;
+        lg += p * (err[j] - ebar);
+        if (dscore) dscore[j] += mwer_weight * inv_g * p * (err[j] - ebar_p);
+      }
+      mw += (double)lg;
+    }
+  }
+  red_md[tid] = md;
+  red_mw[tid] = mw;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (tid < o) { red_md[tid] += red_md[tid + o]; red_mw[tid] += red_mw[tid + o]; }
+    __syncthreads();
+  }
+  if (tid == 0) out_loss[0] = (float)((double)md_weight * red_md[0] / (double)B + (double)mwer_weight * red_mw[0] / (double)G);
+}
+
+// Backward of the head.  Block 0: dlinear_w[c] = sum_b dscore_b * h[b*T, c], dlinear_b = sum_b dscore_b (row
+// order).  Blocks >= 1: the top-layer gradient dh [R, H], zero except row b*T = dscore_b * linear_w.
+__global__ void __launch_bounds__(256)
+cls_bwd_kernel(const float* __restrict__ h, const float* __restrict__ w, const float* __restrict__ dscore, int B, int T,
+               int H, float* __restrict__ dw, float* __restrict__ db, float* __restrict__ dh) {
+  if (blockIdx.x == 0) {
+    for (int c = threadIdx.x; c < H; c += blockDim.x) {
+      float a = 0.f;
+      for (int b = 0; b < B; ++b) a += dscore[b] * h[(size_t)b * T * H + c];
+      dw[c] = a;
+    }
+    if (threadIdx.x == 0) {
+      float a = 0.f;
+      for (int b = 0; b < B; ++b) a += dscore[b];
+      db[0] = a;
+    }
+    return;
+  }
+  const int64_t n = (int64_t)B * T * H;
+  for (int64_t e = (blockIdx.x - 1) * (int64_t)blockDim.x + threadIdx.x; e < n; e += (int64_t)(gridDim.x - 1) * blockDim.x) {
+    const int64_t r = e / H;
+    const int c = (int)(e % H);
+    dh[e] = r % T == 0 ? dscore[r / T] * w[c] : 0.f;
+  }
+}
+
 int grid_for(int64_t n, int block) { return (int)std::min<int64_t>(ceil_div(n, block), 148 * 16); }
 
 }  // namespace
@@ -659,6 +758,31 @@ int launch_train_adamw(float* p, const float* g, float* m, float* v, int64_t n, 
   if (n <= 0) return PLLB_OK;
   adamw_kernel<<<grid_for(n, 256), 256, 0, s>>>(p, g, m, v, n, lr, beta1, beta2, eps, wd, scalars);
   PLLB_LAUNCH_CHECK("adamw_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_cls_fwd(const float* h, const float* w, const float* b, int B, int T, int H, float* scores, cudaStream_t s) {
+  if (B <= 0) return PLLB_OK;
+  const int grid = (int)ceil_div(B, RW);
+  DISPATCH_NV(H, cls_fwd_kernel<NV><<<grid, RW * 32, 0, s>>>(h, w, b, B, T, scores));
+  PLLB_LAUNCH_CHECK("cls_fwd_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_cls_loss(const float* scores, const float* target, const float* am, const float* err, const int32_t* group,
+                          int B, float md_weight, float mwer_weight, float am_weight, float* dscore, float* out_loss,
+                          cudaStream_t s) {
+  if (B <= 0) return PLLB_OK;
+  cls_loss_kernel<<<1, 256, 0, s>>>(scores, target, am, err, group, B, md_weight, mwer_weight, am_weight, dscore, out_loss);
+  PLLB_LAUNCH_CHECK("cls_loss_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_cls_bwd(const float* h, const float* w, const float* dscore, int B, int T, int H, float* dw, float* db,
+                         float* dh, cudaStream_t s) {
+  if (B <= 0) return PLLB_OK;
+  cls_bwd_kernel<<<1 + grid_for((int64_t)B * T * H, 256), 256, 0, s>>>(h, w, dscore, B, T, H, dw, db, dh);
+  PLLB_LAUNCH_CHECK("cls_bwd_kernel");
   return PLLB_OK;
 }
 

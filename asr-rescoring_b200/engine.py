@@ -374,6 +374,158 @@ class MlmTrainer:
         return int(self._lib.pllb_train_graph_replays(self._h))
 
 
+def _prefix_lengths(attention_mask, shape) -> np.ndarray:
+    am = np.asarray(attention_mask)
+    if am.shape != shape:
+        raise ValueError("input_ids and attention_mask must be equal [B, T] arrays")
+    nv = np.ascontiguousarray((am != 0).sum(1), np.int32)
+    if ((am != 0) != (np.arange(shape[1])[None, :] < nv[:, None])).any():
+        raise ValueError("attention_mask must be a prefix mask (ones, then the zero padding)")
+    return nv
+
+
+class ClsTrainer:
+    """RescoreBert distillation on the device: the student of RescoreBert/model.py (BertModel, then
+    Linear(H, 1) on the [CLS] state) trained with the MD loss (MSE to the teacher PLL) and, optionally,
+    the MWER loss over each utterance's N-best list (include/pllb.h, pllb_cls_train_*, states the
+    formulas).  Same encoder, optimizer (AdamW, weight decay on every parameter, linear.* included),
+    stateless dropout and CUDA graphs as :class:`MlmTrainer`; only runs with dropout 0 are comparable
+    value by value with an fp32 reference.
+
+    ``state_dict``: ``bert.*`` (a BertModel, with or without ``bert.pooler.*``), ``linear.weight``
+    [1, H], ``linear.bias`` [1].  The pooler is not used by the score and gets no gradient: it comes
+    back from :meth:`state_dict` unchanged."""
+
+    POOLER = "bert.pooler."
+
+    def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: Optional[dict] = None, device: int = 0,
+                 lr: float = 1e-5, md_weight: float = 1.0, mwer_weight: float = 0.0, am_weight: float = 1.0,
+                 hidden_dropout: float = 0.1, attention_dropout: float = 0.1, seed: int = 0, max_rows: int = 4096,
+                 max_seq: int = 128, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01, pad_id: int = 0):
+        import torch
+        from ._lib import ClsLossDesc, TrainDesc
+        from .synth import config_from_state_dict
+
+        if "linear.weight" not in state_dict or "linear.bias" not in state_dict:
+            raise ValueError("RescoreBert training needs linear.weight [1, H] and linear.bias [1] in the state_dict")
+        self._lib = _lib.load()
+        _lib.require_device()
+        self._h = ctypes.c_void_p()
+        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
+        self.device = device
+        self._dev = torch.device("cuda", device)
+        H = self.cfg["hidden"]
+        if state_dict["linear.weight"].numel() != H or state_dict["linear.bias"].numel() != 1:
+            raise ValueError("linear.weight must have `hidden` elements and linear.bias one")
+        self._keys = list(state_dict.keys())
+        self._passthrough = {k: v for k, v in state_dict.items() if k.endswith("position_ids") or k.startswith(self.POOLER)}
+        self._shapes = {k: tuple(v.shape) for k, v in state_dict.items()}
+        nl = self.cfg["num_layers"]
+        self.max_seq = min(int(max_seq), int(self.cfg["max_position"]), 512)
+        to_dev = lambda t: t.detach().to(device=self._dev, dtype=torch.float32).contiguous()   # noqa: E731
+        enc = [k for k in state_dict.keys() if k.startswith("bert.") and not k.startswith(self.POOLER)]
+        w, keep = weights_struct(lambda key: to_dev(state_dict[key]), nl, enc)
+        lw, lb = to_dev(state_dict["linear.weight"]).reshape(-1), to_dev(state_dict["linear.bias"]).reshape(-1)
+        d = ModelDesc(nl, H, self.cfg["num_heads"], self.cfg["intermediate"], self.cfg["vocab"],
+                      self.cfg["max_position"], float(self.cfg.get("ln_eps", 1e-12)), 101, 102, 103, 0)
+        td = TrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(hidden_dropout),
+                       float(attention_dropout), int(seed) & (2 ** 64 - 1), int(pad_id), int(max_rows), self.max_seq)
+        self.loss_weights = dict(md_weight=float(md_weight), mwer_weight=float(mwer_weight), am_weight=float(am_weight))
+        ld = ClsLossDesc(**self.loss_weights)
+        torch.cuda.synchronize(self._dev)
+        check(self._lib.pllb_cls_train_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w),
+                                              ctypes.c_void_p(lw.data_ptr()), ctypes.c_void_p(lb.data_ptr()),
+                                              ctypes.byref(td), ctypes.byref(ld), device))
+        del keep, lw, lb
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self._lib.pllb_train_destroy(self._h)
+            self._h = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def reset_optimizer(self, lr: float):
+        """A fresh AdamW: zero moments, step count 0, learning rate lr."""
+        check(self._lib.pllb_train_reset_optimizer(self._h, float(lr)))
+
+    def step(self, input_ids, attention_mask, group, target, am, err, mode: int = 1):
+        """One batch of whole utterances: input_ids / attention_mask int [B, T] ([CLS] t [SEP], zero-padded,
+        prefix masks); group int [B] (0, 0, ..., 1, 1, ...: the utterance of each row); target (teacher PLL),
+        am (AM score), err (CER) float [B].  mode 1: forward + backward + AdamW step; 0: loss only (eval);
+        2: forward + backward without the update.  Returns (loss, float32 [B] scores of this forward pass)."""
+        ids = np.ascontiguousarray(input_ids, np.int32)
+        if ids.ndim != 2:
+            raise ValueError("input_ids must be a [B, T] array")
+        nv = _prefix_lengths(attention_mask, ids.shape)
+        B = ids.shape[0]
+        grp = np.ascontiguousarray(group, np.int32)
+        vals = [np.ascontiguousarray(x, np.float32) for x in (target, am, err)]
+        if grp.shape != (B,) or any(v.shape != (B,) for v in vals):
+            raise ValueError("group, target, am and err must have one entry per row of input_ids")
+        loss = ctypes.c_float(0.0)
+        scores = np.zeros(B, np.float32)
+        check(self._lib.pllb_cls_train_step_host(self._h, _np_ptr(ids), _np_ptr(nv), _np_ptr(grp), *map(_np_ptr, vals),
+                                                 B, ids.shape[1], int(mode), ctypes.byref(loss), _np_ptr(scores)))
+        return float(loss.value), scores
+
+    def _export(self, fn, grads: bool) -> Dict[str, "torch.Tensor"]:
+        import torch
+        bufs = {}
+
+        def get(key):
+            if key not in bufs:
+                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
+            return bufs[key]
+
+        enc = [k for k in self._keys if k.startswith("bert.") and k not in self._passthrough]
+        w, keep = weights_struct(get, self.cfg["num_layers"], enc)
+        lw, lb = get("linear.weight"), get("linear.bias")
+        torch.cuda.synchronize(self._dev)
+        check(fn(self._h, ctypes.byref(w), ctypes.c_void_p(lw.data_ptr()), ctypes.c_void_p(lb.data_ptr())))
+        torch.cuda.synchronize(self._dev)
+        out = {}
+        for k in self._keys:
+            if k in bufs:
+                out[k] = bufs[k].cpu()
+            elif grads and k.startswith(self.POOLER):
+                out[k] = torch.zeros(self._shapes[k], dtype=torch.float32)      # the pooler gets no gradient
+            else:
+                out[k] = self._passthrough[k]
+        del keep
+        return out
+
+    def state_dict(self) -> Dict[str, "torch.Tensor"]:
+        """fp32 CPU tensors under the keys of the state_dict given at construction; the pooler and
+        position_ids entries are the given tensors.  ``RescoreBert(trainer.state_dict())`` scores with it."""
+        return self._export(self._lib.pllb_cls_train_export, False)
+
+    def grads(self) -> Dict[str, "torch.Tensor"]:
+        """Gradients of the last mode-1 / mode-2 step under the same keys (zeros for the pooler;
+        position_ids passes through)."""
+        return self._export(self._lib.pllb_cls_train_export_grads, True)
+
+    def workspace_bytes(self) -> int:
+        return int(self._lib.pllb_train_workspace_bytes(self._h))
+
+    def kernel_launches(self) -> int:
+        return int(self._lib.pllb_train_kernel_launches(self._h))
+
+    def graph_replays(self) -> int:
+        """Steps that ran as replays of a captured CUDA graph (PLLB_TRAIN_GRAPH=0 disables capture)."""
+        return int(self._lib.pllb_train_graph_replays(self._h))
+
+
 # ---------------------------------------------------------------------- stage 4
 def pack_strings(strings: Sequence[str]):
     """Strings -> (code points int32[sum len], offsets int64[n+1]); len = Python code points."""

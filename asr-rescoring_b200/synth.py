@@ -243,6 +243,22 @@ def random_init_state_dict(cfg: dict, seed: int = 10, perturb: bool = False):
     return sd
 
 
+def random_rescorebert_state_dict(cfg: dict, seed: int = 10, perturb: bool = False):
+    """fp32 CPU state_dict of the reference's RescoreBert module (RescoreBert/model.py:7-11): the
+    ``bert.*`` encoder of random_init_state_dict, a BertModel pooler (``bert.pooler.dense``) and
+    ``linear.weight`` [1, H] / ``linear.bias`` [1], N(0, 0.02) / 0 (perturb: N(0, 0.5))."""
+    import torch
+
+    sd = {k: v for k, v in random_init_state_dict(cfg, seed, perturb).items() if k.startswith("bert.")}
+    g = torch.Generator().manual_seed(seed + 1)
+    H = cfg["hidden"]
+    sd["bert.pooler.dense.weight"] = torch.empty(H, H).normal_(0.0, 0.02, generator=g)
+    sd["bert.pooler.dense.bias"] = torch.zeros(H)
+    sd["linear.weight"] = torch.empty(1, H).normal_(0.0, 0.02, generator=g)
+    sd["linear.bias"] = torch.empty(1).normal_(0.0, 0.5, generator=g) if perturb else torch.zeros(1)
+    return sd
+
+
 def config_from_state_dict(sd) -> dict:
     """Infer the model shape from a BertForMaskedLM state_dict."""
     H = sd["bert.embeddings.word_embeddings.weight"].shape[1]

@@ -293,6 +293,47 @@ int pllb_train_row_losses_host(pllb_trainer t, float* out, int32_t n);
 int pllb_train_export(pllb_trainer t, const pllb_weights* dst);
 int pllb_train_export_grads(pllb_trainer t, const pllb_weights* dst);
 
+/* ---- RescoreBert distillation: the student of RescoreBert/main.py (BertModel, then Linear(H, 1)
+ * on the [CLS] state; the scorer is pllb_score_cls) trained on the teacher's PLLs.  The
+ * reference's training script is not part of the reference tree, so the losses below are this
+ * library's contract, pinned by an autograd restatement (oracle/rescorebert_train_oracle.py), not
+ * by a reference golden.  A batch is B hypotheses of whole utterances, zero-padded to T positions;
+ * the hypotheses of one utterance are contiguous rows and form one group (G groups).
+ *   s_i  = linear_w . h_L[i, 0, :] + linear_b      (fp32 last-layer output at [CLS])
+ *   MD   = (1/B) sum_i (s_i - y_i)^2               (nn.MSELoss(); y = teacher PLL)
+ *   P    = softmax over the group of (am_weight * a + s)   (a = AM score)
+ *   MWER = (1/G) sum_g sum_{i in g} P_i (e_i - mean_g e)   (e = per-hypothesis CER)
+ *   loss = md_weight * MD + mwer_weight * MWER
+ * A group of one hypothesis has P = 1 and contributes 0 to MWER and to its gradient; it still
+ * counts in G.  Encoder, optimizer, dropout and graphs are those of the MLM trainer above; AdamW
+ * (weight decay on every parameter) also updates linear_w and linear_b.  The pooler of BertModel
+ * gets no gradient and is not held here. */
+typedef struct pllb_cls_loss_desc {
+  float md_weight;          /* >= 0 */
+  float mwer_weight;        /* >= 0; 0 = MD alone */
+  float am_weight;          /* scale of the AM score inside the MWER softmax */
+} pllb_cls_loss_desc;
+
+/* weights: DEVICE fp32 encoder tensors (the head pointers are ignored); linear_w DEVICE fp32 [H],
+ * linear_b DEVICE fp32 [1] (copied).  The handle works with pllb_train_destroy, _reset_optimizer,
+ * _workspace_bytes, _kernel_launches and _graph_replays; pllb_train_step_host, _row_losses_host and
+ * _export* reject it (PLLB_ERR_INVALID), as the pllb_cls_train_* calls reject an MLM trainer. */
+int pllb_cls_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* weights,
+                          const float* linear_w, const float* linear_b, const pllb_train_desc* train,
+                          const pllb_cls_loss_desc* loss, int device);
+/* One batch, HOST buffers.  input_ids int32[B*T] ([CLS] t [SEP], zero-padded); n_valid int32[B];
+ * group int32[B]: 0 for the first row, then each entry equal to the previous one or one more;
+ * target / am / err float[B], finite.  mode as in pllb_train_step_host.  out_loss: the batch loss;
+ * out_scores: float[B] per-hypothesis scores of this forward pass (may be NULL).  Synchronises. */
+int pllb_cls_train_step_host(pllb_trainer t, const int32_t* input_ids, const int32_t* n_valid,
+                             const int32_t* group, const float* target, const float* am,
+                             const float* err, int32_t B, int32_t T, int32_t mode, float* out_loss,
+                             float* out_scores);
+/* Encoder tensors into the caller's DEVICE tensors as pllb_train_export* (NULL skips a tensor),
+ * linear_w [H] and linear_b [1] DEVICE. */
+int pllb_cls_train_export(pllb_trainer t, const pllb_weights* dst, float* linear_w, float* linear_b);
+int pllb_cls_train_export_grads(pllb_trainer t, const pllb_weights* dst, float* linear_w, float* linear_b);
+
 #ifdef __cplusplus
 }
 #endif
