@@ -23,6 +23,14 @@ int fail(int code, const std::string& msg) {
   return code;
 }
 
+int check_model_shape(const pllb_model_desc& d) {
+  if (d.hidden % 256 != 0 || d.hidden < 256 || d.hidden > 1024 || d.num_heads * 64 != d.hidden ||
+      d.intermediate % 256 != 0 || d.num_layers < 1 || d.vocab < 1 || d.max_position < 3)
+    return fail(PLLB_ERR_INVALID, "unsupported model shape: need num_layers >= 1, hidden in {256,512,768,1024}, "
+                                  "head dim 64, intermediate % 256 == 0");
+  return PLLB_OK;
+}
+
 int sm_count() {
   static thread_local int cached_dev = -1, cached = 0;
   int dev = 0;
@@ -566,9 +574,8 @@ int pllb_create(pllb_handle* out, const pllb_model_desc* desc, const pllb_weight
   *out = nullptr;
   RC(check_device());
   const pllb_model_desc& d = *desc;
-  if (d.hidden % 256 != 0 || d.hidden < 256 || d.hidden > 1024 || d.num_heads * 64 != d.hidden ||
-      d.intermediate % 256 != 0 || d.num_layers < 1 || d.vocab < 1 || d.max_position < 3 ||
-      d.operand_dtype < 0 || (d.operand_dtype > 3 && (d.operand_dtype < 16 || d.operand_dtype > 16 + d.num_layers)))
+  RC(check_model_shape(d));
+  if (d.operand_dtype < 0 || (d.operand_dtype > 3 && (d.operand_dtype < 16 || d.operand_dtype > 16 + d.num_layers)))
     return fail(PLLB_ERR_INVALID, "unsupported model shape: need num_layers >= 1, hidden in {256,512,768,1024}, "
                                   "head dim 64, intermediate % 256 == 0");
   PLLB_CUDA(cudaSetDevice(device));

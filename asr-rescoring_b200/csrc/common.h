@@ -16,6 +16,9 @@ namespace pllb {
 void set_error(const std::string& msg);
 int fail(int code, const std::string& msg);
 extern thread_local int64_t g_launch_counter;   // kernels launched by this library on this thread
+// PLLB_ERR_INVALID unless the kernels support the model shape (scoring and training).  Hidden: library-internal,
+// so it does not join the exported symbols.
+__attribute__((visibility("hidden"))) int check_model_shape(const pllb_model_desc& d);
 
 #define PLLB_CUDA(expr)                                                                        \
   do {                                                                                         \

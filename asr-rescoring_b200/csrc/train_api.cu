@@ -160,7 +160,7 @@ int linear_bwd(pllb_trainer_ctx* c, const float* dy32, const __nv_bfloat16* x16,
   return PLLB_OK;
 }
 
-int copy_in(pllb_trainer_ctx* c, Span dst, const float* src, int64_t n, int64_t dst_off = 0) {
+int copy_in(pllb_trainer_ctx* c, Span dst, const float* src, int64_t n, int64_t dst_off) {
   if (!src)
     return fail(PLLB_ERR_INVALID, c->cls ? "pllb_cls_train_create: a weight pointer is null"
                                          : "pllb_train_create: a weight pointer is null (the MLM head is required)");
@@ -173,51 +173,37 @@ int copy_out(const float* buf, Span src, const float* dst, int64_t n, int64_t sr
   return PLLB_OK;
 }
 
-// state_dict tensors <- flat buffer `buf` (parameters or gradients): embeddings and encoder layers
-int export_encoder(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
+// Every external tensor of a trainer with its place in the flat buffers, in one fixed order: the embeddings, the
+// layers (q / k / v stacked in qkv_w and qkv_b), then the MLM head or lin_w / lin_b.  fn(span, ext, n, off) moves the
+// n floats of `ext` to or from span offset `off`.  The word embedding is V x H floats: rows >= vocab of the padded
+// MLM span are not part of any tensor.  The tied decoder weight is not visited.
+template <typename Fn>
+int visit_params(const pllb_trainer_ctx* c, const pllb_weights* w, const float* lin_w, const float* lin_b, Fn fn) {
   const int H = c->d.hidden, I = c->d.intermediate, V = c->d.vocab;
   const int64_t HH = (int64_t)H * H;
-  RC(copy_out(buf, c->word, w->word_emb, (int64_t)V * H));
-  RC(copy_out(buf, c->pos, w->pos_emb, (int64_t)c->d.max_position * H));
-  RC(copy_out(buf, c->type, w->type_emb, 2 * H));
-  RC(copy_out(buf, c->emb_g, w->emb_ln_g, H));
-  RC(copy_out(buf, c->emb_b, w->emb_ln_b, H));
+  RC(fn(c->word, w->word_emb, (int64_t)V * H, 0));
+  RC(fn(c->pos, w->pos_emb, (int64_t)c->d.max_position * H, 0));
+  RC(fn(c->type, w->type_emb, 2 * H, 0));
+  RC(fn(c->emb_g, w->emb_ln_g, H, 0));
+  RC(fn(c->emb_b, w->emb_ln_b, H, 0));
   for (int l = 0; l < c->d.num_layers; ++l) {
     const pllb_layer_weights& lw = w->layers[l];
     const TLayer& t = c->L[l];
-    RC(copy_out(buf, t.qkv_w, lw.q_w, HH, 0));
-    RC(copy_out(buf, t.qkv_w, lw.k_w, HH, HH));
-    RC(copy_out(buf, t.qkv_w, lw.v_w, HH, 2 * HH));
-    RC(copy_out(buf, t.qkv_b, lw.q_b, H, 0));
-    RC(copy_out(buf, t.qkv_b, lw.k_b, H, H));
-    RC(copy_out(buf, t.qkv_b, lw.v_b, H, 2 * H));
-    RC(copy_out(buf, t.ao_w, lw.ao_w, HH));
-    RC(copy_out(buf, t.ao_b, lw.ao_b, H));
-    RC(copy_out(buf, t.ao_g, lw.ao_ln_g, H));
-    RC(copy_out(buf, t.ao_be, lw.ao_ln_b, H));
-    RC(copy_out(buf, t.ff1_w, lw.ff1_w, (int64_t)I * H));
-    RC(copy_out(buf, t.ff1_b, lw.ff1_b, I));
-    RC(copy_out(buf, t.ff2_w, lw.ff2_w, (int64_t)H * I));
-    RC(copy_out(buf, t.ff2_b, lw.ff2_b, H));
-    RC(copy_out(buf, t.out_g, lw.out_ln_g, H));
-    RC(copy_out(buf, t.out_be, lw.out_ln_b, H));
+    RC(fn(t.qkv_w, lw.q_w, HH, 0)); RC(fn(t.qkv_w, lw.k_w, HH, HH)); RC(fn(t.qkv_w, lw.v_w, HH, 2 * HH));
+    RC(fn(t.qkv_b, lw.q_b, H, 0)); RC(fn(t.qkv_b, lw.k_b, H, H)); RC(fn(t.qkv_b, lw.v_b, H, 2 * H));
+    RC(fn(t.ao_w, lw.ao_w, HH, 0)); RC(fn(t.ao_b, lw.ao_b, H, 0));
+    RC(fn(t.ao_g, lw.ao_ln_g, H, 0)); RC(fn(t.ao_be, lw.ao_ln_b, H, 0));
+    RC(fn(t.ff1_w, lw.ff1_w, (int64_t)I * H, 0)); RC(fn(t.ff1_b, lw.ff1_b, I, 0));
+    RC(fn(t.ff2_w, lw.ff2_w, (int64_t)H * I, 0)); RC(fn(t.ff2_b, lw.ff2_b, H, 0));
+    RC(fn(t.out_g, lw.out_ln_g, H, 0)); RC(fn(t.out_be, lw.out_ln_b, H, 0));
   }
-  return PLLB_OK;
-}
-
-// ... plus the MLM head
-int export_flat(pllb_trainer_ctx* c, const float* buf, const pllb_weights* w) {
-  const int H = c->d.hidden, V = c->d.vocab;
-  const int64_t HH = (int64_t)H * H;
-  RC(export_encoder(c, buf, w));
-  RC(copy_out(buf, c->head_w, w->head_w, HH));
-  RC(copy_out(buf, c->head_b, w->head_b, H));
-  RC(copy_out(buf, c->head_g, w->head_ln_g, H));
-  RC(copy_out(buf, c->head_be, w->head_ln_b, H));
-  // the decoder weight is the word-embedding matrix (tied): written only when the caller keeps a separate tensor
-  if (w->decoder_w && w->decoder_w != w->word_emb) RC(copy_out(buf, c->word, w->decoder_w, (int64_t)V * H));
-  RC(copy_out(buf, c->dec_b, w->decoder_b, V));
-  PLLB_CUDA(cudaStreamSynchronize(0));
+  if (c->cls) {
+    RC(fn(c->lin_w, lin_w, H, 0)); RC(fn(c->lin_b, lin_b, 1, 0));
+  } else {
+    RC(fn(c->head_w, w->head_w, HH, 0)); RC(fn(c->head_b, w->head_b, H, 0));
+    RC(fn(c->head_g, w->head_ln_g, H, 0)); RC(fn(c->head_be, w->head_ln_b, H, 0));
+    RC(fn(c->dec_b, w->decoder_b, V, 0));
+  }
   return PLLB_OK;
 }
 
@@ -309,7 +295,7 @@ int optimizer_update(pllb_trainer_ctx* c, cudaStream_t s) {
 
 // Every launch of one MLM step (shape-static arguments only; the per-step scalars are read from params_dev).
 // mode 0: loss only (model.eval()); 1: forward + backward + AdamW step; 2: forward + backward, no update
-int enqueue_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
+int enqueue_mlm_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
   const pllb_model_desc& d = c->d;
   const int H = d.hidden, Vp = c->Vp, V = d.vocab;
   const int R = B * T, Rp = (int)round_up(R, 64);
@@ -371,6 +357,10 @@ int enqueue_cls_step(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s
   return PLLB_OK;
 }
 
+int enqueue(pllb_trainer_ctx* c, int B, int T, int mode, cudaStream_t s) {
+  return c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_mlm_step(c, B, T, mode, s);
+}
+
 int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host, cudaStream_t s) {
   // per-step scalars -> device (the previous step ended with a stream synchronise, so the pinned copy is free)
   c->calls += 1;
@@ -397,7 +387,7 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
     }
     const int64_t before = g_launch_counter;
     PLLB_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    const int rc = c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_step(c, B, T, mode, s);
+    const int rc = enqueue(c, B, T, mode, s);
     cudaGraph_t g = nullptr;
     const cudaError_t e = cudaStreamEndCapture(s, &g);
     if (rc) { if (g) cudaGraphDestroy(g); return rc; }
@@ -413,7 +403,7 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
     c->graph_replays += 1;
   } else {
     const int64_t before = g_launch_counter;
-    RC(c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_step(c, B, T, mode, s));
+    RC(enqueue(c, B, T, mode, s));
     c->launches += g_launch_counter - before;
     if (ge) ge->seen += 1;
   }
@@ -424,16 +414,61 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
   return PLLB_OK;
 }
 
-// state_dict tensors and the Linear(H, 1) head of a CLS trainer <- flat buffer `buf`
-int cls_export(pllb_trainer c, const float* buf, const pllb_weights* dst, float* linear_w, float* linear_b, const char* who) {
-  if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
-  if (!c->cls) return fail(PLLB_ERR_INVALID, std::string(who) + ": an MLM trainer exports with pllb_train_export*");
+// `who` takes a RescoreBert trainer (cls) or an MLM trainer; the other kind is PLLB_ERR_INVALID
+int require_kind(const pllb_trainer_ctx* c, bool cls, const char* who) {
+  if (!c) return fail(PLLB_ERR_INVALID, std::string(who) + ": null trainer");
+  if (c->cls == cls) return PLLB_OK;
+  return fail(PLLB_ERR_INVALID,
+              std::string(who) + (c->cls ? ": a RescoreBert trainer takes pllb_cls_train_step_host / _export / _export_grads"
+                                         : ": an MLM trainer takes pllb_train_step_host / _row_losses_host / _export / _export_grads"));
+}
+
+// state_dict tensors (and lin_w / lin_b of a RescoreBert trainer) <- the parameters or the gradients
+int export_params(pllb_trainer c, bool cls, bool grads, const pllb_weights* w, const float* lin_w, const float* lin_b,
+                  const char* who) {
+  if (!c || !w || !w->layers) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
+  RC(require_kind(c, cls, who));
+  const float* buf = grads ? c->G : c->P;
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaStreamSynchronize(c->stream));
-  RC(export_encoder(c, buf, dst));
-  RC(copy_out(buf, c->lin_w, linear_w, c->d.hidden));
-  RC(copy_out(buf, c->lin_b, linear_b, 1));
+  RC(visit_params(c, w, lin_w, lin_b,
+                  [buf](Span s, const float* dst, int64_t n, int64_t off) { return copy_out(buf, s, dst, n, off); }));
+  // the decoder weight is the word-embedding matrix (tied): written only when the caller keeps a separate tensor
+  if (!c->cls && w->decoder_w && w->decoder_w != w->word_emb)
+    RC(copy_out(buf, c->word, w->decoder_w, (int64_t)c->d.vocab * c->d.hidden));
   PLLB_CUDA(cudaStreamSynchronize(0));
+  return PLLB_OK;
+}
+
+// The checks of a batch both step entry points share.  The reference's embedding lookup raises on an id outside the
+// vocabulary.
+int check_batch(const pllb_trainer_ctx* c, const char* who, const int32_t* ids, const int32_t* n_valid, int B, int T,
+                int mode) {
+  if (!ids || !n_valid || B < 1 || T < 1 || mode < 0 || mode > 2) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (T > c->t.max_seq)
+    return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
+                                       std::to_string(c->t.max_seq));
+  if ((int64_t)B * T > c->cap_rows)
+    return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
+                                  std::to_string(c->cap_rows));
+  for (int i = 0; i < B * T; ++i)
+    if (ids[i] < 0 || ids[i] >= c->d.vocab) return fail(PLLB_ERR_INVALID, "token id outside the vocabulary at row " + std::to_string(i));
+  for (int b = 0; b < B; ++b)
+    if (n_valid[b] < 1 || n_valid[b] > T) return fail(PLLB_ERR_INVALID, "n_valid must be in [1, T]");
+  return PLLB_OK;
+}
+
+struct Upload { void* dst; const void* host; size_t bytes; };
+
+// Host arrays -> device on s through the pinned staging buffer (packed back to back, one copy per array).
+int upload(pllb_trainer_ctx* c, cudaStream_t s, std::initializer_list<Upload> arrays) {
+  PLLB_CUDA(cudaStreamSynchronize(s));       // the pinned staging buffer of the previous call is free
+  char* st = reinterpret_cast<char*>(c->host_stage);
+  for (const Upload& a : arrays) {
+    std::memcpy(st, a.host, a.bytes);
+    PLLB_CUDA(cudaMemcpyAsync(a.dst, st, a.bytes, cudaMemcpyHostToDevice, s));
+    st += a.bytes;
+  }
   return PLLB_OK;
 }
 
@@ -445,10 +480,7 @@ int create_impl(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weigh
   *out = nullptr;
   if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 (B200) device visible; libpllb200 has no CPU fallback");
   const pllb_model_desc& d = *desc;
-  if (d.hidden % 256 != 0 || d.hidden < 256 || d.hidden > 1024 || d.num_heads * 64 != d.hidden || d.intermediate % 256 != 0 ||
-      d.num_layers < 1 || d.vocab < 1 || d.max_position < 3)
-    return fail(PLLB_ERR_INVALID, "unsupported model shape: need num_layers >= 1, hidden in {256,512,768,1024}, head dim 64, "
-                                  "intermediate % 256 == 0");
+  RC(check_model_shape(d));
   if (td->max_rows < 1 || td->max_seq < 1 || td->max_seq > d.max_position || td->max_seq > 512 ||
       td->hidden_dropout < 0.f || td->hidden_dropout >= 1.f || td->attention_dropout < 0.f || td->attention_dropout >= 1.f)
     return fail(PLLB_ERR_INVALID, std::string(who) + ": need max_rows >= 1, 1 <= max_seq <= min(max_position, 512), dropout in [0, 1)");
@@ -500,29 +532,8 @@ int create_impl(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weigh
   TRY(talloc(c, &c->M, cur, true));
   TRY(talloc(c, &c->V, cur, true));
   // ---- parameters in
-  TRY(copy_in(c, c->word, w->word_emb, (int64_t)V * H));
-  TRY(copy_in(c, c->pos, w->pos_emb, (int64_t)d.max_position * H));
-  TRY(copy_in(c, c->type, w->type_emb, 2 * H));
-  TRY(copy_in(c, c->emb_g, w->emb_ln_g, H));
-  TRY(copy_in(c, c->emb_b, w->emb_ln_b, H));
-  for (int l = 0; l < NL; ++l) {
-    const pllb_layer_weights& lw = w->layers[l];
-    TLayer& t = c->L[l];
-    TRY(copy_in(c, t.qkv_w, lw.q_w, HH, 0)); TRY(copy_in(c, t.qkv_w, lw.k_w, HH, HH)); TRY(copy_in(c, t.qkv_w, lw.v_w, HH, 2 * HH));
-    TRY(copy_in(c, t.qkv_b, lw.q_b, H, 0)); TRY(copy_in(c, t.qkv_b, lw.k_b, H, H)); TRY(copy_in(c, t.qkv_b, lw.v_b, H, 2 * H));
-    TRY(copy_in(c, t.ao_w, lw.ao_w, HH)); TRY(copy_in(c, t.ao_b, lw.ao_b, H));
-    TRY(copy_in(c, t.ao_g, lw.ao_ln_g, H)); TRY(copy_in(c, t.ao_be, lw.ao_ln_b, H));
-    TRY(copy_in(c, t.ff1_w, lw.ff1_w, (int64_t)I * H)); TRY(copy_in(c, t.ff1_b, lw.ff1_b, I));
-    TRY(copy_in(c, t.ff2_w, lw.ff2_w, (int64_t)H * I)); TRY(copy_in(c, t.ff2_b, lw.ff2_b, H));
-    TRY(copy_in(c, t.out_g, lw.out_ln_g, H)); TRY(copy_in(c, t.out_be, lw.out_ln_b, H));
-  }
-  if (c->cls) {
-    TRY(copy_in(c, c->lin_w, lin_w, H)); TRY(copy_in(c, c->lin_b, lin_b, 1));
-  } else {
-    TRY(copy_in(c, c->head_w, w->head_w, HH)); TRY(copy_in(c, c->head_b, w->head_b, H));
-    TRY(copy_in(c, c->head_g, w->head_ln_g, H)); TRY(copy_in(c, c->head_be, w->head_ln_b, H));
-    TRY(copy_in(c, c->dec_b, w->decoder_b, V));
-  }
+  TRY(visit_params(c, w, lin_w, lin_b,
+                   [c](Span s, const float* src, int64_t n, int64_t off) { return copy_in(c, s, src, n, off); }));
   // ---- operand copies, stash, scratch
   c->cap_rows = td->max_rows;
   c->cap_rows_pad = round_up(c->cap_rows, 64);
@@ -622,43 +633,26 @@ int pllb_train_reset_optimizer(pllb_trainer c, float lr) {
 
 int pllb_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* labels, int32_t B,
                          int32_t T, int32_t mode, float* out_loss) {
-  if (!c) return fail(PLLB_ERR_INVALID, "null trainer");
-  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_step_host: a RescoreBert trainer takes pllb_cls_train_step_host");
-  if (!input_ids || !n_valid || !labels || B < 1 || T < 1 || mode < 0 || mode > 2)
-    return fail(PLLB_ERR_INVALID, "pllb_train_step_host: bad argument");
-  if (T > c->t.max_seq)
-    return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
-                                       std::to_string(c->t.max_seq));
-  if ((int64_t)B * T > c->cap_rows)
-    return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
-                                  std::to_string(c->cap_rows));
+  const char* who = "pllb_train_step_host";
+  RC(require_kind(c, false, who));
+  if (!labels) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
+  RC(check_batch(c, who, input_ids, n_valid, B, T, mode));
   const int R = B * T;
-  for (int i = 0; i < R; ++i) {
-    // the reference's embedding lookup / CrossEntropyLoss raise on an index outside the vocabulary
-    if (input_ids[i] < 0 || input_ids[i] >= c->d.vocab || labels[i] < 0 || labels[i] >= c->d.vocab)
-      return fail(PLLB_ERR_INVALID, "token id or label outside the vocabulary at row " + std::to_string(i));
-  }
-  for (int b = 0; b < B; ++b)
-    if (n_valid[b] < 1 || n_valid[b] > T) return fail(PLLB_ERR_INVALID, "n_valid must be in [1, T]");
+  for (int i = 0; i < R; ++i)      // the reference's CrossEntropyLoss raises on a label outside the vocabulary
+    if (labels[i] < 0 || labels[i] >= c->d.vocab) return fail(PLLB_ERR_INVALID, "label outside the vocabulary at row " + std::to_string(i));
   PLLB_CUDA(cudaSetDevice(c->device));
-  cudaStream_t s = c->stream;
-  PLLB_CUDA(cudaStreamSynchronize(s));       // the pinned staging buffer of the previous call is free
-  std::memcpy(c->host_stage, input_ids, sizeof(int32_t) * R);
-  std::memcpy(c->host_stage + R, labels, sizeof(int32_t) * R);
-  std::memcpy(c->host_stage + 2 * R, n_valid, sizeof(int32_t) * B);
-  PLLB_CUDA(cudaMemcpyAsync(c->ids, c->host_stage, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->labels, c->host_stage + R, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->n_valid, c->host_stage + 2 * R, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
+  RC(upload(c, c->stream, {{c->ids, input_ids, sizeof(int32_t) * R}, {c->labels, labels, sizeof(int32_t) * R},
+                           {c->n_valid, n_valid, sizeof(int32_t) * B}}));
   float loss = 0.f;
-  RC(step_impl(c, B, T, mode, &loss, s));
+  RC(step_impl(c, B, T, mode, &loss, c->stream));
   c->last_rows = R;
   if (out_loss) *out_loss = loss;
   return PLLB_OK;
 }
 
 int pllb_train_row_losses_host(pllb_trainer c, float* out, int32_t n) {
-  if (c && c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_row_losses_host: a RescoreBert trainer has no per-position losses");
-  if (!c || !out || n < 0 || n > c->last_rows) return fail(PLLB_ERR_INVALID, "pllb_train_row_losses_host: bad argument (n exceeds the rows of the last step)");
+  RC(require_kind(c, false, "pllb_train_row_losses_host"));
+  if (!out || n < 0 || n > c->last_rows) return fail(PLLB_ERR_INVALID, "pllb_train_row_losses_host: bad argument (n exceeds the rows of the last step)");
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaMemcpyAsync(out, c->loss_rows, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, c->stream));
   PLLB_CUDA(cudaStreamSynchronize(c->stream));
@@ -666,19 +660,11 @@ int pllb_train_row_losses_host(pllb_trainer c, float* out, int32_t n) {
 }
 
 int pllb_train_export(pllb_trainer c, const pllb_weights* dst) {
-  if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, "pllb_train_export: null argument");
-  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_export: a RescoreBert trainer exports with pllb_cls_train_export");
-  PLLB_CUDA(cudaSetDevice(c->device));
-  PLLB_CUDA(cudaStreamSynchronize(c->stream));
-  return export_flat(c, c->P, dst);
+  return export_params(c, false, false, dst, nullptr, nullptr, "pllb_train_export");
 }
 
 int pllb_train_export_grads(pllb_trainer c, const pllb_weights* dst) {
-  if (!c || !dst || !dst->layers) return fail(PLLB_ERR_INVALID, "pllb_train_export_grads: null argument");
-  if (c->cls) return fail(PLLB_ERR_INVALID, "pllb_train_export_grads: a RescoreBert trainer exports with pllb_cls_train_export_grads");
-  PLLB_CUDA(cudaSetDevice(c->device));
-  PLLB_CUDA(cudaStreamSynchronize(c->stream));
-  return export_flat(c, c->G, dst);
+  return export_params(c, false, true, dst, nullptr, nullptr, "pllb_train_export_grads");
 }
 
 int pllb_cls_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const float* linear_w,
@@ -690,22 +676,11 @@ int pllb_cls_train_create(pllb_trainer* out, const pllb_model_desc* desc, const 
 int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* group,
                              const float* target, const float* am, const float* err, int32_t B, int32_t T, int32_t mode,
                              float* out_loss, float* out_scores) {
-  if (!c) return fail(PLLB_ERR_INVALID, "null trainer");
-  if (!c->cls) return fail(PLLB_ERR_INVALID, "pllb_cls_train_step_host: an MLM trainer takes pllb_train_step_host");
-  if (!input_ids || !n_valid || !group || !target || !am || !err || B < 1 || T < 1 || mode < 0 || mode > 2)
-    return fail(PLLB_ERR_INVALID, "pllb_cls_train_step_host: bad argument");
-  if (T > c->t.max_seq)
-    return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
-                                       std::to_string(c->t.max_seq));
-  if ((int64_t)B * T > c->cap_rows)
-    return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
-                                  std::to_string(c->cap_rows));
-  const int R = B * T;
-  for (int i = 0; i < R; ++i)
-    if (input_ids[i] < 0 || input_ids[i] >= c->d.vocab)
-      return fail(PLLB_ERR_INVALID, "token id outside the vocabulary at row " + std::to_string(i));
+  const char* who = "pllb_cls_train_step_host";
+  RC(require_kind(c, true, who));
+  if (!group || !target || !am || !err) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
+  RC(check_batch(c, who, input_ids, n_valid, B, T, mode));
   for (int b = 0; b < B; ++b) {
-    if (n_valid[b] < 1 || n_valid[b] > T) return fail(PLLB_ERR_INVALID, "n_valid must be in [1, T]");
     if (b == 0 ? group[0] != 0 : (group[b] != group[b - 1] && group[b] != group[b - 1] + 1))
       return fail(PLLB_ERR_INVALID, "group must start at 0 and number the utterances in row order (each entry equal to the "
                                     "previous one or one more); bad entry at row " + std::to_string(b));
@@ -714,20 +689,9 @@ int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int
   }
   PLLB_CUDA(cudaSetDevice(c->device));
   cudaStream_t s = c->stream;
-  PLLB_CUDA(cudaStreamSynchronize(s));       // the pinned staging buffer of the previous call is free
-  int32_t* st = c->host_stage;
-  std::memcpy(st, input_ids, sizeof(int32_t) * R);
-  std::memcpy(st + R, n_valid, sizeof(int32_t) * B);
-  std::memcpy(st + R + B, group, sizeof(int32_t) * B);
-  std::memcpy(st + R + 2 * B, target, sizeof(float) * B);
-  std::memcpy(st + R + 3 * B, am, sizeof(float) * B);
-  std::memcpy(st + R + 4 * B, err, sizeof(float) * B);
-  PLLB_CUDA(cudaMemcpyAsync(c->ids, st, sizeof(int32_t) * R, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->n_valid, st + R, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->group, st + R + B, sizeof(int32_t) * B, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->target, st + R + 2 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->am, st + R + 3 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
-  PLLB_CUDA(cudaMemcpyAsync(c->err, st + R + 4 * B, sizeof(float) * B, cudaMemcpyHostToDevice, s));
+  RC(upload(c, s, {{c->ids, input_ids, sizeof(int32_t) * B * T}, {c->n_valid, n_valid, sizeof(int32_t) * B},
+                   {c->group, group, sizeof(int32_t) * B}, {c->target, target, sizeof(float) * B},
+                   {c->am, am, sizeof(float) * B}, {c->err, err, sizeof(float) * B}}));
   float loss = 0.f;
   RC(step_impl(c, B, T, mode, &loss, s));
   if (out_scores) {
@@ -739,11 +703,11 @@ int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int
 }
 
 int pllb_cls_train_export(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
-  return cls_export(c, c ? c->P : nullptr, dst, linear_w, linear_b, "pllb_cls_train_export");
+  return export_params(c, true, false, dst, linear_w, linear_b, "pllb_cls_train_export");
 }
 
 int pllb_cls_train_export_grads(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
-  return cls_export(c, c ? c->G : nullptr, dst, linear_w, linear_b, "pllb_cls_train_export_grads");
+  return export_params(c, true, true, dst, linear_w, linear_b, "pllb_cls_train_export_grads");
 }
 
 }  // extern "C"

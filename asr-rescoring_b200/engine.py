@@ -11,7 +11,7 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import LayerWeights, ModelDesc, Stats, Weights, check
+from ._lib import ClsLossDesc, LayerWeights, ModelDesc, Stats, TrainDesc, Weights, check
 
 VARIANTS = {"B": 0, "A": 1, "C": 2, 0: 0, 1: 1, 2: 2}
 OPERAND_DTYPES = {"bf16": 0, "fp16": 1, "bf16+fp16head": 2, "bf16+fp16tail": 3}   # pllb_model_desc.operand_dtype
@@ -77,10 +77,40 @@ def weights_struct(get, num_layers: int, keys):
     return w, keep
 
 
-class PllScorer:
+def _model_desc(cfg: dict, operand_dtype: int = 0, cls_id: int = 101, sep_id: int = 102, mask_id: int = 103) -> ModelDesc:
+    return ModelDesc(cfg["num_layers"], cfg["hidden"], cfg["num_heads"], cfg["intermediate"], cfg["vocab"],
+                     cfg["max_position"], float(cfg.get("ln_eps", 1e-12)), cls_id, sep_id, mask_id, operand_dtype)
+
+
+class _Handle:
+    """Owner of one library handle ``self._h``, released by the symbol ``_DESTROY`` names."""
+
+    _DESTROY = ""
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            getattr(self._lib, self._DESTROY)(self._h)
+            self._h = ctypes.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class PllScorer(_Handle):
     """BERT masked-LM pseudo-log-likelihood scorer; stands in for the
     ``BertForMaskedLM`` + ``run_one_epoch(do_scoring=True)`` pair of
     MLM_PLL/main.py:73-114,184-187."""
+
+    _DESTROY = "pllb_destroy"
 
     def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: Optional[dict] = None, device: int = 0,
                  max_chunk_tokens: int = 0, cls_id: int = 101, sep_id: int = 102, mask_id: int = 103,
@@ -98,31 +128,11 @@ class PllScorer:
         w, keep = weights_struct(lambda key: state_dict[key].detach().to(device=dev, dtype=torch.float32).contiguous(),
                                  nl, state_dict.keys())
         self.has_mlm_head = bool(w.head_w)
-        d = ModelDesc(nl, self.cfg["hidden"], self.cfg["num_heads"], self.cfg["intermediate"], self.cfg["vocab"],
-                      self.cfg["max_position"], float(self.cfg.get("ln_eps", 1e-12)), cls_id, sep_id, mask_id,
-                      operand_dtype_code(operand_dtype))
+        d = _model_desc(self.cfg, operand_dtype_code(operand_dtype), cls_id, sep_id, mask_id)
         self.operand_dtype = operand_dtype
         torch.cuda.synchronize(dev)
         check(self._lib.pllb_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w), int(max_chunk_tokens), device))
         del keep   # the library made its own (bf16 / fp32) copies
-
-    # ------------------------------------------------------------------ lifecycle
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self._lib.pllb_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
 
     # ------------------------------------------------------------------ scoring
     @staticmethod
@@ -244,7 +254,102 @@ class PllScorer:
         return d
 
 
-class MlmTrainer:
+def _prefix_lengths(attention_mask, shape) -> np.ndarray:
+    am = np.asarray(attention_mask)
+    if am.shape != shape:
+        raise ValueError("input_ids and attention_mask must be equal [B, T] arrays")
+    nv = np.ascontiguousarray((am != 0).sum(1), np.int32)
+    if ((am != 0) != (np.arange(shape[1])[None, :] < nv[:, None])).any():
+        raise ValueError("attention_mask must be a prefix mask (ones, then the zero padding)")
+    return nv
+
+
+class _Trainer(_Handle):
+    """One pllb_train_* handle (encoder, AdamW, stateless dropout, CUDA graphs) and the state_dict keys it was
+    created from.  A subclass creates the handle and names its encoder keys, head pointers and aliases."""
+
+    _DESTROY = "pllb_train_destroy"
+    _HEAD_KEYS = ()       # keys passed to the export calls as extra device pointers, after pllb_weights
+
+    def __init__(self, state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+                 weight_decay, pad_id):
+        import torch
+        from .synth import config_from_state_dict
+
+        self._lib = _lib.load()
+        _lib.require_device()
+        self._h = ctypes.c_void_p()
+        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
+        self.device = device
+        self._dev = torch.device("cuda", device)
+        self._keys = list(state_dict.keys())
+        self._passthrough = {k: v for k, v in state_dict.items() if self._passes_through(k)}
+        self._shapes = {k: tuple(v.shape) for k, v in state_dict.items()}
+        self.max_seq = min(int(max_seq), int(self.cfg["max_position"]), 512)
+        self._desc = _model_desc(self.cfg)
+        self._train_desc = TrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay),
+                                     float(hidden_dropout), float(attention_dropout), int(seed) & (2 ** 64 - 1), int(pad_id),
+                                     int(max_rows), self.max_seq)
+
+    def _passes_through(self, key: str) -> bool:
+        """Keys the trainer does not hold: export returns the given tensor."""
+        return key.endswith("position_ids")
+
+    def _encoder_keys(self):
+        return self._keys
+
+    def _alias(self, key: str) -> str:
+        return key
+
+    def _to_dev(self, t):
+        import torch
+        return t.detach().to(device=self._dev, dtype=torch.float32).contiguous()
+
+    def _weights_in(self, state_dict):
+        """pllb_weights over device fp32 copies of the encoder tensors, ready for the create call."""
+        import torch
+        w, keep = weights_struct(lambda key: self._to_dev(state_dict[key]), self.cfg["num_layers"], self._encoder_keys())
+        torch.cuda.synchronize(self._dev)
+        return w, keep
+
+    def _export(self, fn) -> Dict[str, "torch.Tensor"]:
+        """fn(handle, pllb_weights, *head pointers) fills one zeroed device tensor per key (aliased keys share one);
+        returns CPU tensors under the keys given at construction."""
+        import torch
+        bufs = {}
+
+        def get(key):
+            key = self._alias(key)
+            if key not in bufs:
+                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
+            return bufs[key]
+
+        w, keep = weights_struct(get, self.cfg["num_layers"], self._encoder_keys())
+        head = [ctypes.c_void_p(get(k).data_ptr()) for k in self._HEAD_KEYS]
+        torch.cuda.synchronize(self._dev)
+        check(fn(self._h, ctypes.byref(w), *head))
+        torch.cuda.synchronize(self._dev)
+        host = {k: v.cpu() for k, v in bufs.items()}
+        del keep
+        return {k: self._passthrough[k] if k in self._passthrough else host[self._alias(k)] for k in self._keys}
+
+    def reset_optimizer(self, lr: float):
+        """A fresh AdamW: zero moments, step count 0, learning rate lr (the reference creates one per epoch,
+        MLM_PLL/main.py:76)."""
+        check(self._lib.pllb_train_reset_optimizer(self._h, float(lr)))
+
+    def workspace_bytes(self) -> int:
+        return int(self._lib.pllb_train_workspace_bytes(self._h))
+
+    def kernel_launches(self) -> int:
+        return int(self._lib.pllb_train_kernel_launches(self._h))
+
+    def graph_replays(self) -> int:
+        """Steps that ran as replays of a captured CUDA graph (PLLB_TRAIN_GRAPH=0 disables capture)."""
+        return int(self._lib.pllb_train_graph_replays(self._h))
+
+
+class MlmTrainer(_Trainer):
     """BERT masked-LM fine-tuning on the device; stands in for ``BertForMaskedLM`` (train mode) +
     ``torch.optim.AdamW`` inside ``run_one_epoch(train_mode=True)`` (MLM_PLL/main.py:73-99) and for
     the loss-only dev pass (train_mode=False, do_scoring=False).  fp32 master weights, bf16 GEMM
@@ -260,65 +365,28 @@ class MlmTrainer:
                  lr: float = 1e-5, hidden_dropout: float = 0.1, attention_dropout: float = 0.1, seed: int = 0,
                  max_rows: int = 4096, max_seq: int = 128, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 0.01, pad_id: int = 0):
-        import torch
-        from ._lib import TrainDesc
-        from .synth import config_from_state_dict
-
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
-        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
-        self.device = device
-        self._dev = torch.device("cuda", device)
+        super().__init__(state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+                         weight_decay, pad_id)
         if "cls.predictions.transform.dense.weight" not in state_dict:
             raise ValueError("MLM fine-tuning needs a BertForMaskedLM state_dict (cls.predictions.* missing)")
-        self._keys = [k for k in state_dict.keys()]
-        self._passthrough = {k: v for k, v in state_dict.items() if k.endswith("position_ids")}
-        self._shapes = {k: tuple(v.shape) for k, v in state_dict.items()}
-        nl = self.cfg["num_layers"]
-        self.max_seq = min(int(max_seq), int(self.cfg["max_position"]), 512)
-        w, keep = weights_struct(lambda key: state_dict[key].detach().to(device=self._dev, dtype=torch.float32).contiguous(),
-                                 nl, state_dict.keys())
-        d = ModelDesc(nl, self.cfg["hidden"], self.cfg["num_heads"], self.cfg["intermediate"], self.cfg["vocab"],
-                      self.cfg["max_position"], float(self.cfg.get("ln_eps", 1e-12)), 101, 102, 103, 0)
-        td = TrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(hidden_dropout),
-                       float(attention_dropout), int(seed) & (2 ** 64 - 1), int(pad_id), int(max_rows), self.max_seq)
-        torch.cuda.synchronize(self._dev)
-        check(self._lib.pllb_train_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w), ctypes.byref(td), device))
+        w, keep = self._weights_in(state_dict)
+        check(self._lib.pllb_train_create(ctypes.byref(self._h), ctypes.byref(self._desc), ctypes.byref(w),
+                                          ctypes.byref(self._train_desc), device))
         del keep
 
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self._lib.pllb_train_destroy(self._h)
-            self._h = ctypes.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def reset_optimizer(self, lr: float):
-        """A fresh AdamW, as the reference creates one per epoch (MLM_PLL/main.py:76)."""
-        check(self._lib.pllb_train_reset_optimizer(self._h, float(lr)))
+    def _alias(self, key: str) -> str:
+        """Tied entries are one tensor, as in model.state_dict()."""
+        src = self.TIED.get(key, key)
+        return src if src in self._shapes else key
 
     def step(self, input_ids, attention_mask, labels, mode: int = 1) -> float:
         """One zero-padded batch (int arrays [B, T], what collate builds).  mode 1: forward + backward
         + AdamW step; 0: loss only (eval); 2: forward + backward without the update.  Returns the loss."""
         ids = np.ascontiguousarray(input_ids, np.int32)
         lab = np.ascontiguousarray(labels, np.int32)
-        am = np.asarray(attention_mask)
-        if ids.ndim != 2 or lab.shape != ids.shape or am.shape != ids.shape:
+        if ids.ndim != 2 or lab.shape != ids.shape:
             raise ValueError("input_ids, attention_mask and labels must be equal [B, T] arrays")
-        nv = np.ascontiguousarray((am != 0).sum(1), np.int32)
-        if ((am != 0) != (np.arange(ids.shape[1])[None, :] < nv[:, None])).any():
-            raise ValueError("attention_mask must be a prefix mask (ones, then the zero padding of collate)")
+        nv = _prefix_lengths(attention_mask, ids.shape)
         loss = ctypes.c_float(0.0)
         check(self._lib.pllb_train_step_host(self._h, _np_ptr(ids), _np_ptr(nv), _np_ptr(lab), ids.shape[0], ids.shape[1],
                                              int(mode), ctypes.byref(loss)))
@@ -330,33 +398,6 @@ class MlmTrainer:
         check(self._lib.pllb_train_row_losses_host(self._h, _np_ptr(out), int(n_rows)))
         return out
 
-    def _export(self, fn) -> Dict[str, "torch.Tensor"]:
-        import torch
-        bufs = {}
-
-        def get(key):
-            key = self.TIED.get(key, key) if self.TIED.get(key, key) in self._shapes else key
-            if key not in bufs:
-                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
-            return bufs[key]
-
-        w, keep = weights_struct(get, self.cfg["num_layers"], self._keys)
-        torch.cuda.synchronize(self._dev)
-        check(fn(self._h, ctypes.byref(w)))
-        torch.cuda.synchronize(self._dev)
-        out = {}
-        for k in self._keys:
-            if k in self._passthrough:
-                out[k] = self._passthrough[k]
-            else:
-                src = self.TIED.get(k, k)
-                out[k] = bufs[src if src in bufs else k].cpu()
-        for k, src in self.TIED.items():       # tied entries share storage, as in model.state_dict()
-            if k in out and src in out:
-                out[k] = out[src]
-        del keep
-        return out
-
     def state_dict(self) -> Dict[str, "torch.Tensor"]:
         """fp32 CPU tensors under the keys of the state_dict given at construction (model.state_dict(),
         MLM_PLL/main.py:155)."""
@@ -366,25 +407,8 @@ class MlmTrainer:
         """Gradients of the last mode-1 / mode-2 step, same keys (parity tests)."""
         return self._export(self._lib.pllb_train_export_grads)
 
-    def kernel_launches(self) -> int:
-        return int(self._lib.pllb_train_kernel_launches(self._h))
 
-    def graph_replays(self) -> int:
-        """Steps that ran as replays of a captured CUDA graph (PLLB_TRAIN_GRAPH=0 disables capture)."""
-        return int(self._lib.pllb_train_graph_replays(self._h))
-
-
-def _prefix_lengths(attention_mask, shape) -> np.ndarray:
-    am = np.asarray(attention_mask)
-    if am.shape != shape:
-        raise ValueError("input_ids and attention_mask must be equal [B, T] arrays")
-    nv = np.ascontiguousarray((am != 0).sum(1), np.int32)
-    if ((am != 0) != (np.arange(shape[1])[None, :] < nv[:, None])).any():
-        raise ValueError("attention_mask must be a prefix mask (ones, then the zero padding)")
-    return nv
-
-
-class ClsTrainer:
+class ClsTrainer(_Trainer):
     """RescoreBert distillation on the device: the student of RescoreBert/model.py (BertModel, then
     Linear(H, 1) on the [CLS] state) trained with the MD loss (MSE to the teacher PLL) and, optionally,
     the MWER loss over each utterance's N-best list (include/pllb.h, pllb_cls_train_*, states the
@@ -397,67 +421,32 @@ class ClsTrainer:
     back from :meth:`state_dict` unchanged."""
 
     POOLER = "bert.pooler."
+    _HEAD_KEYS = ("linear.weight", "linear.bias")
 
     def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: Optional[dict] = None, device: int = 0,
                  lr: float = 1e-5, md_weight: float = 1.0, mwer_weight: float = 0.0, am_weight: float = 1.0,
                  hidden_dropout: float = 0.1, attention_dropout: float = 0.1, seed: int = 0, max_rows: int = 4096,
                  max_seq: int = 128, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01, pad_id: int = 0):
-        import torch
-        from ._lib import ClsLossDesc, TrainDesc
-        from .synth import config_from_state_dict
-
         if "linear.weight" not in state_dict or "linear.bias" not in state_dict:
             raise ValueError("RescoreBert training needs linear.weight [1, H] and linear.bias [1] in the state_dict")
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
-        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
-        self.device = device
-        self._dev = torch.device("cuda", device)
-        H = self.cfg["hidden"]
-        if state_dict["linear.weight"].numel() != H or state_dict["linear.bias"].numel() != 1:
+        super().__init__(state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+                         weight_decay, pad_id)
+        if state_dict["linear.weight"].numel() != self.cfg["hidden"] or state_dict["linear.bias"].numel() != 1:
             raise ValueError("linear.weight must have `hidden` elements and linear.bias one")
-        self._keys = list(state_dict.keys())
-        self._passthrough = {k: v for k, v in state_dict.items() if k.endswith("position_ids") or k.startswith(self.POOLER)}
-        self._shapes = {k: tuple(v.shape) for k, v in state_dict.items()}
-        nl = self.cfg["num_layers"]
-        self.max_seq = min(int(max_seq), int(self.cfg["max_position"]), 512)
-        to_dev = lambda t: t.detach().to(device=self._dev, dtype=torch.float32).contiguous()   # noqa: E731
-        enc = [k for k in state_dict.keys() if k.startswith("bert.") and not k.startswith(self.POOLER)]
-        w, keep = weights_struct(lambda key: to_dev(state_dict[key]), nl, enc)
-        lw, lb = to_dev(state_dict["linear.weight"]).reshape(-1), to_dev(state_dict["linear.bias"]).reshape(-1)
-        d = ModelDesc(nl, H, self.cfg["num_heads"], self.cfg["intermediate"], self.cfg["vocab"],
-                      self.cfg["max_position"], float(self.cfg.get("ln_eps", 1e-12)), 101, 102, 103, 0)
-        td = TrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), float(hidden_dropout),
-                       float(attention_dropout), int(seed) & (2 ** 64 - 1), int(pad_id), int(max_rows), self.max_seq)
+        lw, lb = (self._to_dev(state_dict[k]).reshape(-1) for k in self._HEAD_KEYS)
+        w, keep = self._weights_in(state_dict)
         self.loss_weights = dict(md_weight=float(md_weight), mwer_weight=float(mwer_weight), am_weight=float(am_weight))
         ld = ClsLossDesc(**self.loss_weights)
-        torch.cuda.synchronize(self._dev)
-        check(self._lib.pllb_cls_train_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w),
+        check(self._lib.pllb_cls_train_create(ctypes.byref(self._h), ctypes.byref(self._desc), ctypes.byref(w),
                                               ctypes.c_void_p(lw.data_ptr()), ctypes.c_void_p(lb.data_ptr()),
-                                              ctypes.byref(td), ctypes.byref(ld), device))
+                                              ctypes.byref(self._train_desc), ctypes.byref(ld), device))
         del keep, lw, lb
 
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self._lib.pllb_train_destroy(self._h)
-            self._h = ctypes.c_void_p()
+    def _passes_through(self, key: str) -> bool:
+        return super()._passes_through(key) or key.startswith(self.POOLER)
 
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def __enter__(self):
-        return self
-
-    def __exit__(self, *exc):
-        self.close()
-
-    def reset_optimizer(self, lr: float):
-        """A fresh AdamW: zero moments, step count 0, learning rate lr."""
-        check(self._lib.pllb_train_reset_optimizer(self._h, float(lr)))
+    def _encoder_keys(self):
+        return [k for k in self._keys if k.startswith("bert.") and not k.startswith(self.POOLER)]
 
     def step(self, input_ids, attention_mask, group, target, am, err, mode: int = 1):
         """One batch of whole utterances: input_ids / attention_mask int [B, T] ([CLS] t [SEP], zero-padded,
@@ -479,51 +468,20 @@ class ClsTrainer:
                                                  B, ids.shape[1], int(mode), ctypes.byref(loss), _np_ptr(scores)))
         return float(loss.value), scores
 
-    def _export(self, fn, grads: bool) -> Dict[str, "torch.Tensor"]:
-        import torch
-        bufs = {}
-
-        def get(key):
-            if key not in bufs:
-                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
-            return bufs[key]
-
-        enc = [k for k in self._keys if k.startswith("bert.") and k not in self._passthrough]
-        w, keep = weights_struct(get, self.cfg["num_layers"], enc)
-        lw, lb = get("linear.weight"), get("linear.bias")
-        torch.cuda.synchronize(self._dev)
-        check(fn(self._h, ctypes.byref(w), ctypes.c_void_p(lw.data_ptr()), ctypes.c_void_p(lb.data_ptr())))
-        torch.cuda.synchronize(self._dev)
-        out = {}
-        for k in self._keys:
-            if k in bufs:
-                out[k] = bufs[k].cpu()
-            elif grads and k.startswith(self.POOLER):
-                out[k] = torch.zeros(self._shapes[k], dtype=torch.float32)      # the pooler gets no gradient
-            else:
-                out[k] = self._passthrough[k]
-        del keep
-        return out
-
     def state_dict(self) -> Dict[str, "torch.Tensor"]:
         """fp32 CPU tensors under the keys of the state_dict given at construction; the pooler and
         position_ids entries are the given tensors.  ``RescoreBert(trainer.state_dict())`` scores with it."""
-        return self._export(self._lib.pllb_cls_train_export, False)
+        return self._export(self._lib.pllb_cls_train_export)
 
     def grads(self) -> Dict[str, "torch.Tensor"]:
         """Gradients of the last mode-1 / mode-2 step under the same keys (zeros for the pooler;
         position_ids passes through)."""
-        return self._export(self._lib.pllb_cls_train_export_grads, True)
-
-    def workspace_bytes(self) -> int:
-        return int(self._lib.pllb_train_workspace_bytes(self._h))
-
-    def kernel_launches(self) -> int:
-        return int(self._lib.pllb_train_kernel_launches(self._h))
-
-    def graph_replays(self) -> int:
-        """Steps that ran as replays of a captured CUDA graph (PLLB_TRAIN_GRAPH=0 disables capture)."""
-        return int(self._lib.pllb_train_graph_replays(self._h))
+        import torch
+        g = self._export(self._lib.pllb_cls_train_export_grads)
+        for k in g:
+            if k.startswith(self.POOLER):
+                g[k] = torch.zeros(self._shapes[k], dtype=torch.float32)      # the pooler gets no gradient
+        return g
 
 
 # ---------------------------------------------------------------------- stage 4

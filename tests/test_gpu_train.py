@@ -300,6 +300,57 @@ def test_scoring_through_the_trainer_matches_the_scoring_path(gold_dir):
             assert abs(got_tr[u][h] - exp[u][h]) <= 0.3          # lr 1e-5: the weights move a little between batches
 
 
+@pytest.mark.parametrize("kind", ["mlm", "cls"])
+def test_state_dict_round_trips_through_the_flat_buffers(gold_dir, kind):
+    """Import and export walk the same tensor list: right after construction state_dict() is the given fp32
+    state_dict bit for bit (tied decoder and pass-through entries included), the gradients of a step come back
+    under the same keys, and a null encoder pointer is rejected by the create call."""
+    import ctypes
+    import torch
+    from asr_rescoring_b200 import _lib
+    case, sd, rows, _ = _case(gold_dir, "tiny_perturbed")
+    cfg = case["cfg"]
+    ids, am, lab = _batch(rows[:8])
+    B = ids.shape[0]
+    kw = dict(hidden_dropout=0.0, attention_dropout=0.0, max_rows=ids.size, max_seq=ids.shape[1])
+    if kind == "mlm":
+        tr = engine.MlmTrainer(sd, cfg, **kw)
+        step = lambda: tr.step(ids, am, lab, mode=2)                                  # noqa: E731
+        create = lambda h, w: tr._lib.pllb_train_create(ctypes.byref(h), ctypes.byref(tr._desc), ctypes.byref(w),  # noqa: E731
+                                                        ctypes.byref(tr._train_desc), 0)
+    else:
+        sd = synth.random_rescorebert_state_dict(cfg, 3, perturb=True)
+        tr = engine.ClsTrainer(sd, cfg, mwer_weight=1.0, **kw)
+        grp = (np.arange(B) * 2 // B).astype(np.int32)
+        vals = [np.linspace(-1.0, 1.0, B, dtype=np.float32) * s for s in (30.0, 10.0, 0.2)]
+        step = lambda: tr.step(ids, am, grp, *vals, mode=2)[0]                        # noqa: E731
+        lin = [sd[k].cuda().reshape(-1) for k in ("linear.weight", "linear.bias")]
+        ld = _lib.ClsLossDesc(1.0, 1.0, 1.0)
+        create = lambda h, w: tr._lib.pllb_cls_train_create(  # noqa: E731
+            ctypes.byref(h), ctypes.byref(tr._desc), ctypes.byref(w), ctypes.c_void_p(lin[0].data_ptr()),
+            ctypes.c_void_p(lin[1].data_ptr()), ctypes.byref(tr._train_desc), ctypes.byref(ld), 0)
+    bits = lambda t: t.contiguous().reshape(-1).view(torch.uint8)                     # noqa: E731
+    with tr:
+        got = tr.state_dict()
+        assert list(got) == list(sd)
+        for k, v in sd.items():
+            assert got[k].dtype == v.dtype and got[k].shape == v.shape and torch.equal(bits(got[k]), bits(v)), k
+        if kind == "mlm":
+            assert got["cls.predictions.decoder.weight"] is got["bert.embeddings.word_embeddings.weight"]
+            assert got["cls.predictions.decoder.bias"] is got["cls.predictions.bias"]
+        else:
+            assert all(got[k] is v for k, v in sd.items() if k.startswith("bert.pooler."))
+        assert np.isfinite(step())
+        g = tr.grads()
+        assert list(g) == list(sd) and all(bool(torch.isfinite(v).all()) for v in g.values())
+        w, keep = tr._weights_in(sd)
+        w.layers[cfg["num_layers"] - 1].out_ln_b = None
+        h = ctypes.c_void_p()
+        assert create(h, w) == 1 and not h.value
+        assert b"null" in tr._lib.pllb_last_error()
+        del keep
+
+
 def test_training_argument_errors(gold_dir):
     case, sd, rows, _ = _case(gold_dir, "tiny_lr1e-5")
     ids, am, lab = _batch(rows[:8])
