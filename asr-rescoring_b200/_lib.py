@@ -75,6 +75,8 @@ SIGNATURES = {
                                    c_void_p]),
     "pllb_debug_gemm_simt": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "pllb_debug_hidden": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
+    "pllb_embed": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
+    "pllb_bertscore": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
     "pllb_tokenize_host": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "pllb_levenshtein": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
     "pllb_levenshtein_host": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),

@@ -19,6 +19,7 @@ UNITS = {
     "encoder_kernels.cu": [],
     "train_kernels.cu": [],
     "train_api.cu": [],
+    "bertscore_kernels.cu": [],
     # fp64 combiner must round like numpy: no FMA contraction, IEEE division
     "rescore_kernels.cu": ["-fmad=false", "-prec-div=true", "-prec-sqrt=true"],
 }

@@ -175,6 +175,9 @@ struct pllb_context {
   int64_t meta_cap = 0;
   cudaEvent_t ev_meta = nullptr;    // recorded after the H2D copy of meta_host: the next call waits on it before refilling
   bool meta_pending = false;
+  // pllb_bertscore: inverse row norms of the last call (grown on demand, part of the workspace)
+  float* bs_norm = nullptr;
+  int64_t bs_norm_cap = 0;
   // The workspace (activations, plan, meta_dev) is shared by every call on this handle: each call
   // records ev_done on its stream when it has enqueued everything, and the next call's stream waits
   // on it, so calls issued on different streams are ordered instead of racing on the workspace.
@@ -418,7 +421,9 @@ int meta_upload(pllb_context* c, int64_t count, cudaStream_t s) {
 // Plans chunks on the host (offsets are control metadata), uploads the metadata once and
 // enqueues every chunk on `s` without synchronising.
 // cls != nullptr: sequence-level scoring ([CLS] t [SEP], one pass per hypothesis, Linear(H,1)
-// on the [CLS] state) instead of masked-copy PLL scoring.
+// on the [CLS] state) instead of masked-copy PLL scoring; with cls->out == nullptr and
+// upto_layer >= 0 only the hidden states of that plan are produced (pllb_embed).
+// out_hidden: every chunk's fp32 rows, row-major, at that chunk's first row.
 int score_impl(pllb_context* c, const int32_t* hyp_tokens, const int64_t* off, int32_t n_hyp, double* out_pll,
                float* out_tok_logp, int upto_layer, float* out_hidden, cudaStream_t s, const ClsHead* cls = nullptr) {
   if (!c) return fail(PLLB_ERR_INVALID, "null handle");
@@ -452,7 +457,7 @@ int score_impl(pllb_context* c, const int32_t* hyp_tokens, const int64_t* off, i
     }
     if (cur.n_hyp > 0) chunks.push_back(cur);
   }
-  if (upto_layer >= 0 && chunks.size() > 1) return fail(PLLB_ERR_OOM, "pllb_debug_hidden: input must fit one chunk");
+  if (upto_layer >= 0 && !cls && chunks.size() > 1) return fail(PLLB_ERR_OOM, "pllb_debug_hidden: input must fit one chunk");
   int64_t meta_need = 0;
   for (auto& ch : chunks) {
     ch.meta_off = meta_need;
@@ -479,6 +484,7 @@ int score_impl(pllb_context* c, const int32_t* hyp_tokens, const int64_t* off, i
     if (!c->ev_begin) { PLLB_CUDA(cudaEventCreate(&c->ev_begin)); PLLB_CUDA(cudaEventCreate(&c->ev_end)); }
     PLLB_CUDA(cudaEventRecord(c->ev_begin, s));
   }
+  int64_t row0 = 0;
   for (const auto& ch : chunks) {
     const int32_t* tok_off = c->meta_dev + ch.meta_off;
     const int32_t* copy_base = tok_off + (ch.n_hyp + 1);
@@ -486,8 +492,9 @@ int score_impl(pllb_context* c, const int32_t* hyp_tokens, const int64_t* off, i
     RC(run_chunk(c, hyp_tokens + (ch.tok_begin - off[0]), tok_off, copy_base, row_base, ch.n_hyp, ch.n_copies, ch.n_rows,
                  ch.max_T, out_pll ? out_pll + ch.hyp_begin : nullptr,
                  out_tok_logp ? out_tok_logp + (ch.tok_begin - off[0]) : nullptr, upto_layer, s, cls,
-                 cls ? cls->out + ch.hyp_begin : nullptr));
-    if (out_hidden) RC(launch_t32_to_rowmajor(c->hidden_f32, out_hidden, ch.n_rows, c->d.hidden, s));
+                 cls && cls->out ? cls->out + ch.hyp_begin : nullptr));
+    if (out_hidden) RC(launch_t32_to_rowmajor(c->hidden_f32, out_hidden + row0 * c->d.hidden, ch.n_rows, c->d.hidden, s));
+    row0 += ch.n_rows;
     c->stats.chunks += 1;
     c->stats.hyps_scored += ch.n_hyp;
     c->stats.copies_scored += ch.n_copies;
@@ -691,6 +698,7 @@ int pllb_destroy(pllb_handle h) {
   for (void* p : h->owned) cudaFree(p);
   if (h->meta_dev) cudaFree(h->meta_dev);
   if (h->meta_host) cudaFreeHost(h->meta_host);
+  if (h->bs_norm) cudaFree(h->bs_norm);
   if (h->ev_meta) cudaEventDestroy(h->ev_meta);
   if (h->ev_done) cudaEventDestroy(h->ev_done);
   if (h->io_dev) cudaFree(h->io_dev);
@@ -892,6 +900,87 @@ int pllb_debug_hidden(pllb_handle h, const int32_t* hyp_tokens, const int64_t* h
   const int64_t o0 = n_hyp > 0 ? hyp_offsets[0] : 0;
   return score_impl(h, hyp_tokens ? hyp_tokens + o0 : nullptr, hyp_offsets, n_hyp, nullptr, nullptr, upto_layer,
                     out_hidden, (cudaStream_t)stream);
+}
+
+int pllb_embed(pllb_handle h, const int32_t* hyp_tokens, const int64_t* hyp_offsets, int32_t n_hyp, int32_t num_layers,
+               float* out_hidden, void* stream) {
+  if (!h) return fail(PLLB_ERR_INVALID, "null handle");
+  if (num_layers < 0 || num_layers > h->d.num_layers)
+    return fail(PLLB_ERR_INVALID, "pllb_embed: num_layers must be in [0, " + std::to_string(h->d.num_layers) + "]");
+  if (n_hyp > 0 && (!hyp_offsets || !out_hidden)) return fail(PLLB_ERR_INVALID, "pllb_embed: null argument");
+  const int64_t o0 = n_hyp > 0 ? hyp_offsets[0] : 0;
+  ClsHead plan_only{nullptr, 0.f, nullptr};     // the [CLS] t [SEP] plan, no head
+  return score_impl(h, hyp_tokens ? hyp_tokens + o0 : nullptr, hyp_offsets, n_hyp, nullptr, nullptr, num_layers,
+                    out_hidden, (cudaStream_t)stream, &plan_only);
+}
+
+int pllb_bertscore(pllb_handle h, const float* emb, const int64_t* row_off, int32_t n_seq, const int32_t* cand,
+                   const int32_t* ref, int32_t n_pairs, float* out_recall, void* stream) {
+  if (!h) return fail(PLLB_ERR_INVALID, "null handle");
+  if (n_seq < 0 || n_pairs < 0) return fail(PLLB_ERR_INVALID, "pllb_bertscore: negative count");
+  if (n_pairs == 0) return PLLB_OK;
+  if (!emb || !row_off || !cand || !ref || !out_recall) return fail(PLLB_ERR_INVALID, "pllb_bertscore: null argument");
+  if (reinterpret_cast<uintptr_t>(emb) % 16 != 0) return fail(PLLB_ERR_INVALID, "pllb_bertscore: emb must be 16-byte aligned");
+  if (row_off[0] < 0 || row_off[n_seq] > INT32_MAX) return fail(PLLB_ERR_INVALID, "pllb_bertscore: row offsets out of range");
+  for (int32_t i = 0; i < n_seq; ++i)
+    if (row_off[i + 1] - row_off[i] < 2)
+      return fail(PLLB_ERR_INVALID, "pllb_bertscore: sequence " + std::to_string(i) +
+                                        (row_off[i + 1] < row_off[i] ? " has non-monotone row offsets"
+                                                                     : " has fewer than 2 rows ([CLS] and [SEP])"));
+  // candidate groups: runs of consecutive pairs with the same candidate (one CTA each)
+  int64_t items = 0;
+  int32_t n_groups = 0;
+  for (int32_t p = 0; p < n_pairs; ++p) {
+    if (cand[p] < 0 || cand[p] >= n_seq || ref[p] < 0 || ref[p] >= n_seq)
+      return fail(PLLB_ERR_INVALID, "pllb_bertscore: pair " + std::to_string(p) + " names a sequence outside [0, " +
+                                        std::to_string(n_seq) + ")");
+    items += row_off[ref[p] + 1] - row_off[ref[p]] - 2;
+    if (p == 0 || cand[p] != cand[p - 1]) ++n_groups;
+  }
+  if (items > INT32_MAX) return fail(PLLB_ERR_INVALID, "pllb_bertscore: too many reference rows in one call");
+  cudaStream_t s = (cudaStream_t)stream;
+  PLLB_CUDA(cudaSetDevice(h->device));
+  const int64_t n_rows = row_off[n_seq] - row_off[0];
+  // metadata (int32): row_off[n_seq+1] | pair_ref[n_pairs] | item_off[n_pairs+1] | grp_pair[n_groups+1] | grp_cand[n_groups]
+  const int64_t meta = (int64_t)(n_seq + 1) + n_pairs + (n_pairs + 1) + (n_groups + 1) + n_groups;
+  RC(ensure_meta(h, meta, s));
+  RC(meta_acquire(h));
+  RC(workspace_acquire(h, s));
+  if (n_rows > h->bs_norm_cap) {
+    PLLB_CUDA(cudaStreamSynchronize(s));
+    PLLB_CUDA(cudaDeviceSynchronize());
+    if (h->bs_norm) cudaFree(h->bs_norm);
+    h->bs_norm = nullptr;
+    h->bs_norm_cap = 0;
+    const int64_t cap = n_rows + n_rows / 2 + 1024;
+    PLLB_CUDA(cudaMalloc(&h->bs_norm, sizeof(float) * cap));
+    h->bs_norm_cap = cap;
+  }
+  int32_t* m_row = h->meta_host;
+  int32_t* m_ref = m_row + (n_seq + 1);
+  int32_t* m_item = m_ref + n_pairs;
+  int32_t* m_gp = m_item + (n_pairs + 1);
+  int32_t* m_gc = m_gp + (n_groups + 1);
+  for (int32_t i = 0; i <= n_seq; ++i) m_row[i] = (int32_t)row_off[i];
+  m_item[0] = 0;
+  for (int32_t p = 0, g = 0; p < n_pairs; ++p) {
+    m_ref[p] = ref[p];
+    m_item[p + 1] = m_item[p] + (int32_t)(row_off[ref[p] + 1] - row_off[ref[p]] - 2);
+    if (p == 0 || cand[p] != cand[p - 1]) { m_gp[g] = p; m_gc[g] = cand[p]; ++g; }
+  }
+  m_gp[n_groups] = n_pairs;
+  RC(meta_upload(h, meta, s));
+  const int32_t* d = h->meta_dev;
+  const int32_t* d_row = d;
+  const int32_t* d_ref = d_row + (n_seq + 1);
+  const int32_t* d_item = d_ref + n_pairs;
+  const int32_t* d_gp = d_item + (n_pairs + 1);
+  const int32_t* d_gc = d_gp + (n_groups + 1);
+  const int64_t launches_before = g_launch_counter;
+  RC(launch_bertscore(emb, d_row, d_ref, d_item, d_gp, d_gc, n_groups, h->d.hidden, (int32_t)row_off[0],
+                      (int32_t)row_off[n_seq], h->bs_norm, out_recall, s));
+  h->stats.kernel_launches += g_launch_counter - launches_before;
+  return workspace_release(h, s);
 }
 
 int pllb_levenshtein(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* hyp_cp, const int64_t* hyp_off,

@@ -177,4 +177,12 @@ int launch_tokenize_write(const int32_t* table, int table_size, const int32_t* c
 int launch_levenshtein(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* hyp_cp, const int64_t* hyp_off,
                        const int32_t* pair_ref, int32_t n_pairs, int32_t max_len, int32_t* out, cudaStream_t s);
 
+// ---- BERTScore recall (bertscore_kernels.cu) ------------------------------------------
+// out[p] = R(cand, ref) of every pair; pairs come in candidate groups (grp_pair / grp_cand), the
+// interior reference rows of pair p are items item_off[p] .. item_off[p+1].  Rows of emb are
+// [row_begin, row_end); inv_norm holds row_end - row_begin floats.  One cooperative launch.
+int launch_bertscore(const float* emb, const int32_t* row_off, const int32_t* pair_ref, const int32_t* item_off,
+                     const int32_t* grp_pair, const int32_t* grp_cand, int32_t n_groups, int H, int32_t row_begin,
+                     int32_t row_end, float* inv_norm, float* out, cudaStream_t s);
+
 }  // namespace pllb

@@ -202,6 +202,49 @@ class PllScorer(_Handle):
                 i += 1
         return out
 
+    # ------------------------------------------------------------------ BERTScore (RMBR)
+    def embed(self, tokens_cuda, offsets: np.ndarray, num_layers: int, out=None):
+        """fp32 hidden states after ``num_layers`` encoder layers (0 = embedding LayerNorm) of every
+        hypothesis as [CLS] t [SEP] (pllb_embed).  tokens_cuda: torch int32 CUDA tensor (no specials);
+        offsets: host int64[n+1].  Returns a torch float32 CUDA tensor [sum (L+2), hidden]; sequence i
+        starts at row offsets[i] - offsets[0] + 2 i.  Asynchronous on the current torch stream."""
+        import torch
+        offsets = self._check_packed(None, offsets)
+        n = len(offsets) - 1
+        rows = int(offsets[-1] - offsets[0]) + 2 * n
+        assert tokens_cuda.is_cuda and tokens_cuda.dtype == torch.int32 and tokens_cuda.is_contiguous()
+        if out is None:
+            out = torch.empty(max(rows, 1), self.cfg["hidden"], dtype=torch.float32, device=tokens_cuda.device)
+        elif out.dtype != torch.float32 or not out.is_contiguous() or out.numel() < rows * self.cfg["hidden"]:
+            raise ValueError("out must be a contiguous float32 CUDA tensor of at least [rows, hidden]")
+        stream = torch.cuda.current_stream(tokens_cuda.device).cuda_stream
+        check(self._lib.pllb_embed(self._h, ctypes.c_void_p(tokens_cuda.data_ptr()), _np_ptr(offsets), n, int(num_layers),
+                                   ctypes.c_void_p(out.data_ptr()), ctypes.c_void_p(stream)))
+        return out[:rows]
+
+    def bertscore(self, emb, row_off: np.ndarray, cand: np.ndarray, ref: np.ndarray, out=None):
+        """BERTScore recall R(cand[p], ref[p]) of every pair (pllb_bertscore).  emb: torch float32 CUDA
+        [rows, hidden] (what :meth:`embed` returns); row_off: host int64[n_seq+1] row ranges of the
+        sequences; cand / ref: host int32[n_pairs] sequence indices, best grouped by candidate.
+        Returns a torch float32 CUDA tensor [n_pairs].  Asynchronous on the current torch stream."""
+        import torch
+        row_off = np.ascontiguousarray(row_off, np.int64)
+        cand = np.ascontiguousarray(cand, np.int32)
+        ref = np.ascontiguousarray(ref, np.int32)
+        if row_off.ndim != 1 or len(row_off) < 1 or cand.shape != ref.shape or cand.ndim != 1:
+            raise ValueError("row_off must be int64[n_seq+1], cand and ref equal int32[n_pairs]")
+        if not (emb.is_cuda and emb.dtype == torch.float32 and emb.is_contiguous() and emb.shape[-1] == self.cfg["hidden"]):
+            raise ValueError("emb must be a contiguous float32 CUDA tensor [rows, hidden]")
+        if len(row_off) > 1 and row_off[-1] > emb.shape[0]:
+            raise ValueError("row_off reaches past the rows of emb")
+        if out is None:
+            out = torch.empty(len(cand), dtype=torch.float32, device=emb.device)
+        stream = torch.cuda.current_stream(emb.device).cuda_stream
+        check(self._lib.pllb_bertscore(self._h, ctypes.c_void_p(emb.data_ptr()), _np_ptr(row_off), len(row_off) - 1,
+                                       _np_ptr(cand), _np_ptr(ref), len(cand), ctypes.c_void_p(out.data_ptr()),
+                                       ctypes.c_void_p(stream)))
+        return out
+
     # ------------------------------------------------------------------ parity hooks
     def expand(self, tokens: np.ndarray, offsets: np.ndarray):
         import torch

@@ -185,6 +185,39 @@ int pllb_debug_gemm_simt(const uint16_t* A, const uint16_t* W, const float* bias
 int pllb_debug_hidden(pllb_handle h, const int32_t* hyp_tokens, const int64_t* hyp_offsets,
                       int32_t n_hyp, int32_t upto_layer, float* out_hidden, void* stream);
 
+/* ---- BERTScore minimum-Bayes-risk (RMBR): replaces bert_score.score(cands, refs, lang="zh") inside
+ * RMBR/utility_functions.py:9-23 (BertScoreFunction).  RMBR/ and bert_score are not in the reference
+ * tree, so this is the library's own contract, following bert_score with its default arguments
+ * (idf=False, no baseline rescaling, bert-base-chinese truncated to num_layers encoder layers; its
+ * model table gives 8):
+ *   E(t)    fp32 output of encoder layer num_layers for all L+2 positions of [CLS] t [SEP]
+ *           (bert_score's model(...)[0] after model.encoder.layer = layer[:num_layers]).
+ *   R(c, r) = mean over x in r[1 .. T_r-2] of max over y in c[0 .. T_c-1] of cos(E_r[x], E_c[y])
+ *           The reference's [CLS] / [SEP] carry weight 0; the candidate's take part in the max
+ *           (bert_score's greedy_cos_idf with uniform idf).  R = 0 when either sentence is empty
+ *           (T == 2).  The max runs over real positions only: bert_score multiplies the similarity
+ *           matrix by the padding mask, so where every real cosine of a column is negative its padded
+ *           batch returns 0 instead (DESIGN.md §3.9).
+ *   P(c, r) = R(r, c): precision is the same call with the roles swapped.
+ *
+ * Embedding pass: hyp_tokens / hyp_offsets as in pllb_score.  num_layers in [0, desc.num_layers]
+ * (0 = the embedding LayerNorm output).  out_hidden DEVICE float[sum (L+2), hidden] row-major;
+ * sequence i starts at row (hyp_offsets[i] - hyp_offsets[0]) + 2 i.  A sequence longer than
+ * max_position returns PLLB_ERR_TOO_LONG.  The handle may be created without MLM head weights.
+ * Asynchronous on `stream` under the one-stream rule of pllb_score. */
+int pllb_embed(pllb_handle h, const int32_t* hyp_tokens, const int64_t* hyp_offsets, int32_t n_hyp,
+               int32_t num_layers, float* out_hidden, void* stream);
+/* Pair recall: out_recall[p] = R(sequence cand[p], sequence ref[p]) for sequences whose rows lie in
+ * emb (DEVICE fp32 [rows, hidden], 16-byte aligned): sequence i is rows row_off[i] .. row_off[i+1]-1.
+ * row_off HOST int64[n_seq+1], cand / ref HOST int32[n_pairs] (control metadata, validated here:
+ * an index outside [0, n_seq), non-monotone offsets or a sequence with fewer than 2 rows return
+ * PLLB_ERR_INVALID) are copied through the handle's pinned metadata buffer.  Consecutive pairs with
+ * the same candidate share one CTA, which keeps the candidate's rows on chip: emit pairs grouped by
+ * candidate (mbr_decode does).  fp32 throughout, one launch, bit-deterministic.  Asynchronous on
+ * `stream` under the one-stream rule of pllb_score. */
+int pllb_bertscore(pllb_handle h, const float* emb, const int64_t* row_off, int32_t n_seq, const int32_t* cand,
+                   const int32_t* ref, int32_t n_pairs, float* out_recall, void* stream);
+
 /* ---- Text front end: replaces BertTokenizer.tokenize + convert_tokens_to_ids
  * (MLM_PLL/preprocess.py:10,16-27,34) for hypotheses made of CJK ideographs,
  * punctuation and whitespace, where BERT's BasicTokenizer makes every character
