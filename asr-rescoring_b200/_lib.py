@@ -80,6 +80,10 @@ SIGNATURES = {
     "pllb_tokenize_host": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),
     "pllb_levenshtein": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
     "pllb_levenshtein_host": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
+    "pllb_align": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p,
+                           c_void_p, c_void_p, c_void_p]),
+    "pllb_align_host": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
+                                c_void_p, c_void_p]),
     "pllb_rescore_sweep": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32, c_int32,
                                    c_void_p, c_void_p, c_void_p]),
     "pllb_rescore_sweep_host": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32,

@@ -50,6 +50,58 @@ def hyps_cer(hyps_text: Dict[str, Dict[str, str]], ref_text: Dict[str, str]) -> 
     return out
 
 
+# The symbol an alignment puts opposite an unmatched one ('D' in aligned_ref, 'I' in aligned_hyp).
+# The reference's own gap symbol is not recorded; the empty string cannot be a character of
+# either side, and "".join(aligned_ref) gives back the (stripped) reference.
+GAP = ""
+
+
+def hyp_alignment(hyps_text: Dict[str, Dict[str, str]], ref_text: Dict[str, str]) -> Dict[str, Dict[str, list]]:
+    """espnet_data/preprocess/main.py's hyp_alignment.json for a whole split, one kernel launch:
+    {utt: {hyp_k: [aligned_ref, aligned_hyp, ops]}}, three lists of equal length per hypothesis
+    over the characters of the stripped strings (DESIGN.md §3.10)."""
+    utts = list(hyps_text)
+    refs = [ref_text[u].strip() for u in utts]
+    hyps, pair_ref = [], []
+    for r, u in enumerate(utts):
+        for h in hyps_text[u].values():
+            hyps.append(h.strip())
+            pair_ref.append(r)
+    rc, ro = engine.pack_strings(refs)
+    hc, ho = engine.pack_strings(hyps)
+    pair_ref = np.asarray(pair_ref, np.int32)
+    al = engine.align_packed(rc, ro, hc, ho, pair_ref)
+    n = len(hyps)
+    # the ops of every pair back to back, and the character each of them consumes on either side
+    n_ops = al.n_ops.astype(np.int64)
+    starts = np.zeros(n + 1, np.int64)
+    np.cumsum(n_ops, out=starts[1:])
+    pos = np.arange(int(starts[-1]), dtype=np.int64) - np.repeat(starts[:-1] - al.off[:-1], n_ops)
+    ops = al.ops[pos]
+    take_ref = ops != ord("D")
+    take_hyp = ops != ord("I")
+    na = np.diff(ro)[pair_ref]
+    nb = np.diff(ho)
+    base_ref = np.repeat(np.cumsum(na) - na, n_ops)        # ref characters consumed before each pair
+    base_hyp = np.repeat(np.cumsum(nb) - nb, n_ops)
+    i_ref = np.cumsum(take_ref) - take_ref - base_ref + np.repeat(ro[pair_ref], n_ops)
+    i_hyp = np.cumsum(take_hyp) - take_hyp - base_hyp + np.repeat(ho[:-1], n_ops)
+    ref_chars = np.array(list("".join(refs)) + [GAP], dtype=object)
+    hyp_chars = np.array(list("".join(hyps)) + [GAP], dtype=object)
+    a_ref = ref_chars[np.where(take_ref, i_ref, len(ref_chars) - 1)].tolist()
+    a_hyp = hyp_chars[np.where(take_hyp, i_hyp, len(hyp_chars) - 1)].tolist()
+    letters = list(ops.tobytes().decode("ascii"))
+    out, p = {}, 0
+    bounds = starts.tolist()
+    for u in utts:
+        out[u] = {}
+        for k in hyps_text[u]:
+            s, e = bounds[p], bounds[p + 1]
+            out[u][k] = [a_ref[s:e], a_hyp[s:e], letters[s:e]]
+            p += 1
+    return out
+
+
 class BaseFunction():
     def __init__(self, config) -> None:
         self.config = config

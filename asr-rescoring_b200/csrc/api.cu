@@ -1077,6 +1077,92 @@ int pllb_levenshtein_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t
   return PLLB_OK;
 }
 
+int pllb_align(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* hyp_cp, const int64_t* hyp_off,
+               const int32_t* pair_ref, int32_t n_pairs, int32_t max_len, const int64_t* ops_off, uint8_t* out_ops,
+               int32_t* out_n_ops, int32_t* out_counts, void* stream) {
+  RC(check_device());
+  if (n_pairs <= 0) return PLLB_OK;
+  if (max_len < 0) return fail(PLLB_ERR_INVALID, "pllb_align: negative max_len");
+  if (max_len > 1024) return fail(PLLB_ERR_TOO_LONG, "pllb_align: max_len above 1024 symbols");
+  NvtxRange r("stage4: align");
+  int32_t warps = 0;
+  int64_t slot_words = 0;
+  align_shape(n_pairs, max_len, max_len, &warps, &slot_words);
+  uint8_t* codes = nullptr;
+  if (slot_words > 0) RC(get_scratch(8 * slot_words * warps, &codes));
+  return launch_align(ref_cp, ref_off, hyp_cp, hyp_off, pair_ref, n_pairs, max_len, max_len, ops_off, out_ops,
+                      out_n_ops, out_counts, reinterpret_cast<uint2*>(codes), (cudaStream_t)stream);
+}
+
+int pllb_align_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t n_ref, const int32_t* hyp_cp,
+                    const int64_t* hyp_off, const int32_t* pair_ref, int32_t n_pairs, const int64_t* ops_off,
+                    uint8_t* out_ops, int32_t* out_n_ops, int32_t* out_counts) {
+  RC(check_device());
+  if (n_pairs <= 0) return PLLB_OK;
+  if (n_ref < 0 || !ref_off || !hyp_off || !pair_ref || !ops_off || !out_n_ops || !out_counts)
+    return fail(PLLB_ERR_INVALID, "pllb_align_host: null argument");
+  if (ref_off[0] < 0 || hyp_off[0] < 0 || ops_off[0] < 0) return fail(PLLB_ERR_INVALID, "pllb_align_host: negative offset");
+  for (int32_t i = 0; i < n_ref; ++i)
+    if (ref_off[i + 1] < ref_off[i]) return fail(PLLB_ERR_INVALID, "pllb_align_host: ref_off not ascending");
+  int32_t max_ref = 0, max_hyp = 0;
+  for (int32_t i = 0; i < n_pairs; ++i) {
+    if (pair_ref[i] < 0 || pair_ref[i] >= n_ref) return fail(PLLB_ERR_INVALID, "pllb_align_host: pair_ref out of range");
+    if (hyp_off[i + 1] < hyp_off[i]) return fail(PLLB_ERR_INVALID, "pllb_align_host: hyp_off not ascending");
+    const int64_t na = ref_off[pair_ref[i] + 1] - ref_off[pair_ref[i]], nb = hyp_off[i + 1] - hyp_off[i];
+    if (na > 1024 || nb > 1024) return fail(PLLB_ERR_TOO_LONG, "pllb_align_host: a side longer than 1024 symbols");
+    if (ops_off[i + 1] - ops_off[i] < na + nb) return fail(PLLB_ERR_INVALID, "pllb_align_host: ops_off slot shorter than na + nb");
+    max_ref = std::max<int32_t>(max_ref, (int32_t)na);
+    max_hyp = std::max<int32_t>(max_hyp, (int32_t)nb);
+  }
+  const int64_t n_rc = ref_off[n_ref], n_hc = hyp_off[n_pairs], n_ops = ops_off[n_pairs];
+  if ((n_rc > 0 && !ref_cp) || (n_hc > 0 && !hyp_cp) || (n_ops > 0 && !out_ops))
+    return fail(PLLB_ERR_INVALID, "pllb_align_host: null argument");
+  int32_t warps = 0;
+  int64_t slot_words = 0;
+  align_shape(n_pairs, max_ref, max_hyp, &warps, &slot_words);
+  const int64_t b0 = align_up(4 * std::max<int64_t>(n_rc, 1), 256), b1 = align_up(8 * (int64_t)(n_ref + 1), 256),
+                b2 = align_up(4 * std::max<int64_t>(n_hc, 1), 256), b3 = align_up(8 * (int64_t)(n_pairs + 1), 256),
+                b4 = align_up(4 * (int64_t)n_pairs, 256), b5 = b3, b6 = align_up(std::max<int64_t>(n_ops, 1), 256),
+                b7 = b4, b8 = align_up(16 * (int64_t)n_pairs, 256), b9 = 8 * slot_words * warps;
+  uint8_t* base = nullptr;
+  RC(get_scratch(b0 + b1 + b2 + b3 + b4 + b5 + b6 + b7 + b8 + b9, &base));
+  int32_t* d_rc = (int32_t*)base;
+  int64_t* d_ro = (int64_t*)(base + b0);
+  int32_t* d_hc = (int32_t*)(base + b0 + b1);
+  int64_t* d_ho = (int64_t*)(base + b0 + b1 + b2);
+  int32_t* d_pr = (int32_t*)(base + b0 + b1 + b2 + b3);
+  int64_t* d_oo = (int64_t*)(base + b0 + b1 + b2 + b3 + b4);
+  uint8_t* d_ops = base + b0 + b1 + b2 + b3 + b4 + b5;
+  int32_t* d_n = (int32_t*)(base + b0 + b1 + b2 + b3 + b4 + b5 + b6);
+  int32_t* d_cnt = (int32_t*)(base + b0 + b1 + b2 + b3 + b4 + b5 + b6 + b7);
+  uint2* d_codes = slot_words > 0 ? (uint2*)(base + b0 + b1 + b2 + b3 + b4 + b5 + b6 + b7 + b8) : nullptr;
+  // ops are addressed relative to the first slot, so the device buffer starts at ops_off[0]
+  std::vector<int64_t> rel(n_pairs + 1);
+  for (int32_t i = 0; i <= n_pairs; ++i) rel[i] = ops_off[i] - ops_off[0];
+  const int64_t n_out = rel[n_pairs];
+  cudaStream_t s = 0;
+  int rc = PLLB_OK;
+  cudaError_t e = cudaSuccess;
+  if (n_rc > 0) e = cudaMemcpyAsync(d_rc, ref_cp, 4 * n_rc, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_ro, ref_off, 8 * (int64_t)(n_ref + 1), cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess && n_hc > 0) e = cudaMemcpyAsync(d_hc, hyp_cp, 4 * n_hc, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_ho, hyp_off, 8 * (int64_t)(n_pairs + 1), cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_pr, pair_ref, 4 * (int64_t)n_pairs, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_oo, rel.data(), 8 * (int64_t)(n_pairs + 1), cudaMemcpyHostToDevice, s);
+  // bytes of a slot past na + nb are not written by the kernel: zero them like its own padding
+  if (e == cudaSuccess && n_out > 0) e = cudaMemsetAsync(d_ops, 0, n_out, s);
+  if (e == cudaSuccess)
+    rc = launch_align(d_rc, d_ro, d_hc, d_ho, d_pr, n_pairs, max_ref, max_hyp, d_oo, d_ops, d_n, d_cnt, d_codes, s);
+  if (e == cudaSuccess && rc == PLLB_OK && n_out > 0)
+    e = cudaMemcpyAsync(out_ops + ops_off[0], d_ops, n_out, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess && rc == PLLB_OK) e = cudaMemcpyAsync(out_n_ops, d_n, 4 * (int64_t)n_pairs, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess && rc == PLLB_OK) e = cudaMemcpyAsync(out_counts, d_cnt, 16 * (int64_t)n_pairs, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess && rc == PLLB_OK) e = cudaStreamSynchronize(s);
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(PLLB_ERR_CUDA, std::string("pllb_align_host: ") + cudaGetErrorString(e));
+  return PLLB_OK;
+}
+
 int pllb_rescore_sweep(const double* am, const double* lm, const int64_t* len, const int32_t* dist, int32_t N,
                        int32_t n_best, const double* weights, int32_t W, int32_t variant, int32_t* out_argmax,
                        int64_t* out_edit_sum, void* stream) {

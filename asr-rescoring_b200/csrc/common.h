@@ -176,6 +176,13 @@ int launch_tokenize_write(const int32_t* table, int table_size, const int32_t* c
                           const uint8_t* needs_host, const int64_t* out_off, int32_t* out_ids, cudaStream_t s);
 int launch_levenshtein(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* hyp_cp, const int64_t* hyp_off,
                        const int32_t* pair_ref, int32_t n_pairs, int32_t max_len, int32_t* out, cudaStream_t s);
+// Edit-operation alignment (pllb_align).  align_shape gives the warps of the launch and the
+// uint2 words of each warp's global code slot (0: every pair fits the shared-memory codes);
+// gcodes must then hold warps * slot_words words.
+void align_shape(int32_t n_pairs, int32_t max_ref, int32_t max_hyp, int32_t* warps, int64_t* slot_words);
+int launch_align(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* hyp_cp, const int64_t* hyp_off,
+                 const int32_t* pair_ref, int32_t n_pairs, int32_t max_ref, int32_t max_hyp, const int64_t* ops_off,
+                 uint8_t* out_ops, int32_t* out_n_ops, int32_t* out_counts, uint2* gcodes, cudaStream_t s);
 
 // ---- BERTScore recall (bertscore_kernels.cu) ------------------------------------------
 // out[p] = R(cand, ref) of every pair; pairs come in candidate groups (grp_pair / grp_cand), the

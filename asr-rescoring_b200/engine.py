@@ -612,6 +612,69 @@ def levenshtein(refs: Sequence[str], hyps: Sequence[str], pair_ref: Optional[Seq
     return levenshtein_packed(rc, ro, hc, ho, pair_ref)
 
 
+class Alignment:
+    """Edit operations of n aligned pairs (DESIGN.md §3.10), as pllb_align_host returns them.
+
+    ops: uint8 ASCII 'U'/'S'/'I'/'D'; pair i's ops are ops[off[i] : off[i] + n_ops[i]] (its slot
+    runs to off[i+1] = off[i] + na + nb).  counts: int32 [n, 4] = (U, S, I, D) per pair."""
+
+    LETTERS = "USID"
+
+    def __init__(self, ops: np.ndarray, off: np.ndarray, n_ops: np.ndarray, counts: np.ndarray):
+        self.ops, self.off, self.n_ops, self.counts = ops, off, n_ops, counts
+
+    def __len__(self) -> int:
+        return len(self.n_ops)
+
+    def __getitem__(self, i: int) -> np.ndarray:
+        o = int(self.off[i])
+        return self.ops[o:o + int(self.n_ops[i])]
+
+    def op_string(self, i: int) -> str:
+        return self[i].tobytes().decode("ascii")
+
+
+def align_packed(ref_cp, ref_off, hyp_cp, hyp_off, pair_ref) -> Alignment:
+    """Edit-operation alignment of (ref[pair_ref[i]], hyp i) pairs on the GPU (host arrays in/out).
+    Symbols are opaque int32; one kernel launch for every pair."""
+    lib = _lib.load()
+    _lib.require_device()
+    ref_cp = np.ascontiguousarray(ref_cp, np.int32)
+    hyp_cp = np.ascontiguousarray(hyp_cp, np.int32)
+    ref_off = np.ascontiguousarray(ref_off, np.int64)
+    hyp_off = np.ascontiguousarray(hyp_off, np.int64)
+    pair_ref = np.ascontiguousarray(pair_ref, np.int32)
+    n = len(pair_ref)
+    n_ref = len(ref_off) - 1
+    # slot of pair i: na + nb bytes.  An out-of-range pair_ref gets a 0-length ref here; the
+    # library rejects it before it reads the offsets.
+    ok = (pair_ref >= 0) & (pair_ref < n_ref)
+    na = np.diff(ref_off)[np.where(ok, pair_ref, 0)] if n_ref > 0 else np.zeros(n, np.int64)
+    off = np.zeros(n + 1, np.int64)
+    if n:
+        np.cumsum(np.where(ok, na, 0) + np.diff(hyp_off), out=off[1:])
+    ops = np.zeros(max(int(off[-1]), 1), np.uint8)
+    n_ops = np.zeros(n, np.int32)
+    counts = np.zeros((n, 4), np.int32)
+    check(lib.pllb_align_host(_np_ptr(ref_cp), _np_ptr(ref_off), n_ref, _np_ptr(hyp_cp), _np_ptr(hyp_off),
+                              _np_ptr(pair_ref), n, _np_ptr(off), _np_ptr(ops), _np_ptr(n_ops), _np_ptr(counts)))
+    return Alignment(ops[:int(off[-1])], off, n_ops, counts)
+
+
+def align(refs: Sequence[str], hyps: Sequence[str], pair_ref: Optional[Sequence[int]] = None) -> Alignment:
+    """Character edit-operation alignment; strings are stripped like engine.levenshtein, so
+    S + I + D of a pair equals its levenshtein distance."""
+    refs = [r.strip() for r in refs]
+    hyps = [h.strip() for h in hyps]
+    rc, ro = pack_strings(refs)
+    hc, ho = pack_strings(hyps)
+    if pair_ref is None:
+        if len(refs) != len(hyps):
+            raise ValueError("reference and hypothesis lists differ in length")
+        pair_ref = np.arange(len(hyps), dtype=np.int32)
+    return align_packed(rc, ro, hc, ho, pair_ref)
+
+
 def rescore_sweep(am, lm, lens, dist, weights, variant="B"):
     """For every weight: per-utterance argmax of the interpolated score and the summed edit
     distance of the chosen hypotheses.  Returns (argmax int32 [W,N], edit_sum int64 [W])."""

@@ -249,6 +249,45 @@ int pllb_levenshtein_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t
                           const int32_t* hyp_cp, const int64_t* hyp_off,
                           const int32_t* pair_ref, int32_t n_pairs, int32_t* out_dist);
 
+/* ---- Edit-operation alignment: the Levenshtein DP with backtrace of the reference's
+ * espnet_data/preprocess/align.py (hyp_alignment.json) and the U/S/I/D counts of its
+ * statistic/error_type_count.py.  DESIGN.md §3.10.
+ * Symbols are opaque int32 (the Python side passes code points of the stripped strings, as
+ * for pllb_levenshtein, so S + I + D is that call's distance; token ids work too).  Same
+ * packing as pllb_levenshtein: pair i aligns ref[pair_ref[i]] (i indexes it) with hyp i (j).
+ * D[i][j] is the unit-cost table of pllb_levenshtein.  The backtrace starts at (na, nb) and
+ * at each cell takes the first predecessor in this order that attains D[i][j]:
+ *   1. diagonal: 'U' if the symbols are equal, 'S' otherwise;
+ *   2. up (i-1): 'I', a reference symbol with no hypothesis counterpart;
+ *   3. left (j-1): 'D', a hypothesis symbol with no reference counterpart.
+ * The letters are the reference's and the reverse of jiwer's naming ('I' is what jiwer calls a
+ * deletion, 'D' an insertion).  Pinned by the reference's own docstring examples
+ * (tests/golden/levenshtein_meta.json): the letters, and diagonal before left on a tie.  Up
+ * before left is this project's reading of align.py; no known-answer test pins it.
+ * ops_off int64[n_pairs+1]: pair i owns out_ops[ops_off[i] .. ops_off[i+1]), at least na + nb
+ * bytes.  The kernel writes the ops as ASCII 'U' 'S' 'I' 'D' in forward order (first symbol
+ * first) at the start of the slot and zeroes the slot's remaining bytes up to na + nb;
+ * out_n_ops[i] = number of ops, in [max(na, nb), na + nb]; out_counts int32[n_pairs*4] =
+ * (U, S, I, D) of pair i.  A side longer than 1024 symbols returns PLLB_ERR_TOO_LONG.
+ * Integer only, no atomics, bit-deterministic.
+ * pllb_align: DEVICE arrays, asynchronous on `stream`.  max_len >= every na and nb (a pair
+ * above it gets out_n_ops = -1 and zero counts).  When max_len > 64 the codes go to the calling
+ * thread's device scratch region, which the *_host entry points share: issue those calls from
+ * one thread on one stream, or synchronise between them.
+ * pllb_align_host: HOST arrays; validates pair_ref, the offsets (non-negative, ascending, slots
+ * of at least na + nb) with PLLB_ERR_INVALID and the lengths with PLLB_ERR_TOO_LONG, copies
+ * through the scratch region and returns when the results are in host memory.  Bytes of a slot
+ * past na + nb are zeroed too. */
+int pllb_align(const int32_t* ref_cp, const int64_t* ref_off,
+               const int32_t* hyp_cp, const int64_t* hyp_off,
+               const int32_t* pair_ref, int32_t n_pairs, int32_t max_len,
+               const int64_t* ops_off, uint8_t* out_ops, int32_t* out_n_ops,
+               int32_t* out_counts, void* stream);
+int pllb_align_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t n_ref,
+                    const int32_t* hyp_cp, const int64_t* hyp_off,
+                    const int32_t* pair_ref, int32_t n_pairs, const int64_t* ops_off,
+                    uint8_t* out_ops, int32_t* out_n_ops, int32_t* out_counts);
+
 /* ---- Combiner: replaces rescore.py:47-58 (rescore + get_highest_score_hyp)
  * and the per-weight CER numerator of rescore.py:37-43 (find_best_weight).
  * variant 0: (1-w)*am/len + w*lm/len   (rescore.py:51, current source)
