@@ -53,6 +53,40 @@ class ClsLossDesc(ctypes.Structure):
     _fields_ = [("md_weight", c_float), ("mwer_weight", c_float), ("am_weight", c_float)]
 
 
+class S2sDesc(ctypes.Structure):
+    _fields_ = [("enc_layers", c_int32), ("dec_layers", c_int32), ("hidden", c_int32), ("num_heads", c_int32),
+                ("enc_intermediate", c_int32), ("dec_intermediate", c_int32), ("vocab", c_int32),
+                ("enc_max_position", c_int32), ("dec_max_position", c_int32), ("ln_eps", c_float),
+                ("embed_scale", c_float), ("cls_id", c_int32), ("sep_id", c_int32), ("operand_dtype", c_int32)]
+
+
+DEC_LAYER_FIELDS = ["q_w", "q_b", "k_w", "k_b", "v_w", "v_b", "o_w", "o_b", "self_ln_g", "self_ln_b",
+                    "cq_w", "cq_b", "ck_w", "ck_b", "cv_w", "cv_b", "co_w", "co_b", "cross_ln_g", "cross_ln_b",
+                    "ff1_w", "ff1_b", "ff2_w", "ff2_b", "final_ln_g", "final_ln_b"]
+
+
+class DecLayerWeights(ctypes.Structure):
+    _fields_ = [(n, c_void_p) for n in DEC_LAYER_FIELDS]
+
+
+class S2sWeights(ctypes.Structure):
+    _fields_ = [("enc", Weights), ("dec_layers", POINTER(DecLayerWeights)), ("shared", c_void_p),
+                ("dec_pos_emb", c_void_p), ("dec_emb_ln_g", c_void_p), ("dec_emb_ln_b", c_void_p),
+                ("final_logits_bias", c_void_p)]
+
+
+class GenDesc(ctypes.Structure):
+    _fields_ = [("max_length", c_int32), ("decoder_start_id", c_int32), ("eos_id", c_int32), ("pad_id", c_int32),
+                ("forced_bos_id", c_int32), ("forced_eos_id", c_int32), ("num_beams", c_int32), ("do_sample", c_int32),
+                ("no_repeat_ngram_size", c_int32), ("min_length", c_int32), ("repetition_penalty", c_float)]
+
+
+class S2sStats(ctypes.Structure):
+    _fields_ = [("kernel_launches", c_int64), ("steps", c_int64), ("chunks", c_int64), ("sentences", c_int64),
+                ("gemm_flops", c_double), ("enc_ms", c_float), ("cross_kv_ms", c_float), ("dec_layers_ms", c_float),
+                ("head_ms", c_float), ("total_ms", c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/pllb.h declares
 SIGNATURES = {
     "pllb_last_error": (c_char_p, []),
@@ -105,6 +139,16 @@ SIGNATURES = {
                                          c_int32, c_int32, POINTER(c_float), c_void_p]),
     "pllb_cls_train_export": (c_int, [c_void_p, POINTER(Weights), c_void_p, c_void_p]),
     "pllb_cls_train_export_grads": (c_int, [c_void_p, POINTER(Weights), c_void_p, c_void_p]),
+    "pllb_s2s_create": (c_int, [POINTER(c_void_p), POINTER(S2sDesc), POINTER(S2sWeights), c_int32, c_int]),
+    "pllb_s2s_destroy": (c_int, [c_void_p]),
+    "pllb_s2s_workspace_bytes": (c_int64, [c_void_p]),
+    "pllb_s2s_set_timing": (c_int, [c_void_p, c_int]),
+    "pllb_s2s_get_stats": (c_int, [c_void_p, POINTER(S2sStats)]),
+    "pllb_s2s_reset_stats": (c_int, [c_void_p]),
+    "pllb_generate": (c_int, [c_void_p, POINTER(GenDesc), c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p,
+                              c_void_p]),
+    "pllb_generate_host": (c_int, [c_void_p, POINTER(GenDesc), c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
+                                   c_void_p]),
 }
 
 _lib = None

@@ -20,6 +20,8 @@ UNITS = {
     "train_kernels.cu": [],
     "train_api.cu": [],
     "bertscore_kernels.cu": [],
+    "seq2seq_kernels.cu": [],
+    "seq2seq_api.cu": [],
     # fp64 combiner must round like numpy: no FMA contraction, IEEE division
     "rescore_kernels.cu": ["-fmad=false", "-prec-div=true", "-prec-sqrt=true"],
 }

@@ -67,7 +67,9 @@ enum GemmEpilogue : int {
   EPI_BIAS_GELU_BF16 = 1,  // out 16-bit = gelu_erf(acc + bias)
   EPI_BIAS_F32 = 2,        // out fp32 = acc + bias
   EPI_BIAS_GELU_F32 = 3,   // out fp32 = gelu_erf(acc + bias)
-  EPI_LSE = 4              // vocab-tiled online logsumexp + label-column pick (no C output)
+  EPI_LSE = 4,             // vocab-tiled online logsumexp + label-column pick (no C output)
+  EPI_ARGMAX = 5           // vocab-tiled (max, first argmax) + label-column pick (no C output); LseArgs.partials
+                           // hold (max, __int_as_float(column)) per 128-column half tile
 };
 
 // Operand-type bits of a GEMM launch:
@@ -191,5 +193,31 @@ int launch_align(const int32_t* ref_cp, const int64_t* ref_off, const int32_t* h
 int launch_bertscore(const float* emb, const int32_t* row_off, const int32_t* pair_ref, const int32_t* item_off,
                      const int32_t* grp_pair, const int32_t* grp_cand, int32_t n_groups, int H, int32_t row_begin,
                      int32_t row_end, float* inv_norm, float* out, cudaStream_t s);
+
+// ---- greedy seq2seq decoding (seq2seq_kernels.cu) ---------------------------------------
+// ids / logit: [rows, max_len] row-major.  done_rows: rows that have emitted EOS (integer counter).
+struct DecodeState {
+  int32_t* ids;            // [rows, max_len] output ids (position 0 = start token)
+  float* logit;            // [rows, max_len] fp32 logit of each chosen token (0 at start / pad positions), or null
+  int32_t* len;            // [rows] 0 while unfinished, else the generated length incl. start and EOS
+  int32_t* force_col;      // [rows] column whose logit the next head launch picks (forced token) or -1
+  int32_t* done_rows;      // [1]
+  int32_t rows, max_len, start_id, eos_id, pad_id, forced_bos, forced_eos;   // forced_*: -1 = none
+};
+int launch_decode_init(DecodeState st, cudaStream_t s);
+// hid_f32 (T32) / hid_16 (row-major) = LayerNorm(word_scaled[ids[:, pos]] + pos_emb[pos])
+int launch_dec_embed(const DecodeState& st, int pos, const float* word_scaled, const float* pos_emb, const float* g,
+                     const float* b, float eps, int H, float* hid_f32, void* hid_16, bool fp16, cudaStream_t s);
+// One query row per (row, head) against n keys of that row.  Self form (key_start == null): keys are the
+// slots 0..t of the row's cache [rows, max_len, 2H] (K | V); the K | V of slot t are first copied there
+// from new_kv ([rows, new_kv_stride], K at column 0, V at H).  Cross form: keys are rows
+// key_start[r] .. + key_len[r] of kv (row stride kv_stride, K at column 0, V at H).
+int launch_decode_attention(const void* q, int q_stride, const void* kv, int64_t kv_stride, const int32_t* key_start,
+                            const int32_t* key_len, int self_t, int max_len, const void* new_kv, int new_kv_stride,
+                            void* kv_cache, void* ctx, int rows, int H, int max_keys, bool fp16, cudaStream_t s);
+// Step t's choice from the EPI_ARGMAX partials: first maximum, forced BOS / EOS, pad after EOS.
+int launch_argmax_finish(const float2* partials, const float* forced_logit, int n_parts, DecodeState st, int t,
+                         cudaStream_t s);
+int launch_scale_copy(const float* src, float* dst, int64_t n, float scale, cudaStream_t s);
 
 }  // namespace pllb

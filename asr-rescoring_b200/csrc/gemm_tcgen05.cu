@@ -18,7 +18,8 @@
 //              — tcgen05.ld (32 lanes x 32 columns per warp), bias / erf-GELU /
 //              dtype conversion in registers, 128-byte-swizzled staging in shared memory
 //              and TMA stores; or, for the decoder, an online logsumexp over the vocab
-//              tile plus the label-column pick, so the [copies x V] logits never exist.
+//              tile plus the label-column pick, so the [copies x V] logits never exist; or, for
+//              greedy generation, the tile's (max, first argmax) pair, with the same column pick.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -152,7 +153,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tmA);
     prefetch_tensormap(&tmB);
-    if (EPI != EPI_LSE) prefetch_tensormap(&tmC);
+    if (EPI != EPI_LSE && EPI != EPI_ARGMAX) prefetch_tensormap(&tmC);
   }
   if (warp == 1) {
     if (lane == 0) {
@@ -302,6 +303,30 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
         if (row < p.M) {
           p.lse.partials[((size_t)row * tiles_n + tn) * 2 + (ew >> 2)] = make_float2(run_max, run_sum);
+          if (has_label) p.lse.label_logit[row] = lab_val;
+        }
+      } else if constexpr (EPI == EPI_ARGMAX) {
+        // greedy decoding: (max, first column attaining it) of this half tile; columns ascend and the
+        // comparison is strict, so a tie keeps the lower column, as torch.argmax does
+        const int label = (row < p.M) ? p.lse.labels[row] : -1;
+        float run_max = -INFINITY, lab_val = 0.f;
+        int run_arg = n0 + cbase;
+        bool has_label = false;
+        for (int c0 = cbase; c0 < cbase + EPI_COLS; c0 += 32) {
+          uint32_t r[32];
+          tmem_ld_32x32b_x32(t_addr + c0, r);
+          tcgen05_wait_ld();
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const int col = n0 + c0 + j;
+            float v = __uint_as_float(r[j]) + __ldg(p.bias + col);
+            if (col >= p.lse.vocab) v = -INFINITY;
+            if (col == label) { lab_val = v; has_label = true; }
+            if (v > run_max) { run_max = v; run_arg = col; }
+          }
+        }
+        if (row < p.M) {
+          p.lse.partials[((size_t)row * tiles_n + tn) * 2 + (ew >> 2)] = make_float2(run_max, __int_as_float(run_arg));
           if (has_label) p.lse.label_logit[row] = lab_val;
         }
       } else if constexpr (EPI == EPI_BIAS_BF16 || EPI == EPI_BIAS_GELU_BF16) {
@@ -476,8 +501,8 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C
   }
   KParams kp{};
   kp.M = (int)M; kp.N = N; kp.K = K; kp.bias = bias;
-  if (epilogue == EPI_LSE) {
-    if (!lse) return fail(PLLB_ERR_INVALID, "gemm: LSE epilogue needs LseArgs");
+  if (epilogue == EPI_LSE || epilogue == EPI_ARGMAX) {
+    if (!lse) return fail(PLLB_ERR_INVALID, "gemm: LSE / argmax epilogue needs LseArgs");
     kp.lse = *lse;
   }
   int grid;
@@ -496,6 +521,7 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C
     case EPI_BIAS_F32: return launch_epi<EPI_BIAS_F32>(ta, tb, tc, kp, grid, dt, mode, stream);
     case EPI_BIAS_GELU_F32: return launch_epi<EPI_BIAS_GELU_F32>(ta, tb, tc, kp, grid, dt, mode, stream);
     case EPI_LSE: return launch_epi<EPI_LSE>(ta, tb, tc, kp, grid, dt, mode, stream);
+    case EPI_ARGMAX: return launch_epi<EPI_ARGMAX>(ta, tb, tc, kp, grid, dt, mode, stream);
   }
   return fail(PLLB_ERR_INVALID, "gemm: unknown epilogue");
 }

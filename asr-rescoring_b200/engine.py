@@ -741,3 +741,221 @@ def debug_gemm(A_bf16, W_bf16, bias_f32, epilogue: int, simt: bool = False, oper
     else:
         check(lib.pllb_debug_gemm_dt(*args, OPERAND_DTYPES[operand_dtype], ctypes.c_void_p(stream)))
     return out
+
+
+# ---------------------------------------------------------------------------------------------- seq2seq
+# BartForConditionalGeneration (CorrectBart, DESIGN.md §3.11): the HF state_dict names of every tensor the
+# library takes, keyed by where it goes.  `cfg` is a BartConfig.to_dict()-style dict.
+_BART_ENC_LAYER = {"q_w": "self_attn.q_proj.weight", "q_b": "self_attn.q_proj.bias",
+                   "k_w": "self_attn.k_proj.weight", "k_b": "self_attn.k_proj.bias",
+                   "v_w": "self_attn.v_proj.weight", "v_b": "self_attn.v_proj.bias",
+                   "ao_w": "self_attn.out_proj.weight", "ao_b": "self_attn.out_proj.bias",
+                   "ao_ln_g": "self_attn_layer_norm.weight", "ao_ln_b": "self_attn_layer_norm.bias",
+                   "ff1_w": "fc1.weight", "ff1_b": "fc1.bias", "ff2_w": "fc2.weight", "ff2_b": "fc2.bias",
+                   "out_ln_g": "final_layer_norm.weight", "out_ln_b": "final_layer_norm.bias"}
+_BART_DEC_LAYER = {"q_w": "self_attn.q_proj.weight", "q_b": "self_attn.q_proj.bias",
+                   "k_w": "self_attn.k_proj.weight", "k_b": "self_attn.k_proj.bias",
+                   "v_w": "self_attn.v_proj.weight", "v_b": "self_attn.v_proj.bias",
+                   "o_w": "self_attn.out_proj.weight", "o_b": "self_attn.out_proj.bias",
+                   "self_ln_g": "self_attn_layer_norm.weight", "self_ln_b": "self_attn_layer_norm.bias",
+                   "cq_w": "encoder_attn.q_proj.weight", "cq_b": "encoder_attn.q_proj.bias",
+                   "ck_w": "encoder_attn.k_proj.weight", "ck_b": "encoder_attn.k_proj.bias",
+                   "cv_w": "encoder_attn.v_proj.weight", "cv_b": "encoder_attn.v_proj.bias",
+                   "co_w": "encoder_attn.out_proj.weight", "co_b": "encoder_attn.out_proj.bias",
+                   "cross_ln_g": "encoder_attn_layer_norm.weight", "cross_ln_b": "encoder_attn_layer_norm.bias",
+                   "ff1_w": "fc1.weight", "ff1_b": "fc1.bias", "ff2_w": "fc2.weight", "ff2_b": "fc2.bias",
+                   "final_ln_g": "final_layer_norm.weight", "final_ln_b": "final_layer_norm.bias"}
+_BART_TOP = {"shared": "model.shared.weight",
+             "enc_pos": "model.encoder.embed_positions.weight",
+             "enc_ln_g": "model.encoder.layernorm_embedding.weight", "enc_ln_b": "model.encoder.layernorm_embedding.bias",
+             "dec_pos": "model.decoder.embed_positions.weight",
+             "dec_ln_g": "model.decoder.layernorm_embedding.weight", "dec_ln_b": "model.decoder.layernorm_embedding.bias",
+             "final_logits_bias": "final_logits_bias"}
+# tied copies of model.shared.weight a checkpoint may carry
+BART_TIED_KEYS = ("model.encoder.embed_tokens.weight", "model.decoder.embed_tokens.weight", "lm_head.weight")
+
+
+def bart_weight_keys(cfg: dict) -> Dict[tuple, str]:
+    """{("top", name) | ("enc", layer, field) | ("dec", layer, field): state_dict key}."""
+    out = {("top", k): v for k, v in _BART_TOP.items()}
+    for i in range(int(cfg["encoder_layers"])):
+        for f, k in _BART_ENC_LAYER.items():
+            out[("enc", i, f)] = f"model.encoder.layers.{i}.{k}"
+    for i in range(int(cfg["decoder_layers"])):
+        for f, k in _BART_DEC_LAYER.items():
+            out[("dec", i, f)] = f"model.decoder.layers.{i}.{k}"
+    return out
+
+
+def bart_state_dict(state_dict) -> Dict[str, "torch.Tensor"]:
+    """The state_dict with one leading module prefix (a wrapper's ``bart.``) stripped, located by
+    ``model.shared.weight``; tied copies of the shared table must equal it (ValueError otherwise)."""
+    import torch
+    anchor = [k for k in state_dict if k == "model.shared.weight" or k.endswith(".model.shared.weight")]
+    if len(anchor) != 1:
+        raise ValueError("state_dict must hold exactly one 'model.shared.weight' (optionally under one prefix)")
+    prefix = anchor[0][:-len("model.shared.weight")]
+    sd = {k[len(prefix):]: v for k, v in state_dict.items() if k.startswith(prefix)}
+    shared = sd["model.shared.weight"]
+    for k in BART_TIED_KEYS:
+        if k in sd and not torch.equal(sd[k].detach().cpu(), shared.detach().cpu()):
+            raise ValueError(f"{k} is not a copy of model.shared.weight: untied embeddings are not supported")
+    return sd
+
+
+def check_bart_config(cfg: dict) -> dict:
+    """The library's s2s shape from a BartConfig dict; ValueError for what the kernels do not implement."""
+    H = int(cfg["d_model"])
+    heads = int(cfg["encoder_attention_heads"])
+    if cfg.get("activation_function", "gelu") != "gelu":
+        raise ValueError("only activation_function 'gelu' (erf form) is supported")
+    if cfg.get("normalize_before", False) or cfg.get("add_final_layer_norm", False):
+        raise ValueError("only post-LN BART (no normalize_before / final layer_norm) is supported")
+    if int(cfg.get("decoder_attention_heads", heads)) != heads or heads * 64 != H:
+        raise ValueError("head dim must be 64 in both stacks")
+    if H % 256 or not 256 <= H <= 1024 or int(cfg["encoder_ffn_dim"]) % 256 or int(cfg["decoder_ffn_dim"]) % 256:
+        raise ValueError("d_model must be 256/512/768/1024 and the FFN widths multiples of 256")
+    return dict(enc_layers=int(cfg["encoder_layers"]), dec_layers=int(cfg["decoder_layers"]), hidden=H, num_heads=heads,
+                enc_intermediate=int(cfg["encoder_ffn_dim"]), dec_intermediate=int(cfg["decoder_ffn_dim"]),
+                vocab=int(cfg["vocab_size"]), max_position=int(cfg["max_position_embeddings"]),
+                embed_scale=float(np.sqrt(H)) if cfg.get("scale_embedding", False) else 1.0)
+
+
+_GEN_KEYS = ("max_length", "decoder_start_token_id", "eos_token_id", "pad_token_id", "forced_bos_token_id",
+             "forced_eos_token_id")
+
+
+def generation_settings(cfg: dict, **overrides) -> dict:
+    """generate()'s settings from a config dict (+ overrides), checked as pllb_generate checks them:
+    ValueError for beam search, sampling, no_repeat_ngram_size, min_length, repetition_penalty != 1 and
+    ids outside the vocabulary."""
+    g = {k: cfg.get(k) for k in _GEN_KEYS}
+    for k in ("num_beams", "do_sample", "no_repeat_ngram_size", "min_length", "repetition_penalty"):
+        if k in cfg:
+            g[k] = cfg[k]
+    g.update(overrides)
+    if g.get("max_length") is None:
+        g["max_length"] = 20
+    if int(g.get("num_beams") or 1) != 1:
+        raise ValueError("beam search (num_beams > 1) is not supported; greedy only")
+    if g.get("do_sample"):
+        raise ValueError("sampling is not supported; greedy only")
+    if int(g.get("no_repeat_ngram_size") or 0) != 0:
+        raise ValueError("no_repeat_ngram_size is not supported")
+    if int(g.get("min_length") or 0) != 0:
+        raise ValueError("min_length is not supported")
+    if float(g.get("repetition_penalty") if g.get("repetition_penalty") is not None else 1.0) != 1.0:
+        raise ValueError("repetition_penalty != 1 is not supported")
+    V = int(cfg["vocab_size"])
+    ml = int(g["max_length"])
+    if not 2 <= ml <= int(cfg["max_position_embeddings"]):
+        raise ValueError(f"max_length must lie in [2, {cfg['max_position_embeddings']}]")
+    for k in ("decoder_start_token_id", "eos_token_id", "pad_token_id"):
+        if g[k] is None or not 0 <= int(g[k]) < V:
+            raise ValueError(f"{k} must be an id inside the vocabulary")
+    for k in ("forced_bos_token_id", "forced_eos_token_id"):
+        if g[k] is not None and not 0 <= int(g[k]) < V:
+            raise ValueError(f"{k} must be None or an id inside the vocabulary")
+    return g
+
+
+def _gen_desc(g: dict) -> "_lib.GenDesc":
+    rp = g.get("repetition_penalty")
+    return _lib.GenDesc(int(g["max_length"]), int(g["decoder_start_token_id"]), int(g["eos_token_id"]),
+                        int(g["pad_token_id"]), -1 if g.get("forced_bos_token_id") is None else int(g["forced_bos_token_id"]),
+                        -1 if g.get("forced_eos_token_id") is None else int(g["forced_eos_token_id"]),
+                        int(g.get("num_beams") or 1), int(bool(g.get("do_sample"))), int(g.get("no_repeat_ngram_size") or 0),
+                        int(g.get("min_length") or 0), float(1.0 if rp is None else rp))
+
+
+class Seq2SeqGenerator(_Handle):
+    """Greedy generation with a BartForConditionalGeneration state_dict (pllb_s2s_* / pllb_generate):
+    the encoder reads [CLS] t [SEP], the decoder emits ids as ``generate(num_beams=1, do_sample=False)``."""
+
+    _DESTROY = "pllb_s2s_destroy"
+
+    def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: dict, device: int = 0, max_rows: int = 0,
+                 operand_dtype: str = "bf16", cls_id: int = 101, sep_id: int = 102):
+        import torch
+        from ._lib import DecLayerWeights, S2sDesc, S2sWeights
+
+        self._lib = _lib.load()
+        _lib.require_device()
+        self._h = ctypes.c_void_p()
+        self.cfg = dict(cfg)
+        self.shape = check_bart_config(self.cfg)
+        if operand_dtype not in ("bf16", "fp16"):
+            raise ValueError("operand_dtype must be 'bf16' or 'fp16'")
+        self.operand_dtype = operand_dtype
+        sd = bart_state_dict(state_dict)
+        dev = torch.device("cuda", device)
+        keep = []
+
+        def dp(key, skip_rows: int = 0):
+            t = sd[key].detach().to(device=dev, dtype=torch.float32)[skip_rows:].contiguous()
+            keep.append(t)
+            return ctypes.c_void_p(t.data_ptr())
+
+        s = self.shape
+        H = s["hidden"]
+        keys = bart_weight_keys(self.cfg)
+        enc_layers = (LayerWeights * s["enc_layers"])()
+        dec_layers = (DecLayerWeights * s["dec_layers"])()
+        keep += [enc_layers, dec_layers]
+        for (kind, *rest), key in keys.items():
+            if kind == "enc":
+                setattr(enc_layers[rest[0]], rest[1], dp(key))
+            elif kind == "dec":
+                setattr(dec_layers[rest[0]], rest[1], dp(key))
+        w = S2sWeights()
+        w.enc.pos_emb = dp(_BART_TOP["enc_pos"], skip_rows=2)       # BartLearnedPositionalEmbedding's offset of 2
+        w.enc.emb_ln_g, w.enc.emb_ln_b = dp(_BART_TOP["enc_ln_g"]), dp(_BART_TOP["enc_ln_b"])
+        w.enc.layers = ctypes.cast(enc_layers, ctypes.POINTER(LayerWeights))
+        w.dec_layers = ctypes.cast(dec_layers, ctypes.POINTER(DecLayerWeights))
+        w.shared = dp(_BART_TOP["shared"])
+        w.dec_pos_emb = dp(_BART_TOP["dec_pos"], skip_rows=2)
+        w.dec_emb_ln_g, w.dec_emb_ln_b = dp(_BART_TOP["dec_ln_g"]), dp(_BART_TOP["dec_ln_b"])
+        if "final_logits_bias" in sd:
+            w.final_logits_bias = dp("final_logits_bias")             # [1, vocab]
+        else:                                                         # a missing buffer loads as zeros in HF
+            z = torch.zeros(s["vocab"], dtype=torch.float32, device=dev)
+            keep.append(z)
+            w.final_logits_bias = ctypes.c_void_p(z.data_ptr())
+        d = S2sDesc(s["enc_layers"], s["dec_layers"], H, s["num_heads"], s["enc_intermediate"], s["dec_intermediate"],
+                    s["vocab"], s["max_position"], s["max_position"],
+                    1e-5, s["embed_scale"], cls_id, sep_id, 0 if operand_dtype == "bf16" else 1)
+        torch.cuda.synchronize(dev)
+        check(self._lib.pllb_s2s_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w), int(max_rows), device))
+        del keep
+
+    def generate_packed(self, tokens: np.ndarray, offsets: np.ndarray, generation: dict, return_logits: bool = False):
+        """HOST arrays in and out.  tokens int32 (no specials), offsets int64[n+1].  Returns
+        (ids int32[n, max_length], lengths int32[n]) and with return_logits the fp32 logit of every chosen
+        token (float32[n, max_length], 0 at position 0 and at pads)."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        tokens = np.ascontiguousarray(tokens, np.int32)
+        if offsets.ndim != 1 or len(offsets) < 1:
+            raise ValueError("offsets must be a 1-D array of n+1 entries")
+        n = len(offsets) - 1
+        ml = int(generation["max_length"])
+        ids = np.zeros((n, ml), np.int32)
+        lens = np.zeros(n, np.int32)
+        lg = np.zeros((n, ml), np.float32) if return_logits else None
+        g = _gen_desc(generation)
+        check(self._lib.pllb_generate_host(self._h, ctypes.byref(g), _np_ptr(tokens) if len(tokens) else None,
+                                           _np_ptr(offsets), n, _np_ptr(ids), _np_ptr(lens),
+                                           _np_ptr(lg) if lg is not None else None))
+        return (ids, lens, lg) if return_logits else (ids, lens)
+
+    def set_timing(self, enable: bool):
+        check(self._lib.pllb_s2s_set_timing(self._h, int(enable)))
+
+    def reset_stats(self):
+        check(self._lib.pllb_s2s_reset_stats(self._h))
+
+    def stats(self) -> dict:
+        s = _lib.S2sStats()
+        check(self._lib.pllb_s2s_get_stats(self._h, ctypes.byref(s)))
+        d = {n: getattr(s, n) for n, _ in _lib.S2sStats._fields_}
+        d["workspace_bytes"] = int(self._lib.pllb_s2s_workspace_bytes(self._h))
+        return d

@@ -139,6 +139,23 @@ class BertCharTokenizer:
     def encode(self, text: str) -> List[int]:
         return self.convert_tokens_to_ids(self.tokenize(text))
 
+    def decode(self, ids: Sequence[int], skip_ids: Sequence[int] = (0, 101, 102)) -> str:
+        """ids -> text for a character error rate: the ids in ``skip_ids`` (pass cls, sep, pad and the
+        decoder's start / eos ids) are dropped, a ``##`` prefix is removed and the pieces are joined
+        WITHOUT spaces.  (HF's decode puts a space between CJK tokens; jiwer.cer compares characters.)"""
+        inv = getattr(self, "_inv", None)
+        if inv is None:
+            inv = self._inv = {i: t for t, i in self.vocab.items()}
+        skip = set(int(i) for i in skip_ids)
+        out = []
+        for i in ids:
+            i = int(i)
+            if i in skip:
+                continue
+            t = inv.get(i, self.unk_token)
+            out.append(t[2:] if t.startswith("##") else t)
+        return "".join(out)
+
     def char_table(self) -> np.ndarray:
         """int32[TABLE_SIZE] for pllb_tokenize_host: the id of every character that BasicTokenizer
         always isolates as its own token (CJK ideographs, punctuation), TOK_SPACE / TOK_REMOVED for

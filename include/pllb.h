@@ -406,6 +406,117 @@ int pllb_cls_train_step_host(pllb_trainer t, const int32_t* input_ids, const int
 int pllb_cls_train_export(pllb_trainer t, const pllb_weights* dst, float* linear_w, float* linear_b);
 int pllb_cls_train_export_grads(pllb_trainer t, const pllb_weights* dst, float* linear_w, float* linear_b);
 
+/* ---- Greedy seq2seq generation: CorrectBart's one_hyp correction (CorrectBart/ in the reference: a
+ * BartForConditionalGeneration reads the 1-best hypothesis and generate()s a corrected sentence).
+ * DESIGN.md §3.11.  The model is BART with post-LN layers (bart-base): no final encoder / decoder
+ * layer_norm, activation "gelu", head dim 64, hidden and both FFN widths multiples of 256, every
+ * LayerNorm with the same eps (1e-5).
+ *   encoder: [CLS] t [SEP] (cls_id / sep_id), token rows * embed_scale + positions (row i + 2 of
+ *            embed_positions), layernorm_embedding, the BERT-form post-LN layers.  It runs through
+ *            the pllb_create / pllb_embed path with a zero token-type row.
+ *   decoder: position 0 holds decoder_start_id.  The step that writes position t feeds the token at
+ *            t - 1 (token row * embed_scale + embed_positions row t - 1 + 2, layernorm_embedding), runs
+ *            every layer against the KV cache of positions 0 .. t - 1 and the sentence's encoder rows,
+ *            and takes logits = h . shared^T + final_logits_bias (embed_scale does not touch the head).
+ *   choice:  the first index of the maximum (torch.argmax); forced_bos_id replaces it at t = 1,
+ *            forced_eos_id at t = max_length - 1 (the EOS one wins when both apply); a sentence that
+ *            has emitted eos_id emits pad_id from then on.  Decoding stops when every sentence has
+ *            emitted EOS or position max_length - 1 has been written.  This equals
+ *            generate(num_beams=1, do_sample=False, max_length=...) with these settings.
+ * Operand type (operand_dtype): 0 = bf16, 1 = IEEE fp16 for every GEMM operand, the self-attention KV
+ * cache and the cross-attention K/V; fp32 accumulation, fp32 residual stream, fp32 softmax. */
+typedef struct pllb_s2s_desc {
+  int32_t enc_layers, dec_layers;
+  int32_t hidden;              /* d_model: 256 / 512 / 768 / 1024                                  */
+  int32_t num_heads;           /* hidden / 64, both stacks                                         */
+  int32_t enc_intermediate;    /* encoder_ffn_dim, multiple of 256                                 */
+  int32_t dec_intermediate;    /* decoder_ffn_dim, multiple of 256                                 */
+  int32_t vocab;
+  int32_t enc_max_position;    /* max_position_embeddings: rows of encoder embed_positions - 2     */
+  int32_t dec_max_position;    /* same for the decoder                                             */
+  float   ln_eps;              /* 1e-5                                                             */
+  float   embed_scale;         /* sqrt(d_model) with scale_embedding, else 1                       */
+  int32_t cls_id, sep_id;      /* the encoder input's [CLS] / [SEP] ids                            */
+  int32_t operand_dtype;       /* 0 bf16, 1 fp16                                                   */
+} pllb_s2s_desc;
+
+/* One decoder layer; DEVICE fp32 tensors in nn.Linear layout (model.decoder.layers.{i}.*). */
+typedef struct pllb_dec_layer_weights {
+  const float *q_w, *q_b, *k_w, *k_b, *v_w, *v_b, *o_w, *o_b;         /* self_attn.{q,k,v,out}_proj        */
+  const float *self_ln_g, *self_ln_b;                                  /* self_attn_layer_norm              */
+  const float *cq_w, *cq_b, *ck_w, *ck_b, *cv_w, *cv_b, *co_w, *co_b; /* encoder_attn.{q,k,v,out}_proj     */
+  const float *cross_ln_g, *cross_ln_b;                                /* encoder_attn_layer_norm           */
+  const float *ff1_w, *ff1_b, *ff2_w, *ff2_b;                          /* fc1, fc2                          */
+  const float *final_ln_g, *final_ln_b;                                /* final_layer_norm                  */
+} pllb_dec_layer_weights;
+
+typedef struct pllb_s2s_weights {
+  /* encoder, DEVICE fp32: word_emb and type_emb are ignored (the token table is `shared`, the
+   * token-type row is zero); pos_emb = model.encoder.embed_positions.weight + 2 * hidden (the offset
+   * rows skipped); emb_ln_* = model.encoder.layernorm_embedding; layers = model.encoder.layers
+   * (self_attn.{q,k,v,out}_proj, self_attn_layer_norm, fc1, fc2, final_layer_norm); head pointers
+   * ignored. */
+  pllb_weights enc;
+  const pllb_dec_layer_weights* dec_layers;   /* HOST array of dec_layers structs                 */
+  const float* shared;                        /* model.shared.weight [vocab, hidden], unscaled     */
+  const float* dec_pos_emb;                   /* model.decoder.embed_positions.weight + 2 * hidden */
+  const float *dec_emb_ln_g, *dec_emb_ln_b;   /* model.decoder.layernorm_embedding                 */
+  const float* final_logits_bias;             /* [vocab]                                           */
+} pllb_s2s_weights;
+
+/* generate() settings.  Everything generate() would apply beyond greedy decoding is rejected with
+ * PLLB_ERR_INVALID: num_beams != 1, do_sample != 0, no_repeat_ngram_size != 0, min_length != 0,
+ * repetition_penalty != 1. */
+typedef struct pllb_gen_desc {
+  int32_t max_length;          /* 2 <= max_length <= dec_max_position                              */
+  int32_t decoder_start_id, eos_id, pad_id;
+  int32_t forced_bos_id;       /* -1 = none */
+  int32_t forced_eos_id;       /* -1 = none */
+  int32_t num_beams, do_sample, no_repeat_ngram_size, min_length;
+  float   repetition_penalty;
+} pllb_gen_desc;
+
+/* Counters since create (or the last reset) and, with timing enabled, the device time of the last
+ * pllb_generate call split by phase. */
+typedef struct pllb_s2s_stats {
+  int64_t kernel_launches;     /* kernels of this library launched                                 */
+  int64_t steps;               /* decoder steps run (summed over chunks)                           */
+  int64_t chunks;
+  int64_t sentences;
+  double  gemm_flops;          /* algorithmic GEMM FLOPs (encoder, cross K/V, decoder, head)       */
+  float   enc_ms, cross_kv_ms, dec_layers_ms, head_ms;   /* last call, timing enabled               */
+  float   total_ms;                                      /* last call, timing enabled               */
+} pllb_s2s_stats;
+
+typedef struct pllb_s2s_ctx* pllb_s2s;
+
+/* weights are copied (16-bit operands, fp32 rest).  max_rows bounds the sentences decoded together
+ * per internal chunk (0 = 8192); the per-call workspace grows with max_rows * max_length: the KV
+ * cache alone is rows * max_length * 2 * hidden * dec_layers * 2 bytes.  Results do not depend on
+ * max_rows. */
+int pllb_s2s_create(pllb_s2s* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* weights, int32_t max_rows,
+                    int device);
+int pllb_s2s_destroy(pllb_s2s h);
+int64_t pllb_s2s_workspace_bytes(pllb_s2s h);
+int pllb_s2s_set_timing(pllb_s2s h, int enable);
+int pllb_s2s_get_stats(pllb_s2s h, pllb_s2s_stats* out);
+int pllb_s2s_reset_stats(pllb_s2s h);
+
+/* tokens DEVICE int32 (ids in [0, vocab): pllb_generate_host checks them), no specials; sentence i is
+ * tokens[offsets[i] .. offsets[i+1]); offsets HOST int64[n+1].  A sentence with more than
+ * enc_max_position - 2 tokens returns PLLB_ERR_TOO_LONG.
+ * out_ids   DEVICE int32[n * max_length]: sentence i's ids at [i * max_length, ...), position 0 = start
+ *           token, pad_id after the end (generate() returns the same up to its own padding width);
+ * out_len   DEVICE int32[n]: positions up to and including EOS (max_length when none was emitted);
+ * out_logit DEVICE float[n * max_length] or NULL: fp32 logit of each chosen token (at a forced position
+ *           the logit of the forced token), 0 at position 0 and at pad positions.
+ * Runs on `stream` and waits for it once per decoder step (the count of finished sentences decides
+ * whether to continue): the call returns when the results are complete. */
+int pllb_generate(pllb_s2s h, const pllb_gen_desc* gen, const int32_t* tokens, const int64_t* offsets, int32_t n,
+                  int32_t* out_ids, int32_t* out_len, float* out_logit, void* stream);
+int pllb_generate_host(pllb_s2s h, const pllb_gen_desc* gen, const int32_t* tokens, const int64_t* offsets, int32_t n,
+                       int32_t* out_ids, int32_t* out_len, float* out_logit);
+
 #ifdef __cplusplus
 }
 #endif
