@@ -2,8 +2,8 @@
 
 The reference generates with ``BartForConditionalGeneration.generate(max_length=50)`` from the 1-best
 hypothesis and scores the outputs with ``jiwer.cer`` (CorrectBart/compute_cer.py:8).  Here the model runs
-through ``engine.Seq2SeqGenerator`` (greedy decoding, pllb_generate) and the CER through the
-Levenshtein kernel of ``cer_clients``."""
+through ``engine.Seq2SeqGenerator`` (greedy decoding, pllb_generate, or beam search, pllb_generate_beam,
+when ``num_beams > 1``) and the CER through the Levenshtein kernel of ``cer_clients``."""
 from __future__ import annotations
 
 from typing import Dict, List, Optional, Sequence
@@ -18,14 +18,19 @@ class CorrectBart:
     """state_dict: a BartForConditionalGeneration state_dict (optionally under one module prefix);
     cfg: its BartConfig as a dict, which also supplies generate()'s settings (decoder_start_token_id,
     eos_token_id, pad_token_id, forced_bos_token_id, forced_eos_token_id); ``generation`` overrides them.
-    tokenizer: a BertCharTokenizer (fnlp/bart-base-chinese uses BertTokenizer)."""
+    tokenizer: a BertCharTokenizer (fnlp/bart-base-chinese uses BertTokenizer).  With ``num_beams > 1`` in
+    the config or in ``generation``, correct() runs beam search (also reading num_return_sequences,
+    length_penalty and early_stopping) and decodes the best hypothesis."""
 
     def __init__(self, state_dict, cfg: dict, tokenizer, device: int = 0, max_length: int = 50,
                  operand_dtype: str = "bf16", max_rows: int = 0, cls_id: int = 101, sep_id: int = 102,
                  generation: Optional[dict] = None):
         self.tokenizer = tokenizer
         self.cls_id, self.sep_id = cls_id, sep_id
-        self.generation = engine.generation_settings(cfg, max_length=max_length, **(generation or {}))
+        gen = dict(generation or {})
+        self.beam = int(gen.get("num_beams", cfg.get("num_beams")) or 1) > 1
+        settings = engine.beam_settings if self.beam else engine.generation_settings
+        self.generation = settings(cfg, max_length=max_length, **gen)
         self.model = engine.Seq2SeqGenerator(state_dict, cfg, device=device, max_rows=max_rows,
                                              operand_dtype=operand_dtype, cls_id=cls_id, sep_id=sep_id)
 
@@ -33,7 +38,13 @@ class CorrectBart:
         self.model.close()
 
     def generate_packed(self, tokens: np.ndarray, offsets: np.ndarray, return_logits: bool = False):
-        """Packed ids (no specials) -> (ids int32[n, max_length], lengths int32[n][, logits])."""
+        """Packed ids (no specials) -> (ids int32[n, max_length], lengths int32[n][, logits]); with beam
+        search the best hypothesis of each sentence (no logits)."""
+        if self.beam:
+            if return_logits:
+                raise ValueError("beam search returns hypothesis scores, not per-token logits")
+            ids, lens, _ = self.model.beam_search_packed(tokens, offsets, self.generation)
+            return ids[:, 0], lens[:, 0]
         return self.model.generate_packed(tokens, offsets, self.generation, return_logits=return_logits)
 
     def skip_ids(self) -> List[int]:

@@ -81,6 +81,10 @@ class GenDesc(ctypes.Structure):
                 ("no_repeat_ngram_size", c_int32), ("min_length", c_int32), ("repetition_penalty", c_float)]
 
 
+class BeamDesc(ctypes.Structure):
+    _fields_ = [("num_return_sequences", c_int32), ("length_penalty", c_float), ("early_stopping", c_int32)]
+
+
 class S2sStats(ctypes.Structure):
     _fields_ = [("kernel_launches", c_int64), ("steps", c_int64), ("chunks", c_int64), ("sentences", c_int64),
                 ("gemm_flops", c_double), ("enc_ms", c_float), ("cross_kv_ms", c_float), ("dec_layers_ms", c_float),
@@ -149,6 +153,12 @@ SIGNATURES = {
                               c_void_p]),
     "pllb_generate_host": (c_int, [c_void_p, POINTER(GenDesc), c_void_p, c_void_p, c_int32, c_void_p, c_void_p,
                                    c_void_p]),
+    "pllb_generate_beam": (c_int, [c_void_p, POINTER(GenDesc), POINTER(BeamDesc), c_void_p, c_void_p, c_int32, c_void_p,
+                                   c_void_p, c_void_p, c_void_p]),
+    "pllb_generate_beam_host": (c_int, [c_void_p, POINTER(GenDesc), POINTER(BeamDesc), c_void_p, c_void_p, c_int32,
+                                        c_void_p, c_void_p, c_void_p]),
+    "pllb_s2s_debug_beam_replay": (c_int, [c_void_p, POINTER(GenDesc), POINTER(BeamDesc), c_int32, c_void_p, c_int32,
+                                           c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

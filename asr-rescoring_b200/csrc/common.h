@@ -68,8 +68,11 @@ enum GemmEpilogue : int {
   EPI_BIAS_F32 = 2,        // out fp32 = acc + bias
   EPI_BIAS_GELU_F32 = 3,   // out fp32 = gelu_erf(acc + bias)
   EPI_LSE = 4,             // vocab-tiled online logsumexp + label-column pick (no C output)
-  EPI_ARGMAX = 5           // vocab-tiled (max, first argmax) + label-column pick (no C output); LseArgs.partials
+  EPI_ARGMAX = 5,          // vocab-tiled (max, first argmax) + label-column pick (no C output); LseArgs.partials
                            // hold (max, __int_as_float(column)) per 128-column half tile
+  EPI_TOPK8 = 6,           // beam search (no C output, labels unused): LseArgs.partials hold the EPI_LSE pairs
+  EPI_TOPK16 = 7           // [M, 2 * n_tiles_n], then the KSEL (8 / 16) largest (logit, __int_as_float(column))
+                           // of every half tile, [M, 2 * n_tiles_n, KSEL], descending, ties to the lower column
 };
 
 // Operand-type bits of a GEMM launch:
@@ -212,12 +215,42 @@ int launch_dec_embed(const DecodeState& st, int pos, const float* word_scaled, c
 // slots 0..t of the row's cache [rows, max_len, 2H] (K | V); the K | V of slot t are first copied there
 // from new_kv ([rows, new_kv_stride], K at column 0, V at H).  Cross form: keys are rows
 // key_start[r] .. + key_len[r] of kv (row stride kv_stride, K at column 0, V at H).
+// slot (beam search, self form only): key j < self_t of row r is cache row slot[r * max_len + j] of
+// the [rows * max_len, 2H] cache instead of row r * max_len + j; key self_t is always the row's own.
 int launch_decode_attention(const void* q, int q_stride, const void* kv, int64_t kv_stride, const int32_t* key_start,
                             const int32_t* key_len, int self_t, int max_len, const void* new_kv, int new_kv_stride,
-                            void* kv_cache, void* ctx, int rows, int H, int max_keys, bool fp16, cudaStream_t s);
+                            void* kv_cache, void* ctx, int rows, int H, int max_keys, bool fp16, cudaStream_t s,
+                            const int32_t* slot = nullptr);
 // Step t's choice from the EPI_ARGMAX partials: first maximum, forced BOS / EOS, pad after EOS.
 int launch_argmax_finish(const float2* partials, const float* forced_logit, int n_parts, DecodeState st, int t,
                          cudaStream_t s);
 int launch_scale_copy(const float* src, float* dst, int64_t n, float scale, cudaStream_t s);
+
+// ---- beam search (seq2seq_kernels.cu, DESIGN.md §3.12) ------------------------------------
+// A chunk of n sentences decodes n * K beam rows; beam b of sentence i is row i * K + b.  Per row
+// [rows, max_len] int32 buffers: running ids and the KV slot table (ping-pong, gathered by parent).
+// Per sentence: K finished slots (ids [n * K, max_len], len, score, flag) and the flags below.
+struct BeamState {
+  int32_t* ids_cur;        // running ids, positions 0 .. t - 1 valid
+  int32_t* ids_next;
+  int32_t* slot_cur;       // KV slot table, entries 0 .. t - 2 valid
+  int32_t* slot_next;
+  float* run_score;        // [rows] running beam scores (read, then rewritten in place)
+  int32_t* parent;         // [rows] parent row of this step's running beams (chunk-local row index)
+  int32_t* fin_ids;        // [rows, max_len]
+  int32_t* fin_len;        // [rows]
+  float* fin_score;        // [rows]
+  int32_t* fin_flag;       // [rows]
+  int32_t* sent_flags;     // [n]: bit 0 early-stop heuristic satisfied, bit 1 frozen
+  int32_t* frozen_count;   // [1] sentences frozen so far (integer atomic)
+  int32_t n, K, max_len, start_id, eos_id, pad_id, forced_bos, forced_eos, early_stopping;   // 0 False 1 True 2 never
+  float length_penalty;
+};
+int launch_beam_init(BeamState st, cudaStream_t s);
+// Step t: merge each row's EPI_TOPK partials (n_parts = 2 * vocab tiles of ksel entries each) into its
+// log-softmax and top 2K, then apply the beam-search bookkeeping of DESIGN.md §3.12; one CTA per sentence.
+int launch_beam_select(const float2* partials, int n_parts, int ksel, int vocab, BeamState st, int t, cudaStream_t s);
+// The best r slots of every sentence: ids [n, r, max_len] (pad after the end), len [n, r], score [n, r].
+int launch_beam_output(BeamState st, int r, int32_t* out_ids, int32_t* out_len, float* out_score, cudaStream_t s);
 
 }  // namespace pllb

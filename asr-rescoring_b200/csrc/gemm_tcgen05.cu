@@ -19,9 +19,12 @@
 //              dtype conversion in registers, 128-byte-swizzled staging in shared memory
 //              and TMA stores; or, for the decoder, an online logsumexp over the vocab
 //              tile plus the label-column pick, so the [copies x V] logits never exist; or, for
-//              greedy generation, the tile's (max, first argmax) pair, with the same column pick.
+//              greedy generation, the tile's (max, first argmax) pair, with the same column pick; or,
+//              for beam search, the logsumexp pair plus the tile's KSEL largest (logit, column) pairs.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+
+#include <climits>
 
 #include "common.h"
 #include "ptx.cuh"
@@ -153,7 +156,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tmA);
     prefetch_tensormap(&tmB);
-    if (EPI != EPI_LSE && EPI != EPI_ARGMAX) prefetch_tensormap(&tmC);
+    if (EPI != EPI_LSE && EPI != EPI_ARGMAX && EPI != EPI_TOPK8 && EPI != EPI_TOPK16) prefetch_tensormap(&tmC);
   }
   if (warp == 1) {
     if (lane == 0) {
@@ -329,6 +332,63 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           p.lse.partials[((size_t)row * tiles_n + tn) * 2 + (ew >> 2)] = make_float2(run_max, __int_as_float(run_arg));
           if (has_label) p.lse.label_logit[row] = lab_val;
         }
+      } else if constexpr (EPI == EPI_TOPK8 || EPI == EPI_TOPK16) {
+        // beam search: the (max, sum of exp) pair exactly as EPI_LSE, plus the KS largest (logit, column)
+        // pairs of this half tile in descending order, ties to the lower column.  The list starts as
+        // (-inf, INT_MAX) placeholders, so masked columns (-inf) still fill it by ascending column.
+        constexpr int KS = EPI == EPI_TOPK16 ? 16 : 8;
+        float run_max = -INFINITY, run_sum = 0.f;
+        float tv[KS];
+        int tc[KS];
+#pragma unroll
+        for (int i = 0; i < KS; ++i) { tv[i] = -INFINITY; tc[i] = INT_MAX; }
+        for (int c0 = cbase; c0 < cbase + EPI_COLS; c0 += 32) {
+          uint32_t r[32];
+          tmem_ld_32x32b_x32(t_addr + c0, r);
+          tcgen05_wait_ld();
+          float x[32];
+          float cmax = -INFINITY;
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const int col = n0 + c0 + j;
+            float v = __uint_as_float(r[j]) + __ldg(p.bias + col);
+            if (col >= p.lse.vocab) v = -INFINITY;
+            x[j] = v;
+            cmax = fmaxf(cmax, v);
+          }
+          if (cmax > -INFINITY) {
+            const float new_max = fmaxf(run_max, cmax);
+            float s = 0.f;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) s += __expf(x[j] - new_max);
+            run_sum = run_sum * __expf(run_max - new_max) + s;
+            run_max = new_max;
+          }
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            // columns ascend: a value equal to the last kept one enters only in front of a placeholder
+            if (x[j] > tv[KS - 1] || (x[j] == tv[KS - 1] && tc[KS - 1] == INT_MAX)) {
+              tv[KS - 1] = x[j];
+              tc[KS - 1] = n0 + c0 + j;
+#pragma unroll
+              for (int i = KS - 1; i > 0; --i) {
+                if (tv[i] > tv[i - 1] || (tv[i] == tv[i - 1] && tc[i] < tc[i - 1])) {
+                  const float fv = tv[i]; tv[i] = tv[i - 1]; tv[i - 1] = fv;
+                  const int fc = tc[i]; tc[i] = tc[i - 1]; tc[i - 1] = fc;
+                }
+              }
+            }
+          }
+        }
+        if (row < p.M) {
+          const size_t slot = ((size_t)row * tiles_n + tn) * 2 + (ew >> 2);
+          p.lse.partials[slot] = make_float2(run_max, run_sum);
+          // the top-KS lists follow the [M, 2 * tiles_n] pairs: [M, 2 * tiles_n, KS] (logit, column)
+          float4* top = reinterpret_cast<float4*>(p.lse.partials + (size_t)p.M * tiles_n * 2 + slot * KS);
+#pragma unroll
+          for (int i = 0; i < KS; i += 2)
+            top[i / 2] = make_float4(tv[i], __int_as_float(tc[i]), tv[i + 1], __int_as_float(tc[i + 1]));
+        }
       } else if constexpr (EPI == EPI_BIAS_BF16 || EPI == EPI_BIAS_GELU_BF16) {
         for (int c0 = cbase; c0 < cbase + EPI_COLS; c0 += 64) {
           uint32_t r0[32], r1[32];
@@ -501,8 +561,8 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C
   }
   KParams kp{};
   kp.M = (int)M; kp.N = N; kp.K = K; kp.bias = bias;
-  if (epilogue == EPI_LSE || epilogue == EPI_ARGMAX) {
-    if (!lse) return fail(PLLB_ERR_INVALID, "gemm: LSE / argmax epilogue needs LseArgs");
+  if (epilogue == EPI_LSE || epilogue == EPI_ARGMAX || epilogue == EPI_TOPK8 || epilogue == EPI_TOPK16) {
+    if (!lse) return fail(PLLB_ERR_INVALID, "gemm: LSE / argmax / top-k epilogue needs LseArgs");
     kp.lse = *lse;
   }
   int grid;
@@ -522,6 +582,8 @@ int launch_gemm_tcgen05(const void* A, const void* W, const float* bias, void* C
     case EPI_BIAS_GELU_F32: return launch_epi<EPI_BIAS_GELU_F32>(ta, tb, tc, kp, grid, dt, mode, stream);
     case EPI_LSE: return launch_epi<EPI_LSE>(ta, tb, tc, kp, grid, dt, mode, stream);
     case EPI_ARGMAX: return launch_epi<EPI_ARGMAX>(ta, tb, tc, kp, grid, dt, mode, stream);
+    case EPI_TOPK8: return launch_epi<EPI_TOPK8>(ta, tb, tc, kp, grid, dt, mode, stream);
+    case EPI_TOPK16: return launch_epi<EPI_TOPK16>(ta, tb, tc, kp, grid, dt, mode, stream);
   }
   return fail(PLLB_ERR_INVALID, "gemm: unknown epilogue");
 }

@@ -5,11 +5,15 @@
 // GEMM, single-query cross-attention over the row's encoder K/V, output GEMM + LayerNorm and the
 // FFN; then the LM head GEMM with the EPI_ARGMAX epilogue and argmax_finish.  The GEMMs are the
 // tcgen05 kernels of gemm_tcgen05.cu / gemm_ln_tcgen05.cu; this file holds everything else.
-// fp32 arithmetic, no atomics except the integer count of finished rows: a run is bit-deterministic.
+// Beam search (pllb_generate_beam) adds beam_select_kernel, which merges the EPI_TOPK8 / EPI_TOPK16
+// partials and carries the beam bookkeeping, and a slot-table form of the self-attention.
+// fp32 arithmetic, no atomics except the integer counts of finished rows / frozen sentences: a run is
+// bit-deterministic.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
 #include <algorithm>
+#include <climits>
 
 #include "common.h"
 
@@ -118,12 +122,15 @@ __global__ void __launch_bounds__(256) dec_embed_kernel(DecodeState st, int pos,
 // One warp per (row, head), four warps per block.  Lane j scores keys j, j + 32, ... (the full
 // 64-wide query sits in registers, each key row is one 128-byte read); the softmax weights go
 // through shared memory; for the weighted sum of V each lane owns two of the 64 dimensions.
-template <bool FP16>
+// SLOT (beam search, self form): key j < self_t of row r is cache row slot[r * max_len + j] instead of
+// r * max_len + j, so beams that share a prefix share its cache rows; the trailing `slot` parameter is
+// unused otherwise.
+template <bool FP16, bool SLOT>
 __global__ void __launch_bounds__(128, 4) decode_attention_kernel(
     const uint16_t* __restrict__ q, int q_stride, const uint16_t* kv, int64_t kv_stride,
     const int32_t* __restrict__ key_start, const int32_t* __restrict__ key_len, int self_t, int max_len,
     const uint16_t* __restrict__ new_kv, int new_kv_stride, uint16_t* kv_cache, uint16_t* __restrict__ ctx, int rows,
-    int H, int NH, int max_keys) {
+    int H, int NH, int max_keys, const int32_t* __restrict__ slot) {
   extern __shared__ float sp[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t item = (int64_t)blockIdx.x * 4 + warp;
@@ -153,9 +160,16 @@ __global__ void __launch_bounds__(128, 4) decode_attention_kernel(
   const uint16_t* qrow = q + (size_t)r * q_stride + h * 64;
 #pragma unroll
   for (int i = 0; i < 8; ++i) ld16x8<FP16>(qrow + 8 * i, qv + 8 * i);
+  // SLOT: cache row of key j (keys before self_t through the slot table, key self_t the row's own)
+  auto key_row = [&](int j) -> const uint16_t* {
+    const int64_t cr = j < self_t ? (int64_t)slot[(size_t)r * max_len + j] : (int64_t)r * max_len + self_t;
+    return kv_cache + (size_t)cr * (size_t)(2 * H);
+  };
   float m = -INFINITY;
   for (int j = lane; j < n; j += 32) {
-    const uint16_t* krow = base + (size_t)j * stride + h * 64;
+    const uint16_t* krow;
+    if constexpr (SLOT) krow = key_row(j) + h * 64;
+    else krow = base + (size_t)j * stride + h * 64;
     float acc = 0.f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -183,7 +197,9 @@ __global__ void __launch_bounds__(128, 4) decode_attention_kernel(
   const uint16_t* vcol = base + H + h * 64 + 2 * lane;
   for (int j = 0; j < n; ++j) {
     const float w = p[j];
-    const uint32_t u = *reinterpret_cast<const uint32_t*>(vcol + (size_t)j * stride);
+    uint32_t u;
+    if constexpr (SLOT) u = *reinterpret_cast<const uint32_t*>(key_row(j) + H + h * 64 + 2 * lane);
+    else u = *reinterpret_cast<const uint32_t*>(vcol + (size_t)j * stride);
     const float2 v = unpack16x2<FP16>(u);
     o0 = fmaf(w, v.x, o0);
     o1 = fmaf(w, v.y, o1);
@@ -221,6 +237,283 @@ __global__ void argmax_finish_kernel(const float2* __restrict__ parts, const flo
   st.force_col[r] = tn == st.max_len - 1 && st.forced_eos >= 0 ? st.forced_eos : tn == 1 ? st.forced_bos : -1;
 }
 
+// ---------------------------------------------------------------------------------------- beam search
+// DESIGN.md §3.12.  (value, index) orders of the selection: higher value first, then lower index.
+__device__ __forceinline__ bool beats(float v, int i, float w, int j) { return v > w || (v == w && i < j); }
+
+__device__ __forceinline__ void lse_merge(float& m, float& s, float m2, float s2) {
+  if (m2 == -INFINITY) return;
+  if (m == -INFINITY) { m = m2; s = s2; return; }
+  const float nm = fmaxf(m, m2);
+  s = s * expf(m - nm) + s2 * expf(m2 - nm);
+  m = nm;
+}
+
+__global__ void beam_init_kernel(BeamState st) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r == 0) *st.frozen_count = 0;
+  if (r < st.n) st.sent_flags[r] = 0;
+  if (r >= st.n * st.K) return;
+  st.ids_cur[(size_t)r * st.max_len] = st.start_id;
+  st.ids_next[(size_t)r * st.max_len] = st.start_id;
+  int32_t* f = st.fin_ids + (size_t)r * st.max_len;
+  f[0] = st.start_id;
+  for (int j = 1; j < st.max_len; ++j) f[j] = st.pad_id;
+  st.fin_len[r] = 1;
+  st.fin_score[r] = -1e9f;
+  st.fin_flag[r] = 0;
+  st.run_score[r] = r % st.K == 0 ? 0.f : -1e9f;
+  st.parent[r] = r;
+}
+
+// One CTA of 256 threads per sentence; warp b < K merges beam row b's partials, warp 0 then selects the
+// sentence's top 2K candidates and thread 0 applies items 3-7 of the contract in fp32, in a fixed order.
+// Dynamic shared memory: K * max_len ints (the old finished ids while the slots are rewritten).
+template <int KS>
+__global__ void __launch_bounds__(256) beam_select_kernel(const float2* __restrict__ parts, int n_parts, int vocab,
+                                                          BeamState st, int t) {
+  extern __shared__ int32_t stage[];
+  __shared__ float c_val[8][KS];
+  __shared__ int c_tok[8][KS];
+  __shared__ float s_val[16];
+  __shared__ int s_tok[16], s_beam[16];
+  __shared__ int n_par[8], n_tok[8], f_src[8], f_flag[8];
+  __shared__ float n_rs[8], f_score[8];
+  __shared__ int s_frozen, s_changed;
+  const int i = blockIdx.x;
+  const int K = st.K, TK = 2 * K, ML = st.max_len, rows = st.n * st.K;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int row0 = i * K;
+  if (threadIdx.x == 0) { s_frozen = (st.sent_flags[i] & 2) != 0; s_changed = 0; }
+  __syncthreads();
+  const bool frozen = s_frozen != 0;
+  const int forced = t == ML - 1 && st.forced_eos >= 0 ? st.forced_eos : t == 1 && st.forced_bos >= 0 ? st.forced_bos : -1;
+  if (!frozen && warp < K) {
+    const int r = row0 + warp;
+    const float rs = st.run_score[r];
+    if (forced >= 0) {
+      // log-probabilities 0 at the forced id and -inf elsewhere: the -inf ones in column order
+      if (lane < TK) {
+        c_val[warp][lane] = lane == 0 ? 0.f + rs : -INFINITY;
+        c_tok[warp][lane] = lane == 0 ? forced : lane - 1 < forced ? lane - 1 : lane;
+      }
+    } else {
+      const float2* lp = parts + (size_t)r * n_parts;
+      float m = -INFINITY, sum = 0.f;
+      for (int q = lane; q < n_parts; q += 32) {
+        const float2 v = lp[q];
+        lse_merge(m, sum, v.x, v.y);
+      }
+#pragma unroll
+      for (int o = 16; o; o >>= 1) {
+        const float m2 = __shfl_xor_sync(0xffffffffu, m, o), s2 = __shfl_xor_sync(0xffffffffu, sum, o);
+        // both lanes of a pair merge the same two values in the same order
+        float a = m, b = sum, c = m2, d = s2;
+        if ((lane & o) != 0) { a = m2; b = s2; c = m; d = sum; }
+        lse_merge(a, b, c, d);
+        m = a;
+        sum = b;
+      }
+      const float logs = logf(sum);
+      float tv[KS];
+      int tc[KS];
+#pragma unroll
+      for (int k = 0; k < KS; ++k) { tv[k] = -INFINITY; tc[k] = INT_MAX; }
+      const float2* tp = parts + (size_t)rows * n_parts + (size_t)r * n_parts * KS;
+      for (int q = lane; q < n_parts; q += 32) {
+        for (int e = 0; e < KS; ++e) {            // each list descends: stop at the first entry that stays out
+          const float2 v = tp[(size_t)q * KS + e];
+          const int col = __float_as_int(v.y);
+          if (!beats(v.x, col, tv[KS - 1], tc[KS - 1])) break;
+          tv[KS - 1] = v.x;
+          tc[KS - 1] = col;
+#pragma unroll
+          for (int k = KS - 1; k > 0; --k)
+            if (beats(tv[k], tc[k], tv[k - 1], tc[k - 1])) {
+              const float fv = tv[k]; tv[k] = tv[k - 1]; tv[k - 1] = fv;
+              const int fc = tc[k]; tc[k] = tc[k - 1]; tc[k - 1] = fc;
+            }
+        }
+      }
+      for (int k = 0; k < TK; ++k) {              // warp merge of the lanes' sorted lists
+        float bv = tv[0];
+        int bc = tc[0], bl = lane;
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+          const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+          const int oc = __shfl_xor_sync(0xffffffffu, bc, o), ol = __shfl_xor_sync(0xffffffffu, bl, o);
+          if (beats(ov, oc, bv, bc) || (ov == bv && oc == bc && ol < bl)) { bv = ov; bc = oc; bl = ol; }
+        }
+        if (lane == bl) {
+#pragma unroll
+          for (int q = 0; q < KS - 1; ++q) { tv[q] = tv[q + 1]; tc[q] = tc[q + 1]; }
+          tv[KS - 1] = -INFINITY;
+          tc[KS - 1] = INT_MAX;
+        }
+        if (lane == 0) {
+          c_val[warp][k] = ((bv - m) - logs) + rs;   // log_softmax as (x - max) - log(sum), plus the beam score
+          c_tok[warp][k] = min(bc, vocab - 1);
+        }
+      }
+    }
+  }
+  __syncthreads();
+  if (!frozen && warp == 0) {
+    // the sentence's top 2K of the K * 2K candidates, flat index beam * vocab + token on ties
+    float v[4];
+    int fl[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int e = lane + 32 * q;
+      const bool ok = e < K * TK;
+      v[q] = ok ? c_val[e / TK][e % TK] : -INFINITY;
+      fl[q] = ok ? (e / TK) * vocab + c_tok[e / TK][e % TK] : INT_MAX;
+    }
+    for (int k = 0; k < TK; ++k) {
+      float bv = -INFINITY;
+      int bf = INT_MAX, bq = -1;
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        if (fl[q] != INT_MAX && (bq < 0 || beats(v[q], fl[q], bv, bf))) { bv = v[q]; bf = fl[q]; bq = q; }
+      int bl = bq >= 0 ? lane : 32;
+#pragma unroll
+      for (int o = 16; o; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int of = __shfl_xor_sync(0xffffffffu, bf, o), ol = __shfl_xor_sync(0xffffffffu, bl, o);
+        if (ol < 32 && (bl == 32 || beats(ov, of, bv, bf))) { bv = ov; bf = of; bl = ol; }
+      }
+      if (lane == bl) fl[bq] = INT_MAX;             // used
+      if (lane == 0) {
+        s_val[k] = bv;
+        s_beam[k] = bf / vocab;
+        s_tok[k] = bf % vocab;
+      }
+    }
+    __syncwarp();
+    if (lane == 0) {
+      const bool last = t == ML - 1;
+      bool hit[16];
+      float pen[16];
+      for (int c = 0; c < TK; ++c) {
+        hit[c] = s_tok[c] == st.eos_id || last;
+        pen[c] = hit[c] ? s_val[c] + -1e9f : s_val[c];
+      }
+      // running beams: top K of the penalised candidates
+      bool used[24];
+      for (int c = 0; c < 24; ++c) used[c] = false;
+      for (int k = 0; k < K; ++k) {
+        int b = -1;
+        for (int c = 0; c < TK; ++c)
+          if (!used[c] && (b < 0 || beats(pen[c], c, pen[b], b))) b = c;
+        used[b] = true;
+        n_par[k] = row0 + s_beam[b];
+        n_tok[k] = s_tok[b];
+        n_rs[k] = pen[b];
+      }
+      // finished slots: top K of the old slots followed by the 2K normalised candidates
+      float fs[24];
+      bool ff[24];
+      bool all_fin = true;
+      for (int j = 0; j < K; ++j) {
+        fs[j] = st.fin_score[row0 + j];
+        ff[j] = st.fin_flag[row0 + j] != 0;
+        all_fin = all_fin && ff[j];
+      }
+      const int flags = st.sent_flags[i];
+      const bool unsat = (flags & 1) == 0;
+      const float norm = (float)pow((double)t, (double)st.length_penalty);
+      for (int c = 0; c < TK; ++c) {
+        float sc = s_val[c] / norm;
+        if (all_fin && st.early_stopping == 1) sc += -1e9f;
+        if (!unsat) sc += -1e9f;
+        const bool jf = c < K && hit[c];
+        if (!jf) sc += -1e9f;
+        fs[K + c] = sc;
+        ff[K + c] = jf;
+      }
+      for (int c = 0; c < 24; ++c) used[c] = false;
+      bool changed = false;
+      for (int k = 0; k < K; ++k) {
+        int b = -1;
+        for (int c = 0; c < K + TK; ++c)
+          if (!used[c] && (b < 0 || beats(fs[c], c, fs[b], b))) b = c;
+        used[b] = true;
+        f_src[k] = b;
+        f_score[k] = fs[b];
+        f_flag[k] = ff[b];
+        changed = changed || b != k;
+      }
+      // early-stop heuristic with t' = t + 1, then freezing
+      const double Lh = st.early_stopping == 2 && st.length_penalty > 0.f ? (double)(ML - 1) : (double)t;
+      const float best = n_rs[0] / (float)pow(Lh, (double)st.length_penalty);
+      float mn = f_score[0];
+      bool all_new = true;
+      for (int k = 0; k < K; ++k) { mn = fminf(mn, f_score[k]); all_new = all_new && f_flag[k]; }
+      bool any = false;
+      for (int k = 0; k < K; ++k) any = any || best > (f_flag[k] ? mn : -1e9f);
+      const bool unsat_new = unsat && any;
+      const bool frz = !unsat_new || (st.early_stopping == 1 && all_new);
+      st.sent_flags[i] = (unsat_new ? 0 : 1) | (frz ? 2 : 0);
+      if (frz) atomicAdd(st.frozen_count, 1);
+      s_changed = changed;
+    }
+  }
+  __syncthreads();
+  // a frozen sentence keeps its rows: each is its own parent and feeds pad_id from here on
+  for (int k = warp; k < K; k += 8) {
+    const int r = row0 + k;
+    const int par = frozen ? r : n_par[k];
+    const int tok = frozen ? st.pad_id : n_tok[k];
+    for (int j = lane; j <= t; j += 32) {
+      st.ids_next[(size_t)r * ML + j] = j < t ? st.ids_cur[(size_t)par * ML + j] : tok;
+      if (j < t) st.slot_next[(size_t)r * ML + j] = j < t - 1 ? st.slot_cur[(size_t)par * ML + j] : par * ML + t - 1;
+    }
+    if (lane == 0) {
+      st.parent[r] = par;
+      if (!frozen) st.run_score[r] = n_rs[k];
+    }
+  }
+  if (frozen || !s_changed) return;
+  for (int e = threadIdx.x; e < K * ML; e += blockDim.x) stage[e] = st.fin_ids[(size_t)row0 * ML + e];
+  __syncthreads();
+  for (int e = threadIdx.x; e < K * ML; e += blockDim.x) {
+    const int k = e / ML, j = e % ML, src = f_src[k];
+    int v;
+    if (src < K) v = stage[src * ML + j];
+    else {
+      const int c = src - K;
+      v = j < t ? st.ids_cur[(size_t)(row0 + s_beam[c]) * ML + j] : j == t ? s_tok[c] : st.pad_id;
+    }
+    st.fin_ids[(size_t)row0 * ML + e] = v;
+  }
+  // lengths before scores: the old values of moved slots are read here first
+  __shared__ int o_len[8];
+  if (threadIdx.x < K) o_len[threadIdx.x] = st.fin_len[row0 + threadIdx.x];
+  __syncthreads();
+  if (threadIdx.x < K) {
+    const int k = threadIdx.x, src = f_src[k];
+    st.fin_len[row0 + k] = src < K ? o_len[src] : t + 1;
+    st.fin_score[row0 + k] = f_score[k];
+    st.fin_flag[row0 + k] = f_flag[k];
+  }
+}
+
+__global__ void beam_output_kernel(BeamState st, int nr, int32_t* __restrict__ out_ids, int32_t* __restrict__ out_len,
+                                   float* __restrict__ out_score) {
+  const int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const int ML = st.max_len;
+  if (e >= (int64_t)st.n * nr * ML) return;
+  const int j = (int)(e % ML);
+  const int64_t h = e / ML;                          // sentence * nr + rank
+  const int64_t r = h / nr * st.K + h % nr;          // finished slot row
+  const int len = st.fin_len[r];
+  out_ids[e] = j < len ? st.fin_ids[r * ML + j] : st.pad_id;
+  if (j == 0) {
+    out_len[h] = len;
+    out_score[h] = st.fin_score[r];
+  }
+}
+
 __global__ void scale_copy_kernel(const float* __restrict__ src, float* __restrict__ dst, int64_t n, float scale) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     dst[i] = src[i] * scale;
@@ -247,7 +540,8 @@ int launch_dec_embed(const DecodeState& st, int pos, const float* word_scaled, c
 
 int launch_decode_attention(const void* q, int q_stride, const void* kv, int64_t kv_stride, const int32_t* key_start,
                             const int32_t* key_len, int self_t, int max_len, const void* new_kv, int new_kv_stride,
-                            void* kv_cache, void* ctx, int rows, int H, int max_keys, bool fp16, cudaStream_t s) {
+                            void* kv_cache, void* ctx, int rows, int H, int max_keys, bool fp16, cudaStream_t s,
+                            const int32_t* slot) {
   if (rows <= 0) return PLLB_OK;
   const int NH = H / 64;
   const int64_t items = (int64_t)rows * NH;
@@ -259,12 +553,24 @@ int launch_decode_attention(const void* q, int q_stride, const void* kv, int64_t
   auto* nk = reinterpret_cast<const uint16_t*>(new_kv);
   auto* kc = reinterpret_cast<uint16_t*>(kv_cache);
   auto* cc = reinterpret_cast<uint16_t*>(ctx);
-  if (fp16)
-    decode_attention_kernel<true><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len, self_t, max_len,
-                                                          nk, new_kv_stride, kc, cc, rows, H, NH, max_keys);
+  if (slot && key_start) return fail(PLLB_ERR_INVALID, "decode_attention: a slot table needs the self form");
+  if (slot) {
+    if (fp16)
+      decode_attention_kernel<true, true><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len, self_t,
+                                                                  max_len, nk, new_kv_stride, kc, cc, rows, H, NH, max_keys,
+                                                                  slot);
+    else
+      decode_attention_kernel<false, true><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len,
+                                                                   self_t, max_len, nk, new_kv_stride, kc, cc, rows, H, NH,
+                                                                   max_keys, slot);
+  } else if (fp16)
+    decode_attention_kernel<true, false><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len, self_t,
+                                                                 max_len, nk, new_kv_stride, kc, cc, rows, H, NH, max_keys,
+                                                                 nullptr);
   else
-    decode_attention_kernel<false><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len, self_t,
-                                                           max_len, nk, new_kv_stride, kc, cc, rows, H, NH, max_keys);
+    decode_attention_kernel<false, false><<<grid, 128, smem, s>>>(qq, q_stride, kk, kv_stride, key_start, key_len, self_t,
+                                                                  max_len, nk, new_kv_stride, kc, cc, rows, H, NH, max_keys,
+                                                                  nullptr);
   PLLB_LAUNCH_CHECK("decode_attention_kernel");
   return PLLB_OK;
 }
@@ -282,6 +588,33 @@ int launch_scale_copy(const float* src, float* dst, int64_t n, float scale, cuda
   const int64_t blocks = std::min<int64_t>(ceil_div(n, 256), 4096);
   scale_copy_kernel<<<(unsigned)blocks, 256, 0, s>>>(src, dst, n, scale);
   PLLB_LAUNCH_CHECK("scale_copy_kernel");
+  return PLLB_OK;
+}
+
+int launch_beam_init(BeamState st, cudaStream_t s) {
+  const int rows = std::max(st.n * st.K, 1);
+  beam_init_kernel<<<(unsigned)ceil_div(rows, 128), 128, 0, s>>>(st);
+  PLLB_LAUNCH_CHECK("beam_init_kernel");
+  return PLLB_OK;
+}
+
+int launch_beam_select(const float2* partials, int n_parts, int ksel, int vocab, BeamState st, int t, cudaStream_t s) {
+  if (st.n <= 0) return PLLB_OK;
+  if (st.K < 2 || 2 * st.K > ksel || st.K > 8) return fail(PLLB_ERR_INVALID, "beam_select: need 2 <= K <= 8, 2K <= ksel");
+  const size_t smem = sizeof(int32_t) * (size_t)st.K * st.max_len;
+  if (smem > 48 * 1024) return fail(PLLB_ERR_INVALID, "beam_select: num_beams * max_length > 12288");
+  if (ksel == 8) beam_select_kernel<8><<<st.n, 256, smem, s>>>(partials, n_parts, vocab, st, t);
+  else if (ksel == 16) beam_select_kernel<16><<<st.n, 256, smem, s>>>(partials, n_parts, vocab, st, t);
+  else return fail(PLLB_ERR_INVALID, "beam_select: ksel must be 8 or 16");
+  PLLB_LAUNCH_CHECK("beam_select_kernel");
+  return PLLB_OK;
+}
+
+int launch_beam_output(BeamState st, int r, int32_t* out_ids, int32_t* out_len, float* out_score, cudaStream_t s) {
+  const int64_t total = (int64_t)st.n * r * st.max_len;
+  if (total <= 0) return PLLB_OK;
+  beam_output_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(st, r, out_ids, out_len, out_score);
+  PLLB_LAUNCH_CHECK("beam_output_kernel");
   return PLLB_OK;
 }
 

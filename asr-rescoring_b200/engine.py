@@ -859,6 +859,51 @@ def generation_settings(cfg: dict, **overrides) -> dict:
     return g
 
 
+_EARLY_STOPPING = {False: 0, True: 1, "never": 2}
+
+
+def beam_settings(cfg: dict, **overrides) -> dict:
+    """generate()'s beam-search settings from a config dict (+ overrides), checked as pllb_generate_beam
+    checks them: num_beams in [2, 8] with vocab >= 2 * num_beams, num_return_sequences in [1, num_beams]
+    (default 1), a finite length_penalty (default 1.0) and early_stopping False / True / "never" (default
+    False); everything else as generation_settings checks it.  ValueError otherwise."""
+    g = {k: cfg.get(k) for k in _GEN_KEYS}
+    for k in ("do_sample", "no_repeat_ngram_size", "min_length", "repetition_penalty"):
+        if k in cfg:
+            g[k] = cfg[k]
+    for k, default in (("num_beams", None), ("num_return_sequences", 1), ("length_penalty", 1.0),
+                       ("early_stopping", False)):
+        g[k] = cfg.get(k, default) if cfg.get(k) is not None else default
+    g.update(overrides)
+    K = int(g.get("num_beams") or 1)
+    if not 2 <= K <= 8:
+        raise ValueError("num_beams must lie in [2, 8] for beam search")
+    if int(cfg["vocab_size"]) < 2 * K:
+        raise ValueError("beam search needs vocab_size >= 2 * num_beams")
+    r = int(g["num_return_sequences"] if g["num_return_sequences"] is not None else 1)
+    if not 1 <= r <= K:
+        raise ValueError("num_return_sequences must lie in [1, num_beams]")
+    lp = float(g["length_penalty"] if g["length_penalty"] is not None else 1.0)
+    if not np.isfinite(lp):
+        raise ValueError("length_penalty must be finite")
+    es = g["early_stopping"]
+    if not any(es is k or (isinstance(es, str) and es == k) for k in _EARLY_STOPPING):
+        raise ValueError('early_stopping must be False, True or "never"')
+    if K * int(g.get("max_length") or 20) > 12288:
+        raise ValueError("num_beams * max_length must not exceed 12288")
+    rest = generation_settings(cfg, **{k: v for k, v in g.items()
+                                       if k not in ("num_beams", "num_return_sequences", "length_penalty",
+                                                    "early_stopping")}, num_beams=1)
+    rest.update(num_beams=K, num_return_sequences=r, length_penalty=lp, early_stopping=es)
+    return rest
+
+
+def _beam_desc(g: dict) -> "_lib.BeamDesc":
+    es = g["early_stopping"]
+    code = 2 if isinstance(es, str) else int(bool(es))
+    return _lib.BeamDesc(int(g["num_return_sequences"]), float(g["length_penalty"]), code)
+
+
 def _gen_desc(g: dict) -> "_lib.GenDesc":
     rp = g.get("repetition_penalty")
     return _lib.GenDesc(int(g["max_length"]), int(g["decoder_start_token_id"]), int(g["eos_token_id"]),
@@ -946,6 +991,43 @@ class Seq2SeqGenerator(_Handle):
                                            _np_ptr(offsets), n, _np_ptr(ids), _np_ptr(lens),
                                            _np_ptr(lg) if lg is not None else None))
         return (ids, lens, lg) if return_logits else (ids, lens)
+
+    def beam_search_packed(self, tokens: np.ndarray, offsets: np.ndarray, settings: dict):
+        """Beam search (pllb_generate_beam_host) with ``beam_settings``.  HOST arrays in and out; returns
+        (ids int32[n, r, max_length], lengths int32[n, r], scores float32[n, r]), r = num_return_sequences,
+        hypotheses in descending score order."""
+        offsets = np.ascontiguousarray(offsets, np.int64)
+        tokens = np.ascontiguousarray(tokens, np.int32)
+        if offsets.ndim != 1 or len(offsets) < 1:
+            raise ValueError("offsets must be a 1-D array of n+1 entries")
+        n, ml, r = len(offsets) - 1, int(settings["max_length"]), int(settings["num_return_sequences"])
+        ids = np.zeros((n, r, ml), np.int32)
+        lens = np.zeros((n, r), np.int32)
+        scores = np.zeros((n, r), np.float32)
+        g, b = _gen_desc(settings), _beam_desc(settings)
+        check(self._lib.pllb_generate_beam_host(self._h, ctypes.byref(g), ctypes.byref(b),
+                                                _np_ptr(tokens) if len(tokens) else None, _np_ptr(offsets), n,
+                                                _np_ptr(ids), _np_ptr(lens), _np_ptr(scores)))
+        return ids, lens, scores
+
+    def debug_beam_replay(self, hidden: np.ndarray, settings: dict):
+        """Test hook (pllb_s2s_debug_beam_replay): the LM head and beam selection alone on given decoder
+        outputs hidden float32[max_length - 1, n * num_beams, d_model].  Returns (ids, lengths, scores) as
+        beam_search_packed plus parents int32[steps, n * K] and running scores float32[steps, n * K]."""
+        hidden = np.ascontiguousarray(hidden, np.float32)
+        steps, rows, _ = hidden.shape
+        K, ml, r = int(settings["num_beams"]), int(settings["max_length"]), int(settings["num_return_sequences"])
+        n = rows // K
+        ids = np.zeros((n, r, ml), np.int32)
+        lens = np.zeros((n, r), np.int32)
+        scores = np.zeros((n, r), np.float32)
+        par = np.zeros((steps, rows), np.int32)
+        rs = np.zeros((steps, rows), np.float32)
+        g, b = _gen_desc(settings), _beam_desc(settings)
+        check(self._lib.pllb_s2s_debug_beam_replay(self._h, ctypes.byref(g), ctypes.byref(b), n, _np_ptr(hidden), steps,
+                                                   _np_ptr(ids), _np_ptr(lens), _np_ptr(scores), _np_ptr(par),
+                                                   _np_ptr(rs)))
+        return ids, lens, scores, par, rs
 
     def set_timing(self, enable: bool):
         check(self._lib.pllb_s2s_set_timing(self._h, int(enable)))

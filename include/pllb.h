@@ -465,8 +465,8 @@ typedef struct pllb_s2s_weights {
 } pllb_s2s_weights;
 
 /* generate() settings.  Everything generate() would apply beyond greedy decoding is rejected with
- * PLLB_ERR_INVALID: num_beams != 1, do_sample != 0, no_repeat_ngram_size != 0, min_length != 0,
- * repetition_penalty != 1. */
+ * PLLB_ERR_INVALID: num_beams != 1 (beam search is pllb_generate_beam), do_sample != 0,
+ * no_repeat_ngram_size != 0, min_length != 0, repetition_penalty != 1. */
 typedef struct pllb_gen_desc {
   int32_t max_length;          /* 2 <= max_length <= dec_max_position                              */
   int32_t decoder_start_id, eos_id, pad_id;
@@ -516,6 +516,58 @@ int pllb_generate(pllb_s2s h, const pllb_gen_desc* gen, const int32_t* tokens, c
                   int32_t* out_ids, int32_t* out_len, float* out_logit, void* stream);
 int pllb_generate_host(pllb_s2s h, const pllb_gen_desc* gen, const int32_t* tokens, const int64_t* offsets, int32_t n,
                        int32_t* out_ids, int32_t* out_len, float* out_logit);
+
+/* ---- Beam search (DESIGN.md §3.12): generate(num_beams=K, do_sample=False) of transformers 5.5.0
+ * (GenerationMixin._beam_search) with one EOS id.  K = pllb_gen_desc.num_beams, 2 <= K <= 8,
+ * vocab >= 2K, K * max_length <= 12288; every other pllb_gen_desc field is checked as pllb_generate
+ * checks it.  t is the position being written (the start token is at 0), ML = max_length.
+ *  1. logp = log_softmax(fp32 logits) of each running beam, logits as greedy; forced BOS (t = 1) and
+ *     forced EOS (t = ML - 1, wins when both apply) set the forced id to 0 and every other id to -inf.
+ *  2. cand = logp + running_score[beam] (fp32); running scores start [0, -1e9, ...].  The step keeps
+ *     the top 2K of the K * V candidates of a sentence.
+ *  3. A candidate hits the stopping criteria when its token is eos_id or t = ML - 1.
+ *  4. The next running beams are the top K of cand + hit * -1e9 (fp32), each with its parent beam.
+ *  5. K finished slots per sentence start at score -1e9, not finished.  Candidate c of the 2K enters
+ *     with cand / (float)(t ** length_penalty), then -1e9 is added (fp32, in this order) when every
+ *     slot is finished and early_stopping is 1; when the early-stop heuristic is satisfied; and
+ *     unless c < K and c hit.  The new slots are the top K of [old slots ++ 2K candidates].
+ *  6. Early-stop heuristic, after the step: it stays unsatisfied only while it was unsatisfied and,
+ *     for some slot, best_running / L ** length_penalty > (slot finished ? min(slot scores) : -1e9),
+ *     with L = t (L = ML - 1 when early_stopping is 2 and length_penalty > 0).
+ *  7. A sentence is frozen once the heuristic is satisfied, or early_stopping is 1 and every slot is
+ *     finished; its slots cannot change from then on.  Decoding stops when every sentence is frozen
+ *     or position ML - 1 has been written.
+ *  8. The result is the best num_return_sequences slots in descending score order.
+ *  9. Ties: higher value first, then lower flat index (beam * V + token; slot before candidate).
+ * max_rows of pllb_s2s_create counts decoder rows (beams): a chunk holds max_rows / K sentences, and
+ * max_rows < K is PLLB_ERR_INVALID.  Results do not depend on max_rows.  The time of the selection
+ * kernel is part of pllb_s2s_stats.head_ms. */
+typedef struct pllb_beam_desc {
+  int32_t num_return_sequences;   /* 1 <= r <= num_beams                                             */
+  float   length_penalty;         /* finite                                                          */
+  int32_t early_stopping;         /* 0 False, 1 True, 2 "never"                                      */
+} pllb_beam_desc;
+
+/* tokens / offsets as pllb_generate.  Outputs (DEVICE):
+ * out_ids   int32[n * r * max_length]: hypothesis k of sentence i at [(i * r + k) * max_length, ...),
+ *           position 0 = start token, pad_id after the end;
+ * out_len   int32[n * r]: positions up to and including EOS, start included;
+ * out_score float[n * r]: the finished-slot score (sum of logp / (len - 1) ** length_penalty). */
+int pllb_generate_beam(pllb_s2s h, const pllb_gen_desc* gen, const pllb_beam_desc* beam, const int32_t* tokens,
+                       const int64_t* offsets, int32_t n, int32_t* out_ids, int32_t* out_len, float* out_score,
+                       void* stream);
+/* The same with HOST tokens and outputs; token ids are checked against the vocabulary. */
+int pllb_generate_beam_host(pllb_s2s h, const pllb_gen_desc* gen, const pllb_beam_desc* beam, const int32_t* tokens,
+                            const int64_t* offsets, int32_t n, int32_t* out_ids, int32_t* out_len, float* out_score);
+/* Test hook: the selection alone on given decoder outputs.  hidden HOST fp32 [steps = max_length - 1,
+ * n * K, hidden] (row i * K + b is beam b of sentence i at that step), rounded to the operand type and
+ * fed to the LM head with EPI_TOPK, beam_select_kernel and the bookkeeping; no decoder layers, and
+ * n * K <= max_rows.  HOST outputs as pllb_generate_beam_host, plus out_parent int32[steps, n * K]
+ * (chunk row of each running beam's parent) and out_run_score float[steps, n * K]; steps not run
+ * hold -1 / 0. */
+int pllb_s2s_debug_beam_replay(pllb_s2s h, const pllb_gen_desc* gen, const pllb_beam_desc* beam, int32_t n,
+                               const float* hidden, int32_t steps, int32_t* out_ids, int32_t* out_len,
+                               float* out_score, int32_t* out_parent, float* out_run_score);
 
 #ifdef __cplusplus
 }
