@@ -75,6 +75,12 @@ class S2sWeights(ctypes.Structure):
                 ("final_logits_bias", c_void_p)]
 
 
+class S2sTrainDesc(ctypes.Structure):
+    _fields_ = [("lr", c_float), ("beta1", c_float), ("beta2", c_float), ("adam_eps", c_float), ("weight_decay", c_float),
+                ("dropout", c_float), ("attention_dropout", c_float), ("seed", c_uint64), ("pad_id", c_int32),
+                ("decoder_start_id", c_int32), ("max_batch", c_int32), ("max_enc_len", c_int32), ("max_dec_len", c_int32)]
+
+
 class GenDesc(ctypes.Structure):
     _fields_ = [("max_length", c_int32), ("decoder_start_id", c_int32), ("eos_id", c_int32), ("pad_id", c_int32),
                 ("forced_bos_id", c_int32), ("forced_eos_id", c_int32), ("num_beams", c_int32), ("do_sample", c_int32),
@@ -159,6 +165,12 @@ SIGNATURES = {
                                         c_void_p, c_void_p, c_void_p]),
     "pllb_s2s_debug_beam_replay": (c_int, [c_void_p, POINTER(GenDesc), POINTER(BeamDesc), c_int32, c_void_p, c_int32,
                                            c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "pllb_s2s_train_create": (c_int, [POINTER(c_void_p), POINTER(S2sDesc), POINTER(S2sWeights), POINTER(S2sTrainDesc),
+                                      c_int]),
+    "pllb_s2s_train_step_host": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32,
+                                         POINTER(c_float)]),
+    "pllb_s2s_train_export": (c_int, [c_void_p, POINTER(S2sWeights)]),
+    "pllb_s2s_train_export_grads": (c_int, [c_void_p, POINTER(S2sWeights)]),
 }
 
 _lib = None

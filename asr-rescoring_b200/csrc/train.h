@@ -64,4 +64,33 @@ int launch_train_cls_loss(const float* scores, const float* target, const float*
 int launch_train_cls_bwd(const float* h, const float* w, const float* dscore, int B, int T, int H, float* dw, float* db,
                          float* dh, cudaStream_t s);
 
+// ---- BART fine-tuning (pllb_s2s_train_*)
+// out = [dropout](LN(word[ids] * scale + pos[r % T]))   (BART embeddings; pos = row 2 of embed_positions)
+int launch_train_bart_embed(const int32_t* ids, int T, const float* word, float scale, const float* pos, const float* g,
+                            const float* b, float eps, int R, int H, TrainDrop drop, uint32_t site, float* out32, void* out16,
+                            float* xhat, float* rstd, cudaStream_t s);
+// dpos[p] = sum_b dz[b*T + p] for p < pos_rows (0 past T); then dz *= scale (in place) and dword[id] += the
+// occurrences of id, pad_id excluded
+int launch_train_bart_embed_bwd(float* dz, const int32_t* ids, int B, int T, int H, int pos_rows, int pad_id, float scale,
+                                float* dword, float* dpos, cudaStream_t s);
+// One attention of B sequences: Tq bf16 query rows (q, row stride ldq) over Tk key / value rows (k, v, stride ldkv),
+// head h at columns h*64.  causal: Tq == Tk, query i sees keys <= i; otherwise keys < n_valid[seq] (DEVICE int32[B]).
+struct S2sAttn {
+  const void *q, *k, *v;
+  int ldq, ldkv;
+  int B, Tq, Tk, NH;
+  bool causal;
+  const int32_t* n_valid;
+};
+// ctx bf16 [B*Tq, NH*64], lse [B*Tq*NH]
+int launch_train_attn_s2s_fwd(const S2sAttn& a, TrainDrop drop, uint32_t site, void* ctx, float* lse, cudaStream_t s);
+// dq fp32 (row stride lddq), dk / dv fp32 (row stride lddkv); Dscratch [B*Tq*NH]
+int launch_train_attn_s2s_bwd(const S2sAttn& a, const float* dctx, const float* lse, TrainDrop drop, uint32_t site, float* dq,
+                              int lddq, float* dk, float* dv, int lddkv, float* Dscratch, cudaStream_t s);
+// cross entropy with ignore_index -100 (loss 0, zero dlogits row); out_loss2[0] = mean over the N labelled rows,
+// out_loss2[1] = 1 / N (fp32, DEVICE: read by launch_train_scale_dev)
+int launch_train_ce_ignore(const float* logits, const int32_t* labels, int R, int V, int Vp, float* loss_rows, void* dlogits,
+                           float* out_loss2, cudaStream_t s);
+int launch_train_scale_dev(float* x, int64_t n, const float* alpha, cudaStream_t s);
+
 }  // namespace pllb

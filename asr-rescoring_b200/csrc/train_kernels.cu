@@ -786,4 +786,360 @@ int launch_train_cls_bwd(const float* h, const float* w, const float* dscore, in
   return PLLB_OK;
 }
 
+// ================================================================== BART fine-tuning (pllb_s2s_train_*)
+namespace {
+
+// out = [dropout](LN(shared[id] * scale + pos[r % T]))   (BART embeddings; pos already points at row 2 of the table)
+template <int NV>
+__global__ void __launch_bounds__(RW * 32)
+bart_embed_kernel(const int32_t* __restrict__ ids, int T, const float* __restrict__ word, float scale,
+                  const float* __restrict__ pos, const float* __restrict__ g, const float* __restrict__ b, float eps, int R,
+                  TrainDrop drop, uint32_t site, float* __restrict__ out32, __nv_bfloat16* __restrict__ out16,
+                  float* __restrict__ xhat, float* __restrict__ rstd) {
+  constexpr int H = NV * 32;
+  const int r = blockIdx.x * RW + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (r >= R) return;
+  const int id = ids[r], p = r % T;
+  float v[NV];
+  float s = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = lane + 32 * i;
+    v[i] = word[(size_t)id * H + c] * scale + pos[(size_t)p * H + c];
+    s += v[i];
+  }
+  const float mean = wsum(s) * (1.f / H);
+  float q = 0.f;
+#pragma unroll
+  for (int i = 0; i < NV; ++i) { const float d = v[i] - mean; q += d * d; }
+  const float rs = rsqrtf(wsum(q) * (1.f / H) + eps);
+#pragma unroll
+  for (int i = 0; i < NV; ++i) {
+    const int c = lane + 32 * i;
+    const size_t e = (size_t)r * H + c;
+    const float xh = (v[i] - mean) * rs;
+    const float o = (xh * g[c] + b[c]) * drop_factor(drop, site, e);
+    xhat[e] = xh;
+    out32[e] = o;
+    out16[e] = __float2bfloat16_rn(o);
+  }
+  if (lane == 0) rstd[r] = rs;
+}
+
+// Attention of B sequences whose Tq query rows (q, row stride ldq) attend to Tk key / value rows of the same
+// sequence (k, v, row stride ldkv), warp per (query row, head).  CAUSAL: Tq == Tk and query i sees keys <= i
+// (the decoder's self-attention); otherwise the keys < n_valid[seq] (cross-attention over the encoder rows).
+__device__ __forceinline__ int s2s_key_limit(bool causal, int i, const int32_t* n_valid, int seq) {
+  return causal ? i + 1 : n_valid[seq];
+}
+
+template <bool CAUSAL>
+__global__ void __launch_bounds__(RW * 32, 8)     // without the occupancy hint ptxas spills 4 bytes in the cross form
+attn_fwd_s2s_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
+                    const __nv_bfloat16* __restrict__ v, int ldq, int ldkv, const int32_t* __restrict__ n_valid, int Rq,
+                    int Tq, int Tk, int NH, TrainDrop drop, uint32_t site, __nv_bfloat16* __restrict__ ctx,
+                    float* __restrict__ lse_out) {
+  extern __shared__ float smem[];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int item = blockIdx.x * RW + w;
+  if (item >= Rq * NH) return;
+  const int r = item / NH, h = item % NH, seq = r / Tq, i = r % Tq, H = NH * 64;
+  const int nk = s2s_key_limit(CAUSAL, i, n_valid, seq);
+  float* sq = smem + (size_t)w * (64 + Tk);
+  float* sp = sq + 64;
+  const __nv_bfloat16* kb = k + (size_t)seq * Tk * ldkv + h * 64;
+  const __nv_bfloat16* vb = v + (size_t)seq * Tk * ldkv + h * 64;
+  {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(q + (size_t)r * ldq + h * 64 + 2 * lane));
+    sq[2 * lane] = f.x; sq[2 * lane + 1] = f.y;
+  }
+  __syncwarp();
+  float m = -INFINITY;
+  for (int j = lane; j < nk; j += 32) {
+    const float s = dot64_bf16(sq, kb + (size_t)j * ldkv) * 0.125f;
+    sp[j] = s;
+    m = fmaxf(m, s);
+  }
+  m = wmax(m);
+  float l = 0.f;
+  for (int j = lane; j < nk; j += 32) l += __expf(sp[j] - m);
+  const float lse = m + __logf(wsum(l));
+  const uint64_t pbase = ((uint64_t)(seq * NH + h) * Tq + i) * Tk;
+  for (int j = lane; j < nk; j += 32) sp[j] = __expf(sp[j] - lse) * drop_factor(drop, site, pbase + j);
+  __syncwarp();
+  float a0 = 0.f, a1 = 0.f;
+#pragma unroll 4
+  for (int j = 0; j < nk; ++j) {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(vb + (size_t)j * ldkv + 2 * lane));
+    a0 += sp[j] * f.x; a1 += sp[j] * f.y;
+  }
+  *reinterpret_cast<__nv_bfloat162*>(ctx + (size_t)r * H + h * 64 + 2 * lane) = __floats2bfloat162_rn(a0, a1);
+  if (lane == 0) lse_out[item] = lse;
+}
+
+// dq of query row r (fp32, row stride lddq) and D_r = sum_j P_rj dP_rj for the dk / dv pass
+template <bool CAUSAL>
+__global__ void __launch_bounds__(RW * 32)
+attn_bwd_q_s2s_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
+                      const __nv_bfloat16* __restrict__ v, int ldq, int ldkv, const float* __restrict__ dctx,
+                      const float* __restrict__ lse, const int32_t* __restrict__ n_valid, int Rq, int Tq, int Tk, int NH,
+                      TrainDrop drop, uint32_t site, float* __restrict__ dq, int lddq, float* __restrict__ Dout) {
+  extern __shared__ float smem[];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int item = blockIdx.x * RW + w;
+  if (item >= Rq * NH) return;
+  const int r = item / NH, h = item % NH, seq = r / Tq, i = r % Tq, H = NH * 64;
+  const int nk = s2s_key_limit(CAUSAL, i, n_valid, seq);
+  float* sq = smem + (size_t)w * (128 + 2 * Tk);
+  float* sdo = sq + 64;
+  float* sp = sdo + 64;
+  float* sds = sp + Tk;
+  const __nv_bfloat16* kb = k + (size_t)seq * Tk * ldkv + h * 64;
+  const __nv_bfloat16* vb = v + (size_t)seq * Tk * ldkv + h * 64;
+  {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(q + (size_t)r * ldq + h * 64 + 2 * lane));
+    sq[2 * lane] = f.x; sq[2 * lane + 1] = f.y;
+    const float2 g = *reinterpret_cast<const float2*>(dctx + (size_t)r * H + h * 64 + 2 * lane);
+    sdo[2 * lane] = g.x; sdo[2 * lane + 1] = g.y;
+  }
+  __syncwarp();
+  const float ls = lse[item];
+  const uint64_t pbase = ((uint64_t)(seq * NH + h) * Tq + i) * Tk;
+  float dpart = 0.f;
+  for (int j = lane; j < nk; j += 32) {
+    const float p = __expf(dot64_bf16(sq, kb + (size_t)j * ldkv) * 0.125f - ls);
+    const float dp = dot64_bf16(sdo, vb + (size_t)j * ldkv) * drop_factor(drop, site, pbase + j);
+    sp[j] = p; sds[j] = dp;
+    dpart += p * dp;
+  }
+  const float D = wsum(dpart);
+  for (int j = lane; j < nk; j += 32) sds[j] = sp[j] * (sds[j] - D);
+  __syncwarp();
+  float a0 = 0.f, a1 = 0.f;
+#pragma unroll 4
+  for (int j = 0; j < nk; ++j) {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(kb + (size_t)j * ldkv + 2 * lane));
+    a0 += sds[j] * f.x; a1 += sds[j] * f.y;
+  }
+  *reinterpret_cast<float2*>(dq + (size_t)r * lddq + h * 64 + 2 * lane) = make_float2(a0 * 0.125f, a1 * 0.125f);
+  if (lane == 0) Dout[item] = D;
+}
+
+// dk and dv of key row rk (fp32, row stride lddkv): sums over the queries that see it, in query order (CAUSAL: i >= j;
+// cross: all Tq decoder rows of the sentence).  A masked key gets zero.
+template <bool CAUSAL>
+__global__ void __launch_bounds__(RW * 32)
+attn_bwd_kv_s2s_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
+                       const __nv_bfloat16* __restrict__ v, int ldq, int ldkv, const float* __restrict__ dctx,
+                       const float* __restrict__ lse, const float* __restrict__ Dq, const int32_t* __restrict__ n_valid,
+                       int Rk, int Tq, int Tk, int NH, TrainDrop drop, uint32_t site, float* __restrict__ dk,
+                       float* __restrict__ dv, int lddkv) {
+  extern __shared__ float smem[];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int item = blockIdx.x * RW + w;
+  if (item >= Rk * NH) return;
+  const int rk = item / NH, h = item % NH, seq = rk / Tk, j = rk % Tk, H = NH * 64;
+  float2* dk_out = reinterpret_cast<float2*>(dk + (size_t)rk * lddkv + h * 64 + 2 * lane);
+  float2* dv_out = reinterpret_cast<float2*>(dv + (size_t)rk * lddkv + h * 64 + 2 * lane);
+  if (!CAUSAL && j >= n_valid[seq]) {
+    *dk_out = make_float2(0.f, 0.f);
+    *dv_out = make_float2(0.f, 0.f);
+    return;
+  }
+  const int i0 = CAUSAL ? j : 0;
+  float* sk = smem + (size_t)w * (128 + 2 * Tq);
+  float* sv = sk + 64;
+  float* sds = sv + 64;
+  float* spd = sds + Tq;
+  const __nv_bfloat16* qb = q + (size_t)seq * Tq * ldq + h * 64;
+  {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(k + (size_t)rk * ldkv + h * 64 + 2 * lane));
+    sk[2 * lane] = f.x; sk[2 * lane + 1] = f.y;
+    const float2 g = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(v + (size_t)rk * ldkv + h * 64 + 2 * lane));
+    sv[2 * lane] = g.x; sv[2 * lane + 1] = g.y;
+  }
+  __syncwarp();
+  for (int i = i0 + lane; i < Tq; i += 32) {
+    const int ri = seq * Tq + i;
+    const float p = __expf(dot64_bf16(sk, qb + (size_t)i * ldq) * 0.125f - lse[(size_t)ri * NH + h]);
+    const float sc = drop_factor(drop, site, ((uint64_t)(seq * NH + h) * Tq + i) * Tk + j);
+    const float dp = dot64_f32(sv, dctx + (size_t)ri * H + h * 64) * sc;
+    sds[i] = p * (dp - Dq[(size_t)ri * NH + h]);
+    spd[i] = p * sc;
+  }
+  __syncwarp();
+  float k0 = 0.f, k1 = 0.f, v0 = 0.f, v1 = 0.f;
+#pragma unroll 4
+  for (int i = i0; i < Tq; ++i) {
+    const int ri = seq * Tq + i;
+    const float2 qq = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(qb + (size_t)i * ldq + 2 * lane));
+    const float2 g = *reinterpret_cast<const float2*>(dctx + (size_t)ri * H + h * 64 + 2 * lane);
+    k0 += sds[i] * qq.x; k1 += sds[i] * qq.y;
+    v0 += spd[i] * g.x; v1 += spd[i] * g.y;
+  }
+  *dk_out = make_float2(k0 * 0.125f, k1 * 0.125f);
+  *dv_out = make_float2(v0, v1);
+}
+
+// Cross entropy with ignore_index -100: as ce_kernel on a row whose label is in [0, V); an ignored row has loss 0
+// and a zero dlogits row (bf16, unscaled: the 1/N of the mean is applied in fp32 by the consumers).
+__global__ void __launch_bounds__(256)
+ce_ignore_kernel(const float* __restrict__ logits, const int32_t* __restrict__ labels, int V, int Vp,
+                 float* __restrict__ loss_rows, __nv_bfloat16* __restrict__ dlogits) {
+  __shared__ float red[8];
+  __shared__ float bc;
+  const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const int label = labels[r];
+  if (label < 0) {
+    if (tid == 0) loss_rows[r] = 0.f;
+    if (dlogits)
+      for (int c = tid; c < Vp; c += 256) dlogits[(size_t)r * Vp + c] = __float2bfloat16_rn(0.f);
+    return;
+  }
+  const float* x = logits + (size_t)r * Vp;
+  float m = -INFINITY;
+  for (int c = tid; c < V; c += 256) m = fmaxf(m, x[c]);
+  m = wmax(m);
+  if (lane == 0) red[w] = m;
+  __syncthreads();
+  if (tid == 0) { float t = red[0]; for (int k = 1; k < 8; ++k) t = fmaxf(t, red[k]); bc = t; }
+  __syncthreads();
+  m = bc;
+  float s = 0.f;
+  for (int c = tid; c < V; c += 256) s += __expf(x[c] - m);
+  s = wsum(s);
+  __syncthreads();
+  if (lane == 0) red[w] = s;
+  __syncthreads();
+  if (tid == 0) { float t = 0.f; for (int k = 0; k < 8; ++k) t += red[k]; bc = m + logf(t); }
+  __syncthreads();
+  const float lse = bc;
+  if (tid == 0) loss_rows[r] = lse - x[label];
+  if (dlogits) {
+    __nv_bfloat16* d = dlogits + (size_t)r * Vp;
+    for (int c = tid; c < Vp; c += 256) {
+      float g = 0.f;
+      if (c < V) g = __expf(x[c] - lse) - (c == label ? 1.f : 0.f);
+      d[c] = __float2bfloat16_rn(g);
+    }
+  }
+}
+
+// out[0] = the mean of the per-row losses over the N rows with a label (fixed order, double accumulation);
+// out[1] = 1 / N in fp32, the factor the backward pass applies.  Single block; N >= 1 is checked on the host.
+__global__ void __launch_bounds__(256)
+loss_mean_valid_kernel(const float* __restrict__ loss_rows, const int32_t* __restrict__ labels, int R, float* __restrict__ out) {
+  __shared__ double red[256];
+  __shared__ int cnt[256];
+  double a = 0.0;
+  int n = 0;
+  for (int r = threadIdx.x; r < R; r += 256)
+    if (labels[r] >= 0) { a += (double)loss_rows[r]; ++n; }
+  red[threadIdx.x] = a;
+  cnt[threadIdx.x] = n;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) { red[threadIdx.x] += red[threadIdx.x + o]; cnt[threadIdx.x] += cnt[threadIdx.x + o]; }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    out[0] = (float)(red[0] / (double)cnt[0]);
+    out[1] = 1.f / (float)cnt[0];
+  }
+}
+
+// x *= alpha[0], alpha read from device memory (the 1 / N of a batch inside a captured graph)
+__global__ void scale_dev_kernel(float* __restrict__ x, int64_t n, const float* __restrict__ alpha) {
+  const float a = *alpha;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) x[i] *= a;
+}
+
+}  // namespace
+
+int launch_train_bart_embed(const int32_t* ids, int T, const float* word, float scale, const float* pos, const float* g,
+                            const float* b, float eps, int R, int H, TrainDrop drop, uint32_t site, float* out32, void* out16,
+                            float* xhat, float* rstd, cudaStream_t s) {
+  if (R <= 0) return PLLB_OK;
+  const int grid = (int)ceil_div(R, RW);
+  DISPATCH_NV(H, bart_embed_kernel<NV><<<grid, RW * 32, 0, s>>>(ids, T, word, scale, pos, g, b, eps, R, drop, site, out32,
+                                                               reinterpret_cast<__nv_bfloat16*>(out16), xhat, rstd));
+  PLLB_LAUNCH_CHECK("bart_embed_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_bart_embed_bwd(float* dz, const int32_t* ids, int B, int T, int H, int pos_rows, int pad_id, float scale,
+                                float* dword, float* dpos, cudaStream_t s) {
+  const int R = B * T;
+  if (R <= 0) return PLLB_OK;
+  pos_grad_kernel<<<grid_for((int64_t)pos_rows * H, 256), 256, 0, s>>>(dz, B, T, H, pos_rows, dpos);
+  PLLB_LAUNCH_CHECK("pos_grad_kernel");
+  if (scale != 1.f) {           // the lookup is shared[id] * scale: each occurrence sends dz * scale
+    scale_kernel<<<grid_for((int64_t)R * H, 256), 256, 0, s>>>(dz, (int64_t)R * H, scale);
+    PLLB_LAUNCH_CHECK("scale_kernel");
+  }
+  word_grad_kernel<<<R, 256, 0, s>>>(dz, ids, R, H, pad_id, dword);
+  PLLB_LAUNCH_CHECK("word_grad_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_attn_s2s_fwd(const S2sAttn& a, TrainDrop drop, uint32_t site, void* ctx, float* lse, cudaStream_t s) {
+  const int Rq = a.B * a.Tq;
+  if (Rq <= 0) return PLLB_OK;
+  const size_t smem = sizeof(float) * RW * (64 + (size_t)a.Tk);
+  const int grid = (int)ceil_div((int64_t)Rq * a.NH, RW);
+  const auto* q = reinterpret_cast<const __nv_bfloat16*>(a.q);
+  const auto* k = reinterpret_cast<const __nv_bfloat16*>(a.k);
+  const auto* v = reinterpret_cast<const __nv_bfloat16*>(a.v);
+  auto* c16 = reinterpret_cast<__nv_bfloat16*>(ctx);
+  if (a.causal)
+    attn_fwd_s2s_kernel<true><<<grid, RW * 32, smem, s>>>(q, k, v, a.ldq, a.ldkv, a.n_valid, Rq, a.Tq, a.Tk, a.NH, drop, site, c16, lse);
+  else
+    attn_fwd_s2s_kernel<false><<<grid, RW * 32, smem, s>>>(q, k, v, a.ldq, a.ldkv, a.n_valid, Rq, a.Tq, a.Tk, a.NH, drop, site, c16, lse);
+  PLLB_LAUNCH_CHECK("attn_fwd_s2s_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_attn_s2s_bwd(const S2sAttn& a, const float* dctx, const float* lse, TrainDrop drop, uint32_t site, float* dq,
+                              int lddq, float* dk, float* dv, int lddkv, float* Dscratch, cudaStream_t s) {
+  const int Rq = a.B * a.Tq, Rk = a.B * a.Tk;
+  if (Rq <= 0) return PLLB_OK;
+  const auto* q = reinterpret_cast<const __nv_bfloat16*>(a.q);
+  const auto* k = reinterpret_cast<const __nv_bfloat16*>(a.k);
+  const auto* v = reinterpret_cast<const __nv_bfloat16*>(a.v);
+  const size_t smem_q = sizeof(float) * RW * (128 + 2 * (size_t)a.Tk), smem_kv = sizeof(float) * RW * (128 + 2 * (size_t)a.Tq);
+  const int grid_q = (int)ceil_div((int64_t)Rq * a.NH, RW), grid_kv = (int)ceil_div((int64_t)Rk * a.NH, RW);
+  if (a.causal)
+    attn_bwd_q_s2s_kernel<true><<<grid_q, RW * 32, smem_q, s>>>(q, k, v, a.ldq, a.ldkv, dctx, lse, a.n_valid, Rq, a.Tq, a.Tk,
+                                                               a.NH, drop, site, dq, lddq, Dscratch);
+  else
+    attn_bwd_q_s2s_kernel<false><<<grid_q, RW * 32, smem_q, s>>>(q, k, v, a.ldq, a.ldkv, dctx, lse, a.n_valid, Rq, a.Tq, a.Tk,
+                                                                a.NH, drop, site, dq, lddq, Dscratch);
+  PLLB_LAUNCH_CHECK("attn_bwd_q_s2s_kernel");
+  if (a.causal)
+    attn_bwd_kv_s2s_kernel<true><<<grid_kv, RW * 32, smem_kv, s>>>(q, k, v, a.ldq, a.ldkv, dctx, lse, Dscratch, a.n_valid, Rk,
+                                                                  a.Tq, a.Tk, a.NH, drop, site, dk, dv, lddkv);
+  else
+    attn_bwd_kv_s2s_kernel<false><<<grid_kv, RW * 32, smem_kv, s>>>(q, k, v, a.ldq, a.ldkv, dctx, lse, Dscratch, a.n_valid, Rk,
+                                                                   a.Tq, a.Tk, a.NH, drop, site, dk, dv, lddkv);
+  PLLB_LAUNCH_CHECK("attn_bwd_kv_s2s_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_ce_ignore(const float* logits, const int32_t* labels, int R, int V, int Vp, float* loss_rows, void* dlogits,
+                           float* out_loss2, cudaStream_t s) {
+  if (R <= 0) return PLLB_OK;
+  ce_ignore_kernel<<<R, 256, 0, s>>>(logits, labels, V, Vp, loss_rows, reinterpret_cast<__nv_bfloat16*>(dlogits));
+  PLLB_LAUNCH_CHECK("ce_ignore_kernel");
+  loss_mean_valid_kernel<<<1, 256, 0, s>>>(loss_rows, labels, R, out_loss2);
+  PLLB_LAUNCH_CHECK("loss_mean_valid_kernel");
+  return PLLB_OK;
+}
+
+int launch_train_scale_dev(float* x, int64_t n, const float* alpha, cudaStream_t s) {
+  if (n <= 0) return PLLB_OK;
+  scale_dev_kernel<<<grid_for(n, 256), 256, 0, s>>>(x, n, alpha);
+  PLLB_LAUNCH_CHECK("scale_dev_kernel");
+  return PLLB_OK;
+}
+
 }  // namespace pllb

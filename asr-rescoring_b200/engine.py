@@ -821,6 +821,39 @@ def check_bart_config(cfg: dict) -> dict:
                 embed_scale=float(np.sqrt(H)) if cfg.get("scale_embedding", False) else 1.0)
 
 
+def s2s_weights_struct(get, cfg: dict, pos_skip_rows: int):
+    """pllb_s2s_weights over the device fp32 tensors ``get(key)`` returns for the BART state_dict names; the two
+    position tables start ``pos_skip_rows`` rows in (2 for pllb_s2s_create, 0 for pllb_s2s_train_create).  Returns
+    (struct, list keeping the tensors and the layer arrays alive)."""
+    from ._lib import DecLayerWeights, S2sWeights
+    s = check_bart_config(cfg)
+    keep = []
+
+    def dp(key, skip_rows: int = 0):
+        t = get(key)[skip_rows:].contiguous()
+        keep.append(t)
+        return ctypes.c_void_p(t.data_ptr())
+
+    enc_layers = (LayerWeights * s["enc_layers"])()
+    dec_layers = (DecLayerWeights * s["dec_layers"])()
+    keep += [enc_layers, dec_layers]
+    for (kind, *rest), key in bart_weight_keys(cfg).items():
+        if kind == "enc":
+            setattr(enc_layers[rest[0]], rest[1], dp(key))
+        elif kind == "dec":
+            setattr(dec_layers[rest[0]], rest[1], dp(key))
+    w = S2sWeights()
+    w.enc.pos_emb = dp(_BART_TOP["enc_pos"], pos_skip_rows)
+    w.enc.emb_ln_g, w.enc.emb_ln_b = dp(_BART_TOP["enc_ln_g"]), dp(_BART_TOP["enc_ln_b"])
+    w.enc.layers = ctypes.cast(enc_layers, ctypes.POINTER(LayerWeights))
+    w.dec_layers = ctypes.cast(dec_layers, ctypes.POINTER(DecLayerWeights))
+    w.shared = dp(_BART_TOP["shared"])
+    w.dec_pos_emb = dp(_BART_TOP["dec_pos"], pos_skip_rows)
+    w.dec_emb_ln_g, w.dec_emb_ln_b = dp(_BART_TOP["dec_ln_g"]), dp(_BART_TOP["dec_ln_b"])
+    w.final_logits_bias = dp("final_logits_bias")                     # [1, vocab] or [vocab]
+    return w, keep
+
+
 _GEN_KEYS = ("max_length", "decoder_start_token_id", "eos_token_id", "pad_token_id", "forced_bos_token_id",
              "forced_eos_token_id")
 
@@ -922,7 +955,7 @@ class Seq2SeqGenerator(_Handle):
     def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: dict, device: int = 0, max_rows: int = 0,
                  operand_dtype: str = "bf16", cls_id: int = 101, sep_id: int = 102):
         import torch
-        from ._lib import DecLayerWeights, S2sDesc, S2sWeights
+        from ._lib import S2sDesc
 
         self._lib = _lib.load()
         _lib.require_device()
@@ -934,38 +967,15 @@ class Seq2SeqGenerator(_Handle):
         self.operand_dtype = operand_dtype
         sd = bart_state_dict(state_dict)
         dev = torch.device("cuda", device)
-        keep = []
-
-        def dp(key, skip_rows: int = 0):
-            t = sd[key].detach().to(device=dev, dtype=torch.float32)[skip_rows:].contiguous()
-            keep.append(t)
-            return ctypes.c_void_p(t.data_ptr())
-
         s = self.shape
         H = s["hidden"]
-        keys = bart_weight_keys(self.cfg)
-        enc_layers = (LayerWeights * s["enc_layers"])()
-        dec_layers = (DecLayerWeights * s["dec_layers"])()
-        keep += [enc_layers, dec_layers]
-        for (kind, *rest), key in keys.items():
-            if kind == "enc":
-                setattr(enc_layers[rest[0]], rest[1], dp(key))
-            elif kind == "dec":
-                setattr(dec_layers[rest[0]], rest[1], dp(key))
-        w = S2sWeights()
-        w.enc.pos_emb = dp(_BART_TOP["enc_pos"], skip_rows=2)       # BartLearnedPositionalEmbedding's offset of 2
-        w.enc.emb_ln_g, w.enc.emb_ln_b = dp(_BART_TOP["enc_ln_g"]), dp(_BART_TOP["enc_ln_b"])
-        w.enc.layers = ctypes.cast(enc_layers, ctypes.POINTER(LayerWeights))
-        w.dec_layers = ctypes.cast(dec_layers, ctypes.POINTER(DecLayerWeights))
-        w.shared = dp(_BART_TOP["shared"])
-        w.dec_pos_emb = dp(_BART_TOP["dec_pos"], skip_rows=2)
-        w.dec_emb_ln_g, w.dec_emb_ln_b = dp(_BART_TOP["dec_ln_g"]), dp(_BART_TOP["dec_ln_b"])
-        if "final_logits_bias" in sd:
-            w.final_logits_bias = dp("final_logits_bias")             # [1, vocab]
-        else:                                                         # a missing buffer loads as zeros in HF
-            z = torch.zeros(s["vocab"], dtype=torch.float32, device=dev)
-            keep.append(z)
-            w.final_logits_bias = ctypes.c_void_p(z.data_ptr())
+
+        def get(key):
+            if key not in sd:                                         # final_logits_bias: a missing buffer loads as zeros
+                return torch.zeros(s["vocab"], dtype=torch.float32, device=dev)
+            return sd[key].detach().to(device=dev, dtype=torch.float32)
+
+        w, keep = s2s_weights_struct(get, self.cfg, pos_skip_rows=2)  # BartLearnedPositionalEmbedding's offset of 2
         d = S2sDesc(s["enc_layers"], s["dec_layers"], H, s["num_heads"], s["enc_intermediate"], s["dec_intermediate"],
                     s["vocab"], s["max_position"], s["max_position"],
                     1e-5, s["embed_scale"], cls_id, sep_id, 0 if operand_dtype == "bf16" else 1)
@@ -1041,3 +1051,137 @@ class Seq2SeqGenerator(_Handle):
         d = {n: getattr(s, n) for n, _ in _lib.S2sStats._fields_}
         d["workspace_bytes"] = int(self._lib.pllb_s2s_workspace_bytes(self._h))
         return d
+
+
+def shift_tokens_right(labels, pad_id: int, decoder_start_id: int) -> np.ndarray:
+    """The decoder input pllb_s2s_train_step_host builds from labels [B, T_dec] (transformers'
+    ``shift_tokens_right``): the start id at position 0, the labels shifted right by one, -100 -> pad_id."""
+    lab = np.asarray(labels)
+    out = np.empty(lab.shape, np.int64)
+    out[:, 0] = decoder_start_id
+    out[:, 1:] = lab[:, :-1]
+    out[out == -100] = pad_id
+    return out
+
+
+class Seq2SeqTrainer(_Trainer):
+    """CorrectBart fine-tuning on the device (pllb_s2s_train_*; include/pllb.h and DESIGN.md §3.13 state the
+    contract): ``BartForConditionalGeneration.forward(input_ids, attention_mask, labels=labels)`` in train mode,
+    ``loss.backward()`` and ``torch.optim.AdamW`` over ``model.parameters()``.  fp32 master weights, bf16 GEMM
+    operands, fp32 accumulation.  ``dropout`` / ``attention_dropout`` default to the config's; the masks come from
+    a stateless hash, so only runs with dropout 0 are comparable value by value with torch.
+
+    ``state_dict``: a BartForConditionalGeneration state_dict (one wrapper prefix allowed, as
+    :class:`Seq2SeqGenerator` takes it); ``cfg`` its BartConfig dict.  ``max_batch`` / ``max_enc_len`` /
+    ``max_dec_len`` bound the batches :meth:`step` takes."""
+
+    def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: dict, device: int = 0, lr: float = 1e-5,
+                 dropout: Optional[float] = None, attention_dropout: Optional[float] = None, seed: int = 0,
+                 max_batch: int = 64, max_enc_len: int = 128, max_dec_len: int = 128, betas=(0.9, 0.999),
+                 eps: float = 1e-8, weight_decay: float = 0.01, operand_dtype: str = "bf16"):
+        import torch
+        from ._lib import S2sDesc, S2sTrainDesc
+
+        self.cfg = dict(cfg)
+        self.shape = check_bart_config(self.cfg)
+        if float(self.cfg.get("activation_dropout") or 0.0) != 0.0:
+            raise ValueError("activation_dropout != 0 is not supported (bart-base's default is 0)")
+        if operand_dtype != "bf16":
+            raise ValueError("training takes bf16 GEMM operands only (no fp16 training)")
+        sd = bart_state_dict(state_dict)
+        # the handle is created here, not by _Trainer.__init__ (which builds the BERT descriptors)
+        self._lib = _lib.load()
+        _lib.require_device()
+        self._h = ctypes.c_void_p()
+        self.device = device
+        self._dev = torch.device("cuda", device)
+        self._keys = list(state_dict.keys())
+        # bart_state_dict located exactly one model.shared.weight; its prefix maps the given keys to sd's
+        self._prefix = next(k for k in state_dict if k == "model.shared.weight" or k.endswith(".model.shared.weight"))[
+            :-len("model.shared.weight")]
+        self._given = {k: v for k, v in state_dict.items()}
+        self._shapes = {k: tuple(v.shape) for k, v in sd.items()}
+        self.pad_id = int(self.cfg.get("pad_token_id", 0) if self.cfg.get("pad_token_id") is not None else 0)
+        self.decoder_start_id = int(self.cfg["decoder_start_token_id"])
+        s = self.shape
+        if "final_logits_bias" not in sd:                              # a missing buffer loads as zeros in HF
+            sd["final_logits_bias"] = torch.zeros(1, s["vocab"])
+            self._shapes["final_logits_bias"] = (1, s["vocab"])
+        w, keep = s2s_weights_struct(lambda k: self._to_dev(sd[k]), self.cfg, pos_skip_rows=0)
+        self._desc = S2sDesc(s["enc_layers"], s["dec_layers"], s["hidden"], s["num_heads"], s["enc_intermediate"],
+                             s["dec_intermediate"], s["vocab"], s["max_position"], s["max_position"], 1e-5,
+                             s["embed_scale"], 101, 102, 0)
+        drop = float(self.cfg.get("dropout", 0.1) if dropout is None else dropout)
+        adrop = float(self.cfg.get("attention_dropout", 0.0) if attention_dropout is None else attention_dropout)
+        self.max_batch, self.max_enc_len, self.max_dec_len = int(max_batch), int(max_enc_len), int(max_dec_len)
+        self._train_desc = S2sTrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), drop,
+                                        adrop, int(seed) & (2 ** 64 - 1), self.pad_id, self.decoder_start_id,
+                                        self.max_batch, self.max_enc_len, self.max_dec_len)
+        torch.cuda.synchronize(self._dev)
+        check(self._lib.pllb_s2s_train_create(ctypes.byref(self._h), ctypes.byref(self._desc), ctypes.byref(w),
+                                              ctypes.byref(self._train_desc), device))
+        del keep
+        self._last_shape = None
+
+    def step(self, input_ids, attention_mask, labels, mode: int = 1) -> float:
+        """One batch: input_ids / attention_mask int [B, T_enc] ([CLS] hyp [SEP], right-padded, prefix masks),
+        labels int [B, T_dec] (-100 = ignored).  mode 1: forward + backward + AdamW step; 0: loss only (eval);
+        2: forward + backward without the update.  Returns the loss."""
+        ids = np.ascontiguousarray(input_ids, np.int32)
+        lab = np.ascontiguousarray(labels, np.int32)
+        if ids.ndim != 2 or lab.ndim != 2 or lab.shape[0] != ids.shape[0]:
+            raise ValueError("input_ids [B, T_enc] and labels [B, T_dec] must be 2-D with the same B")
+        nv = _prefix_lengths(attention_mask, ids.shape)
+        loss = ctypes.c_float(0.0)
+        check(self._lib.pllb_s2s_train_step_host(self._h, _np_ptr(ids), _np_ptr(nv), _np_ptr(lab), ids.shape[0],
+                                                 ids.shape[1], lab.shape[1], int(mode), ctypes.byref(loss)))
+        self._last_shape = lab.shape
+        return float(loss.value)
+
+    def token_losses(self) -> np.ndarray:
+        """float32 [B, T_dec]: -log_softmax(logits)[label] of every decoder position of the last step, 0 where the
+        label is -100."""
+        if self._last_shape is None:
+            raise RuntimeError("no step has run")
+        out = np.zeros(self._last_shape, np.float32)
+        check(self._lib.pllb_train_row_losses_host(self._h, _np_ptr(out), out.size))
+        return out
+
+    def _export(self, fn) -> Dict[str, "torch.Tensor"]:
+        import torch
+        bufs = {}
+
+        def get(key):
+            if key not in bufs:
+                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
+            return bufs[key]
+
+        w, keep = s2s_weights_struct(get, self.cfg, pos_skip_rows=0)
+        torch.cuda.synchronize(self._dev)
+        check(fn(self._h, ctypes.byref(w)))
+        torch.cuda.synchronize(self._dev)
+        host = {k: v.cpu() for k, v in bufs.items()}
+        del keep
+        out = {}
+        for k in self._keys:
+            name = k[len(self._prefix):] if k.startswith(self._prefix) else k
+            if name in BART_TIED_KEYS:
+                name = _BART_TOP["shared"]
+            out[k] = host[name].reshape(self._given[k].shape) if name in host else self._given[k]
+        return out
+
+    def state_dict(self) -> Dict[str, "torch.Tensor"]:
+        """fp32 CPU tensors under the keys given at construction: the tied aliases hold the ``model.shared``
+        values and ``final_logits_bias`` (a buffer) passes through.  ``CorrectBart(trainer.state_dict(), cfg,
+        tokenizer)`` decodes with it."""
+        return self._export(self._lib.pllb_s2s_train_export)
+
+    def grads(self) -> Dict[str, "torch.Tensor"]:
+        """Gradients of the last mode-1 / mode-2 step under the same keys (the tied aliases hold the one
+        ``model.shared`` gradient; zeros for ``final_logits_bias``)."""
+        import torch
+        g = self._export(self._lib.pllb_s2s_train_export_grads)
+        for k in g:
+            if k.endswith("final_logits_bias"):
+                g[k] = torch.zeros(self._given[k].shape, dtype=torch.float32)
+        return g

@@ -569,6 +569,69 @@ int pllb_s2s_debug_beam_replay(pllb_s2s h, const pllb_gen_desc* gen, const pllb_
                                const float* hidden, int32_t steps, int32_t* out_ids, int32_t* out_len,
                                float* out_score, int32_t* out_parent, float* out_run_score);
 
+/* ---- CorrectBart fine-tuning (DESIGN.md §3.13): one step is what transformers 5.5.0 computes for
+ * BartForConditionalGeneration.forward(input_ids, attention_mask, labels=labels) in train mode, then
+ * loss.backward() and torch.optim.AdamW over model.parameters().  The reference's training script is
+ * not part of the reference tree, so this is the library's contract, pinned by an fp32 autograd
+ * restatement (oracle/bart_train_oracle.py).
+ *   encoder input  input_ids int32[B, T_enc] ([CLS] hyp [SEP], right-padded), n_valid int32[B] (prefix
+ *                  mask): self-attention and cross-attention keys >= n_valid are masked; padded query
+ *                  rows are computed.
+ *   labels         int32[B, T_dec]; -100 = ignored.
+ *   decoder input  shift_tokens_right(labels, pad_id, decoder_start_id): position 0 holds the start id,
+ *                  -100 becomes pad_id.  Built inside the library.  Decoder self-attention is causal only
+ *                  (no decoder padding mask).
+ *   embeddings     LN(shared[id] * embed_scale + embed_positions[i + 2]) then dropout, both stacks.
+ *   loss           CrossEntropyLoss() of h . shared^T + final_logits_bias at every decoder position: the
+ *                  mean over the positions whose label is not -100.
+ *   gradients      shared gets the LM head's part, then the decoder lookup's, then the encoder lookup's
+ *                  (the lookups carry embed_scale and send nothing to the pad_id row).  final_logits_bias
+ *                  is a buffer: no gradient, no update.  Position rows 0 and 1 get no gradient but are
+ *                  decayed by AdamW, like every parameter.
+ *   dropout        `dropout` after each embedding LayerNorm, each attention / cross-attention output and
+ *                  fc2; `attention_dropout` on the self, causal and cross probabilities.  Stateless hash
+ *                  as in pllb_train_*; parity with torch is defined at dropout 0.
+ * bf16 GEMM operands, fp32 master weights / gradients / moments, fp32 residual stream, LayerNorm and
+ * softmax.  Training takes operand_dtype 0 only; the exported fp32 weights feed pllb_s2s_create with
+ * either operand type.  A step is bit-deterministic. */
+typedef struct pllb_s2s_train_desc {
+  float lr;
+  float beta1, beta2;         /* torch.optim.AdamW defaults 0.9, 0.999                              */
+  float adam_eps;             /* 1e-8                                                                */
+  float weight_decay;         /* applied to every parameter                                          */
+  float dropout;              /* BartConfig.dropout (0.1); 0 for parity runs                          */
+  float attention_dropout;    /* BartConfig.attention_dropout                                         */
+  uint64_t seed;              /* dropout stream                                                       */
+  int32_t pad_id;             /* BartConfig.pad_token_id: lookup padding_idx and shifted -100         */
+  int32_t decoder_start_id;   /* BartConfig.decoder_start_token_id                                    */
+  int32_t max_batch;          /* capacity: sentences per batch                                        */
+  int32_t max_enc_len;        /* capacity: T_enc, <= min(enc_max_position, 1024)                      */
+  int32_t max_dec_len;        /* capacity: T_dec, <= min(dec_max_position, 1024)                      */
+} pllb_s2s_train_desc;
+
+/* desc / weights as pllb_s2s_create, except that enc.pos_emb and dec_pos_emb point at the WHOLE
+ * embed_positions tables (max_position + 2 rows: rows 0 and 1 are parameters too) and every pointer,
+ * final_logits_bias included, is required.  operand_dtype must be 0 (PLLB_ERR_INVALID otherwise).
+ * The handle works with pllb_train_destroy, _reset_optimizer, _workspace_bytes, _kernel_launches,
+ * _graph_replays and _row_losses_host; the MLM and RescoreBert calls reject it (PLLB_ERR_INVALID), and
+ * the pllb_s2s_train_* calls reject their handles. */
+int pllb_s2s_train_create(pllb_trainer* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* weights,
+                          const pllb_s2s_train_desc* train, int device);
+/* One batch, HOST buffers: input_ids int32[B * T_enc], n_valid int32[B], labels int32[B * T_dec].
+ * mode as in pllb_train_step_host (0 loss only, no dropout; 1 update; 2 gradients, no update).
+ * PLLB_ERR_INVALID: an id or label outside [0, vocab) other than label -100, n_valid outside [1, T_enc],
+ * no label other than -100.  PLLB_ERR_TOO_LONG: T_enc or T_dec above its position table.
+ * PLLB_ERR_OOM: B, T_enc or T_dec above the capacity given at create.  One CUDA graph per
+ * (B, T_enc, T_dec, mode).  out_loss: the batch loss.  Synchronises.  pllb_train_row_losses_host then
+ * returns the B * T_dec per-position losses, 0 where the label is -100. */
+int pllb_s2s_train_step_host(pllb_trainer t, const int32_t* input_ids, const int32_t* n_valid, const int32_t* labels,
+                             int32_t B, int32_t T_enc, int32_t T_dec, int32_t mode, float* out_loss);
+/* The fp32 master weights / the gradients of the last mode-1/2 step into the caller's DEVICE tensors
+ * (layout of pllb_s2s_train_create; a NULL pointer skips a tensor).  final_logits_bias: the given
+ * values (export) or zeros (export_grads). */
+int pllb_s2s_train_export(pllb_trainer t, const pllb_s2s_weights* dst);
+int pllb_s2s_train_export_grads(pllb_trainer t, const pllb_s2s_weights* dst);
+
 #ifdef __cplusplus
 }
 #endif
