@@ -5,7 +5,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint16, c_uint64, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint16, c_uint32, c_uint64, c_void_p
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PLLB_LIB") or os.path.join(HERE, "libpllb200.so")   # PLLB_LIB: A/B testing of builds
@@ -119,6 +119,25 @@ SIGNATURES = {
                                    c_void_p]),
     "pllb_debug_gemm_simt": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p]),
     "pllb_debug_hidden": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
+    "pllb_debug_train_attn": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_float, c_uint32,
+                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "pllb_debug_s2s_attn": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_int32, c_int32, c_int32,
+                                    c_int32, c_int32, c_void_p, c_void_p, c_float, c_uint32, c_void_p, c_void_p, c_void_p,
+                                    c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
+    "pllb_debug_train_ln_fwd": (c_int, [c_int32, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_void_p,
+                                        c_void_p, c_float, c_void_p, c_void_p, c_float, c_int32, c_int32, c_void_p, c_float,
+                                        c_uint32, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "pllb_debug_train_ln_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p,
+                                        c_float, c_int32, c_int32, c_void_p, c_void_p, c_void_p]),
+    "pllb_debug_train_ce": (c_int, [c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                    c_void_p]),
+    "pllb_debug_train_embed_bwd": (c_int, [c_int32, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,
+                                           c_float, c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "pllb_debug_train_colsum": (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_int32, c_void_p, c_void_p, c_void_p,
+                                        c_void_p]),
+    "pllb_debug_train_cast_transpose": (c_int, [c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p,
+                                                c_void_p]),
+    "pllb_debug_train_gelu": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "pllb_embed": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_void_p, c_void_p]),
     "pllb_bertscore": (c_int, [c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p]),
     "pllb_tokenize_host": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),

@@ -293,10 +293,11 @@ int visit_params(const pllb_trainer_ctx* c, const pllb_weights* w, const float* 
   return PLLB_OK;
 }
 
-TrainDrop make_drop(const pllb_trainer_ctx* c, float p, bool train) {
+// drop probability p (0: no dropout) over the DEVICE seed; shared by the trainers and the kernel test hooks
+TrainDrop drop_of(const uint64_t* seed, float p) {
   TrainDrop d{};
-  d.seed = &c->params_dev->seed;
-  if (train && p > 0.f) {
+  d.seed = seed;
+  if (p > 0.f) {
     d.thresh = (uint32_t)std::min<double>(4294967295.0, (double)p * 4294967296.0);
     d.inv_keep = 1.f / (1.f - p);
   } else {
@@ -304,6 +305,10 @@ TrainDrop make_drop(const pllb_trainer_ctx* c, float p, bool train) {
     d.inv_keep = 1.f;
   }
   return d;
+}
+
+TrainDrop make_drop(const pllb_trainer_ctx* c, float p, bool train) {
+  return drop_of(&c->params_dev->seed, train ? p : 0.f);
 }
 
 // The encoder forward of one step: embeddings and every layer.  On return h32 holds the fp32 output of the
@@ -1116,6 +1121,190 @@ int pllb_s2s_train_export(pllb_trainer c, const pllb_s2s_weights* dst) {
 
 int pllb_s2s_train_export_grads(pllb_trainer c, const pllb_s2s_weights* dst) {
   return export_s2s(c, true, dst, "pllb_s2s_train_export_grads");
+}
+
+// ---------------------------------------------------------------- kernel test hooks (pllb_debug_train_*)
+// Thin wrappers over the launchers of train.h on caller buffers, so each kernel can be checked alone against a
+// high-precision reference.  Scalars and pointers are checked first; then the DEVICE index arrays a kernel reads
+// without bounds (n_valid, ids, labels) are copied back and checked, so a bad argument never reaches a launch.
+namespace {
+bool hidden_ok(int H) { return H == 256 || H == 512 || H == 768 || H == 1024; }
+
+int bad(const char* who, const std::string& what) { return fail(PLLB_ERR_INVALID, std::string(who) + ": " + what); }
+
+int need_device(const char* who) {
+  if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, std::string(who) + ": no sm_100 (B200) device visible");
+  return PLLB_OK;
+}
+
+// every entry of the DEVICE int32[n] in [lo, hi], or equal to `also` (when also_ok)
+int check_dev_ints(const char* who, const char* name, const int32_t* d, int64_t n, int lo, int hi, cudaStream_t s,
+                   bool also_ok = false, int also = 0, int* count_also = nullptr) {
+  std::vector<int32_t> h((size_t)n);
+  PLLB_CUDA(cudaMemcpyAsync(h.data(), d, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, s));
+  PLLB_CUDA(cudaStreamSynchronize(s));
+  int k = 0;
+  for (int64_t i = 0; i < n; ++i) {
+    if (also_ok && h[i] == also) { ++k; continue; }
+    if (h[i] < lo || h[i] > hi)
+      return bad(who, std::string(name) + "[" + std::to_string(i) + "] = " + std::to_string(h[i]) + " outside [" +
+                          std::to_string(lo) + ", " + std::to_string(hi) + "]");
+  }
+  if (count_also) *count_also = k;
+  return PLLB_OK;
+}
+
+bool drop_ok(const uint64_t* seed, float p) { return p >= 0.f && p < 1.f && (p == 0.f || seed); }
+
+// the attention kernels read bf16 rows and the fp32 dctx 16 bytes at a time and write the fp32 gradients as pairs
+bool aligned(const void* p, uintptr_t bytes) { return p == nullptr || reinterpret_cast<uintptr_t>(p) % bytes == 0; }
+}  // namespace
+
+int pllb_debug_train_attn(const uint16_t* qkv, const int32_t* n_valid, int32_t B, int32_t T, int32_t H, const float* dctx,
+                          const uint64_t* seed, float p, uint32_t site, uint16_t* ctx, float* lse, float* dqkv, float* Dscratch,
+                          void* stream) {
+  const char* who = "pllb_debug_train_attn";
+  if (!qkv || !n_valid || !ctx || !lse) return bad(who, "null pointer");
+  if (dctx && (!dqkv || !Dscratch)) return bad(who, "the backward pass needs dqkv and Dscratch");
+  if (B < 1 || T < 1 || T > 512) return bad(who, "need B >= 1 and T in [1, 512]");
+  if (!hidden_ok(H)) return bad(who, "hidden must be 256, 512, 768 or 1024");
+  if (!drop_ok(seed, p)) return bad(who, "need p in [0, 1) and a seed when p > 0");
+  if (!aligned(qkv, 16) || !aligned(dctx, 16) || !aligned(ctx, 4) || !aligned(lse, 4) || !aligned(dqkv, 8) ||
+      !aligned(Dscratch, 4))
+    return bad(who, "misaligned pointer (qkv and dctx: 16 bytes, dqkv: 8, ctx, lse and Dscratch: 4)");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  RC(check_dev_ints(who, "n_valid", n_valid, B, 1, T, s));
+  const TrainDrop d = drop_of(seed, p);
+  const int R = B * T, NH = H / 64;
+  RC(launch_train_attn_fwd(qkv, n_valid, R, T, H, NH, d, site, ctx, lse, s));
+  if (dctx) RC(launch_train_attn_bwd(qkv, dctx, lse, n_valid, R, T, H, NH, d, site, dqkv, Dscratch, s));
+  return PLLB_OK;
+}
+
+int pllb_debug_s2s_attn(const uint16_t* q, const uint16_t* k, const uint16_t* v, int32_t ldq, int32_t ldkv,
+                        const int32_t* n_valid, int32_t B, int32_t Tq, int32_t Tk, int32_t NH, int32_t causal,
+                        const float* dctx, const uint64_t* seed, float p, uint32_t site, uint16_t* ctx, float* lse, float* dq,
+                        int32_t lddq, float* dk, float* dv, int32_t lddkv, float* Dscratch, void* stream) {
+  const char* who = "pllb_debug_s2s_attn";
+  if (!q || !k || !v || !ctx || !lse || (!causal && !n_valid)) return bad(who, "null pointer");
+  if (dctx && (!dq || !dk || !dv || !Dscratch)) return bad(who, "the backward pass needs dq, dk, dv and Dscratch");
+  if (B < 1 || Tq < 1 || Tq > 512 || Tk < 1 || Tk > 512 || (causal && Tq != Tk))
+    return bad(who, "need B >= 1, Tq and Tk in [1, 512], Tq == Tk when causal");
+  const int H = NH * 64;
+  if (NH < 1 || !hidden_ok(H)) return bad(who, "NH * 64 must be 256, 512, 768 or 1024");
+  // 16-byte rows for the vector loads of Q, K and V (the dk / dv pass reads Q rows as K rows are read), 8-byte rows
+  // (fp32 pairs) for the gradients
+  if (ldq < H || ldkv < H || ldq % 8 || ldkv % 8 || (dctx && (lddq < H || lddkv < H || lddq % 2 || lddkv % 2)))
+    return bad(who, "bad row stride");
+  if (!drop_ok(seed, p)) return bad(who, "need p in [0, 1) and a seed when p > 0");
+  if (!aligned(q, 16) || !aligned(k, 16) || !aligned(v, 16) || !aligned(dctx, 16) || !aligned(ctx, 4) ||
+      !aligned(lse, 4) || !aligned(dq, 8) || !aligned(dk, 8) || !aligned(dv, 8) || !aligned(Dscratch, 4))
+    return bad(who, "misaligned pointer (q, k, v and dctx: 16 bytes, dq, dk and dv: 8, ctx, lse and Dscratch: 4)");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!causal) RC(check_dev_ints(who, "n_valid", n_valid, B, 1, Tk, s));
+  const S2sAttn a{q, k, v, ldq, ldkv, B, Tq, Tk, NH, causal != 0, causal ? nullptr : n_valid};
+  const TrainDrop d = drop_of(seed, p);
+  RC(launch_train_attn_s2s_fwd(a, d, site, ctx, lse, s));
+  if (dctx) RC(launch_train_attn_s2s_bwd(a, dctx, lse, d, site, dq, lddq, dk, dv, lddkv, Dscratch, s));
+  return PLLB_OK;
+}
+
+int pllb_debug_train_ln_fwd(int32_t form, const float* y, const float* res, const int32_t* ids, int32_t T, const float* word,
+                            int32_t vocab, const float* pos, const float* type, float embed_scale, const float* g, const float* b,
+                            float eps, int32_t R, int32_t H, const uint64_t* seed, float p, uint32_t site, float* out32,
+                            uint16_t* out16, float* xhat, float* rstd, void* stream) {
+  const char* who = "pllb_debug_train_ln_fwd";
+  if (form < 0 || form > 2) return bad(who, "form must be 0 (plain), 1 (BERT embedding) or 2 (BART embedding)");
+  if (!g || !b || (form == 0 && !y) || (form != 0 && (!ids || !word || !pos || (form == 1 && !type))) ||
+      (form == 2 && (!out32 || !out16 || !xhat || !rstd)))
+    return bad(who, "null pointer");
+  if (R < 1 || !(eps > 0.f)) return bad(who, "need R >= 1 and eps > 0");
+  if (form != 0 && (T < 1 || T > 512 || vocab < 1)) return bad(who, "need T in [1, 512] and vocab >= 1");
+  if (!hidden_ok(H)) return bad(who, "hidden must be 256, 512, 768 or 1024");
+  if (!drop_ok(seed, p)) return bad(who, "need p in [0, 1) and a seed when p > 0");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (form != 0) RC(check_dev_ints(who, "ids", ids, R, 0, vocab - 1, s));
+  const TrainDrop d = drop_of(seed, p);
+  if (form == 0) return launch_train_ln_fwd(y, res, g, b, eps, R, H, d, site, out32, out16, xhat, rstd, s);
+  if (form == 1) return launch_train_embed(ids, T, word, pos, type, g, b, eps, R, H, d, site, out32, out16, xhat, rstd, s);
+  return launch_train_bart_embed(ids, T, word, embed_scale, pos, g, b, eps, R, H, d, site, out32, out16, xhat, rstd, s);
+}
+
+int pllb_debug_train_ln_bwd(float* dy, const float* add, const float* g, const float* xhat, const float* rstd, int32_t R,
+                            int32_t H, const uint64_t* seed, float p, int32_t site_in, int32_t site_out, float* dz,
+                            float* dz_drop, void* stream) {
+  const char* who = "pllb_debug_train_ln_bwd";
+  if (!dy || !g || !xhat || !rstd || !dz) return bad(who, "null pointer");
+  if (R < 1) return bad(who, "need R >= 1");
+  if (!hidden_ok(H)) return bad(who, "hidden must be 256, 512, 768 or 1024");
+  if (!drop_ok(seed, p) || site_in < -1 || site_out < -1) return bad(who, "need p in [0, 1), a seed when p > 0, sites >= -1");
+  RC(need_device(who));
+  return launch_train_ln_bwd(dy, add, g, xhat, rstd, R, H, drop_of(seed, p), site_in, site_out, dz, dz_drop,
+                             (cudaStream_t)stream);
+}
+
+int pllb_debug_train_ce(const float* logits, const int32_t* labels, int32_t R, int32_t V, int32_t Vp, int32_t ignore_index,
+                        float* loss_rows, uint16_t* dlogits, float* out_loss, void* stream) {
+  const char* who = "pllb_debug_train_ce";
+  if (!logits || !labels || !loss_rows || !out_loss) return bad(who, "null pointer");
+  if (R < 1 || V < 1 || Vp < V) return bad(who, "need R >= 1 and 1 <= V <= Vp");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!ignore_index) {
+    RC(check_dev_ints(who, "labels", labels, R, 0, V - 1, s));
+    return launch_train_ce(logits, labels, R, V, Vp, loss_rows, dlogits, out_loss, s);
+  }
+  int ignored = 0;
+  RC(check_dev_ints(who, "labels", labels, R, 0, V - 1, s, true, -100, &ignored));
+  if (ignored == R) return bad(who, "every label is -100");
+  return launch_train_ce_ignore(logits, labels, R, V, Vp, loss_rows, dlogits, out_loss, s);
+}
+
+int pllb_debug_train_embed_bwd(int32_t form, float* dz, const int32_t* ids, int32_t B, int32_t T, int32_t H, int32_t pos_rows,
+                               int32_t pad_id, float scale, float* dword, int32_t vocab, float* dpos, float* dtype0,
+                               float* scratch, void* stream) {
+  const char* who = "pllb_debug_train_embed_bwd";
+  if (form < 0 || form > 1) return bad(who, "form must be 0 (BERT embedding) or 1 (BART embedding)");
+  if (!dz || !ids || !dword || !dpos || (form == 0 && !dtype0)) return bad(who, "null pointer");
+  if (B < 1 || T < 1 || T > 512 || pos_rows < T || vocab < 1) return bad(who, "need B >= 1, T in [1, 512], pos_rows >= T");
+  if (!hidden_ok(H)) return bad(who, "hidden must be 256, 512, 768 or 1024");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  RC(check_dev_ints(who, "ids", ids, (int64_t)B * T, 0, vocab - 1, s));
+  if (form == 0) return launch_train_embed_bwd(dz, ids, B, T, H, pos_rows, pad_id, dword, dpos, dtype0, scratch, s);
+  return launch_train_bart_embed_bwd(dz, ids, B, T, H, pos_rows, pad_id, scale, dword, dpos, s);
+}
+
+int pllb_debug_train_colsum(const void* dy, int32_t dy_bf16, const float* xhat, int32_t R, int32_t C, float* out_sum,
+                            float* out_dot, float* scratch, void* stream) {
+  const char* who = "pllb_debug_train_colsum";
+  if (!dy || (!out_sum && !out_dot) || (out_dot && !xhat)) return bad(who, "null pointer");
+  if (R < 1 || C < 1) return bad(who, "need R >= 1 and C >= 1");
+  RC(need_device(who));
+  return launch_train_colsum(dy, dy_bf16 != 0, xhat, R, C, out_sum, out_dot, scratch, (cudaStream_t)stream);
+}
+
+int pllb_debug_train_cast_transpose(const void* src, int32_t src_bf16, int32_t R, int32_t C, int32_t Rp, uint16_t* dst16,
+                                    uint16_t* dstT, void* stream) {
+  const char* who = "pllb_debug_train_cast_transpose";
+  if (!src || (!dst16 && !dstT)) return bad(who, "null pointer");
+  if (R < 1 || C < 1 || Rp < R) return bad(who, "need R >= 1, C >= 1 and Rp >= R");
+  RC(need_device(who));
+  return launch_train_cast_transpose(src, src_bf16 != 0, R, C, Rp, dst16, dstT, (cudaStream_t)stream);
+}
+
+int pllb_debug_train_gelu(const float* f, int64_t n, uint16_t* out16, float* out32, float* dg, void* stream) {
+  const char* who = "pllb_debug_train_gelu";
+  if (!f || (!out16 && !out32 && !dg)) return bad(who, "null pointer");
+  if (n < 1) return bad(who, "need n >= 1");
+  RC(need_device(who));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (out16 || out32) RC(launch_train_gelu_fwd(f, n, out16, out32, s));
+  if (dg) RC(launch_train_gelu_bwd(dg, f, n, s));
+  return PLLB_OK;
 }
 
 }  // extern "C"

@@ -185,6 +185,67 @@ int pllb_debug_gemm_simt(const uint16_t* A, const uint16_t* W, const float* bias
 int pllb_debug_hidden(pllb_handle h, const int32_t* hyp_tokens, const int64_t* hyp_offsets,
                       int32_t n_hyp, int32_t upto_layer, float* out_hidden, void* stream);
 
+/* Kernel hooks of the training path (the non-GEMM kernels the MLM, RescoreBert and CorrectBart
+ * trainers share; used by tests only).  Every pointer is a caller DEVICE buffer; the launches are
+ * those of a training step.  bf16 buffers are raw uint16.  Dropout: probability p in [0, 1) over the
+ * DEVICE uint64 *seed (may be NULL when p == 0) at dropout site `site`, as in a step.  Bad scalars or
+ * pointers, H outside {256, 512, 768, 1024}, T outside [1, 512], and device index arrays out of range
+ * (n_valid outside [1, T], ids outside [0, vocab), labels outside [0, V) and not -100 where allowed)
+ * return PLLB_ERR_INVALID before anything is launched; the index checks synchronise the stream.  The
+ * attention hooks also refuse misaligned pointers: bf16 q / k / v (qkv) and fp32 dctx on 16 bytes,
+ * fp32 dq / dk / dv (dqkv) on 8, the rest on 4.
+ *
+ * Padded self-attention of B sequences of T rows, NH = H / 64 heads: qkv bf16 [B*T, 3H] (q | k | v),
+ * n_valid int32[B].  Forward: ctx bf16 [B*T, H], lse fp32 [B*T*NH].  With dctx (fp32 [B*T, H]) also the
+ * backward: dqkv fp32 [B*T, 3H], Dscratch fp32 [B*T*NH] (D = sum_j P dP of every (row, head)). */
+int pllb_debug_train_attn(const uint16_t* qkv, const int32_t* n_valid, int32_t B, int32_t T, int32_t H,
+                          const float* dctx, const uint64_t* seed, float p, uint32_t site, uint16_t* ctx,
+                          float* lse, float* dqkv, float* Dscratch, void* stream);
+/* The decoder's attention: Tq query rows (q, row stride ldq) over Tk key / value rows (k, v, row stride
+ * ldkv) per sequence.  causal != 0: Tq == Tk, query i sees keys <= i (n_valid unused); otherwise keys
+ * < n_valid[b].  ctx bf16 [B*Tq, NH*64], lse [B*Tq*NH]; with dctx (fp32 [B*Tq, NH*64]) also dq (row
+ * stride lddq), dk and dv (row stride lddkv) and Dscratch [B*Tq*NH].  ldq % 8 == ldkv % 8 == 0. */
+int pllb_debug_s2s_attn(const uint16_t* q, const uint16_t* k, const uint16_t* v, int32_t ldq, int32_t ldkv,
+                        const int32_t* n_valid, int32_t B, int32_t Tq, int32_t Tk, int32_t NH, int32_t causal,
+                        const float* dctx, const uint64_t* seed, float p, uint32_t site, uint16_t* ctx, float* lse,
+                        float* dq, int32_t lddq, float* dk, float* dv, int32_t lddkv, float* Dscratch, void* stream);
+/* LayerNorm forward over R rows of H, saving xhat and rstd (either may be NULL in form 0).
+ * form 0: LN(dropout(y) + res)            (res may be NULL; out32 / out16 may be NULL)
+ * form 1: dropout(LN(word[ids[r]] + pos[r % T] + type[0]))        (BERT embeddings)
+ * form 2: dropout(LN(word[ids[r]] * embed_scale + pos[r % T]))    (BART embeddings; every output required) */
+int pllb_debug_train_ln_fwd(int32_t form, const float* y, const float* res, const int32_t* ids, int32_t T,
+                            const float* word, int32_t vocab, const float* pos, const float* type, float embed_scale,
+                            const float* g, const float* b, float eps, int32_t R, int32_t H, const uint64_t* seed,
+                            float p, uint32_t site, float* out32, uint16_t* out16, float* xhat, float* rstd,
+                            void* stream);
+/* LayerNorm backward: dy <- (dy + add) [* mask site_in]; dz = the input gradient; dz_drop = dz [* mask
+ * site_out] (may be NULL).  add may be NULL or alias dz; site -1 = no mask. */
+int pllb_debug_train_ln_bwd(float* dy, const float* add, const float* g, const float* xhat, const float* rstd,
+                            int32_t R, int32_t H, const uint64_t* seed, float p, int32_t site_in, int32_t site_out,
+                            float* dz, float* dz_drop, void* stream);
+/* Cross entropy over the first V of Vp logit columns (fp32 [R, Vp]): loss_rows [R]; dlogits bf16 [R, Vp]
+ * = softmax - onehot, 0 past V (may be NULL).  ignore_index 0: out_loss[0] = the mean loss.
+ * ignore_index != 0: label -100 gives loss 0 and a zero dlogits row; out_loss[0] = the mean over the N
+ * labelled rows, out_loss[1] = 1 / N. */
+int pllb_debug_train_ce(const float* logits, const int32_t* labels, int32_t R, int32_t V, int32_t Vp,
+                        int32_t ignore_index, float* loss_rows, uint16_t* dlogits, float* out_loss, void* stream);
+/* Embedding backward from dz fp32 [B*T, H]: dpos [pos_rows, H] (rows >= T zero); dword [vocab, H] += the
+ * rows of each id except pad_id.  form 0 (BERT): dtype0 [H] = the column sums (scratch: 128 * H floats
+ * or NULL).  form 1 (BART): dz is scaled by `scale` in place before the word scatter. */
+int pllb_debug_train_embed_bwd(int32_t form, float* dz, const int32_t* ids, int32_t B, int32_t T, int32_t H,
+                               int32_t pos_rows, int32_t pad_id, float scale, float* dword, int32_t vocab,
+                               float* dpos, float* dtype0, float* scratch, void* stream);
+/* Column sums of dy [R, C] (fp32, or bf16 when dy_bf16): out_sum[c] = sum_r dy, out_dot[c] = sum_r
+ * dy * xhat (either may be NULL).  scratch: 128 * C floats for the row-sliced form, or NULL. */
+int pllb_debug_train_colsum(const void* dy, int32_t dy_bf16, const float* xhat, int32_t R, int32_t C,
+                            float* out_sum, float* out_dot, float* scratch, void* stream);
+/* src [R, C] (fp32, or bf16 when src_bf16) -> dst16 bf16 [R, C] and / or dstT bf16 [C, Rp], columns
+ * >= R of dstT zero.  Rp >= R. */
+int pllb_debug_train_cast_transpose(const void* src, int32_t src_bf16, int32_t R, int32_t C, int32_t Rp,
+                                    uint16_t* dst16, uint16_t* dstT, void* stream);
+/* GELU (erf form) of f [n]: out16 bf16 and / or out32; then dg[i] *= GELU'(f[i]) when dg != NULL. */
+int pllb_debug_train_gelu(const float* f, int64_t n, uint16_t* out16, float* out32, float* dg, void* stream);
+
 /* ---- BERTScore minimum-Bayes-risk (RMBR): replaces bert_score.score(cands, refs, lang="zh") inside
  * RMBR/utility_functions.py:9-23 (BertScoreFunction).  RMBR/ and bert_score are not in the reference
  * tree, so this is the library's own contract, following bert_score with its default arguments

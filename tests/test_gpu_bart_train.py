@@ -94,7 +94,7 @@ def check_parity(kind, cfg, m, ids, mask, labels):
     assert errs["model.shared.weight"] <= SHARED_REL[kind] and dec_rows <= SHARED_REL[kind]
     for k in ("model.encoder.embed_positions.weight", "model.decoder.embed_positions.weight"):
         assert float(g[k][:2].abs().max()) == 0.0          # rows 0 and 1 are never looked up
-    return errs
+    return errs, tl, tl_o, g, g_o
 
 
 @pytest.mark.parametrize("scale", [False, True])
@@ -104,6 +104,23 @@ def test_parity_tiny(scale, label_pad):
     rng = np.random.default_rng(11 + scale + 2 * (label_pad == 0))
     ids, mask, labels = batch(rng, 5, 13, 9, 300, label_pad=label_pad)
     check_parity("tiny", cfg, m, ids, mask, labels)
+
+
+def test_parity_long_sequences():
+    """T_enc 129 and T_dec 65 (max_position 160), ragged, so the attention loops take several 32-key and 32-query
+    passes.  The tiny-shape tolerances (every per-position loss, those at positions >= 32 included, within TOKEN_ABS);
+    and separately the position-embedding gradients of rows >= 32 (table rows >= 34: the tables start at offset 2), so
+    an error at long positions cannot be averaged away in the whole table's norm."""
+    cfg = bo.bart_config(d_model=256, layers=2, ffn=1024, vocab=300, max_position=160)
+    m = bo.make_model(cfg, seed=8)
+    ids, mask, labels = batch(np.random.default_rng(8), 3, 129, 65, 300)
+    _, tl, tl_o, g, g_o = check_parity("tiny", cfg, m, ids, mask, labels)     # every position within TOKEN_ABS
+    assert int((labels[:, 32:] != -100).sum()) > 0
+    pos = {k: rel_l2(g[k].numpy()[34:], g_o[k].numpy()[34:]) for k in
+           ("model.encoder.embed_positions.weight", "model.decoder.embed_positions.weight")}
+    print(f"[parity long] per-position loss |d| at positions >= 32: {float(np.abs(tl - tl_o)[:, 32:].max()):.4f}; "
+          f"position rows >= 32: {pos}")
+    assert all(v <= GRAD_REL["tiny"] for v in pos.values()), pos
 
 
 def c2_pairs(n):

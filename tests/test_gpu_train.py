@@ -97,6 +97,48 @@ def test_bert_base_shape_two_layers_vs_oracle():
     print(f"bert-base shape, 2 layers: loss {loss:.5f} (oracle {o_loss:.5f}), worst gradient rel L2 error {worst:.4f}")
 
 
+def test_long_ragged_batch_vs_oracle():
+    """Rows up to T = 128 (BERT_TINY's max_position), so every attention loop takes several 32-key passes, with ragged
+    lengths from 3 to 128.  The existing tolerances; every per-position loss within 0.1 nats, the positions >= 32
+    included; and separately the position-embedding gradient of rows >= 32, so an error at long positions cannot be
+    averaged away in the whole table's norm."""
+    import torch
+    import torch.nn.functional as F
+    cfg = synth.BERT_TINY
+    sd = synth.random_init_state_dict(cfg, 12, perturb=True)
+    rng = np.random.default_rng(12)
+    rows = []
+    for n in (128, 97, 3, 65, 33, 120):
+        toks = [int(t) for t in rng.integers(104, cfg["vocab"], n - 2)]
+        rows.append(pll_oracle.expand_rows(toks, "u", None)[int(rng.integers(0, n - 2))])
+    ids, am, lab = _batch(rows)
+    assert ids.shape == (6, 128)
+    o_loss, o_grads = train_oracle.loss_and_grads(sd, cfg, rows)
+    with torch.no_grad():
+        logits = pll_oracle.bert_mlm_logits(train_oracle._full(train_oracle.parameters(sd)), cfg, torch.from_numpy(ids).long(),
+                                            torch.from_numpy(am).long())
+    o_tok = F.cross_entropy(logits.reshape(-1, cfg["vocab"]), torch.from_numpy(lab).long().reshape(-1), reduction="none")
+    with engine.MlmTrainer(sd, cfg, hidden_dropout=0.0, attention_dropout=0.0, max_rows=ids.size, max_seq=ids.shape[1]) as tr:
+        loss = tr.step(ids, am, lab, mode=2)
+        tok = tr.row_losses(ids.size).reshape(ids.shape)
+        g = tr.grads()
+    o_tok = o_tok.reshape(ids.shape).numpy()
+    tok_err = np.abs(tok - o_tok)
+    worst = 0.0
+    for k, og in o_grads.items():
+        if k.endswith(KEY_BIAS):
+            continue
+        d, og = g[k].double(), og.double()
+        worst = max(worst, float((d - og).norm() / (og.norm() + 1e-30)))
+    P = "bert.embeddings.position_embeddings.weight"
+    d, og = g[P][32:].double(), o_grads[P][32:].double()
+    pos_rel = float((d - og).norm() / (og.norm() + 1e-30))
+    print(f"long batch T=128: loss {loss:.5f} (oracle {o_loss:.5f}); worst gradient rel L2 {worst:.4f}; position rows >= 32 "
+          f"{pos_rel:.4f}; per-position loss |d| max {tok_err.max():.4f}, at positions >= 32 {tok_err[:, 32:].max():.4f}")
+    assert abs(loss - o_loss) <= 0.02 and worst <= 0.06 and pos_rel <= 0.06
+    assert float(og.norm()) > 0 and tok_err.max() <= 0.1
+
+
 def test_bert_base_twelve_layers_three_steps_vs_oracle():
     """The shape and depth the reference fine-tunes (bert-base-chinese, train.yaml:23-24), three AdamW steps at
     lr 1e-4 on batches of 32 rows: the batch losses follow the fp32 autograd oracle within 0.02 nats, and the
