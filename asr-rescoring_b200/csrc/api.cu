@@ -31,6 +31,15 @@ int check_model_shape(const pllb_model_desc& d) {
   return PLLB_OK;
 }
 
+int check_create_device(int device) {
+  if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 (B200) device visible; libpllb200 has no CPU fallback");
+  PLLB_CUDA(cudaSetDevice(device));
+  int major = 0;
+  PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
+  if (major != 10) return fail(PLLB_ERR_NO_DEVICE, "device is not sm_100 (B200); libpllb200 has no other code path");
+  return PLLB_OK;
+}
+
 int sm_count() {
   static thread_local int cached_dev = -1, cached = 0;
   int dev = 0;
@@ -199,39 +208,16 @@ struct pllb_context {
 
 namespace {
 
-template <typename T>
-int dev_alloc(pllb_context* c, T** out, int64_t count) {
-  void* p = nullptr;
-  const int64_t bytes = std::max<int64_t>(count, 1) * (int64_t)sizeof(T);
-  cudaError_t e = cudaMalloc(&p, (size_t)bytes);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail(PLLB_ERR_OOM, "cudaMalloc of " + std::to_string(bytes) + " bytes failed: " + cudaGetErrorString(e));
-  }
-  c->owned.push_back(p);
-  c->owned_bytes += bytes;
-  *out = reinterpret_cast<T*>(p);
-  return PLLB_OK;
-}
-
 int copy_f32(pllb_context* c, float** dst, const float* src, int64_t n, cudaStream_t s) {
-  int rc = dev_alloc(c, dst, n);
-  if (rc) return rc;
+  RC(owned_alloc(c, dst, n));
   PLLB_CUDA(cudaMemcpyAsync(*dst, src, sizeof(float) * n, cudaMemcpyDeviceToDevice, s));
   return PLLB_OK;
 }
 
 int conv_16(pllb_context* c, __nv_bfloat16** dst, const float* src, int64_t n, bool fp16, cudaStream_t s) {
-  int rc = dev_alloc(c, dst, n);
-  if (rc) return rc;
+  RC(owned_alloc(c, dst, n));
   return launch_f32_to_bf16(src, *dst, n, fp16, s);
 }
-
-#define RC(expr)            \
-  do {                      \
-    int _rc = (expr);       \
-    if (_rc) return _rc;    \
-  } while (0)
 
 // Enqueues one GEMM launch (`launch`) on s between the timing events of a timed call, and counts
 // its FLOPs towards the stats and its kind.
@@ -525,8 +511,6 @@ int check_device() {
   return PLLB_OK;
 }
 
-inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
-
 // Grow-only device scratch for the stage-4 host entry points (one per host thread and
 // device): repeated sweeps must not pay cudaMalloc / cudaFree (an implicit device sync).
 struct Scratch {
@@ -551,6 +535,93 @@ int get_scratch(int64_t bytes, uint8_t** out) {
     g_scratch.dev = dev;
   }
   *out = reinterpret_cast<uint8_t*>(g_scratch.p);
+  return PLLB_OK;
+}
+
+// The weights and the workspace of a new scoring handle (c->d and c->device set); on failure pllb_create destroys it.
+int build_context(pllb_context* c, const pllb_weights* w, int64_t max_chunk_tokens) {
+  const pllb_model_desc& d = c->d;
+  c->fp16_from = d.operand_dtype == 1 ? 0 : d.operand_dtype == 3 ? d.num_layers / 2
+               : d.operand_dtype >= 16 ? d.operand_dtype - 16 : d.num_layers;
+  c->head_fp16 = d.operand_dtype >= 1;
+  c->dt_head = c->head_fp16 ? DT_FP16 : DT_BF16;
+  if (const char* e = getenv("PLLB_SHARE_L0")) c->share_l0 = atoi(e) != 0;
+  cudaStream_t s = 0;
+  const int H = d.hidden, I = d.intermediate, V = d.vocab;
+  RC(copy_f32(c, &c->word_emb, w->word_emb, (int64_t)V * H, s));
+  RC(copy_f32(c, &c->pos_emb, w->pos_emb, (int64_t)d.max_position * H, s));
+  RC(copy_f32(c, &c->type_emb, w->type_emb, H, s));   // token_type 0 only (MLM_PLL/main.py:89-94 passes none)
+  RC(copy_f32(c, &c->emb_g, w->emb_ln_g, H, s));
+  RC(copy_f32(c, &c->emb_b, w->emb_ln_b, H, s));
+  c->layers.resize(d.num_layers);
+  for (int l = 0; l < d.num_layers; ++l) {
+    const pllb_layer_weights& lw = w->layers[l];
+    LayerDev& L = c->layers[l];
+    RC(owned_alloc(c, &L.qkv_w, (int64_t)3 * H * H));
+    RC(launch_f32_to_bf16(lw.q_w, L.qkv_w, (int64_t)H * H, c->lfp16(l), s));
+    RC(launch_f32_to_bf16(lw.k_w, L.qkv_w + (int64_t)H * H, (int64_t)H * H, c->lfp16(l), s));
+    RC(launch_f32_to_bf16(lw.v_w, L.qkv_w + (int64_t)2 * H * H, (int64_t)H * H, c->lfp16(l), s));
+    RC(owned_alloc(c, &L.qkv_b, 3 * H));
+    cudaMemcpyAsync(L.qkv_b, lw.q_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
+    cudaMemcpyAsync(L.qkv_b + H, lw.k_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
+    cudaMemcpyAsync(L.qkv_b + 2 * H, lw.v_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
+    RC(conv_16(c, &L.ao_w, lw.ao_w, (int64_t)H * H, c->lfp16(l), s));
+    RC(copy_f32(c, &L.ao_b, lw.ao_b, H, s));
+    RC(copy_f32(c, &L.ao_g, lw.ao_ln_g, H, s));
+    RC(copy_f32(c, &L.ao_be, lw.ao_ln_b, H, s));
+    RC(conv_16(c, &L.ff1_w, lw.ff1_w, (int64_t)I * H, c->lfp16(l), s));
+    RC(copy_f32(c, &L.ff1_b, lw.ff1_b, I, s));
+    RC(conv_16(c, &L.ff2_w, lw.ff2_w, (int64_t)H * I, c->lfp16(l), s));
+    RC(copy_f32(c, &L.ff2_b, lw.ff2_b, H, s));
+    RC(copy_f32(c, &L.out_g, lw.out_ln_g, H, s));
+    RC(copy_f32(c, &L.out_be, lw.out_ln_b, H, s));
+  }
+  c->vocab_pad = (int)round_up(V, 256);
+  c->tiles_v = c->vocab_pad / 256;
+  // the MLM head is optional: a RescoreBert checkpoint (BertModel + Linear) has none
+  c->has_head = w->head_w && w->head_b && w->head_ln_g && w->head_ln_b && w->decoder_w && w->decoder_b;
+  if (c->has_head) {
+    RC(owned_alloc(c, &c->head_w, (int64_t)H * H));
+    RC(launch_f32_to_bf16(w->head_w, c->head_w, (int64_t)H * H, c->head_fp16, s));
+    RC(copy_f32(c, &c->head_b, w->head_b, H, s));
+    RC(copy_f32(c, &c->head_g, w->head_ln_g, H, s));
+    RC(copy_f32(c, &c->head_be, w->head_ln_b, H, s));
+    RC(owned_alloc(c, &c->dec_w, (int64_t)c->vocab_pad * H));
+    cudaMemsetAsync(c->dec_w, 0, sizeof(__nv_bfloat16) * (size_t)c->vocab_pad * H, s);
+    RC(launch_f32_to_bf16(w->decoder_w, c->dec_w, (int64_t)V * H, c->head_fp16, s));
+    RC(owned_alloc(c, &c->dec_b, c->vocab_pad));
+    cudaMemsetAsync(c->dec_b, 0, sizeof(float) * c->vocab_pad, s);
+    cudaMemcpyAsync(c->dec_b, w->decoder_b, sizeof(float) * V, cudaMemcpyDeviceToDevice, s);
+  }
+
+  // workspace: sized by the expanded-token budget of one chunk
+  if (max_chunk_tokens <= 0) max_chunk_tokens = (int64_t)1 << 20;
+  c->cap_rows = round_up(std::max<int64_t>(max_chunk_tokens, 1024), 256);   // the paired LayerNorm clusters work on 256-row blocks
+  c->cap_copies = c->cap_rows / 4 + 128;
+  c->cap_hyps = c->cap_rows / 4 + 128;
+  const int64_t R = c->cap_rows, C = c->cap_copies;
+  const int wide = std::max(3 * H, I);
+  RC(owned_alloc(c, &c->hidden_f32, R * H));
+  RC(owned_alloc(c, &c->hidden_bf16, R * H));
+  RC(owned_alloc(c, &c->wide, R * wide));
+  RC(owned_alloc(c, &c->ctx, R * H));
+  RC(owned_alloc(c, &c->y_f32, R * H));
+  RC(owned_alloc(c, &c->plan.seq_start, C));
+  RC(owned_alloc(c, &c->plan.seq_len, C));
+  RC(owned_alloc(c, &c->plan.mask_row, C));
+  RC(owned_alloc(c, &c->plan.label, C));
+  RC(owned_alloc(c, &c->plan.hyp, C));
+  RC(owned_alloc(c, &c->plan.uniq_base, C));
+  RC(owned_alloc(c, &c->plan.row_src, R));
+  RC(owned_alloc(c, &c->hg, C * H));
+  RC(owned_alloc(c, &c->t_f32, C * H));
+  RC(owned_alloc(c, &c->hid_c, round_up(C, 256) * H));
+  RC(owned_alloc(c, &c->t_bf16, C * H));
+  RC(owned_alloc(c, &c->partials, C * c->tiles_v * 2));
+  RC(owned_alloc(c, &c->label_logit, C));
+  RC(owned_alloc(c, &c->tok_logp, C));
+  cudaError_t e = cudaStreamSynchronize(s);
+  if (e != cudaSuccess) return fail(PLLB_ERR_CUDA, std::string("pllb_create: ") + cudaGetErrorString(e));
   return PLLB_OK;
 }
 
@@ -579,113 +650,19 @@ int pllb_create(pllb_handle* out, const pllb_model_desc* desc, const pllb_weight
                 int device) {
   if (!out || !desc || !w || !w->layers) return fail(PLLB_ERR_INVALID, "pllb_create: null argument");
   *out = nullptr;
-  RC(check_device());
   const pllb_model_desc& d = *desc;
   RC(check_model_shape(d));
   if (d.operand_dtype < 0 || (d.operand_dtype > 3 && (d.operand_dtype < 16 || d.operand_dtype > 16 + d.num_layers)))
     return fail(PLLB_ERR_INVALID, "unsupported model shape: need num_layers >= 1, hidden in {256,512,768,1024}, "
                                   "head dim 64, intermediate % 256 == 0");
-  PLLB_CUDA(cudaSetDevice(device));
-  int major = 0;
-  PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
-  if (major != 10) return fail(PLLB_ERR_NO_DEVICE, "device is not sm_100 (B200); libpllb200 has no other code path");
+  RC(check_create_device(device));
   pllb_context* c = new pllb_context();
   c->d = d;
   c->device = device;
-  c->fp16_from = d.operand_dtype == 1 ? 0 : d.operand_dtype == 3 ? d.num_layers / 2
-               : d.operand_dtype >= 16 ? d.operand_dtype - 16 : d.num_layers;
-  c->head_fp16 = d.operand_dtype >= 1;
-  c->dt_head = c->head_fp16 ? DT_FP16 : DT_BF16;
-  if (const char* e = getenv("PLLB_SHARE_L0")) c->share_l0 = atoi(e) != 0;
-  cudaStream_t s = 0;
-  const int H = d.hidden, I = d.intermediate, V = d.vocab;
-  int rc = PLLB_OK;
-  auto bail = [&](int code) {
+  const int rc = build_context(c, w, max_chunk_tokens);
+  if (rc) {
     pllb_destroy(c);
-    return code;
-  };
-#define TRY(expr)                  \
-  do {                             \
-    rc = (expr);                   \
-    if (rc) return bail(rc);       \
-  } while (0)
-  TRY(copy_f32(c, &c->word_emb, w->word_emb, (int64_t)V * H, s));
-  TRY(copy_f32(c, &c->pos_emb, w->pos_emb, (int64_t)d.max_position * H, s));
-  TRY(copy_f32(c, &c->type_emb, w->type_emb, H, s));   // token_type 0 only (MLM_PLL/main.py:89-94 passes none)
-  TRY(copy_f32(c, &c->emb_g, w->emb_ln_g, H, s));
-  TRY(copy_f32(c, &c->emb_b, w->emb_ln_b, H, s));
-  c->layers.resize(d.num_layers);
-  for (int l = 0; l < d.num_layers; ++l) {
-    const pllb_layer_weights& lw = w->layers[l];
-    LayerDev& L = c->layers[l];
-    TRY(dev_alloc(c, &L.qkv_w, (int64_t)3 * H * H));
-    TRY(launch_f32_to_bf16(lw.q_w, L.qkv_w, (int64_t)H * H, c->lfp16(l), s));
-    TRY(launch_f32_to_bf16(lw.k_w, L.qkv_w + (int64_t)H * H, (int64_t)H * H, c->lfp16(l), s));
-    TRY(launch_f32_to_bf16(lw.v_w, L.qkv_w + (int64_t)2 * H * H, (int64_t)H * H, c->lfp16(l), s));
-    TRY(dev_alloc(c, &L.qkv_b, 3 * H));
-    cudaMemcpyAsync(L.qkv_b, lw.q_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
-    cudaMemcpyAsync(L.qkv_b + H, lw.k_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
-    cudaMemcpyAsync(L.qkv_b + 2 * H, lw.v_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s);
-    TRY(conv_16(c, &L.ao_w, lw.ao_w, (int64_t)H * H, c->lfp16(l), s));
-    TRY(copy_f32(c, &L.ao_b, lw.ao_b, H, s));
-    TRY(copy_f32(c, &L.ao_g, lw.ao_ln_g, H, s));
-    TRY(copy_f32(c, &L.ao_be, lw.ao_ln_b, H, s));
-    TRY(conv_16(c, &L.ff1_w, lw.ff1_w, (int64_t)I * H, c->lfp16(l), s));
-    TRY(copy_f32(c, &L.ff1_b, lw.ff1_b, I, s));
-    TRY(conv_16(c, &L.ff2_w, lw.ff2_w, (int64_t)H * I, c->lfp16(l), s));
-    TRY(copy_f32(c, &L.ff2_b, lw.ff2_b, H, s));
-    TRY(copy_f32(c, &L.out_g, lw.out_ln_g, H, s));
-    TRY(copy_f32(c, &L.out_be, lw.out_ln_b, H, s));
-  }
-  c->vocab_pad = (int)align_up(V, 256);
-  c->tiles_v = c->vocab_pad / 256;
-  // the MLM head is optional: a RescoreBert checkpoint (BertModel + Linear) has none
-  c->has_head = w->head_w && w->head_b && w->head_ln_g && w->head_ln_b && w->decoder_w && w->decoder_b;
-  if (c->has_head) {
-    TRY(dev_alloc(c, &c->head_w, (int64_t)H * H));
-    TRY(launch_f32_to_bf16(w->head_w, c->head_w, (int64_t)H * H, c->head_fp16, s));
-    TRY(copy_f32(c, &c->head_b, w->head_b, H, s));
-    TRY(copy_f32(c, &c->head_g, w->head_ln_g, H, s));
-    TRY(copy_f32(c, &c->head_be, w->head_ln_b, H, s));
-    TRY(dev_alloc(c, &c->dec_w, (int64_t)c->vocab_pad * H));
-    cudaMemsetAsync(c->dec_w, 0, sizeof(__nv_bfloat16) * (size_t)c->vocab_pad * H, s);
-    TRY(launch_f32_to_bf16(w->decoder_w, c->dec_w, (int64_t)V * H, c->head_fp16, s));
-    TRY(dev_alloc(c, &c->dec_b, c->vocab_pad));
-    cudaMemsetAsync(c->dec_b, 0, sizeof(float) * c->vocab_pad, s);
-    cudaMemcpyAsync(c->dec_b, w->decoder_b, sizeof(float) * V, cudaMemcpyDeviceToDevice, s);
-  }
-
-  // workspace: sized by the expanded-token budget of one chunk
-  if (max_chunk_tokens <= 0) max_chunk_tokens = (int64_t)1 << 20;
-  c->cap_rows = align_up(std::max<int64_t>(max_chunk_tokens, 1024), 256);   // the paired LayerNorm clusters work on 256-row blocks
-  c->cap_copies = c->cap_rows / 4 + 128;
-  c->cap_hyps = c->cap_rows / 4 + 128;
-  const int64_t R = c->cap_rows, C = c->cap_copies;
-  const int wide = std::max(3 * H, I);
-  TRY(dev_alloc(c, &c->hidden_f32, R * H));
-  TRY(dev_alloc(c, &c->hidden_bf16, R * H));
-  TRY(dev_alloc(c, &c->wide, R * wide));
-  TRY(dev_alloc(c, &c->ctx, R * H));
-  TRY(dev_alloc(c, &c->y_f32, R * H));
-  TRY(dev_alloc(c, &c->plan.seq_start, C));
-  TRY(dev_alloc(c, &c->plan.seq_len, C));
-  TRY(dev_alloc(c, &c->plan.mask_row, C));
-  TRY(dev_alloc(c, &c->plan.label, C));
-  TRY(dev_alloc(c, &c->plan.hyp, C));
-  TRY(dev_alloc(c, &c->plan.uniq_base, C));
-  TRY(dev_alloc(c, &c->plan.row_src, R));
-  TRY(dev_alloc(c, &c->hg, C * H));
-  TRY(dev_alloc(c, &c->t_f32, C * H));
-  TRY(dev_alloc(c, &c->hid_c, align_up(C, 256) * H));
-  TRY(dev_alloc(c, &c->t_bf16, C * H));
-  TRY(dev_alloc(c, &c->partials, C * c->tiles_v * 2));
-  TRY(dev_alloc(c, &c->label_logit, C));
-  TRY(dev_alloc(c, &c->tok_logp, C));
-#undef TRY
-  cudaError_t e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) {
-    pllb_destroy(c);
-    return fail(PLLB_ERR_CUDA, std::string("pllb_create: ") + cudaGetErrorString(e));
+    return rc;
   }
   *out = c;
   return PLLB_OK;
@@ -734,9 +711,9 @@ int pllb_score_host(pllb_handle h, const int32_t* hyp_tokens, const int64_t* off
     if (hyp_tokens[i] < 0 || hyp_tokens[i] >= h->d.vocab)
       return fail(PLLB_ERR_INVALID, "token id " + std::to_string(hyp_tokens[i]) + " at position " + std::to_string(i) +
                                         " is outside the vocabulary [0, " + std::to_string(h->d.vocab) + ")");
-  const int64_t b_tok = align_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
-  const int64_t b_pll = align_up(sizeof(double) * n_hyp, 256);
-  const int64_t b_lp = align_up(sizeof(float) * std::max<int64_t>(n_tok, 1), 256);
+  const int64_t b_tok = round_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
+  const int64_t b_pll = round_up(sizeof(double) * n_hyp, 256);
+  const int64_t b_lp = round_up(sizeof(float) * std::max<int64_t>(n_tok, 1), 256);
   RC(ensure_io(h, b_tok + b_pll + b_lp));
   uint8_t* base = reinterpret_cast<uint8_t*>(h->io_dev);
   int32_t* d_tok = reinterpret_cast<int32_t*>(base);
@@ -774,8 +751,8 @@ int pllb_score_cls_host(pllb_handle h, const int32_t* hyp_tokens, const int64_t*
     if (hyp_tokens[i] < 0 || hyp_tokens[i] >= h->d.vocab)
       return fail(PLLB_ERR_INVALID, "token id " + std::to_string(hyp_tokens[i]) + " is outside the vocabulary");
   const int H = h->d.hidden;
-  const int64_t b_tok = align_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
-  const int64_t b_out = align_up(sizeof(float) * n_hyp, 256), b_w = align_up(sizeof(float) * H, 256);
+  const int64_t b_tok = round_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
+  const int64_t b_out = round_up(sizeof(float) * n_hyp, 256), b_w = round_up(sizeof(float) * H, 256);
   RC(ensure_io(h, b_tok + b_out + b_w));
   uint8_t* base = reinterpret_cast<uint8_t*>(h->io_dev);
   int32_t* d_tok = reinterpret_cast<int32_t*>(base);
@@ -1001,9 +978,9 @@ int pllb_tokenize_host(const int32_t* table, int32_t table_size, const int32_t* 
   if (n_cp < 0 || (n_cp > 0 && (!cp || !out_ids))) return fail(PLLB_ERR_INVALID, "pllb_tokenize_host: bad offsets");
   for (int32_t i = 0; i < n_hyp; ++i)
     if (cp_off[i + 1] < cp_off[i]) return fail(PLLB_ERR_INVALID, "pllb_tokenize_host: offsets not ascending");
-  const int64_t b0 = align_up(4 * (int64_t)table_size, 256), b1 = align_up(4 * std::max<int64_t>(n_cp, 1), 256),
-                b2 = align_up(8 * (int64_t)(n_hyp + 1), 256), b3 = align_up(4 * (int64_t)n_hyp, 256),
-                b4 = align_up((int64_t)n_hyp, 256), b5 = b2, b6 = b1;
+  const int64_t b0 = round_up(4 * (int64_t)table_size, 256), b1 = round_up(4 * std::max<int64_t>(n_cp, 1), 256),
+                b2 = round_up(8 * (int64_t)(n_hyp + 1), 256), b3 = round_up(4 * (int64_t)n_hyp, 256),
+                b4 = round_up((int64_t)n_hyp, 256), b5 = b2, b6 = b1;
   uint8_t* base = nullptr;
   RC(get_scratch(b0 + b1 + b2 + b3 + b4 + b5 + b6, &base));
   int32_t* d_table = (int32_t*)base;
@@ -1050,9 +1027,9 @@ int pllb_levenshtein_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t
     if (pair_ref[i] < 0 || pair_ref[i] >= n_ref) return fail(PLLB_ERR_INVALID, "pllb_levenshtein_host: pair_ref out of range");
   }
   const int64_t n_rc = ref_off[n_ref], n_hc = hyp_off[n_pairs];
-  const int64_t b0 = align_up(4 * std::max<int64_t>(n_rc, 1), 256), b1 = align_up(8 * (int64_t)(n_ref + 1), 256),
-                b2 = align_up(4 * std::max<int64_t>(n_hc, 1), 256), b3 = align_up(8 * (int64_t)(n_pairs + 1), 256),
-                b4 = align_up(4 * (int64_t)n_pairs, 256), b5 = b4;
+  const int64_t b0 = round_up(4 * std::max<int64_t>(n_rc, 1), 256), b1 = round_up(8 * (int64_t)(n_ref + 1), 256),
+                b2 = round_up(4 * std::max<int64_t>(n_hc, 1), 256), b3 = round_up(8 * (int64_t)(n_pairs + 1), 256),
+                b4 = round_up(4 * (int64_t)n_pairs, 256), b5 = b4;
   uint8_t* base = nullptr;
   RC(get_scratch(b0 + b1 + b2 + b3 + b4 + b5, &base));
   int32_t* d_rc = (int32_t*)base;
@@ -1120,10 +1097,10 @@ int pllb_align_host(const int32_t* ref_cp, const int64_t* ref_off, int32_t n_ref
   int32_t warps = 0;
   int64_t slot_words = 0;
   align_shape(n_pairs, max_ref, max_hyp, &warps, &slot_words);
-  const int64_t b0 = align_up(4 * std::max<int64_t>(n_rc, 1), 256), b1 = align_up(8 * (int64_t)(n_ref + 1), 256),
-                b2 = align_up(4 * std::max<int64_t>(n_hc, 1), 256), b3 = align_up(8 * (int64_t)(n_pairs + 1), 256),
-                b4 = align_up(4 * (int64_t)n_pairs, 256), b5 = b3, b6 = align_up(std::max<int64_t>(n_ops, 1), 256),
-                b7 = b4, b8 = align_up(16 * (int64_t)n_pairs, 256), b9 = 8 * slot_words * warps;
+  const int64_t b0 = round_up(4 * std::max<int64_t>(n_rc, 1), 256), b1 = round_up(8 * (int64_t)(n_ref + 1), 256),
+                b2 = round_up(4 * std::max<int64_t>(n_hc, 1), 256), b3 = round_up(8 * (int64_t)(n_pairs + 1), 256),
+                b4 = round_up(4 * (int64_t)n_pairs, 256), b5 = b3, b6 = round_up(std::max<int64_t>(n_ops, 1), 256),
+                b7 = b4, b8 = round_up(16 * (int64_t)n_pairs, 256), b9 = 8 * slot_words * warps;
   uint8_t* base = nullptr;
   RC(get_scratch(b0 + b1 + b2 + b3 + b4 + b5 + b6 + b7 + b8 + b9, &base));
   int32_t* d_rc = (int32_t*)base;
@@ -1179,8 +1156,8 @@ int pllb_rescore_sweep_host(const double* am, const double* lm, const int64_t* l
   if (N <= 0 || W <= 0) return PLLB_OK;
   if (!am || !lm || !len || !weights || !out_argmax) return fail(PLLB_ERR_INVALID, "pllb_rescore_sweep_host: null argument");
   const int64_t n = (int64_t)N * n_best;
-  const int64_t b_d = align_up(8 * n, 256), b_i = align_up(4 * n, 256), b_w = align_up(8 * (int64_t)W, 256),
-                b_a = align_up(4 * (int64_t)W * N, 256);
+  const int64_t b_d = round_up(8 * n, 256), b_i = round_up(4 * n, 256), b_w = round_up(8 * (int64_t)W, 256),
+                b_a = round_up(4 * (int64_t)W * N, 256);
   uint8_t* base = nullptr;
   RC(get_scratch(3 * b_d + b_i + 2 * b_w + b_a, &base));
   double* d_am = (double*)base;

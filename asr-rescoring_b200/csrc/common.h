@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <cstdio>
 #include <string>
 #include <utility>
@@ -19,6 +20,9 @@ extern thread_local int64_t g_launch_counter;   // kernels launched by this libr
 // PLLB_ERR_INVALID unless the kernels support the model shape (scoring and training).  Hidden: library-internal,
 // so it does not join the exported symbols.
 __attribute__((visibility("hidden"))) int check_model_shape(const pllb_model_desc& d);
+// The device check of every create: PLLB_ERR_NO_DEVICE unless an sm_100 device is visible and `device` is sm_100.
+// Makes `device` current.
+__attribute__((visibility("hidden"))) int check_create_device(int device);
 
 #define PLLB_CUDA(expr)                                                                        \
   do {                                                                                         \
@@ -26,6 +30,31 @@ __attribute__((visibility("hidden"))) int check_model_shape(const pllb_model_des
     if (_e != cudaSuccess)                                                                     \
       return ::pllb::fail(PLLB_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));  \
   } while (0)
+
+// returns the error code of a library call that failed
+#define RC(expr)            \
+  do {                      \
+    int _rc = (expr);       \
+    if (_rc) return _rc;    \
+  } while (0)
+
+// cudaMalloc of max(count, 1) elements, zeroed when asked, recorded in the handle's owned / owned_bytes (its destroy
+// frees them; owned_bytes is what the workspace_bytes calls report).
+template <typename Ctx, typename T>
+int owned_alloc(Ctx* c, T** out, int64_t count, bool zero = false) {
+  void* p = nullptr;
+  const int64_t bytes = std::max<int64_t>(count, 1) * (int64_t)sizeof(T);
+  cudaError_t e = cudaMalloc(&p, (size_t)bytes);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(PLLB_ERR_OOM, "cudaMalloc of " + std::to_string(bytes) + " bytes failed: " + cudaGetErrorString(e));
+  }
+  if (zero) cudaMemset(p, 0, (size_t)bytes);
+  c->owned.push_back(p);
+  c->owned_bytes += bytes;
+  *out = reinterpret_cast<T*>(p);
+  return PLLB_OK;
+}
 
 #define PLLB_LAUNCH_CHECK(name)                                                                \
   do {                                                                                         \

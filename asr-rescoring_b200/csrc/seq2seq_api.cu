@@ -20,14 +20,6 @@ struct DecLayer {
   float *qkv_b, *o_b, *ln1_g, *ln1_b, *cq_b, *co_b, *ln2_g, *ln2_b, *ff1_b, *ff2_b, *ln3_g, *ln3_b;
 };
 
-#define RC(expr)            \
-  do {                      \
-    int _rc = (expr);       \
-    if (_rc) return _rc;    \
-  } while (0)
-
-inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
-
 }  // namespace
 
 struct pllb_s2s_ctx {
@@ -74,31 +66,16 @@ struct pllb_s2s_ctx {
 
 namespace {
 
-template <typename T>
-int s2s_alloc(pllb_s2s_ctx* c, T** out, int64_t count) {
-  void* p = nullptr;
-  const int64_t bytes = std::max<int64_t>(count, 1) * (int64_t)sizeof(T);
-  cudaError_t e = cudaMalloc(&p, (size_t)bytes);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail(PLLB_ERR_OOM, "cudaMalloc of " + std::to_string(bytes) + " bytes failed: " + cudaGetErrorString(e));
-  }
-  c->owned.push_back(p);
-  c->owned_bytes += bytes;
-  *out = reinterpret_cast<T*>(p);
-  return PLLB_OK;
-}
-
 int copy_f32(pllb_s2s_ctx* c, float** dst, const float* src, int64_t n, cudaStream_t s) {
   if (!src) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null weight pointer");
-  RC(s2s_alloc(c, dst, n));
+  RC(owned_alloc(c, dst, n));
   PLLB_CUDA(cudaMemcpyAsync(*dst, src, sizeof(float) * n, cudaMemcpyDeviceToDevice, s));
   return PLLB_OK;
 }
 
 // 16-bit copies of the row blocks srcs[i] ([rows_i, K] each) stacked in one [sum rows, K] operand
 int conv_stack(pllb_s2s_ctx* c, uint16_t** dst, std::initializer_list<const float*> srcs, int64_t block, cudaStream_t s) {
-  RC(s2s_alloc(c, dst, block * (int64_t)srcs.size()));
+  RC(owned_alloc(c, dst, block * (int64_t)srcs.size()));
   int64_t i = 0;
   for (const float* p : srcs) {
     if (!p) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null weight pointer");
@@ -109,7 +86,7 @@ int conv_stack(pllb_s2s_ctx* c, uint16_t** dst, std::initializer_list<const floa
 }
 
 int bias_stack(pllb_s2s_ctx* c, float** dst, std::initializer_list<const float*> srcs, int64_t block, cudaStream_t s) {
-  RC(s2s_alloc(c, dst, block * (int64_t)srcs.size()));
+  RC(owned_alloc(c, dst, block * (int64_t)srcs.size()));
   int64_t i = 0;
   for (const float* p : srcs) {
     if (!p) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null weight pointer");
@@ -353,8 +330,8 @@ int beam_state(pllb_s2s_ctx* c, const pllb_gen_desc* g, const pllb_beam_desc* bd
   const int K = g->num_beams, ML = g->max_length;
   const int64_t R = c->max_rows;
   const int64_t parts = R * 2 * c->tiles_v * (1 + ksel_of(K));
-  const int64_t b_i32 = align_up(sizeof(int32_t) * (R * ML * 5 + R * 3 + R + 1), 256);
-  const int64_t b_f32 = align_up(sizeof(float) * R * 2, 256);
+  const int64_t b_i32 = round_up(sizeof(int32_t) * (R * ML * 5 + R * 3 + R + 1), 256);
+  const int64_t b_f32 = round_up(sizeof(float) * R * 2, 256);
   const int64_t need = b_i32 + b_f32 + (int64_t)sizeof(float2) * parts;
   if (need > c->beam_cap) {
     PLLB_CUDA(cudaDeviceSynchronize());
@@ -551,44 +528,23 @@ int generate_beam_impl(pllb_s2s_ctx* c, const pllb_gen_desc* g, const pllb_beam_
   return PLLB_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int pllb_s2s_create(pllb_s2s* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* w, int32_t max_rows, int device) {
-  if (!out || !desc || !w || !w->enc.layers || !w->dec_layers || !w->shared)
-    return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null argument");
-  *out = nullptr;
-  const pllb_s2s_desc& d = *desc;
-  RC(check_s2s_desc(d));
-  if (max_rows < 0) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: max_rows < 0");
-  if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 device visible; libpllb200 has no CPU fallback");
-  PLLB_CUDA(cudaSetDevice(device));
-  int major = 0;
-  PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
-  if (major != 10) return fail(PLLB_ERR_NO_DEVICE, "device is not sm_100 (B200); libpllb200 has no other code path");
-  pllb_s2s_ctx* c = new pllb_s2s_ctx();
-  c->d = d;
-  c->device = device;
+// The weights and the workspace of a new generation handle (c->d and c->device set); on failure pllb_s2s_create
+// destroys it.
+int build_s2s_ctx(pllb_s2s_ctx* c, const pllb_s2s_weights* w, int32_t max_rows) {
+  const pllb_s2s_desc& d = c->d;
   c->fp16 = d.operand_dtype == 1;
   c->dt = c->fp16 ? DT_FP16 : DT_BF16;
   c->max_rows = max_rows > 0 ? max_rows : 8192;
   c->enc_cap = std::max<int64_t>((int64_t)c->max_rows * 32, d.enc_max_position);
   const int H = d.hidden, V = d.vocab, NL = d.dec_layers, I = d.dec_intermediate;
-  c->vocab_pad = (int)align_up(V, 256);
+  c->vocab_pad = (int)round_up(V, 256);
   c->tiles_v = c->vocab_pad / 256;
   cudaStream_t s = 0;
-  int rc = PLLB_OK;
-#define TRY(expr)                            \
-  do {                                       \
-    rc = (expr);                             \
-    if (rc) { pllb_s2s_destroy(c); return rc; } \
-  } while (0)
   // token table * embed_scale: the lookups of both embeddings (never the LM head)
-  TRY(s2s_alloc(c, &c->word, (int64_t)V * H));
-  TRY(launch_scale_copy(w->shared, c->word, (int64_t)V * H, d.embed_scale, s));
-  TRY(s2s_alloc(c, &c->type_zero, H));
-  if (cudaMemsetAsync(c->type_zero, 0, sizeof(float) * H, s) != cudaSuccess) TRY(fail(PLLB_ERR_CUDA, "memset"));
+  RC(owned_alloc(c, &c->word, (int64_t)V * H));
+  RC(launch_scale_copy(w->shared, c->word, (int64_t)V * H, d.embed_scale, s));
+  RC(owned_alloc(c, &c->type_zero, H));
+  if (cudaMemsetAsync(c->type_zero, 0, sizeof(float) * H, s) != cudaSuccess) return fail(PLLB_ERR_CUDA, "memset");
   {
     pllb_model_desc ed{};
     ed.num_layers = d.enc_layers;
@@ -606,80 +562,99 @@ int pllb_s2s_create(pllb_s2s* out, const pllb_s2s_desc* desc, const pllb_s2s_wei
     ew.word_emb = c->word;
     ew.type_emb = c->type_zero;
     ew.head_w = ew.head_b = ew.head_ln_g = ew.head_ln_b = ew.decoder_w = ew.decoder_b = nullptr;
-    if (cudaStreamSynchronize(s) != cudaSuccess) TRY(fail(PLLB_ERR_CUDA, "pllb_s2s_create: weight copy failed"));
-    TRY(pllb_create(&c->enc, &ed, &ew, c->enc_cap, device));
+    if (cudaStreamSynchronize(s) != cudaSuccess) return fail(PLLB_ERR_CUDA, "pllb_s2s_create: weight copy failed");
+    RC(pllb_create(&c->enc, &ed, &ew, c->enc_cap, c->device));
   }
-  TRY(copy_f32(c, &c->dec_pos, w->dec_pos_emb, (int64_t)d.dec_max_position * H, s));
-  TRY(copy_f32(c, &c->dec_ln_g, w->dec_emb_ln_g, H, s));
-  TRY(copy_f32(c, &c->dec_ln_b, w->dec_emb_ln_b, H, s));
+  RC(copy_f32(c, &c->dec_pos, w->dec_pos_emb, (int64_t)d.dec_max_position * H, s));
+  RC(copy_f32(c, &c->dec_ln_g, w->dec_emb_ln_g, H, s));
+  RC(copy_f32(c, &c->dec_ln_b, w->dec_emb_ln_b, H, s));
   c->layers.resize(NL);
   const int64_t HH = (int64_t)H * H;
   std::vector<const float*> ckw, ckb;
   for (int l = 0; l < NL; ++l) {
     const pllb_dec_layer_weights& lw = w->dec_layers[l];
     DecLayer& L = c->layers[l];
-    TRY(conv_stack(c, &L.qkv_w, {lw.q_w, lw.k_w, lw.v_w}, HH, s));
-    TRY(bias_stack(c, &L.qkv_b, {lw.q_b, lw.k_b, lw.v_b}, H, s));
-    TRY(conv_stack(c, &L.o_w, {lw.o_w}, HH, s));
-    TRY(copy_f32(c, &L.o_b, lw.o_b, H, s));
-    TRY(copy_f32(c, &L.ln1_g, lw.self_ln_g, H, s));
-    TRY(copy_f32(c, &L.ln1_b, lw.self_ln_b, H, s));
-    TRY(conv_stack(c, &L.cq_w, {lw.cq_w}, HH, s));
-    TRY(copy_f32(c, &L.cq_b, lw.cq_b, H, s));
-    TRY(conv_stack(c, &L.co_w, {lw.co_w}, HH, s));
-    TRY(copy_f32(c, &L.co_b, lw.co_b, H, s));
-    TRY(copy_f32(c, &L.ln2_g, lw.cross_ln_g, H, s));
-    TRY(copy_f32(c, &L.ln2_b, lw.cross_ln_b, H, s));
-    TRY(conv_stack(c, &L.ff1_w, {lw.ff1_w}, (int64_t)I * H, s));
-    TRY(copy_f32(c, &L.ff1_b, lw.ff1_b, I, s));
-    TRY(conv_stack(c, &L.ff2_w, {lw.ff2_w}, (int64_t)H * I, s));
-    TRY(copy_f32(c, &L.ff2_b, lw.ff2_b, H, s));
-    TRY(copy_f32(c, &L.ln3_g, lw.final_ln_g, H, s));
-    TRY(copy_f32(c, &L.ln3_b, lw.final_ln_b, H, s));
+    RC(conv_stack(c, &L.qkv_w, {lw.q_w, lw.k_w, lw.v_w}, HH, s));
+    RC(bias_stack(c, &L.qkv_b, {lw.q_b, lw.k_b, lw.v_b}, H, s));
+    RC(conv_stack(c, &L.o_w, {lw.o_w}, HH, s));
+    RC(copy_f32(c, &L.o_b, lw.o_b, H, s));
+    RC(copy_f32(c, &L.ln1_g, lw.self_ln_g, H, s));
+    RC(copy_f32(c, &L.ln1_b, lw.self_ln_b, H, s));
+    RC(conv_stack(c, &L.cq_w, {lw.cq_w}, HH, s));
+    RC(copy_f32(c, &L.cq_b, lw.cq_b, H, s));
+    RC(conv_stack(c, &L.co_w, {lw.co_w}, HH, s));
+    RC(copy_f32(c, &L.co_b, lw.co_b, H, s));
+    RC(copy_f32(c, &L.ln2_g, lw.cross_ln_g, H, s));
+    RC(copy_f32(c, &L.ln2_b, lw.cross_ln_b, H, s));
+    RC(conv_stack(c, &L.ff1_w, {lw.ff1_w}, (int64_t)I * H, s));
+    RC(copy_f32(c, &L.ff1_b, lw.ff1_b, I, s));
+    RC(conv_stack(c, &L.ff2_w, {lw.ff2_w}, (int64_t)H * I, s));
+    RC(copy_f32(c, &L.ff2_b, lw.ff2_b, H, s));
+    RC(copy_f32(c, &L.ln3_g, lw.final_ln_g, H, s));
+    RC(copy_f32(c, &L.ln3_b, lw.final_ln_b, H, s));
   }
-  TRY(s2s_alloc(c, &c->ckv_w, (int64_t)NL * 2 * HH));
-  TRY(s2s_alloc(c, &c->ckv_b, (int64_t)NL * 2 * H));
+  RC(owned_alloc(c, &c->ckv_w, (int64_t)NL * 2 * HH));
+  RC(owned_alloc(c, &c->ckv_b, (int64_t)NL * 2 * H));
   for (int l = 0; l < NL; ++l) {
     const pllb_dec_layer_weights& lw = w->dec_layers[l];
-    if (!lw.ck_w || !lw.cv_w || !lw.ck_b || !lw.cv_b) TRY(fail(PLLB_ERR_INVALID, "pllb_s2s_create: null weight pointer"));
-    TRY(launch_f32_to_bf16(lw.ck_w, c->ckv_w + (int64_t)l * 2 * HH, HH, c->fp16, s));
-    TRY(launch_f32_to_bf16(lw.cv_w, c->ckv_w + (int64_t)l * 2 * HH + HH, HH, c->fp16, s));
+    if (!lw.ck_w || !lw.cv_w || !lw.ck_b || !lw.cv_b) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null weight pointer");
+    RC(launch_f32_to_bf16(lw.ck_w, c->ckv_w + (int64_t)l * 2 * HH, HH, c->fp16, s));
+    RC(launch_f32_to_bf16(lw.cv_w, c->ckv_w + (int64_t)l * 2 * HH + HH, HH, c->fp16, s));
     if (cudaMemcpyAsync(c->ckv_b + (int64_t)l * 2 * H, lw.ck_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s) ||
         cudaMemcpyAsync(c->ckv_b + (int64_t)l * 2 * H + H, lw.cv_b, sizeof(float) * H, cudaMemcpyDeviceToDevice, s))
-      TRY(fail(PLLB_ERR_CUDA, "pllb_s2s_create: bias copy failed"));
+      return fail(PLLB_ERR_CUDA, "pllb_s2s_create: bias copy failed");
   }
-  if (!w->final_logits_bias) TRY(fail(PLLB_ERR_INVALID, "pllb_s2s_create: final_logits_bias is null"));
-  TRY(s2s_alloc(c, &c->head_w, (int64_t)c->vocab_pad * H));
-  TRY(s2s_alloc(c, &c->head_b, c->vocab_pad));
+  if (!w->final_logits_bias) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: final_logits_bias is null");
+  RC(owned_alloc(c, &c->head_w, (int64_t)c->vocab_pad * H));
+  RC(owned_alloc(c, &c->head_b, c->vocab_pad));
   if (cudaMemsetAsync(c->head_w, 0, sizeof(uint16_t) * (size_t)c->vocab_pad * H, s) ||
       cudaMemsetAsync(c->head_b, 0, sizeof(float) * c->vocab_pad, s) ||
       cudaMemcpyAsync(c->head_b, w->final_logits_bias, sizeof(float) * V, cudaMemcpyDeviceToDevice, s))
-    TRY(fail(PLLB_ERR_CUDA, "pllb_s2s_create: head copy failed"));
-  TRY(launch_f32_to_bf16(w->shared, c->head_w, (int64_t)V * H, c->fp16, s));
+    return fail(PLLB_ERR_CUDA, "pllb_s2s_create: head copy failed");
+  RC(launch_f32_to_bf16(w->shared, c->head_w, (int64_t)V * H, c->fp16, s));
   // chunk workspace
   const int64_t R = c->max_rows, E = c->enc_cap;
-  TRY(s2s_alloc(c, &c->enc_f32, E * H));
-  TRY(s2s_alloc(c, &c->enc16, E * H));
-  TRY(s2s_alloc(c, &c->ckv, E * 2 * H * NL));
-  TRY(s2s_alloc(c, &c->hid32, align_up(R, 256) * H));     // T32 layout, padded to the LayerNorm clusters' blocks
-  TRY(s2s_alloc(c, &c->hid16, R * H));
-  TRY(s2s_alloc(c, &c->wide, R * std::max(3 * H, I)));
-  TRY(s2s_alloc(c, &c->ctx, R * H));
-  TRY(s2s_alloc(c, &c->partials, R * 2 * c->tiles_v));
-  TRY(s2s_alloc(c, &c->forced_logit, R));
-  TRY(s2s_alloc(c, &c->force_col, R));
-  TRY(s2s_alloc(c, &c->done, 1));
-  TRY(s2s_alloc(c, &c->enc_meta, 2 * R));
+  RC(owned_alloc(c, &c->enc_f32, E * H));
+  RC(owned_alloc(c, &c->enc16, E * H));
+  RC(owned_alloc(c, &c->ckv, E * 2 * H * NL));
+  RC(owned_alloc(c, &c->hid32, round_up(R, 256) * H));     // T32 layout, padded to the LayerNorm clusters' blocks
+  RC(owned_alloc(c, &c->hid16, R * H));
+  RC(owned_alloc(c, &c->wide, R * std::max(3 * H, I)));
+  RC(owned_alloc(c, &c->ctx, R * H));
+  RC(owned_alloc(c, &c->partials, R * 2 * c->tiles_v));
+  RC(owned_alloc(c, &c->forced_logit, R));
+  RC(owned_alloc(c, &c->force_col, R));
+  RC(owned_alloc(c, &c->done, 1));
+  RC(owned_alloc(c, &c->enc_meta, 2 * R));
   if (cudaHostAlloc(&c->meta_host, sizeof(int32_t) * 2 * R, cudaHostAllocDefault) != cudaSuccess ||
       cudaHostAlloc(&c->done_host, sizeof(int32_t) * 2, cudaHostAllocDefault) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_done[0], cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&c->ev_done[1], cudaEventDisableTiming) != cudaSuccess)
-    TRY(fail(PLLB_ERR_CUDA, "pllb_s2s_create: pinned buffers / events"));
-#undef TRY
+    return fail(PLLB_ERR_CUDA, "pllb_s2s_create: pinned buffers / events");
   cudaError_t e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) {
+  if (e != cudaSuccess) return fail(PLLB_ERR_CUDA, std::string("pllb_s2s_create: ") + cudaGetErrorString(e));
+  return PLLB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int pllb_s2s_create(pllb_s2s* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* w, int32_t max_rows, int device) {
+  if (!out || !desc || !w || !w->enc.layers || !w->dec_layers || !w->shared)
+    return fail(PLLB_ERR_INVALID, "pllb_s2s_create: null argument");
+  *out = nullptr;
+  const pllb_s2s_desc& d = *desc;
+  RC(check_s2s_desc(d));
+  if (max_rows < 0) return fail(PLLB_ERR_INVALID, "pllb_s2s_create: max_rows < 0");
+  RC(check_create_device(device));
+  pllb_s2s_ctx* c = new pllb_s2s_ctx();
+  c->d = d;
+  c->device = device;
+  const int rc = build_s2s_ctx(c, w, max_rows);
+  if (rc) {
     pllb_s2s_destroy(c);
-    return fail(PLLB_ERR_CUDA, std::string("pllb_s2s_create: ") + cudaGetErrorString(e));
+    return rc;
   }
   *out = c;
   return PLLB_OK;
@@ -747,10 +722,10 @@ int pllb_generate_host(pllb_s2s h, const pllb_gen_desc* gen, const int32_t* toke
                                         " is outside the vocabulary [0, " + std::to_string(h->d.vocab) + ")");
   PLLB_CUDA(cudaSetDevice(h->device));
   const int64_t ML = gen->max_length;
-  const int64_t b_tok = align_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
-  const int64_t b_ids = align_up(sizeof(int32_t) * n * ML, 256);
-  const int64_t b_len = align_up(sizeof(int32_t) * n, 256);
-  const int64_t b_lg = out_logit ? align_up(sizeof(float) * n * ML, 256) : 0;
+  const int64_t b_tok = round_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
+  const int64_t b_ids = round_up(sizeof(int32_t) * n * ML, 256);
+  const int64_t b_len = round_up(sizeof(int32_t) * n, 256);
+  const int64_t b_lg = out_logit ? round_up(sizeof(float) * n * ML, 256) : 0;
   const int64_t need = b_tok + b_ids + b_len + b_lg;
   if (need > h->io_cap) {
     PLLB_CUDA(cudaDeviceSynchronize());
@@ -798,10 +773,10 @@ int pllb_generate_beam_host(pllb_s2s h, const pllb_gen_desc* gen, const pllb_bea
                                         " is outside the vocabulary [0, " + std::to_string(h->d.vocab) + ")");
   PLLB_CUDA(cudaSetDevice(h->device));
   const int64_t ML = gen->max_length, nr = beam->num_return_sequences;
-  const int64_t b_tok = align_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
-  const int64_t b_ids = align_up(sizeof(int32_t) * n * nr * ML, 256);
-  const int64_t b_len = align_up(sizeof(int32_t) * n * nr, 256);
-  const int64_t b_sc = align_up(sizeof(float) * n * nr, 256);
+  const int64_t b_tok = round_up(sizeof(int32_t) * std::max<int64_t>(n_tok, 1), 256);
+  const int64_t b_ids = round_up(sizeof(int32_t) * n * nr * ML, 256);
+  const int64_t b_len = round_up(sizeof(int32_t) * n * nr, 256);
+  const int64_t b_sc = round_up(sizeof(float) * n * nr, 256);
   const int64_t need = b_tok + b_ids + b_len + b_sc;
   if (need > h->io_cap) {
     PLLB_CUDA(cudaDeviceSynchronize());

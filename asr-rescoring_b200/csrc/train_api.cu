@@ -55,29 +55,35 @@ struct DLayer {
 // decoder layer l at 8 * (enc_layers + 1 + l) + {SITE_ATT, SITE_AO, SITE_FF2, DSITE_XATT, DSITE_XAO}
 enum DSite : uint32_t { DSITE_XATT = 5, DSITE_XAO = 6 };
 
+// MLM: pllb_train_create; CLS: RescoreBert, pllb_cls_train_create; S2S: CorrectBart, pllb_s2s_train_create
+enum Kind { KIND_MLM, KIND_CLS, KIND_S2S };
+
 }  // namespace
 
 struct pllb_trainer_ctx {
-  pllb_model_desc d{};
+  Kind kind = KIND_MLM;
+  pllb_model_desc d{};     // an s2s trainer's encoder, in BERT form
   pllb_train_desc t{};
   int device = 0;
   int Vp = 0;
-  int64_t cap_rows = 0, cap_rows_pad = 0;
+  int64_t cap_rows = 0;
   std::vector<void*> owned;
   int64_t owned_bytes = 0;
   // flat fp32 buffers, one layout: parameters, gradients, Adam first / second moments
   float *P = nullptr, *G = nullptr, *M = nullptr, *V = nullptr;
   int64_t n_flat = 0;
-  Span word, pos, type, emb_g, emb_b, head_w, head_b, head_g, head_be, dec_b;
+  Span word, pos, type, emb_g, emb_b;
   std::vector<TLayer> L;
-  __nv_bfloat16 *head16 = nullptr, *headT16 = nullptr, *E16 = nullptr, *ET16 = nullptr;
   // batch inputs
-  int32_t *ids = nullptr, *labels = nullptr, *n_valid = nullptr;
+  int32_t *ids = nullptr, *n_valid = nullptr;
   int32_t* host_stage = nullptr;     // pinned
   // stash outside the layers
-  float *xhat_e = nullptr, *rstd_e = nullptr, *t_f32 = nullptr, *xhat_h = nullptr, *rstd_h = nullptr;
-  __nv_bfloat16 *xlast16 = nullptr, *tn16 = nullptr, *dlogits16 = nullptr;
-  float *logits = nullptr, *loss_rows = nullptr, *loss_dev = nullptr;
+  float *xhat_e = nullptr, *rstd_e = nullptr, *loss_dev = nullptr;
+  __nv_bfloat16* xlast16 = nullptr;       // bf16 encoder output (MLM and S2S)
+  // the LM head over the word embedding (MLM and S2S): operand copies, labels, [R, Vp] logits and their gradient
+  __nv_bfloat16 *E16 = nullptr, *ET16 = nullptr, *dlogits16 = nullptr;
+  int32_t* labels = nullptr;
+  float *logits = nullptr, *loss_rows = nullptr;
   // scratch
   float *h32 = nullptr, *y32 = nullptr, *dh32 = nullptr, *dz32 = nullptr, *dzd32 = nullptr, *Dq = nullptr, *zeros = nullptr,
         *colsum_scratch = nullptr;
@@ -97,16 +103,18 @@ struct pllb_trainer_ctx {
   struct GraphEntry { int seen = 0; cudaGraphExec_t exec = nullptr; int64_t launches = 0; };
   std::unordered_map<uint64_t, GraphEntry> graphs;
   int64_t graph_replays = 0;
-  // RescoreBert trainer (pllb_cls_train_create): Linear(H, 1) on the [CLS] row instead of the MLM head.  The flat
-  // buffers hold the embeddings, the layers and lin_w / lin_b; there are no head / decoder copies and no logits.
-  bool cls = false;
+  // KIND_MLM: the BertForMaskedLM head; the decoder weight is `word` (tied), its operand copies are E16 / ET16.
+  Span head_w, head_b, head_g, head_be, dec_b;
+  __nv_bfloat16 *head16 = nullptr, *headT16 = nullptr, *tn16 = nullptr;
+  float *t_f32 = nullptr, *xhat_h = nullptr, *rstd_h = nullptr;
+  // KIND_CLS: Linear(H, 1) on the [CLS] row instead of the MLM head.  The flat buffers hold the embeddings, the layers
+  // and lin_w / lin_b; there are no head / decoder copies and no logits.
   Span lin_w, lin_b;
   pllb_cls_loss_desc loss{};
   int32_t* group = nullptr;                                                 // [max_rows]
   float *target = nullptr, *am = nullptr, *err = nullptr, *scores = nullptr, *dscore = nullptr;   // [max_rows] each
-  // CorrectBart trainer (pllb_s2s_train_create): word = model.shared (Vp rows, rows >= vocab zero), pos / emb_g / emb_b
-  // = the encoder's embed_positions (whole table) and layernorm_embedding, L = the encoder layers (BERT form).
-  bool s2s = false;
+  // KIND_S2S: word = model.shared (Vp rows, rows >= vocab zero), pos / emb_g / emb_b = the encoder's embed_positions
+  // (whole table) and layernorm_embedding, L = the encoder layers (BERT form); the decoder below.
   pllb_s2s_desc sd{};
   int32_t decoder_start_id = 0;
   int cap_batch = 0, cap_enc = 0, cap_dec = 0;
@@ -121,28 +129,6 @@ struct pllb_trainer_ctx {
 };
 
 namespace {
-
-#define RC(expr)            \
-  do {                      \
-    int _rc = (expr);       \
-    if (_rc) return _rc;    \
-  } while (0)
-
-template <typename T>
-int talloc(pllb_trainer_ctx* c, T** out, int64_t count, bool zero = false) {
-  void* p = nullptr;
-  const int64_t bytes = std::max<int64_t>(count, 1) * (int64_t)sizeof(T);
-  cudaError_t e = cudaMalloc(&p, (size_t)bytes);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail(PLLB_ERR_OOM, "cudaMalloc of " + std::to_string(bytes) + " bytes failed: " + cudaGetErrorString(e));
-  }
-  if (zero) cudaMemset(p, 0, (size_t)bytes);
-  c->owned.push_back(p);
-  c->owned_bytes += bytes;
-  *out = reinterpret_cast<T*>(p);
-  return PLLB_OK;
-}
 
 Span take(int64_t& cursor, int64_t n) {
   Span s{cursor, n};
@@ -167,7 +153,7 @@ int refresh_all(pllb_trainer_ctx* c, cudaStream_t s) {
     RC(refresh_weight(c, l.ff1_w, I, H, l.ff116, l.ff1T16, s));
     RC(refresh_weight(c, l.ff2_w, H, I, l.ff216, l.ff2T16, s));
   }
-  if (c->s2s) {
+  if (c->kind == KIND_S2S) {
     const int Id = c->sd.dec_intermediate;
     for (auto& l : c->D) {
       RC(refresh_weight(c, l.qkv_w, 3 * H, H, l.qkv16, l.qkvT16, s));
@@ -180,7 +166,7 @@ int refresh_all(pllb_trainer_ctx* c, cudaStream_t s) {
     RC(refresh_weight(c, c->ckv_w, 2 * H * c->sd.dec_layers, H, c->ckv16, c->ckvT16, s));
     return refresh_weight(c, c->word, c->Vp, H, c->E16, c->ET16, s);     // the LM head is model.shared
   }
-  if (c->cls) return PLLB_OK;     // no MLM head, no tied decoder
+  if (c->kind == KIND_CLS) return PLLB_OK;     // no MLM head, no tied decoder
   RC(refresh_weight(c, c->head_w, H, H, c->head16, c->headT16, s));
   RC(refresh_weight(c, c->word, c->Vp, H, c->E16, c->ET16, s));
   return PLLB_OK;
@@ -202,9 +188,9 @@ int linear_bwd(pllb_trainer_ctx* c, const float* dy32, const __nv_bfloat16* x16,
 
 int copy_in(pllb_trainer_ctx* c, Span dst, const float* src, int64_t n, int64_t dst_off) {
   if (!src)
-    return fail(PLLB_ERR_INVALID, c->s2s ? "pllb_s2s_train_create: a weight pointer is null"
-                                  : c->cls ? "pllb_cls_train_create: a weight pointer is null"
-                                           : "pllb_train_create: a weight pointer is null (the MLM head is required)");
+    return fail(PLLB_ERR_INVALID, c->kind == KIND_S2S ? "pllb_s2s_train_create: a weight pointer is null"
+                                  : c->kind == KIND_CLS ? "pllb_cls_train_create: a weight pointer is null"
+                                                        : "pllb_train_create: a weight pointer is null (the MLM head is required)");
   PLLB_CUDA(cudaMemcpyAsync(c->P + dst.off + dst_off, src, sizeof(float) * n, cudaMemcpyDeviceToDevice, 0));
   return PLLB_OK;
 }
@@ -283,7 +269,7 @@ int visit_params(const pllb_trainer_ctx* c, const pllb_weights* w, const float* 
   RC(fn(c->emb_g, w->emb_ln_g, H, 0));
   RC(fn(c->emb_b, w->emb_ln_b, H, 0));
   RC(visit_enc_layers(c, w, fn));
-  if (c->cls) {
+  if (c->kind == KIND_CLS) {
     RC(fn(c->lin_w, lin_w, H, 0)); RC(fn(c->lin_b, lin_b, 1, 0));
   } else {
     RC(fn(c->head_w, w->head_w, HH, 0)); RC(fn(c->head_b, w->head_b, H, 0));
@@ -318,7 +304,7 @@ int encoder_fwd(pllb_trainer_ctx* c, int B, int T, const TrainDrop& hd, const Tr
   const int H = d.hidden, I = d.intermediate, NH = d.num_heads, NL = d.num_layers;
   const int R = B * T;
   float* P = c->P;
-  if (c->s2s)
+  if (c->kind == KIND_S2S)
     RC(launch_train_bart_embed(c->ids, T, P + c->word.off, c->sd.embed_scale, P + c->pos.off + 2 * H, P + c->emb_g.off,
                                P + c->emb_b.off, d.ln_eps, R, H, hd, SITE_EMB, c->h32, c->L[0].x16, c->xhat_e, c->rstd_e, s));
   else
@@ -377,7 +363,7 @@ int encoder_bwd(pllb_trainer_ctx* c, int B, int T, const TrainDrop& hd, const Tr
   RC(launch_train_ln_bwd(c->dh32, have_res ? c->dz32 : nullptr, P + c->emb_g.off, c->xhat_e, c->rstd_e, R, H, hd,
                          hd.thresh != 0 ? (int)SITE_EMB : -1, -1, c->dz32, nullptr, s));
   RC(launch_train_colsum(c->dh32, false, c->xhat_e, R, H, G + c->emb_b.off, G + c->emb_g.off, c->colsum_scratch, s));
-  if (c->s2s)      // adds to G[shared] after the LM head and the decoder lookup
+  if (c->kind == KIND_S2S)      // adds to G[shared] after the LM head and the decoder lookup
     return launch_train_bart_embed_bwd(c->dz32, c->ids, B, T, H, d.max_position, c->t.pad_id, c->sd.embed_scale,
                                        G + c->word.off, G + c->pos.off + 2 * H, s);
   RC(launch_train_embed_bwd(c->dz32, c->ids, B, T, H, d.max_position, c->t.pad_id, G + c->word.off, G + c->pos.off,
@@ -552,8 +538,8 @@ int enqueue_s2s_step(pllb_trainer_ctx* c, int B, int Te, int Td, int mode, cudaS
 }
 
 int enqueue(pllb_trainer_ctx* c, int B, int T, int T2, int mode, cudaStream_t s) {
-  if (c->s2s) return enqueue_s2s_step(c, B, T, T2, mode, s);
-  return c->cls ? enqueue_cls_step(c, B, T, mode, s) : enqueue_mlm_step(c, B, T, mode, s);
+  if (c->kind == KIND_S2S) return enqueue_s2s_step(c, B, T, T2, mode, s);
+  return c->kind == KIND_CLS ? enqueue_cls_step(c, B, T, mode, s) : enqueue_mlm_step(c, B, T, mode, s);
 }
 
 // T2: the decoder length of an s2s step (0 otherwise); one graph per (B, T, T2, mode)
@@ -567,8 +553,8 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
   c->params_host->adam_step_size = (float)((double)c->t.lr / bc1);
   c->params_host->adam_bc2_sqrt = (float)std::sqrt(bc2);
   PLLB_CUDA(cudaMemcpyAsync(c->params_dev, c->params_host, sizeof(TrainStepParams), cudaMemcpyHostToDevice, s));
-  const uint64_t key = c->s2s ? ((uint64_t)(uint32_t)B << 42) | ((uint64_t)(uint32_t)T << 22) | ((uint64_t)(uint32_t)T2 << 2) | (uint64_t)mode
-                              : ((uint64_t)(uint32_t)B << 34) | ((uint64_t)(uint32_t)T << 2) | (uint64_t)mode;
+  // T and T2 are at most 1024 for every kind (the limits of the create calls) and mode < 3: one key per shape
+  const uint64_t key = (((uint64_t)B * 1025 + (uint64_t)T) * 1025 + (uint64_t)T2) * 3 + (uint64_t)mode;
   pllb_trainer_ctx::GraphEntry* ge = c->use_graph ? &c->graphs[key] : nullptr;
   if (ge && ge->exec) {
     PLLB_CUDA(cudaGraphLaunch(ge->exec, s));
@@ -611,49 +597,68 @@ int step_impl(pllb_trainer_ctx* c, int B, int T, int mode, float* out_loss_host,
   return PLLB_OK;
 }
 
-enum Kind { KIND_MLM, KIND_CLS, KIND_S2S };
-Kind kind_of(const pllb_trainer_ctx* c) { return c->s2s ? KIND_S2S : c->cls ? KIND_CLS : KIND_MLM; }
-
 // `who` takes trainers of kind k (k2 too when given); any other kind is PLLB_ERR_INVALID
 int require_kind(const pllb_trainer_ctx* c, Kind k, const char* who, int k2 = -1) {
   if (!c) return fail(PLLB_ERR_INVALID, std::string(who) + ": null trainer");
-  const Kind ck = kind_of(c);
-  if (ck == k || (int)ck == k2) return PLLB_OK;
+  if (c->kind == k || (int)c->kind == k2) return PLLB_OK;
   static const char* takes[] = {": an MLM trainer takes pllb_train_step_host / _row_losses_host / _export / _export_grads",
                                 ": a RescoreBert trainer takes pllb_cls_train_step_host / _export / _export_grads",
                                 ": a CorrectBart trainer takes pllb_s2s_train_step_host / _export / _export_grads and "
                                 "pllb_train_row_losses_host"};
-  return fail(PLLB_ERR_INVALID, std::string(who) + takes[ck]);
+  return fail(PLLB_ERR_INVALID, std::string(who) + takes[c->kind]);
 }
 
-// state_dict tensors (and lin_w / lin_b of a RescoreBert trainer) <- the parameters or the gradients
-int export_params(pllb_trainer c, bool cls, bool grads, const pllb_weights* w, const float* lin_w, const float* lin_b,
-                  const char* who) {
-  if (!c || !w || !w->layers) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
-  RC(require_kind(c, cls ? KIND_CLS : KIND_MLM, who));
+// The caller's state_dict tensors <- the parameters or (grads) the gradients of the last step: w (and lin_w / lin_b of
+// a RescoreBert trainer) as visit_params walks them, or sw of a CorrectBart trainer as visit_s2s_params walks them.
+int export_params(pllb_trainer c, Kind kind, bool grads, const pllb_weights* w, const float* lin_w, const float* lin_b,
+                  const pllb_s2s_weights* sw, const char* who) {
+  RC(require_kind(c, kind, who));
+  if (kind == KIND_S2S ? !sw || !sw->enc.layers || !sw->dec_layers : !w || !w->layers)
+    return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
   const float* buf = grads ? c->G : c->P;
+  auto out = [buf](Span s, const float* dst, int64_t n, int64_t off) { return copy_out(buf, s, dst, n, off); };
   PLLB_CUDA(cudaSetDevice(c->device));
   PLLB_CUDA(cudaStreamSynchronize(c->stream));
-  RC(visit_params(c, w, lin_w, lin_b,
-                  [buf](Span s, const float* dst, int64_t n, int64_t off) { return copy_out(buf, s, dst, n, off); }));
-  // the decoder weight is the word-embedding matrix (tied): written only when the caller keeps a separate tensor
-  if (!c->cls && w->decoder_w && w->decoder_w != w->word_emb)
-    RC(copy_out(buf, c->word, w->decoder_w, (int64_t)c->d.vocab * c->d.hidden));
+  if (kind == KIND_S2S) {
+    RC(visit_s2s_params(c, sw, out));
+    if (sw->final_logits_bias) {       // a buffer: the given values, no gradient
+      float* dst = const_cast<float*>(sw->final_logits_bias);
+      if (grads) PLLB_CUDA(cudaMemsetAsync(dst, 0, sizeof(float) * c->sd.vocab, 0));
+      else PLLB_CUDA(cudaMemcpyAsync(dst, c->flb, sizeof(float) * c->sd.vocab, cudaMemcpyDeviceToDevice, 0));
+    }
+  } else {
+    RC(visit_params(c, w, lin_w, lin_b, out));
+    // the decoder weight is the word-embedding matrix (tied): written only when the caller keeps a separate tensor
+    if (kind == KIND_MLM && w->decoder_w != w->word_emb) RC(out(c->word, w->decoder_w, (int64_t)c->d.vocab * c->d.hidden, 0));
+  }
   PLLB_CUDA(cudaStreamSynchronize(0));
   return PLLB_OK;
 }
 
-// The checks of a batch both step entry points share.  The reference's embedding lookup raises on an id outside the
-// vocabulary.
+// The checks of a batch every step entry point shares, in this order: the arguments, the length limit
+// (PLLB_ERR_TOO_LONG), the capacity (PLLB_ERR_OOM), the token ids, n_valid.  T2: the decoder length of an s2s batch
+// (0 otherwise).  The reference's embedding lookup raises on an id outside the vocabulary.
 int check_batch(const pllb_trainer_ctx* c, const char* who, const int32_t* ids, const int32_t* n_valid, int B, int T,
-                int mode) {
-  if (!ids || !n_valid || B < 1 || T < 1 || mode < 0 || mode > 2) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
-  if (T > c->t.max_seq)
-    return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
-                                       std::to_string(c->t.max_seq));
-  if ((int64_t)B * T > c->cap_rows)
-    return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
-                                  std::to_string(c->cap_rows));
+                int T2, int mode) {
+  if (!ids || !n_valid || B < 1 || T < 1 || (c->kind == KIND_S2S && T2 < 1) || mode < 0 || mode > 2)
+    return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
+  if (c->kind == KIND_S2S) {
+    if (T > c->sd.enc_max_position || T2 > c->sd.dec_max_position)
+      return fail(PLLB_ERR_TOO_LONG, std::string(who) + ": T_enc " + std::to_string(T) + " / T_dec " + std::to_string(T2) +
+                                         " above the position tables (" + std::to_string(c->sd.enc_max_position) + " / " +
+                                         std::to_string(c->sd.dec_max_position) + ")");
+    if (B > c->cap_batch || T > c->cap_enc || T2 > c->cap_dec)
+      return fail(PLLB_ERR_OOM, std::string(who) + ": batch [" + std::to_string(B) + ", " + std::to_string(T) + ", " +
+                                    std::to_string(T2) + "] above the capacity given at create [" + std::to_string(c->cap_batch) +
+                                    ", " + std::to_string(c->cap_enc) + ", " + std::to_string(c->cap_dec) + "]");
+  } else {
+    if (T > c->t.max_seq)
+      return fail(PLLB_ERR_TOO_LONG, "batch of " + std::to_string(T) + " positions; the trainer was created for " +
+                                         std::to_string(c->t.max_seq));
+    if ((int64_t)B * T > c->cap_rows)
+      return fail(PLLB_ERR_OOM, "batch of " + std::to_string((int64_t)B * T) + " rows; the trainer was created for " +
+                                    std::to_string(c->cap_rows));
+  }
   for (int i = 0; i < B * T; ++i)
     if (ids[i] < 0 || ids[i] >= c->d.vocab) return fail(PLLB_ERR_INVALID, "token id outside the vocabulary at row " + std::to_string(i));
   for (int b = 0; b < B; ++b)
@@ -675,38 +680,85 @@ int upload(pllb_trainer_ctx* c, cudaStream_t s, std::initializer_list<Upload> ar
   return PLLB_OK;
 }
 
+// the flat layout of the encoder layers (q / k / v stacked in qkv_w and qkv_b)
+void take_enc_layers(pllb_trainer_ctx* c, int64_t& cur) {
+  const int H = c->d.hidden, I = c->d.intermediate;
+  const int64_t HH = (int64_t)H * H;
+  c->L.resize(c->d.num_layers);
+  for (auto& l : c->L) {
+    l.qkv_w = take(cur, 3 * HH); l.qkv_b = take(cur, 3 * H);
+    l.ao_w = take(cur, HH); l.ao_b = take(cur, H); l.ao_g = take(cur, H); l.ao_be = take(cur, H);
+    l.ff1_w = take(cur, (int64_t)I * H); l.ff1_b = take(cur, I);
+    l.ff2_w = take(cur, (int64_t)H * I); l.ff2_b = take(cur, H); l.out_g = take(cur, H); l.out_be = take(cur, H);
+  }
+}
+
+// the flat buffers P / G / M / V of the n floats the layout took, zeroed
+int alloc_flat(pllb_trainer_ctx* c, int64_t n) {
+  c->n_flat = n;
+  RC(owned_alloc(c, &c->P, n, true));
+  RC(owned_alloc(c, &c->G, n, true));
+  RC(owned_alloc(c, &c->M, n, true));
+  return owned_alloc(c, &c->V, n, true);
+}
+
 // operand copies and stash of the encoder layers, R rows
 int alloc_enc_layers(pllb_trainer_ctx* c, int64_t R) {
   const int H = c->d.hidden, I = c->d.intermediate, NH = c->d.num_heads;
   const int64_t HH = (int64_t)H * H;
   for (auto& l : c->L) {
-    RC(talloc(c, &l.qkv16, 3 * HH)); RC(talloc(c, &l.qkvT16, 3 * HH));
-    RC(talloc(c, &l.ao16, HH)); RC(talloc(c, &l.aoT16, HH));
-    RC(talloc(c, &l.ff116, (int64_t)I * H)); RC(talloc(c, &l.ff1T16, (int64_t)I * H));
-    RC(talloc(c, &l.ff216, (int64_t)I * H)); RC(talloc(c, &l.ff2T16, (int64_t)I * H));
-    RC(talloc(c, &l.x16, R * H)); RC(talloc(c, &l.qkv, R * 3 * H)); RC(talloc(c, &l.ctx, R * H));
-    RC(talloc(c, &l.h1_16, R * H)); RC(talloc(c, &l.g16, R * I));
-    RC(talloc(c, &l.lse, R * NH)); RC(talloc(c, &l.xhat1, R * H)); RC(talloc(c, &l.rstd1, R));
-    RC(talloc(c, &l.f, R * I)); RC(talloc(c, &l.xhat2, R * H)); RC(talloc(c, &l.rstd2, R));
+    RC(owned_alloc(c, &l.qkv16, 3 * HH)); RC(owned_alloc(c, &l.qkvT16, 3 * HH));
+    RC(owned_alloc(c, &l.ao16, HH)); RC(owned_alloc(c, &l.aoT16, HH));
+    RC(owned_alloc(c, &l.ff116, (int64_t)I * H)); RC(owned_alloc(c, &l.ff1T16, (int64_t)I * H));
+    RC(owned_alloc(c, &l.ff216, (int64_t)I * H)); RC(owned_alloc(c, &l.ff2T16, (int64_t)I * H));
+    RC(owned_alloc(c, &l.x16, R * H)); RC(owned_alloc(c, &l.qkv, R * 3 * H)); RC(owned_alloc(c, &l.ctx, R * H));
+    RC(owned_alloc(c, &l.h1_16, R * H)); RC(owned_alloc(c, &l.g16, R * I));
+    RC(owned_alloc(c, &l.lse, R * NH)); RC(owned_alloc(c, &l.xhat1, R * H)); RC(owned_alloc(c, &l.rstd1, R));
+    RC(owned_alloc(c, &l.f, R * I)); RC(owned_alloc(c, &l.xhat2, R * H)); RC(owned_alloc(c, &l.rstd2, R));
   }
   return PLLB_OK;
 }
 
-// The buffers every trainer has (R rows; `wide` = the widest GEMM output of a layer, Vw = the widest vocabulary-sized
-// one, kmax = the widest GEMM input, stage_ints = int32 slots of the pinned upload buffer), the stream, the pinned
-// buffers and the first operand refresh.  On failure the caller destroys the trainer.
-int alloc_rest(pllb_trainer_ctx* c, int64_t R, int wide, int Vw, int kmax, int64_t stage_ints, const char* who) {
+// operand copies and stash of the decoder layers, R rows
+int alloc_dec_layers(pllb_trainer_ctx* c, int64_t R) {
+  const int H = c->sd.hidden, Id = c->sd.dec_intermediate, NH = c->sd.num_heads;
+  const int64_t HH = (int64_t)H * H;
+  for (auto& l : c->D) {
+    RC(owned_alloc(c, &l.qkv16, 3 * HH)); RC(owned_alloc(c, &l.qkvT16, 3 * HH));
+    RC(owned_alloc(c, &l.o16, HH)); RC(owned_alloc(c, &l.oT16, HH)); RC(owned_alloc(c, &l.cq16, HH)); RC(owned_alloc(c, &l.cqT16, HH));
+    RC(owned_alloc(c, &l.co16, HH)); RC(owned_alloc(c, &l.coT16, HH));
+    RC(owned_alloc(c, &l.ff116, (int64_t)Id * H)); RC(owned_alloc(c, &l.ff1T16, (int64_t)Id * H));
+    RC(owned_alloc(c, &l.ff216, (int64_t)Id * H)); RC(owned_alloc(c, &l.ff2T16, (int64_t)Id * H));
+    RC(owned_alloc(c, &l.x16, R * H)); RC(owned_alloc(c, &l.qkv, R * 3 * H)); RC(owned_alloc(c, &l.ctx, R * H));
+    RC(owned_alloc(c, &l.h1_16, R * H)); RC(owned_alloc(c, &l.cq, R * H)); RC(owned_alloc(c, &l.cctx, R * H));
+    RC(owned_alloc(c, &l.h2_16, R * H)); RC(owned_alloc(c, &l.g16, R * Id));
+    RC(owned_alloc(c, &l.lse, R * NH)); RC(owned_alloc(c, &l.clse, R * NH));
+    RC(owned_alloc(c, &l.xhat1, R * H)); RC(owned_alloc(c, &l.rstd1, R)); RC(owned_alloc(c, &l.xhat2, R * H)); RC(owned_alloc(c, &l.rstd2, R));
+    RC(owned_alloc(c, &l.f, R * Id)); RC(owned_alloc(c, &l.xhat3, R * H)); RC(owned_alloc(c, &l.rstd3, R));
+  }
+  return PLLB_OK;
+}
+
+// The buffers every trainer has (R = cap_rows rows; `wide` = the widest GEMM output of a layer, Vw = the widest
+// vocabulary-sized one, kmax = the widest GEMM input, stage_ints = int32 slots of the pinned upload buffer), the LM
+// head's, the stream, the pinned buffers and the first operand refresh.  On failure the caller destroys the trainer.
+int alloc_rest(pllb_trainer_ctx* c, int wide, int Vw, int kmax, int64_t stage_ints, const char* who) {
   const int H = c->d.hidden, NH = c->d.num_heads;
-  const int64_t Rp = c->cap_rows_pad;
-  RC(talloc(c, &c->ids, R)); RC(talloc(c, &c->n_valid, R));
-  RC(talloc(c, &c->xhat_e, R * H)); RC(talloc(c, &c->rstd_e, R)); RC(talloc(c, &c->loss_dev, 2));
-  RC(talloc(c, &c->h32, R * H)); RC(talloc(c, &c->y32, R * wide)); RC(talloc(c, &c->dh32, R * H));
-  RC(talloc(c, &c->dz32, R * H)); RC(talloc(c, &c->dzd32, R * H)); RC(talloc(c, &c->Dq, R * NH));
-  RC(talloc(c, &c->zeros, std::max(Vw, wide), true));
-  RC(talloc(c, &c->colsum_scratch, (int64_t)2 * TRAIN_COLSUM_SPLITS * std::max(Vw, wide)));
-  RC(talloc(c, &c->d16, R * std::max(wide, H))); RC(talloc(c, &c->dT16, (int64_t)std::max(wide, Vw) * Rp));
-  RC(talloc(c, &c->xT16, (int64_t)kmax * Rp));
-  RC(talloc(c, &c->params_dev, 1, true));
+  const int64_t R = c->cap_rows, Rp = round_up(R, 64);
+  if (c->kind != KIND_CLS) {      // the LM head over the word embedding
+    RC(owned_alloc(c, &c->E16, (int64_t)c->Vp * H)); RC(owned_alloc(c, &c->ET16, (int64_t)c->Vp * H));
+    RC(owned_alloc(c, &c->labels, R)); RC(owned_alloc(c, &c->xlast16, R * H));
+    RC(owned_alloc(c, &c->dlogits16, R * c->Vp)); RC(owned_alloc(c, &c->logits, R * c->Vp)); RC(owned_alloc(c, &c->loss_rows, R));
+  }
+  RC(owned_alloc(c, &c->ids, R)); RC(owned_alloc(c, &c->n_valid, R));
+  RC(owned_alloc(c, &c->xhat_e, R * H)); RC(owned_alloc(c, &c->rstd_e, R)); RC(owned_alloc(c, &c->loss_dev, 2));
+  RC(owned_alloc(c, &c->h32, R * H)); RC(owned_alloc(c, &c->y32, R * wide)); RC(owned_alloc(c, &c->dh32, R * H));
+  RC(owned_alloc(c, &c->dz32, R * H)); RC(owned_alloc(c, &c->dzd32, R * H)); RC(owned_alloc(c, &c->Dq, R * NH));
+  RC(owned_alloc(c, &c->zeros, std::max(Vw, wide), true));
+  RC(owned_alloc(c, &c->colsum_scratch, (int64_t)2 * TRAIN_COLSUM_SPLITS * std::max(Vw, wide)));
+  RC(owned_alloc(c, &c->d16, R * std::max(wide, H))); RC(owned_alloc(c, &c->dT16, (int64_t)std::max(wide, Vw) * Rp));
+  RC(owned_alloc(c, &c->xT16, (int64_t)kmax * Rp));
+  RC(owned_alloc(c, &c->params_dev, 1, true));
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) {
     cudaGetLastError();
     return fail(PLLB_ERR_CUDA, std::string(who) + ": cudaStreamCreate failed");
@@ -723,13 +775,74 @@ int alloc_rest(pllb_trainer_ctx* c, int64_t R, int wide, int Vw, int kmax, int64
   return PLLB_OK;
 }
 
+// The start of every create, after its argument checks: a null `out`, the device check, then a new trainer of `kind`.
+int new_trainer(pllb_trainer* out, Kind kind, int device, const char* who, pllb_trainer_ctx** c) {
+  if (!out) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
+  *out = nullptr;
+  RC(check_create_device(device));
+  *c = new pllb_trainer_ctx();
+  (*c)->kind = kind;
+  (*c)->device = device;
+  return PLLB_OK;
+}
+
+// The end of every create: rc is what the trainer's build returned; a trainer whose build failed is destroyed.
+int finish_create(pllb_trainer* out, pllb_trainer_ctx* c, int rc) {
+  if (rc) {
+    pllb_train_destroy(c);
+    return rc;
+  }
+  *out = c;
+  return PLLB_OK;
+}
+
+// The flat layout, the parameters and the buffers of an MLM or RescoreBert trainer
+int build_bert(pllb_trainer_ctx* c, const pllb_weights* w, const float* lin_w, const float* lin_b, const char* who) {
+  const pllb_model_desc& d = c->d;
+  c->Vp = (int)round_up(d.vocab, 256);
+  const int H = d.hidden, I = d.intermediate, V = d.vocab, Vp = c->Vp;
+  const int64_t HH = (int64_t)H * H;
+  // ---- flat layout
+  int64_t cur = 0;
+  c->word = take(cur, (int64_t)(c->kind == KIND_CLS ? V : Vp) * H);    // MLM: rows >= vocab stay zero (zero gradient, zero moments)
+  c->pos = take(cur, (int64_t)d.max_position * H);
+  c->type = take(cur, 2 * H);
+  c->emb_g = take(cur, H);
+  c->emb_b = take(cur, H);
+  take_enc_layers(c, cur);
+  if (c->kind == KIND_CLS) {
+    c->lin_w = take(cur, H); c->lin_b = take(cur, 1);
+  } else {
+    c->head_w = take(cur, HH); c->head_b = take(cur, H); c->head_g = take(cur, H); c->head_be = take(cur, H);
+    c->dec_b = take(cur, Vp);
+  }
+  RC(alloc_flat(c, cur));
+  // ---- parameters in
+  RC(visit_params(c, w, lin_w, lin_b,
+                  [c](Span s, const float* src, int64_t n, int64_t off) { return copy_in(c, s, src, n, off); }));
+  // ---- operand copies, stash, scratch
+  c->cap_rows = c->t.max_rows;
+  const int64_t R = c->cap_rows;
+  const int wide = std::max(3 * H, I);
+  RC(alloc_enc_layers(c, R));
+  // the MLM head's transform: operand copies and stash; a CLS trainer has no MLM head
+  const int Vw = c->kind == KIND_CLS ? 0 : Vp;       // widest vocabulary-sized GEMM / column sum
+  if (c->kind != KIND_CLS) {
+    RC(owned_alloc(c, &c->head16, HH)); RC(owned_alloc(c, &c->headT16, HH));
+    RC(owned_alloc(c, &c->t_f32, R * H)); RC(owned_alloc(c, &c->xhat_h, R * H)); RC(owned_alloc(c, &c->rstd_h, R));
+    RC(owned_alloc(c, &c->tn16, R * H));
+  } else {
+    RC(owned_alloc(c, &c->group, R)); RC(owned_alloc(c, &c->target, R)); RC(owned_alloc(c, &c->am, R)); RC(owned_alloc(c, &c->err, R));
+    RC(owned_alloc(c, &c->scores, R)); RC(owned_alloc(c, &c->dscore, R));
+  }
+  return alloc_rest(c, wide, Vw, std::max(I, H), (c->kind == KIND_CLS ? 6 : 3) * R, who);
+}
+
 // lin_w / lin_b / loss given: a RescoreBert (CLS) trainer; otherwise an MLM trainer (the head pointers of w are required)
-int create_impl(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td, int device,
+int create_bert(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td, int device,
                 const float* lin_w, const float* lin_b, const pllb_cls_loss_desc* loss) {
   const char* who = loss ? "pllb_cls_train_create" : "pllb_train_create";
-  if (!out || !desc || !w || !w->layers || !td) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
-  *out = nullptr;
-  if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 (B200) device visible; libpllb200 has no CPU fallback");
+  if (!desc || !w || !w->layers || !td) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
   const pllb_model_desc& d = *desc;
   RC(check_model_shape(d));
   if (td->max_rows < 1 || td->max_seq < 1 || td->max_seq > d.max_position || td->max_seq > 512 ||
@@ -738,139 +851,28 @@ int create_impl(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weigh
   if (loss && (!lin_w || !lin_b || !std::isfinite(loss->md_weight) || !std::isfinite(loss->mwer_weight) ||
                !std::isfinite(loss->am_weight) || loss->md_weight < 0.f || loss->mwer_weight < 0.f))
     return fail(PLLB_ERR_INVALID, "pllb_cls_train_create: need linear_w, linear_b and finite loss weights, md / mwer >= 0");
-  PLLB_CUDA(cudaSetDevice(device));
-  int major = 0;
-  PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
-  if (major != 10) return fail(PLLB_ERR_NO_DEVICE, "device is not sm_100 (B200); libpllb200 has no other code path");
-  pllb_trainer_ctx* c = new pllb_trainer_ctx();
+  pllb_trainer_ctx* c = nullptr;
+  RC(new_trainer(out, loss ? KIND_CLS : KIND_MLM, device, who, &c));
   c->d = d;
   c->t = *td;
-  c->device = device;
-  c->cls = loss != nullptr;
   if (loss) c->loss = *loss;
-  c->Vp = (int)round_up(d.vocab, 256);
-  const int H = d.hidden, I = d.intermediate, V = d.vocab, NL = d.num_layers, Vp = c->Vp;
-  const int64_t HH = (int64_t)H * H;
-  int rc = PLLB_OK;
-#define TRY(expr)                        \
-  do {                                   \
-    rc = (expr);                         \
-    if (rc) { pllb_train_destroy(c); return rc; } \
-  } while (0)
-  // ---- flat layout
-  int64_t cur = 0;
-  c->word = take(cur, (int64_t)(c->cls ? V : Vp) * H);    // MLM: rows >= vocab stay zero (zero gradient, zero moments)
-  c->pos = take(cur, (int64_t)d.max_position * H);
-  c->type = take(cur, 2 * H);
-  c->emb_g = take(cur, H);
-  c->emb_b = take(cur, H);
-  c->L.resize(NL);
-  for (auto& l : c->L) {
-    l.qkv_w = take(cur, 3 * HH); l.qkv_b = take(cur, 3 * H);
-    l.ao_w = take(cur, HH); l.ao_b = take(cur, H); l.ao_g = take(cur, H); l.ao_be = take(cur, H);
-    l.ff1_w = take(cur, (int64_t)I * H); l.ff1_b = take(cur, I);
-    l.ff2_w = take(cur, (int64_t)H * I); l.ff2_b = take(cur, H); l.out_g = take(cur, H); l.out_be = take(cur, H);
-  }
-  if (c->cls) {
-    c->lin_w = take(cur, H); c->lin_b = take(cur, 1);
-  } else {
-    c->head_w = take(cur, HH); c->head_b = take(cur, H); c->head_g = take(cur, H); c->head_be = take(cur, H);
-    c->dec_b = take(cur, Vp);
-  }
-  c->n_flat = cur;
-  TRY(talloc(c, &c->P, cur, true));
-  TRY(talloc(c, &c->G, cur, true));
-  TRY(talloc(c, &c->M, cur, true));
-  TRY(talloc(c, &c->V, cur, true));
-  // ---- parameters in
-  TRY(visit_params(c, w, lin_w, lin_b,
-                   [c](Span s, const float* src, int64_t n, int64_t off) { return copy_in(c, s, src, n, off); }));
-  // ---- operand copies, stash, scratch
-  c->cap_rows = td->max_rows;
-  c->cap_rows_pad = round_up(c->cap_rows, 64);
-  const int64_t R = c->cap_rows;
-  const int wide = std::max(3 * H, I);
-  TRY(alloc_enc_layers(c, R));
-  // the MLM head's operand copies, stash, [R, Vp] logits and their gradient; a CLS trainer has none of them
-  const int Vw = c->cls ? 0 : Vp;       // widest vocabulary-sized GEMM / column sum
-  if (!c->cls) {
-    TRY(talloc(c, &c->head16, HH)); TRY(talloc(c, &c->headT16, HH));
-    TRY(talloc(c, &c->E16, (int64_t)Vp * H)); TRY(talloc(c, &c->ET16, (int64_t)Vp * H));
-    TRY(talloc(c, &c->labels, R));
-    TRY(talloc(c, &c->t_f32, R * H)); TRY(talloc(c, &c->xhat_h, R * H)); TRY(talloc(c, &c->rstd_h, R));
-    TRY(talloc(c, &c->xlast16, R * H)); TRY(talloc(c, &c->tn16, R * H)); TRY(talloc(c, &c->dlogits16, R * Vp));
-    TRY(talloc(c, &c->logits, R * Vp)); TRY(talloc(c, &c->loss_rows, R));
-  } else {
-    TRY(talloc(c, &c->group, R)); TRY(talloc(c, &c->target, R)); TRY(talloc(c, &c->am, R)); TRY(talloc(c, &c->err, R));
-    TRY(talloc(c, &c->scores, R)); TRY(talloc(c, &c->dscore, R));
-  }
-  TRY(alloc_rest(c, R, wide, Vw, std::max(I, H), (c->cls ? 6 : 3) * R, who));
-#undef TRY
-  *out = c;
-  return PLLB_OK;
+  return finish_create(out, c, build_bert(c, w, lin_w, lin_b, who));
 }
 
-// BART: the encoder layers above, the decoder layers, the stacked cross K / V and the LM head over shared
-int create_s2s_impl(pllb_trainer* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* w, const pllb_s2s_train_desc* td,
-                    int device) {
-  const char* who = "pllb_s2s_train_create";
-  if (!out || !desc || !w || !w->enc.layers || !w->dec_layers || !td) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
-  *out = nullptr;
-  if (pllb_device_count() < 1) return fail(PLLB_ERR_NO_DEVICE, "no sm_100 (B200) device visible; libpllb200 has no CPU fallback");
-  const pllb_s2s_desc& sd = *desc;
-  const int H = sd.hidden, V = sd.vocab;
-  if (H % 256 != 0 || H < 256 || H > 1024 || sd.num_heads * 64 != H || sd.enc_intermediate % 256 != 0 ||
-      sd.dec_intermediate % 256 != 0 || sd.enc_intermediate < 256 || sd.dec_intermediate < 256 || sd.enc_layers < 1 ||
-      sd.dec_layers < 1 || V < 1 || sd.enc_max_position < 1 || sd.dec_max_position < 1 || !std::isfinite(sd.embed_scale) ||
-      !(sd.ln_eps > 0.f))
-    return fail(PLLB_ERR_INVALID, std::string(who) + ": unsupported shape: need hidden in {256,512,768,1024}, head dim 64, "
-                                                     "FFN widths % 256 == 0, >= 1 layer per stack");
-  if (sd.operand_dtype != 0) return fail(PLLB_ERR_INVALID, std::string(who) + ": training takes operand_dtype 0 (bf16) only");
-  if (td->max_batch < 1 || td->max_enc_len < 1 || td->max_dec_len < 1 || td->max_enc_len > std::min(sd.enc_max_position, 1024) ||
-      td->max_dec_len > std::min(sd.dec_max_position, 1024) || !(td->dropout >= 0.f && td->dropout < 1.f) ||
-      !(td->attention_dropout >= 0.f && td->attention_dropout < 1.f) || td->pad_id < 0 || td->pad_id >= V ||
-      td->decoder_start_id < 0 || td->decoder_start_id >= V)
-    return fail(PLLB_ERR_INVALID, std::string(who) + ": need capacities >= 1 with lengths <= min(max_position, 1024), "
-                                                     "dropout in [0, 1), pad / decoder start ids in the vocabulary");
-  PLLB_CUDA(cudaSetDevice(device));
-  int major = 0;
-  PLLB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
-  if (major != 10) return fail(PLLB_ERR_NO_DEVICE, "device is not sm_100 (B200); libpllb200 has no other code path");
-  pllb_trainer_ctx* c = new pllb_trainer_ctx();
-  c->s2s = true;
-  c->sd = sd;
-  c->device = device;
-  c->decoder_start_id = td->decoder_start_id;
-  c->cap_batch = td->max_batch;
-  c->cap_enc = td->max_enc_len;
-  c->cap_dec = td->max_dec_len;
-  // the shared encoder / optimizer code reads these two descriptors
-  c->d = pllb_model_desc{sd.enc_layers, H, sd.num_heads, sd.enc_intermediate, V, sd.enc_max_position, sd.ln_eps,
-                         sd.cls_id, sd.sep_id, 0, 0};
-  c->t = pllb_train_desc{td->lr, td->beta1, td->beta2, td->adam_eps, td->weight_decay, td->dropout, td->attention_dropout,
-                         td->seed, td->pad_id, 0, 0};
-  c->Vp = (int)round_up(V, 256);
-  const int NL = sd.dec_layers, Id = sd.dec_intermediate, Vp = c->Vp, NH = sd.num_heads;
+// The flat layout, the parameters and the buffers of a CorrectBart trainer: the encoder layers above, the decoder
+// layers, the stacked cross K / V and the LM head over shared
+int build_s2s(pllb_trainer_ctx* c, const pllb_s2s_weights* w, const char* who) {
+  const pllb_s2s_desc& sd = c->sd;
+  c->Vp = (int)round_up(sd.vocab, 256);
+  const int H = sd.hidden, V = sd.vocab, NL = sd.dec_layers, Id = sd.dec_intermediate, Vp = c->Vp;
   const int64_t HH = (int64_t)H * H;
-  int rc = PLLB_OK;
-#define TRY(expr)                        \
-  do {                                   \
-    rc = (expr);                         \
-    if (rc) { pllb_train_destroy(c); return rc; } \
-  } while (0)
   // ---- flat layout
   int64_t cur = 0;
   c->word = take(cur, (int64_t)Vp * H);            // shared; rows >= vocab stay zero
   c->pos = take(cur, (int64_t)(sd.enc_max_position + 2) * H);
   c->emb_g = take(cur, H);
   c->emb_b = take(cur, H);
-  c->L.resize(sd.enc_layers);
-  for (auto& l : c->L) {
-    l.qkv_w = take(cur, 3 * HH); l.qkv_b = take(cur, 3 * H);
-    l.ao_w = take(cur, HH); l.ao_b = take(cur, H); l.ao_g = take(cur, H); l.ao_be = take(cur, H);
-    l.ff1_w = take(cur, (int64_t)sd.enc_intermediate * H); l.ff1_b = take(cur, sd.enc_intermediate);
-    l.ff2_w = take(cur, (int64_t)H * sd.enc_intermediate); l.ff2_b = take(cur, H); l.out_g = take(cur, H); l.out_be = take(cur, H);
-  }
+  take_enc_layers(c, cur);
   c->dec_pos = take(cur, (int64_t)(sd.dec_max_position + 2) * H);
   c->dec_emb_g = take(cur, H);
   c->dec_emb_b = take(cur, H);
@@ -886,48 +888,25 @@ int create_s2s_impl(pllb_trainer* out, const pllb_s2s_desc* desc, const pllb_s2s
   const int KV = 2 * H * NL;
   c->ckv_w = take(cur, (int64_t)KV * H);
   c->ckv_b = take(cur, KV);
-  c->n_flat = cur;
-  TRY(talloc(c, &c->P, cur, true));
-  TRY(talloc(c, &c->G, cur, true));      // position rows 0 and 1 are never written: their gradient stays 0
-  TRY(talloc(c, &c->M, cur, true));
-  TRY(talloc(c, &c->V, cur, true));
-  TRY(visit_s2s_params(c, w, [c](Span s, const float* src, int64_t n, int64_t off) { return copy_in(c, s, src, n, off); }));
-  TRY(talloc(c, &c->flb, Vp, true));
-  if (!w->final_logits_bias) TRY(fail(PLLB_ERR_INVALID, std::string(who) + ": final_logits_bias is null"));
+  RC(alloc_flat(c, cur));      // position rows 0 and 1 are never written: their gradient stays 0
+  RC(visit_s2s_params(c, w, [c](Span s, const float* src, int64_t n, int64_t off) { return copy_in(c, s, src, n, off); }));
+  RC(owned_alloc(c, &c->flb, Vp, true));
+  if (!w->final_logits_bias) return fail(PLLB_ERR_INVALID, std::string(who) + ": final_logits_bias is null");
   if (cudaMemcpyAsync(c->flb, w->final_logits_bias, sizeof(float) * V, cudaMemcpyDeviceToDevice, 0) != cudaSuccess) {
     cudaGetLastError();
-    TRY(fail(PLLB_ERR_CUDA, std::string(who) + ": copy of final_logits_bias failed"));
+    return fail(PLLB_ERR_CUDA, std::string(who) + ": copy of final_logits_bias failed");
   }
   // ---- operand copies, stash, scratch: the encoder and the decoder share row-sized buffers of max(T_enc, T_dec) rows
-  c->cap_rows = (int64_t)td->max_batch * std::max(td->max_enc_len, td->max_dec_len);
-  c->cap_rows_pad = round_up(c->cap_rows, 64);
+  c->cap_rows = (int64_t)c->cap_batch * std::max(c->cap_enc, c->cap_dec);
   const int64_t R = c->cap_rows;
-  TRY(alloc_enc_layers(c, R));
-  for (auto& l : c->D) {
-    TRY(talloc(c, &l.qkv16, 3 * HH)); TRY(talloc(c, &l.qkvT16, 3 * HH));
-    TRY(talloc(c, &l.o16, HH)); TRY(talloc(c, &l.oT16, HH)); TRY(talloc(c, &l.cq16, HH)); TRY(talloc(c, &l.cqT16, HH));
-    TRY(talloc(c, &l.co16, HH)); TRY(talloc(c, &l.coT16, HH));
-    TRY(talloc(c, &l.ff116, (int64_t)Id * H)); TRY(talloc(c, &l.ff1T16, (int64_t)Id * H));
-    TRY(talloc(c, &l.ff216, (int64_t)Id * H)); TRY(talloc(c, &l.ff2T16, (int64_t)Id * H));
-    TRY(talloc(c, &l.x16, R * H)); TRY(talloc(c, &l.qkv, R * 3 * H)); TRY(talloc(c, &l.ctx, R * H));
-    TRY(talloc(c, &l.h1_16, R * H)); TRY(talloc(c, &l.cq, R * H)); TRY(talloc(c, &l.cctx, R * H));
-    TRY(talloc(c, &l.h2_16, R * H)); TRY(talloc(c, &l.g16, R * Id));
-    TRY(talloc(c, &l.lse, R * NH)); TRY(talloc(c, &l.clse, R * NH));
-    TRY(talloc(c, &l.xhat1, R * H)); TRY(talloc(c, &l.rstd1, R)); TRY(talloc(c, &l.xhat2, R * H)); TRY(talloc(c, &l.rstd2, R));
-    TRY(talloc(c, &l.f, R * Id)); TRY(talloc(c, &l.xhat3, R * H)); TRY(talloc(c, &l.rstd3, R));
-  }
-  TRY(talloc(c, &c->ckv16, (int64_t)KV * H)); TRY(talloc(c, &c->ckvT16, (int64_t)KV * H));
-  TRY(talloc(c, &c->E16, (int64_t)Vp * H)); TRY(talloc(c, &c->ET16, (int64_t)Vp * H));
-  TRY(talloc(c, &c->labels, R)); TRY(talloc(c, &c->dec_ids, R));
-  TRY(talloc(c, &c->xlast16, R * H)); TRY(talloc(c, &c->dlast16, R * H)); TRY(talloc(c, &c->ckv, R * KV));
-  TRY(talloc(c, &c->dckv32, R * KV)); TRY(talloc(c, &c->dq32, R * H));
-  TRY(talloc(c, &c->xhat_d, R * H)); TRY(talloc(c, &c->rstd_d, R));
-  TRY(talloc(c, &c->dlogits16, R * Vp)); TRY(talloc(c, &c->logits, R * Vp)); TRY(talloc(c, &c->loss_rows, R));
+  RC(alloc_enc_layers(c, R));
+  RC(alloc_dec_layers(c, R));
+  RC(owned_alloc(c, &c->ckv16, (int64_t)KV * H)); RC(owned_alloc(c, &c->ckvT16, (int64_t)KV * H));
+  RC(owned_alloc(c, &c->dec_ids, R)); RC(owned_alloc(c, &c->dlast16, R * H)); RC(owned_alloc(c, &c->ckv, R * KV));
+  RC(owned_alloc(c, &c->dckv32, R * KV)); RC(owned_alloc(c, &c->dq32, R * H));
+  RC(owned_alloc(c, &c->xhat_d, R * H)); RC(owned_alloc(c, &c->rstd_d, R));
   const int wide = std::max({3 * H, sd.enc_intermediate, Id, KV});
-  TRY(alloc_rest(c, R, wide, Vp, std::max({sd.enc_intermediate, Id, H}), 4 * R, who));
-#undef TRY
-  *out = c;
-  return PLLB_OK;
+  return alloc_rest(c, wide, Vp, std::max({sd.enc_intermediate, Id, H}), 4 * R, who);
 }
 
 }  // namespace
@@ -936,7 +915,7 @@ extern "C" {
 
 int pllb_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const pllb_train_desc* td,
                       int device) {
-  return create_impl(out, desc, w, td, device, nullptr, nullptr, nullptr);
+  return create_bert(out, desc, w, td, device, nullptr, nullptr, nullptr);
 }
 
 int pllb_train_destroy(pllb_trainer c) {
@@ -972,7 +951,7 @@ int pllb_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t
   const char* who = "pllb_train_step_host";
   RC(require_kind(c, KIND_MLM, who));
   if (!labels) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
-  RC(check_batch(c, who, input_ids, n_valid, B, T, mode));
+  RC(check_batch(c, who, input_ids, n_valid, B, T, 0, mode));
   const int R = B * T;
   for (int i = 0; i < R; ++i)      // the reference's CrossEntropyLoss raises on a label outside the vocabulary
     if (labels[i] < 0 || labels[i] >= c->d.vocab) return fail(PLLB_ERR_INVALID, "label outside the vocabulary at row " + std::to_string(i));
@@ -996,17 +975,17 @@ int pllb_train_row_losses_host(pllb_trainer c, float* out, int32_t n) {
 }
 
 int pllb_train_export(pllb_trainer c, const pllb_weights* dst) {
-  return export_params(c, false, false, dst, nullptr, nullptr, "pllb_train_export");
+  return export_params(c, KIND_MLM, false, dst, nullptr, nullptr, nullptr, "pllb_train_export");
 }
 
 int pllb_train_export_grads(pllb_trainer c, const pllb_weights* dst) {
-  return export_params(c, false, true, dst, nullptr, nullptr, "pllb_train_export_grads");
+  return export_params(c, KIND_MLM, true, dst, nullptr, nullptr, nullptr, "pllb_train_export_grads");
 }
 
 int pllb_cls_train_create(pllb_trainer* out, const pllb_model_desc* desc, const pllb_weights* w, const float* linear_w,
                           const float* linear_b, const pllb_train_desc* td, const pllb_cls_loss_desc* loss, int device) {
   if (!loss) return fail(PLLB_ERR_INVALID, "pllb_cls_train_create: null loss descriptor");
-  return create_impl(out, desc, w, td, device, linear_w, linear_b, loss);
+  return create_bert(out, desc, w, td, device, linear_w, linear_b, loss);
 }
 
 int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* group,
@@ -1015,7 +994,7 @@ int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int
   const char* who = "pllb_cls_train_step_host";
   RC(require_kind(c, KIND_CLS, who));
   if (!group || !target || !am || !err) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
-  RC(check_batch(c, who, input_ids, n_valid, B, T, mode));
+  RC(check_batch(c, who, input_ids, n_valid, B, T, 0, mode));
   for (int b = 0; b < B; ++b) {
     if (b == 0 ? group[0] != 0 : (group[b] != group[b - 1] && group[b] != group[b - 1] + 1))
       return fail(PLLB_ERR_INVALID, "group must start at 0 and number the utterances in row order (each entry equal to the "
@@ -1039,37 +1018,54 @@ int pllb_cls_train_step_host(pllb_trainer c, const int32_t* input_ids, const int
 }
 
 int pllb_cls_train_export(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
-  return export_params(c, true, false, dst, linear_w, linear_b, "pllb_cls_train_export");
+  return export_params(c, KIND_CLS, false, dst, linear_w, linear_b, nullptr, "pllb_cls_train_export");
 }
 
 int pllb_cls_train_export_grads(pllb_trainer c, const pllb_weights* dst, float* linear_w, float* linear_b) {
-  return export_params(c, true, true, dst, linear_w, linear_b, "pllb_cls_train_export_grads");
+  return export_params(c, KIND_CLS, true, dst, linear_w, linear_b, nullptr, "pllb_cls_train_export_grads");
 }
 
-int pllb_s2s_train_create(pllb_trainer* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* weights,
-                          const pllb_s2s_train_desc* train, int device) {
-  return create_s2s_impl(out, desc, weights, train, device);
+int pllb_s2s_train_create(pllb_trainer* out, const pllb_s2s_desc* desc, const pllb_s2s_weights* w,
+                          const pllb_s2s_train_desc* td, int device) {
+  const char* who = "pllb_s2s_train_create";
+  if (!desc || !w || !w->enc.layers || !w->dec_layers || !td) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
+  const pllb_s2s_desc& sd = *desc;
+  const int H = sd.hidden, V = sd.vocab;
+  if (H % 256 != 0 || H < 256 || H > 1024 || sd.num_heads * 64 != H || sd.enc_intermediate % 256 != 0 ||
+      sd.dec_intermediate % 256 != 0 || sd.enc_intermediate < 256 || sd.dec_intermediate < 256 || sd.enc_layers < 1 ||
+      sd.dec_layers < 1 || V < 1 || sd.enc_max_position < 1 || sd.dec_max_position < 1 || !std::isfinite(sd.embed_scale) ||
+      !(sd.ln_eps > 0.f))
+    return fail(PLLB_ERR_INVALID, std::string(who) + ": unsupported shape: need hidden in {256,512,768,1024}, head dim 64, "
+                                                     "FFN widths % 256 == 0, >= 1 layer per stack");
+  if (sd.operand_dtype != 0) return fail(PLLB_ERR_INVALID, std::string(who) + ": training takes operand_dtype 0 (bf16) only");
+  if (td->max_batch < 1 || td->max_enc_len < 1 || td->max_dec_len < 1 || td->max_enc_len > std::min(sd.enc_max_position, 1024) ||
+      td->max_dec_len > std::min(sd.dec_max_position, 1024) || !(td->dropout >= 0.f && td->dropout < 1.f) ||
+      !(td->attention_dropout >= 0.f && td->attention_dropout < 1.f) || td->pad_id < 0 || td->pad_id >= V ||
+      td->decoder_start_id < 0 || td->decoder_start_id >= V)
+    return fail(PLLB_ERR_INVALID, std::string(who) + ": need capacities >= 1 with lengths <= min(max_position, 1024), "
+                                                     "dropout in [0, 1), pad / decoder start ids in the vocabulary");
+  pllb_trainer_ctx* c = nullptr;
+  RC(new_trainer(out, KIND_S2S, device, who, &c));
+  c->sd = sd;
+  c->decoder_start_id = td->decoder_start_id;
+  c->cap_batch = td->max_batch;
+  c->cap_enc = td->max_enc_len;
+  c->cap_dec = td->max_dec_len;
+  // the shared encoder / optimizer code reads these two descriptors
+  c->d = pllb_model_desc{sd.enc_layers, H, sd.num_heads, sd.enc_intermediate, V, sd.enc_max_position, sd.ln_eps,
+                         sd.cls_id, sd.sep_id, 0, 0};
+  c->t = pllb_train_desc{td->lr, td->beta1, td->beta2, td->adam_eps, td->weight_decay, td->dropout, td->attention_dropout,
+                         td->seed, td->pad_id, 0, 0};
+  return finish_create(out, c, build_s2s(c, w, who));
 }
 
 int pllb_s2s_train_step_host(pllb_trainer c, const int32_t* input_ids, const int32_t* n_valid, const int32_t* labels,
                              int32_t B, int32_t T_enc, int32_t T_dec, int32_t mode, float* out_loss) {
   const char* who = "pllb_s2s_train_step_host";
   RC(require_kind(c, KIND_S2S, who));
-  if (!input_ids || !n_valid || !labels || B < 1 || T_enc < 1 || T_dec < 1 || mode < 0 || mode > 2)
-    return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
-  if (T_enc > c->sd.enc_max_position || T_dec > c->sd.dec_max_position)
-    return fail(PLLB_ERR_TOO_LONG, std::string(who) + ": T_enc " + std::to_string(T_enc) + " / T_dec " + std::to_string(T_dec) +
-                                       " above the position tables (" + std::to_string(c->sd.enc_max_position) + " / " +
-                                       std::to_string(c->sd.dec_max_position) + ")");
-  if (B > c->cap_batch || T_enc > c->cap_enc || T_dec > c->cap_dec)
-    return fail(PLLB_ERR_OOM, std::string(who) + ": batch [" + std::to_string(B) + ", " + std::to_string(T_enc) + ", " +
-                                  std::to_string(T_dec) + "] above the capacity given at create [" + std::to_string(c->cap_batch) +
-                                  ", " + std::to_string(c->cap_enc) + ", " + std::to_string(c->cap_dec) + "]");
+  if (!labels) return fail(PLLB_ERR_INVALID, std::string(who) + ": bad argument");
+  RC(check_batch(c, who, input_ids, n_valid, B, T_enc, T_dec, mode));
   const int V = c->sd.vocab, Re = B * T_enc, Rd = B * T_dec;
-  for (int i = 0; i < Re; ++i)
-    if (input_ids[i] < 0 || input_ids[i] >= V) return fail(PLLB_ERR_INVALID, "token id outside the vocabulary at row " + std::to_string(i));
-  for (int b = 0; b < B; ++b)
-    if (n_valid[b] < 1 || n_valid[b] > T_enc) return fail(PLLB_ERR_INVALID, "n_valid must be in [1, T_enc]");
   int n_lab = 0;
   for (int i = 0; i < Rd; ++i) {
     if (labels[i] == -100) continue;
@@ -1097,30 +1093,12 @@ int pllb_s2s_train_step_host(pllb_trainer c, const int32_t* input_ids, const int
   return PLLB_OK;
 }
 
-namespace {
-int export_s2s(pllb_trainer c, bool grads, const pllb_s2s_weights* w, const char* who) {
-  RC(require_kind(c, KIND_S2S, who));
-  if (!w || !w->enc.layers || !w->dec_layers) return fail(PLLB_ERR_INVALID, std::string(who) + ": null argument");
-  const float* buf = grads ? c->G : c->P;
-  PLLB_CUDA(cudaSetDevice(c->device));
-  PLLB_CUDA(cudaStreamSynchronize(c->stream));
-  RC(visit_s2s_params(c, w, [buf](Span s, const float* dst, int64_t n, int64_t off) { return copy_out(buf, s, dst, n, off); }));
-  if (w->final_logits_bias) {       // a buffer: the given values, no gradient
-    float* dst = const_cast<float*>(w->final_logits_bias);
-    if (grads) PLLB_CUDA(cudaMemsetAsync(dst, 0, sizeof(float) * c->sd.vocab, 0));
-    else PLLB_CUDA(cudaMemcpyAsync(dst, c->flb, sizeof(float) * c->sd.vocab, cudaMemcpyDeviceToDevice, 0));
-  }
-  PLLB_CUDA(cudaStreamSynchronize(0));
-  return PLLB_OK;
-}
-}  // namespace
-
 int pllb_s2s_train_export(pllb_trainer c, const pllb_s2s_weights* dst) {
-  return export_s2s(c, false, dst, "pllb_s2s_train_export");
+  return export_params(c, KIND_S2S, false, nullptr, nullptr, nullptr, dst, "pllb_s2s_train_export");
 }
 
 int pllb_s2s_train_export_grads(pllb_trainer c, const pllb_s2s_weights* dst) {
-  return export_s2s(c, true, dst, "pllb_s2s_train_export_grads");
+  return export_params(c, KIND_S2S, true, nullptr, nullptr, nullptr, dst, "pllb_s2s_train_export_grads");
 }
 
 // ---------------------------------------------------------------- kernel test hooks (pllb_debug_train_*)

@@ -83,9 +83,15 @@ def _model_desc(cfg: dict, operand_dtype: int = 0, cls_id: int = 101, sep_id: in
 
 
 class _Handle:
-    """Owner of one library handle ``self._h``, released by the symbol ``_DESTROY`` names."""
+    """Owner of one library handle ``self._h``, released by the symbol ``_DESTROY`` names.  The library is loaded and
+    a device required before a subclass creates the handle."""
 
     _DESTROY = ""
+
+    def __init__(self):
+        self._lib = _lib.load()
+        _lib.require_device()
+        self._h = ctypes.c_void_p()
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -118,9 +124,7 @@ class PllScorer(_Handle):
         import torch
         from .synth import config_from_state_dict
 
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
+        super().__init__()
         self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
         self.device = device
         dev = torch.device("cuda", device)
@@ -309,72 +313,78 @@ def _prefix_lengths(attention_mask, shape) -> np.ndarray:
 
 class _Trainer(_Handle):
     """One pllb_train_* handle (encoder, AdamW, stateless dropout, CUDA graphs) and the state_dict keys it was
-    created from.  A subclass creates the handle and names its encoder keys, head pointers and aliases."""
+    created from.  A subclass builds its descriptors, creates the handle and says which tensor each given key names."""
 
     _DESTROY = "pllb_train_destroy"
-    _HEAD_KEYS = ()       # keys passed to the export calls as extra device pointers, after pllb_weights
+    _HEAD_KEYS = ()       # keys passed to the export calls as extra device pointers, after the weights struct
 
-    def __init__(self, state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
-                 weight_decay, pad_id):
+    def __init__(self, state_dict, device):
         import torch
-        from .synth import config_from_state_dict
 
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
-        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
+        super().__init__()
         self.device = device
         self._dev = torch.device("cuda", device)
         self._keys = list(state_dict.keys())
-        self._passthrough = {k: v for k, v in state_dict.items() if self._passes_through(k)}
         self._shapes = {k: tuple(v.shape) for k, v in state_dict.items()}
+        self._passthrough = {k: v for k, v in state_dict.items() if self._internal_key(k) is None}
+
+    def _bert_descs(self, state_dict, cfg, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+                    weight_decay, pad_id):
+        """The config and the descriptors of an MLM or RescoreBert trainer."""
+        from .synth import config_from_state_dict
+
+        self.cfg = dict(cfg) if cfg is not None else config_from_state_dict(state_dict)
         self.max_seq = min(int(max_seq), int(self.cfg["max_position"]), 512)
         self._desc = _model_desc(self.cfg)
         self._train_desc = TrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay),
                                      float(hidden_dropout), float(attention_dropout), int(seed) & (2 ** 64 - 1), int(pad_id),
                                      int(max_rows), self.max_seq)
 
-    def _passes_through(self, key: str) -> bool:
-        """Keys the trainer does not hold: export returns the given tensor."""
-        return key.endswith("position_ids")
+    def _internal_key(self, key: str) -> Optional[str]:
+        """The key of the tensor the trainer holds for the given ``key`` (tied keys name one tensor), or None for a
+        tensor it does not hold: export returns the given tensor."""
+        return None if key.endswith("position_ids") else key
 
-    def _encoder_keys(self):
-        return self._keys
+    def _no_grad(self, key: str) -> bool:
+        """Keys that get no gradient: grads() returns zeros for them."""
+        return False
 
-    def _alias(self, key: str) -> str:
-        return key
+    def _weights_struct(self, get):
+        """The weights struct of the create and export calls over ``get(internal key)``: (struct, keep-alive list)."""
+        return weights_struct(get, self.cfg["num_layers"], self._keys)
 
     def _to_dev(self, t):
         import torch
         return t.detach().to(device=self._dev, dtype=torch.float32).contiguous()
 
     def _weights_in(self, state_dict):
-        """pllb_weights over device fp32 copies of the encoder tensors, ready for the create call."""
+        """The weights struct over device fp32 copies of the given tensors, ready for the create call."""
         import torch
-        w, keep = weights_struct(lambda key: self._to_dev(state_dict[key]), self.cfg["num_layers"], self._encoder_keys())
+        w, keep = self._weights_struct(lambda key: self._to_dev(state_dict[key]))
         torch.cuda.synchronize(self._dev)
         return w, keep
 
-    def _export(self, fn) -> Dict[str, "torch.Tensor"]:
-        """fn(handle, pllb_weights, *head pointers) fills one zeroed device tensor per key (aliased keys share one);
-        returns CPU tensors under the keys given at construction."""
+    def _export(self, fn, grads: bool = False) -> Dict[str, "torch.Tensor"]:
+        """fn(handle, weights struct, *head pointers) fills one zeroed device tensor per internal key; returns CPU
+        tensors under the keys given at construction (tied keys share one tensor, pass-through keys the given one,
+        zeros under the keys that get no gradient when ``grads``)."""
         import torch
         bufs = {}
 
         def get(key):
-            key = self._alias(key)
             if key not in bufs:
                 bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
             return bufs[key]
 
-        w, keep = weights_struct(get, self.cfg["num_layers"], self._encoder_keys())
+        w, keep = self._weights_struct(get)
         head = [ctypes.c_void_p(get(k).data_ptr()) for k in self._HEAD_KEYS]
         torch.cuda.synchronize(self._dev)
         check(fn(self._h, ctypes.byref(w), *head))
         torch.cuda.synchronize(self._dev)
         host = {k: v.cpu() for k, v in bufs.items()}
         del keep
-        return {k: self._passthrough[k] if k in self._passthrough else host[self._alias(k)] for k in self._keys}
+        return {k: torch.zeros(self._shapes[k], dtype=torch.float32) if grads and self._no_grad(k)
+                else self._passthrough[k] if k in self._passthrough else host[self._internal_key(k)] for k in self._keys}
 
     def reset_optimizer(self, lr: float):
         """A fresh AdamW: zero moments, step count 0, learning rate lr (the reference creates one per epoch,
@@ -408,7 +418,8 @@ class MlmTrainer(_Trainer):
                  lr: float = 1e-5, hidden_dropout: float = 0.1, attention_dropout: float = 0.1, seed: int = 0,
                  max_rows: int = 4096, max_seq: int = 128, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 0.01, pad_id: int = 0):
-        super().__init__(state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+        super().__init__(state_dict, device)
+        self._bert_descs(state_dict, cfg, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
                          weight_decay, pad_id)
         if "cls.predictions.transform.dense.weight" not in state_dict:
             raise ValueError("MLM fine-tuning needs a BertForMaskedLM state_dict (cls.predictions.* missing)")
@@ -417,10 +428,10 @@ class MlmTrainer(_Trainer):
                                           ctypes.byref(self._train_desc), device))
         del keep
 
-    def _alias(self, key: str) -> str:
+    def _internal_key(self, key: str) -> Optional[str]:
         """Tied entries are one tensor, as in model.state_dict()."""
-        src = self.TIED.get(key, key)
-        return src if src in self._shapes else key
+        src = self.TIED.get(key)
+        return src if src in self._shapes else super()._internal_key(key)
 
     def step(self, input_ids, attention_mask, labels, mode: int = 1) -> float:
         """One zero-padded batch (int arrays [B, T], what collate builds).  mode 1: forward + backward
@@ -448,7 +459,7 @@ class MlmTrainer(_Trainer):
 
     def grads(self) -> Dict[str, "torch.Tensor"]:
         """Gradients of the last mode-1 / mode-2 step, same keys (parity tests)."""
-        return self._export(self._lib.pllb_train_export_grads)
+        return self._export(self._lib.pllb_train_export_grads, grads=True)
 
 
 class ClsTrainer(_Trainer):
@@ -472,7 +483,8 @@ class ClsTrainer(_Trainer):
                  max_seq: int = 128, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 0.01, pad_id: int = 0):
         if "linear.weight" not in state_dict or "linear.bias" not in state_dict:
             raise ValueError("RescoreBert training needs linear.weight [1, H] and linear.bias [1] in the state_dict")
-        super().__init__(state_dict, cfg, device, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
+        super().__init__(state_dict, device)
+        self._bert_descs(state_dict, cfg, lr, hidden_dropout, attention_dropout, seed, max_rows, max_seq, betas, eps,
                          weight_decay, pad_id)
         if state_dict["linear.weight"].numel() != self.cfg["hidden"] or state_dict["linear.bias"].numel() != 1:
             raise ValueError("linear.weight must have `hidden` elements and linear.bias one")
@@ -485,11 +497,15 @@ class ClsTrainer(_Trainer):
                                               ctypes.byref(self._train_desc), ctypes.byref(ld), device))
         del keep, lw, lb
 
-    def _passes_through(self, key: str) -> bool:
-        return super()._passes_through(key) or key.startswith(self.POOLER)
+    def _internal_key(self, key: str) -> Optional[str]:
+        return None if key.startswith(self.POOLER) else super()._internal_key(key)
 
-    def _encoder_keys(self):
-        return [k for k in self._keys if k.startswith("bert.") and not k.startswith(self.POOLER)]
+    def _no_grad(self, key: str) -> bool:
+        return key.startswith(self.POOLER)
+
+    def _weights_struct(self, get):
+        keys = [k for k in self._keys if k.startswith("bert.") and not k.startswith(self.POOLER)]
+        return weights_struct(get, self.cfg["num_layers"], keys)
 
     def step(self, input_ids, attention_mask, group, target, am, err, mode: int = 1):
         """One batch of whole utterances: input_ids / attention_mask int [B, T] ([CLS] t [SEP], zero-padded,
@@ -519,12 +535,7 @@ class ClsTrainer(_Trainer):
     def grads(self) -> Dict[str, "torch.Tensor"]:
         """Gradients of the last mode-1 / mode-2 step under the same keys (zeros for the pooler;
         position_ids passes through)."""
-        import torch
-        g = self._export(self._lib.pllb_cls_train_export_grads)
-        for k in g:
-            if k.startswith(self.POOLER):
-                g[k] = torch.zeros(self._shapes[k], dtype=torch.float32)      # the pooler gets no gradient
-        return g
+        return self._export(self._lib.pllb_cls_train_export_grads, grads=True)
 
 
 # ---------------------------------------------------------------------- stage 4
@@ -854,6 +865,14 @@ def s2s_weights_struct(get, cfg: dict, pos_skip_rows: int):
     return w, keep
 
 
+def _s2s_desc(shape: dict, cls_id: int, sep_id: int, operand_dtype: int) -> "_lib.S2sDesc":
+    """pllb_s2s_desc of a check_bart_config shape (one position table size for both stacks, ln_eps 1e-5)."""
+    s = shape
+    return _lib.S2sDesc(s["enc_layers"], s["dec_layers"], s["hidden"], s["num_heads"], s["enc_intermediate"],
+                        s["dec_intermediate"], s["vocab"], s["max_position"], s["max_position"], 1e-5, s["embed_scale"],
+                        cls_id, sep_id, operand_dtype)
+
+
 _GEN_KEYS = ("max_length", "decoder_start_token_id", "eos_token_id", "pad_token_id", "forced_bos_token_id",
              "forced_eos_token_id")
 
@@ -955,11 +974,8 @@ class Seq2SeqGenerator(_Handle):
     def __init__(self, state_dict: Dict[str, "torch.Tensor"], cfg: dict, device: int = 0, max_rows: int = 0,
                  operand_dtype: str = "bf16", cls_id: int = 101, sep_id: int = 102):
         import torch
-        from ._lib import S2sDesc
 
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
+        super().__init__()
         self.cfg = dict(cfg)
         self.shape = check_bart_config(self.cfg)
         if operand_dtype not in ("bf16", "fp16"):
@@ -968,7 +984,6 @@ class Seq2SeqGenerator(_Handle):
         sd = bart_state_dict(state_dict)
         dev = torch.device("cuda", device)
         s = self.shape
-        H = s["hidden"]
 
         def get(key):
             if key not in sd:                                         # final_logits_bias: a missing buffer loads as zeros
@@ -976,9 +991,7 @@ class Seq2SeqGenerator(_Handle):
             return sd[key].detach().to(device=dev, dtype=torch.float32)
 
         w, keep = s2s_weights_struct(get, self.cfg, pos_skip_rows=2)  # BartLearnedPositionalEmbedding's offset of 2
-        d = S2sDesc(s["enc_layers"], s["dec_layers"], H, s["num_heads"], s["enc_intermediate"], s["dec_intermediate"],
-                    s["vocab"], s["max_position"], s["max_position"],
-                    1e-5, s["embed_scale"], cls_id, sep_id, 0 if operand_dtype == "bf16" else 1)
+        d = _s2s_desc(s, cls_id, sep_id, 0 if operand_dtype == "bf16" else 1)
         torch.cuda.synchronize(dev)
         check(self._lib.pllb_s2s_create(ctypes.byref(self._h), ctypes.byref(d), ctypes.byref(w), int(max_rows), device))
         del keep
@@ -1080,7 +1093,7 @@ class Seq2SeqTrainer(_Trainer):
                  max_batch: int = 64, max_enc_len: int = 128, max_dec_len: int = 128, betas=(0.9, 0.999),
                  eps: float = 1e-8, weight_decay: float = 0.01, operand_dtype: str = "bf16"):
         import torch
-        from ._lib import S2sDesc, S2sTrainDesc
+        from ._lib import S2sTrainDesc
 
         self.cfg = dict(cfg)
         self.shape = check_bart_config(self.cfg)
@@ -1088,36 +1101,27 @@ class Seq2SeqTrainer(_Trainer):
             raise ValueError("activation_dropout != 0 is not supported (bart-base's default is 0)")
         if operand_dtype != "bf16":
             raise ValueError("training takes bf16 GEMM operands only (no fp16 training)")
-        sd = bart_state_dict(state_dict)
-        # the handle is created here, not by _Trainer.__init__ (which builds the BERT descriptors)
-        self._lib = _lib.load()
-        _lib.require_device()
-        self._h = ctypes.c_void_p()
-        self.device = device
-        self._dev = torch.device("cuda", device)
-        self._keys = list(state_dict.keys())
-        # bart_state_dict located exactly one model.shared.weight; its prefix maps the given keys to sd's
+        bart_state_dict(state_dict)             # ValueError unless one model.shared.weight with equal tied copies
+        # the prefix of that one model.shared.weight maps the given keys to the BART names
         self._prefix = next(k for k in state_dict if k == "model.shared.weight" or k.endswith(".model.shared.weight"))[
             :-len("model.shared.weight")]
-        self._given = {k: v for k, v in state_dict.items()}
-        self._shapes = {k: tuple(v.shape) for k, v in sd.items()}
+        self._held = set(bart_weight_keys(self.cfg).values())
+        super().__init__(state_dict, device)
         self.pad_id = int(self.cfg.get("pad_token_id", 0) if self.cfg.get("pad_token_id") is not None else 0)
         self.decoder_start_id = int(self.cfg["decoder_start_token_id"])
         s = self.shape
-        if "final_logits_bias" not in sd:                              # a missing buffer loads as zeros in HF
-            sd["final_logits_bias"] = torch.zeros(1, s["vocab"])
-            self._shapes["final_logits_bias"] = (1, s["vocab"])
-        w, keep = s2s_weights_struct(lambda k: self._to_dev(sd[k]), self.cfg, pos_skip_rows=0)
-        self._desc = S2sDesc(s["enc_layers"], s["dec_layers"], s["hidden"], s["num_heads"], s["enc_intermediate"],
-                             s["dec_intermediate"], s["vocab"], s["max_position"], s["max_position"], 1e-5,
-                             s["embed_scale"], 101, 102, 0)
+        flb = self._prefix + "final_logits_bias"
+        if flb not in state_dict:                                      # a missing buffer loads as zeros in HF
+            state_dict = {**state_dict, flb: torch.zeros(1, s["vocab"])}
+            self._shapes[flb] = (1, s["vocab"])
+        self._desc = _s2s_desc(s, 101, 102, 0)
         drop = float(self.cfg.get("dropout", 0.1) if dropout is None else dropout)
         adrop = float(self.cfg.get("attention_dropout", 0.0) if attention_dropout is None else attention_dropout)
         self.max_batch, self.max_enc_len, self.max_dec_len = int(max_batch), int(max_enc_len), int(max_dec_len)
         self._train_desc = S2sTrainDesc(float(lr), float(betas[0]), float(betas[1]), float(eps), float(weight_decay), drop,
                                         adrop, int(seed) & (2 ** 64 - 1), self.pad_id, self.decoder_start_id,
                                         self.max_batch, self.max_enc_len, self.max_dec_len)
-        torch.cuda.synchronize(self._dev)
+        w, keep = self._weights_in(state_dict)
         check(self._lib.pllb_s2s_train_create(ctypes.byref(self._h), ctypes.byref(self._desc), ctypes.byref(w),
                                               ctypes.byref(self._train_desc), device))
         del keep
@@ -1147,28 +1151,18 @@ class Seq2SeqTrainer(_Trainer):
         check(self._lib.pllb_train_row_losses_host(self._h, _np_ptr(out), out.size))
         return out
 
-    def _export(self, fn) -> Dict[str, "torch.Tensor"]:
-        import torch
-        bufs = {}
+    def _internal_key(self, key: str) -> Optional[str]:
+        """The tied aliases name model.shared; keys outside the BART names pass through."""
+        name = key[len(self._prefix):] if key.startswith(self._prefix) else None
+        if name in BART_TIED_KEYS:
+            return self._prefix + _BART_TOP["shared"]
+        return key if name in self._held else None
 
-        def get(key):
-            if key not in bufs:
-                bufs[key] = torch.zeros(self._shapes[key], dtype=torch.float32, device=self._dev)
-            return bufs[key]
+    def _no_grad(self, key: str) -> bool:
+        return key.endswith("final_logits_bias")
 
-        w, keep = s2s_weights_struct(get, self.cfg, pos_skip_rows=0)
-        torch.cuda.synchronize(self._dev)
-        check(fn(self._h, ctypes.byref(w)))
-        torch.cuda.synchronize(self._dev)
-        host = {k: v.cpu() for k, v in bufs.items()}
-        del keep
-        out = {}
-        for k in self._keys:
-            name = k[len(self._prefix):] if k.startswith(self._prefix) else k
-            if name in BART_TIED_KEYS:
-                name = _BART_TOP["shared"]
-            out[k] = host[name].reshape(self._given[k].shape) if name in host else self._given[k]
-        return out
+    def _weights_struct(self, get):
+        return s2s_weights_struct(lambda name: get(self._prefix + name), self.cfg, pos_skip_rows=0)
 
     def state_dict(self) -> Dict[str, "torch.Tensor"]:
         """fp32 CPU tensors under the keys given at construction: the tied aliases hold the ``model.shared``
@@ -1179,9 +1173,4 @@ class Seq2SeqTrainer(_Trainer):
     def grads(self) -> Dict[str, "torch.Tensor"]:
         """Gradients of the last mode-1 / mode-2 step under the same keys (the tied aliases hold the one
         ``model.shared`` gradient; zeros for ``final_logits_bias``)."""
-        import torch
-        g = self._export(self._lib.pllb_s2s_train_export_grads)
-        for k in g:
-            if k.endswith("final_logits_bias"):
-                g[k] = torch.zeros(self._given[k].shape, dtype=torch.float32)
-        return g
+        return self._export(self._lib.pllb_s2s_train_export_grads, grads=True)
